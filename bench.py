@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200-native segmentation hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 One JSON line on stdout (rank 0).  Metric (BASELINE.json): ASPP+CE train Mpx/s -- label pixels per second
 through  features -> ASPP head fwd -> upsample+CE fwd -> CE/upsample bwd -> head dgrad+wgrad (+ mean
@@ -10,6 +10,10 @@ confusion matrix) reported in the same line under "eval".  Synthetic Cityscapes-
 
 Under torchrun (N > 1) every rank runs the same per-GPU workload (weak scaling, batch sharded by image,
 frames rank::world); time is the max over ranks, measured with CUDA events between barriers.
+
+--dump-outputs DIR writes what the headline train step returned in its last timed step (loss, low-res logits, parameter
+gradients, a fixed seeded sample of the feature gradient) as DIR/<name>.npy.  The inputs are seeded, so two builds can be
+compared output for output.
 """
 from __future__ import annotations
 
@@ -148,6 +152,33 @@ def timed(step_fn, steps, warmup, sampler=None):
     return max_over_ranks(e0.elapsed_time(e1)), clocks
 
 
+DUMP_SAMPLE = 1 << 22                    # elements kept of an output larger than this (16 MB in float32)
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def seeded_sample(t, n=DUMP_SAMPLE, seed=0):
+    """n elements of t at positions drawn from a fixed CPU generator: the same positions on every run for the same shape."""
+    flat = t.detach().reshape(-1)
+    if flat.numel() <= n:
+        return flat
+    idx = torch.randint(0, flat.numel(), (n,), generator=torch.Generator().manual_seed(seed))
+    return flat[idx.to(flat.device)]
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each tensor as out_dir/<name>.npy: float64 stays float64, everything else becomes float32."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    host = {name: t.detach().to(torch.float64 if t.dtype == torch.float64 else torch.float32).cpu().numpy()
+            for name, t in arrays.items()}
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    log(f"dumped {len(host)} arrays ({total / 2 ** 20:.1f} MB) to {out_dir}")
+
+
 class HostPipelinedStep:
     """End-to-end step from HOST buffers: every call copies that call's inputs host->device from pinned memory and reads the
     step's scalar result back (both inside the caller's timed region).  Double-buffered: the copy of call k+1's inputs is
@@ -207,6 +238,10 @@ def run_ours(args):
     bucket = D.HeadGradBucket(head) if world > 1 else None
     label_px = n * H * W
     head_params = list(head.parameters())                  # (an optimizer holds this list; zero_grad() walks it)
+    # --dump-outputs: what the last timed step returned, kept from that step only, so that no earlier step's outputs stay
+    # alive into the next timed step (timed() makes warmup + steps calls)
+    last = {} if args.dump_outputs else None
+    calls_left = [args.warmup + args.steps]
 
     def train_step(x_in=x, labels_in=labels):
         xg = x_in.detach().requires_grad_(True)            # the backbone needs d loss / d features
@@ -215,10 +250,14 @@ def run_ours(args):
         # (the module is in training mode: the bf16 weight pack is rebuilt on every call, as after every optimizer step)
         # N > 1: weight gradients land in the flat bucket and its NCCL mean all-reduce runs on a second stream underneath
         # the data-gradient GEMM; wait() joins the streams (the all-reduce is inside the timed step)
-        loss, _ = head.forward_loss(xg, labels_in, grad_bucket=bucket)
+        loss, logits_lr = head.forward_loss(xg, labels_in, grad_bucket=bucket)
         loss.backward()
         if bucket is not None:
             bucket.wait()
+        if last is not None:
+            calls_left[0] -= 1
+            if calls_left[0] == 0:                           # (detached: a live autograd graph would break the graph-capture leg)
+                last.update(loss=loss.detach(), logits_lr=logits_lr, grad_x=xg.grad)
         return loss, xg.grad
 
     launches0 = _lib.launch_count()
@@ -226,6 +265,12 @@ def run_ours(args):
     ms, clocks = timed(train_step, args.steps, args.warmup, sampler)
     launches = _lib.launch_count() - launches0 - 0
     launches_timed = launches * args.steps // (args.steps + args.warmup)
+    if last is not None and rank == 0:
+        # the later legs call train_step again: dump the headline's last timed step now.  The feature gradient has as many
+        # elements as the features (8 x 2048 x 64 x 128 by default): a fixed seeded sample of it is kept.
+        dump_outputs(args.dump_outputs, {"loss": last["loss"], "logits_lr": last["logits_lr"], "grad_x_sample": seeded_sample(last["grad_x"]),
+                                         **{"grad." + name: p.grad for name, p in head.named_parameters()}})
+    last = None
     ms_per_step = ms / args.steps
     value = world * label_px / (ms_per_step * 1e-3) / 1e6
 
@@ -923,12 +968,22 @@ def main():
     _claim_stdout()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps K of the headline train step and of the unmodified-trainer, graph-replay, seam, adversarial and "
+                         "per-config legs.  Side legs derive or fix their own counts: end to end from host buffers "
+                         "max(2, min(K, 10)) steps, eval max(4K, 24) frames rounded down to a multiple of 8, the single-kernel legs "
+                         "fixed counts")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="train_b8_512x1024")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the headline train step returned in its last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)

@@ -244,27 +244,22 @@ def test_distributed_gloo_world2(tmp_path):
 
 
 def test_color_palette_png_round_trip(tmp_path):
-    """get_color_palette (utility.py:211-217): mode-'P' image whose indices are the label ids and whose palette is the given one;
-    equal to the reference's own function when the reference tree is present."""
+    """get_color_palette (utility.py:211-217: Image.fromarray(pred.astype('uint8')).convert('P'), putpalette(palette)): a mode-'P'
+    image whose indices are the label ids and whose palette is the given one, all 256 entries of it."""
     import rnd_semantic_segmentation_b200 as b200
     from PIL import Image
-    from oracle.ref_loader import load_reference, reference_available
     rng = np.random.default_rng(0)
     pred = rng.integers(0, 19, size=(37, 53)).astype(np.int64)
     palette = [int(v) for v in rng.integers(0, 256, size=19 * 3)] + [0] * (256 * 3 - 19 * 3)
     img = b200.get_color_palette(pred, palette)
-    assert img.mode == "P" and img.size == (53, 37)
+    assert img.mode == "P" and img.size == (53, 37) and img.palette.mode == "RGB"
     np.testing.assert_array_equal(np.asarray(img), pred.astype(np.uint8))
-    assert img.getpalette()[:57] == palette[:57]
+    assert img.getpalette() == palette
     path = tmp_path / "mask.png"
     img.save(path)
     back = Image.open(path)
     np.testing.assert_array_equal(np.asarray(back), pred.astype(np.uint8))
     np.testing.assert_array_equal(np.asarray(back.convert("RGB")), np.asarray(palette[:57], dtype=np.uint8).reshape(19, 3)[pred])
-    if reference_available():
-        ref_img = load_reference().get_color_palette(pred, palette)
-        assert ref_img.mode == img.mode and ref_img.getpalette() == img.getpalette()
-        np.testing.assert_array_equal(np.asarray(ref_img), np.asarray(img))
 
 
 def test_fused_optimizers_pickle_and_state_dict_contract():

@@ -6,7 +6,6 @@ import torch
 
 from oracle import np_oracle as npo
 from oracle import torch_oracle as to
-from oracle.ref_loader import load_reference, reference_available
 
 RATES = [6, 12, 18, 24]
 
@@ -94,8 +93,9 @@ def test_discriminator_and_soft_label_builder_golden(golden):
         scaled = torch.from_numpy(g["seg_hr"]).div(1.8)
         q0 = to.build_soft_label(scaled, slot=0)
         q1 = to.build_soft_label(scaled, slot=1)
-        np.testing.assert_array_equal(q0[:, :ncls].numpy(), g["soft"])
-        np.testing.assert_array_equal(q1[:, ncls:].numpy(), g["soft"])
+        # CPU softmax rounds the last bit differently from host to host (vector width, thread split): a few ulp, not bit for bit
+        np.testing.assert_allclose(q0[:, :ncls].numpy(), g["soft"], rtol=1e-6, atol=0)
+        np.testing.assert_allclose(q1[:, ncls:].numpy(), g["soft"], rtol=1e-6, atol=0)
         assert float(q0[:, ncls:].abs().max()) == 0.0 and float(q1[:, :ncls].abs().max()) == 0.0
         assert abs(to.soft_label_cross_entropy(out_hr, q0).item() - float(g["loss_slot0"])) < 1e-6
         assert abs(to.soft_label_cross_entropy(out_hr, q1).item() - float(g["loss_slot1"])) < 1e-6
@@ -145,25 +145,34 @@ def test_anchor_known_answer_full_size():
     assert abs(loss.item() - 4.04814) < 5e-5
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference tree not mounted (GPU box)")
-def test_oracle_equals_live_reference():
-    """In the authoring container: same seed, same init order => identical parameters and outputs."""
-    ref = load_reference()
-    torch.manual_seed(5)
-    a = ref.ASPP_Classifier_V2(12, RATES, RATES, 7)
-    torch.manual_seed(5)
-    b = to.AsppHeadOracle(12, RATES, RATES, 7)
-    for (ka, va), (kb, vb) in zip(a.state_dict().items(), b.state_dict().items()):
-        assert ka == kb and torch.equal(va, vb)
-    x = torch.relu(torch.randn(2, 12, 10, 14))
-    assert torch.equal(a(x, (33, 47)), b(x, (33, 47)))
-    torch.manual_seed(6)
-    da = ref.PixelDiscriminator(12, 8, num_classes=7)
-    torch.manual_seed(6)
-    db = to.PixelDiscriminatorOracle(12, 8, num_classes=7)
-    assert torch.equal(da(x, (20, 20)), db(x, (20, 20)))
-    p = torch.randn(2, 14, 5, 6); q = torch.rand(2, 14, 5, 6)
-    assert torch.equal(ref.soft_label_cross_entropy(p, q), to.soft_label_cross_entropy(p, q))
+def _assert_state_dict_equal(module, g):
+    sd = {k[3:]: v for k, v in g.items() if k.startswith("sd.")}
+    assert list(module.state_dict().keys()) == list(sd.keys())
+    for k, v in module.state_dict().items():
+        np.testing.assert_array_equal(v.numpy(), sd[k], err_msg=k)
+
+
+@pytest.mark.parametrize("name,seed,cin,ncls", [("head_c19", 1, 24, 19), ("head_c2", 2, 16, 2), ("head_c19_T18", 3, 32, 19)])
+def test_oracle_seeded_init_matches_reference_golden(golden, name, seed, cin, ncls):
+    """Same seed, same init order as the reference (oracle/gen_golden.py seeds its modules the same way) => identical
+    parameters; the seeded module then reproduces the reference's outputs (to the golden tolerance: CPU convolutions may
+    round differently from machine to machine)."""
+    g = golden(name)
+    torch.manual_seed(seed)
+    head = to.AsppHeadOracle(cin, RATES, RATES, ncls)
+    _assert_state_dict_equal(head, g)
+    x = torch.from_numpy(g["x"])
+    with torch.no_grad():
+        np.testing.assert_allclose(head(x, g["labels"].shape[-2:]).numpy(), g["logits_hr"], rtol=1e-5, atol=1e-6)
+
+
+def test_discriminator_oracle_seeded_init_matches_reference_golden(golden):
+    g = golden("discriminator")
+    torch.manual_seed(21)
+    D = to.PixelDiscriminatorOracle(24, 16, num_classes=int(g["num_classes"]))
+    _assert_state_dict_equal(D, g)
+    with torch.no_grad():
+        np.testing.assert_allclose(D(torch.from_numpy(g["x"]), (20, 27)).numpy(), g["out_hr"], rtol=1e-5, atol=1e-6)
 
 
 # ------------------------------------------------------------------ 8f-3: test-time augmentation (flip / multi-scale)
@@ -195,7 +204,9 @@ def test_tta_oracle_matches_reference_golden(golden):
     # inference(flip=True): the oracle's line-by-line restatement fed the recorded head outputs, and the from-members form
     both = torch.cat([torch.from_numpy(g["flip.member0"]), torch.from_numpy(g["flip.member1"])], 0)
     probs = to.inference(torch.nn.Identity(), _Replay([both]), image, label, flip=True)
-    np.testing.assert_array_equal(probs.numpy(), g["flip.probs"])
+    # CPU softmax rounds the last bit differently from host to host (vector width, thread split): a few ulp, not bit for bit
+    np.testing.assert_allclose(probs.numpy(), g["flip.probs"], rtol=1e-6, atol=0)
+    _assert_pred_equal_off_ties(probs, g["flip.pred"])
     # member by member the CPU kernels vectorise differently than on the batch of two: equal to an ulp, not bit for bit
     probs2 = to.tta_probabilities([both[0:1], both[1:2]], [False, True], size, divisors=(2,))
     np.testing.assert_allclose(probs2.numpy(), g["flip.probs"], rtol=1e-6, atol=1e-7)
@@ -206,25 +217,32 @@ def test_tta_oracle_matches_reference_golden(golden):
         members = [torch.from_numpy(g[f"{name}.member{k}"]) for k in range(int(g[f"{name}.n_members"]))]
         scales = [float(s) for s in g["scales"]]
         probs = to.multi_scale_inference(torch.nn.Identity(), _Replay(members), image, label, flip=flip, scales=scales)
-        np.testing.assert_array_equal(probs.numpy(), g[f"{name}.probs"])
+        np.testing.assert_allclose(probs.numpy(), g[f"{name}.probs"], rtol=1e-6, atol=0)
+        _assert_pred_equal_off_ties(probs, g[f"{name}.pred"])
         flips = [bool(k % 2) for k in range(len(members))] if flip else [False] * len(members)
         probs2 = to.tta_probabilities(members, flips, size, divisors=(len(scales), 2) if flip else (len(scales),))
         np.testing.assert_allclose(probs2.numpy(), g[f"{name}.probs"], rtol=1e-6, atol=1e-7)
         _assert_pred_equal_off_ties(probs2, g[f"{name}.pred"])
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference tree not present")
-def test_tta_oracle_matches_live_reference():
-    ref = load_reference()
-    torch.manual_seed(5)
-    fe = torch.nn.Sequential(torch.nn.Conv2d(3, 8, 3, stride=4, padding=1), torch.nn.ReLU())
-    head = to.AsppHeadOracle(8, RATES, RATES, 5)
-    image, label = torch.randn(1, 3, 40, 56), torch.zeros(1, 37, 61, dtype=torch.int64)
-    for flip in (True, False):
-        assert torch.equal(to.inference(fe, head, image, label, flip=flip), ref.inference(fe, head, image, label, flip=flip))
-        assert torch.equal(to.multi_scale_inference(fe, head, image, label, flip=flip),
-                           ref.multi_scale_inference(fe, head, image, label, flip=flip))
-    assert to.adjust_learning_rate('poly', 2.5e-4, 7, 100, 0.9) == ref.adjust_learning_rate('poly', 2.5e-4, 7, 100, 0.9)
+def test_tta_oracle_end_to_end_matches_reference_golden(golden):
+    """inference / multi_scale_inference driven through a backbone and head (rebuilt from the seeds oracle/gen_golden_tta.py
+    used), so that the images the oracle feeds them -- mirrored, rescaled -- are checked too, not only the ensemble arithmetic."""
+    g = golden("tta")
+    torch.manual_seed(51)
+    fe = torch.nn.Sequential(torch.nn.Conv2d(3, 12, 3, stride=4, padding=1), torch.nn.ReLU())
+    head = to.AsppHeadOracle(12, RATES, RATES, int(g["num_classes"]))
+    with torch.no_grad():
+        for m in head.conv2d_list:
+            m.weight.mul_(40.0)
+    image, label = torch.from_numpy(g["image"]), torch.from_numpy(g["label"])
+    scales = [float(s) for s in g["scales"]]
+    for name, probs in (("flip", to.inference(fe, head, image, label, flip=True)),
+                        ("ms", to.multi_scale_inference(fe, head, image, label, flip=True, scales=scales)),
+                        ("ms_noflip", to.multi_scale_inference(fe, head, image, label, flip=False, scales=scales))):
+        np.testing.assert_allclose(probs.numpy(), g[f"{name}.probs"], rtol=1e-5, atol=1e-6, err_msg=name)
+        _assert_pred_equal_off_ties(probs, g[f"{name}.pred"], gap=1e-5)
+    # the poly schedule itself is pinned by the reference's learning rates in optim.npz (test_optimizer_oracle_matches_reference_golden)
     with pytest.raises(NotImplementedError):
         to.adjust_learning_rate('step', 1.0, 1, 2, 0.9)
 
