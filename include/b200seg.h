@@ -312,6 +312,24 @@ B200SEG_API int64_t b200seg_nhwc_colsum_scratch_bytes(int pitch);
 B200SEG_API int b200seg_nhwc_bf16_colsum(const void* g_nhwc_bf16, int64_t P, int C, int pitch, void* scratch, float* out, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Seam-format producer: the fused tail of the backbone's last Bottleneck (SURVEY 8f rank 2)
+ * b200seg_seam_tail_forward  replaces  out = self.bn3(out); out += identity; out = self.relu(out)
+ *                                      (core/models/feature_extractor/resnet.py:106-113, bn3 a FrozenBatchNorm2d: x * scale + bias,
+ *                                      core/models/layers.py:17-23) and the bf16 channels_last cast the head's seam format takes:
+ *   y bf16 NHWC [N][hw][C] = bf16_rn(relu((c * scale + bias) + identity)), c / identity fp32 NCHW [N][C][hw], scale / bias fp32 [C]
+ *   (the folded norm).  Each step rounded in fp32 in that order, no FMA contraction: y is bit-identical to the stock output cast
+ *   with .to(torch.bfloat16).
+ * b200seg_seam_tail_backward  replaces  the autograd backward of the same lines:
+ *   g = dy * (y > 0);  dc fp32 NCHW = g * scale;  didentity fp32 NCHW = g     (dy, y bf16 NHWC as above)
+ *   dc or didentity may be NULL when that gradient is not wanted.
+ * C % 8 == 0, any hw >= 1, any N; y and dy 16-byte aligned.  No scratch.
+ * ------------------------------------------------------------------------------------------- */
+B200SEG_API int b200seg_seam_tail_forward(const float* c, const float* identity, const float* scale, const float* bias, int N, int C,
+                                          int hw, void* y, void* stream);
+B200SEG_API int b200seg_seam_tail_backward(const void* dy, const void* y, const float* scale, int N, int C, int hw, float* dc,
+                                           float* didentity, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * K7  test-time augmentation fused with argmax + confusion matrix (SURVEY 8f rank 3).
  * Replaces inference(..., flip=True) (core/utils/utility.py:179-191), multi_scale_inference (utility.py:193-209), the
  * output.max(1)[1] / output.argmax(0) that follow (core/testers/aspp_tester.py:63,42) and confusion_matrix /

@@ -19,7 +19,8 @@ ROOT = os.path.dirname(PKG_DIR)
 LIB_PATH = os.path.join(PKG_DIR, "libb200seg.so")
 OBJ_DIR = os.path.join(PKG_DIR, "_obj")
 SOURCES = ["api.cu", "eval_kernels.cu", "ce_kernels.cu", "ce_v2_kernels.cu", "softce_kernels.cu",
-           "gemm_sm100.cu", "aspp_head.cu", "conv_sm100.cu", "tta_kernels.cu", "optim_kernels.cu", "p2p_allreduce.cu"]
+           "gemm_sm100.cu", "aspp_head.cu", "conv_sm100.cu", "tta_kernels.cu", "optim_kernels.cu", "p2p_allreduce.cu",
+           "seam_tail_kernels.cu"]
 HEADERS = ["common.cuh", "ce_geom.cuh", "gemm_sm100.cuh", os.path.join(ROOT, "include", "b200seg.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "--expt-relaxed-constexpr"]

@@ -101,6 +101,8 @@ SIGNATURES = {
     "b200seg_conv3x3_wgrad": (c_int, [c_vp, c_int, c_i64, c_vp, c_int, c_i64, c_int, c_int, c_int, c_int, c_int, c_vp, c_i64, c_vp,
                                       c_vp, c_int, c_vp]),
     "b200seg_nchw_to_nhwc_bf16": (c_int, [c_vp, c_int, c_int, c_int, c_vp, c_int, c_vp]),
+    "b200seg_seam_tail_forward": (c_int, [c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_vp, c_vp]),
+    "b200seg_seam_tail_backward": (c_int, [c_vp, c_vp, c_vp, c_int, c_int, c_int, c_vp, c_vp, c_vp]),
     "b200seg_nhwc_colsum_scratch_bytes": (c_i64, [c_int]),
     "b200seg_nhwc_bf16_colsum": (c_int, [c_vp, c_i64, c_int, c_int, c_vp, c_vp, c_vp]),
     "b200seg_gemm_set_overlap_sms": (None, [c_int]),
@@ -1194,6 +1196,61 @@ def nchw_to_nhwc_bf16(src: torch.Tensor, pitch: Optional[int] = None) -> torch.T
     with _on_device(src.device):
         _check(lib.b200seg_nchw_to_nhwc_bf16(src.data_ptr(), N, C, h * w, dst.data_ptr(), pitch, _stream()))
     return dst
+
+
+def _need_channels_last_bf16(t: torch.Tensor, name: str) -> torch.Tensor:
+    if not isinstance(t, torch.Tensor):
+        raise TypeError(f"{name}: expected a torch.Tensor, got {type(t)}")
+    if not t.is_cuda:
+        raise B200SegError(f"{name}: expected a CUDA tensor (b200seg has no CPU fallback), got device {t.device}")
+    if t.dtype != torch.bfloat16 or t.dim() != 4 or not t.is_contiguous(memory_format=torch.channels_last):
+        raise B200SegError(f"{name}: expected a bf16 channels_last contiguous [N,C,h,w] tensor")
+    return t
+
+
+def _need_channel_vector(t: torch.Tensor, C: int, name: str) -> torch.Tensor:
+    _need(t, torch.float32, name)
+    if t.numel() != C:
+        raise B200SegError(f"{name}: expected {C} values, got {t.numel()}")
+    return t
+
+
+def seam_tail_forward(c: torch.Tensor, identity: torch.Tensor, scale: torch.Tensor, bias: torch.Tensor) -> torch.Tensor:
+    """bf16 channels_last y = bf16_rn(relu((c * scale + bias) + identity)) from fp32 NCHW c / identity (the last Bottleneck's
+    bn3 + residual + relu, resnet.py:106-113, with the cast the head's seam format takes); bit-identical to the stock fp32
+    result .to(torch.bfloat16).  C % 8 == 0."""
+    lib = load()
+    _need(c, torch.float32, "c")
+    _need(identity, torch.float32, "identity")
+    if c.dim() != 4 or identity.shape != c.shape:
+        raise B200SegError(f"seam_tail_forward: c {tuple(c.shape)} and identity {tuple(identity.shape)} must be equal [N,C,h,w]")
+    N, C, h, w = c.shape
+    _need_channel_vector(scale, C, "scale")
+    _need_channel_vector(bias, C, "bias")
+    y = torch.empty((N, C, h, w), dtype=torch.bfloat16, device=c.device, memory_format=torch.channels_last)
+    with _on_device(c.device):
+        _check(lib.b200seg_seam_tail_forward(c.data_ptr(), identity.data_ptr(), scale.data_ptr(), bias.data_ptr(), N, C, h * w,
+                                             y.data_ptr(), _stream()))
+    return y
+
+
+def seam_tail_backward(dy: torch.Tensor, y: torch.Tensor, scale: torch.Tensor, need_c: bool = True, need_identity: bool = True):
+    """(dc, didentity), fp32 NCHW: g = dy * (y > 0), dc = g * scale, didentity = g; dy / y bf16 channels_last.  An output that is
+    not needed is None (and not written)."""
+    lib = load()
+    _need_channels_last_bf16(dy, "dy")
+    _need_channels_last_bf16(y, "y")
+    if dy.shape != y.shape:
+        raise B200SegError(f"seam_tail_backward: dy {tuple(dy.shape)} and y {tuple(y.shape)} differ")
+    N, C, h, w = y.shape
+    _need_channel_vector(scale, C, "scale")
+    dc = torch.empty((N, C, h, w), dtype=torch.float32, device=y.device) if need_c else None
+    di = torch.empty((N, C, h, w), dtype=torch.float32, device=y.device) if need_identity else None
+    if dc is None and di is None:
+        return None, None
+    with _on_device(y.device):
+        _check(lib.b200seg_seam_tail_backward(dy.data_ptr(), y.data_ptr(), scale.data_ptr(), N, C, h * w, _ptr(dc), _ptr(di), _stream()))
+    return dc, di
 
 
 def nhwc_bf16_colsum(g: torch.Tensor, C: Optional[int] = None) -> torch.Tensor:

@@ -94,6 +94,8 @@ long long conv3x3_wgrad_scratch_bytes(int, int, int, int, int, int);
 int conv3x3_wgrad(const void*, int, long long, const void*, int, long long, int, int, int, int, int, void*, long long, float* const*,
                   const int*, int, cudaStream_t);
 int nchw_to_nhwc_bf16(const float*, int, int, int, void*, int, cudaStream_t);
+int seam_tail_forward(const float*, const float*, const float*, const float*, int, int, int, void*, cudaStream_t);
+int seam_tail_backward(const void*, const void*, const float*, int, int, int, float*, float*, cudaStream_t);
 long long nhwc_colsum_scratch_bytes(int);
 int nhwc_bf16_colsum(const void*, long long, int, int, void*, float*, cudaStream_t);
 int tta_launch(const float* const*, const int*, const int*, const int*, int, int, const void*, int, int, int, int, const float*, int, int,
@@ -526,6 +528,18 @@ int b200seg_conv3x3_wgrad(const void* g, int Co, int64_t g_pitch, const void* x,
 int b200seg_nchw_to_nhwc_bf16(const float* src, int N, int C, int hw, void* dst, int pitch, void* stream) {
   REQUIRE_DEVICE();
   return nchw_to_nhwc_bf16(src, N, C, hw, dst, pitch, S(stream));
+}
+
+int b200seg_seam_tail_forward(const float* c, const float* identity, const float* scale, const float* bias, int N, int C, int hw, void* y,
+                              void* stream) {
+  REQUIRE_DEVICE();
+  return seam_tail_forward(c, identity, scale, bias, N, C, hw, y, S(stream));
+}
+
+int b200seg_seam_tail_backward(const void* dy, const void* y, const float* scale, int N, int C, int hw, float* dc, float* didentity,
+                               void* stream) {
+  REQUIRE_DEVICE();
+  return seam_tail_backward(dy, y, scale, N, C, hw, dc, didentity, S(stream));
 }
 
 int b200seg_tta_argmax_confusion(const float* const* logits_lr, const int* h, const int* w, const int* flip, int n_members, int C,

@@ -8,7 +8,9 @@ After this, ``core.models.build.build_classifier`` / ``build_adversarial_discrim
 AverageMeter,get_color_palette}`` and ``core.utils.adapt_lr.adjust_learning_rate`` resolve to this package's implementations; the
 scripts themselves stay unmodified (INTEGRATION.md).  ``install(optimizers=True)`` additionally makes the trainers'
 ``torch.optim.SGD`` / ``torch.optim.Adam`` constructions (aspp_trainer.py:25-26, fada_adapter.py:24) build FusedSGD / FusedAdam for
-parameter sets that live on a CUDA device (everything else keeps the stock classes).
+parameter sets that live on a CUDA device (everything else keeps the stock classes).  ``install(seam=True)`` additionally wraps
+``core.models.build.build_feature_extractor`` (same signature) so that the backbone it returns emits the head's seam format, bf16
+channels_last, from its last Bottleneck (seam.fuse_backbone_tail; INTEGRATION.md "Seam format").
 """
 from __future__ import annotations
 
@@ -19,6 +21,7 @@ import torch
 
 from . import build as _build
 from . import optim as _optim
+from . import seam as _seam
 from . import utility as _utility
 
 _BUILD_NAMES = ("build_classifier", "build_adversarial_discriminator")
@@ -73,8 +76,32 @@ def uninstall_optimizers():
         torch.optim.SGD, torch.optim.Adam = _stock_optimizers.pop("SGD"), _stock_optimizers.pop("Adam")
 
 
-def install(strict: bool = False, optimizers: bool = False):
-    """Returns the list of 'module.attr' names that were patched."""
+def _install_seam(patched):
+    """core.models(.build).build_feature_extractor -> the same factory with fuse_backbone_tail applied to its result, also in
+    modules that imported the name before."""
+    wrapped = {}                     # id(stock function) -> wrapper (core.models re-exports core.models.build's function)
+    for modname in ("core.models.build", "core.models"):
+        mod = sys.modules.get(modname)
+        stock = getattr(mod, "build_feature_extractor", None) if mod is not None else None
+        if stock is None:
+            continue
+        fn = wrapped.setdefault(id(stock), _seam.wrap_feature_extractor_factory(stock))
+        wrapped[id(fn)] = fn
+        setattr(mod, "build_feature_extractor", fn)
+        patched.append(f"{modname}.build_feature_extractor")
+    for mod in list(sys.modules.values()):
+        name = getattr(mod, "__name__", "")
+        if not name.startswith("core.") or name in ("core.models.build", "core.models"):
+            continue
+        fn = getattr(mod, "__dict__", {}).get("build_feature_extractor")
+        if fn is not None and id(fn) in wrapped:
+            setattr(mod, "build_feature_extractor", wrapped[id(fn)])
+            patched.append(f"{name}.build_feature_extractor")
+
+
+def install(strict: bool = False, optimizers: bool = False, seam: bool = False):
+    """Returns the list of 'module.attr' names that were patched.  ``seam=True``: the reference's build_feature_extractor returns
+    a backbone whose last Bottleneck emits bf16 channels_last features (seam.fuse_backbone_tail)."""
     patched = install_optimizers() if optimizers else []
     targets = (("core.models.build", _build, _BUILD_NAMES), ("core.models", _build, _BUILD_NAMES),
                ("core.utils.utility", _utility, _UTIL_NAMES), ("core.utils.adapt_lr", _optim, _LR_NAMES))
@@ -100,4 +127,6 @@ def install(strict: bool = False, optimizers: bool = False):
                 if n in getattr(mod, "__dict__", {}):
                     setattr(mod, n, getattr(src, n))
                     patched.append(f"{name}.{n}")
+    if seam:
+        _install_seam(patched)
     return patched

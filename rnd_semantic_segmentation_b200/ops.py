@@ -243,6 +243,41 @@ def pixel_discriminator_logits(x, w1, b1, w2, b2, wc1, bc1, wc2, bc2, slope: flo
 
 
 # --------------------------------------------------------------------------------------------
+# seam-format producer: the last Bottleneck's bn3 + residual + relu, emitted as bf16 channels_last
+# --------------------------------------------------------------------------------------------
+class _SeamTailFn(torch.autograd.Function):
+    """bf16 channels_last relu((c * scale + bias) + identity)  (resnet.py:106-113 with a folded FrozenBatchNorm2d, layers.py:17-23).
+    Saves only y (and the [C] scale): when the head consumes y it keeps the same storage as its GEMM operand, so the stock tail's
+    fp32 relu output is not kept at all."""
+
+    @staticmethod
+    def forward(ctx, c, identity, scale, bias):
+        y = _lib.seam_tail_forward(c.detach().contiguous(), identity.detach().contiguous(), scale.detach().contiguous(),
+                                   bias.detach().contiguous())
+        ctx.save_for_backward(y, scale.detach())
+        return y
+
+    @staticmethod
+    def backward(ctx, dy):
+        y, scale = ctx.saved_tensors
+        need_c, need_id = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
+        dy = dy.detach()
+        # the head's seam-format dgrad already writes bf16 channels_last; a sum of two consumers' gradients or the NCHW bf16
+        # gradient of the plain head call is converted once
+        if dy.dtype != torch.bfloat16 or not dy.is_contiguous(memory_format=torch.channels_last):
+            dy = dy.to(torch.bfloat16).contiguous(memory_format=torch.channels_last)
+        dc, di = _lib.seam_tail_backward(dy, y, scale.contiguous(), need_c, need_id)
+        return dc, di, None, None
+
+
+def seam_tail(c: torch.Tensor, identity: torch.Tensor, scale: torch.Tensor, bias: torch.Tensor) -> torch.Tensor:
+    """bf16 channels_last ``relu((c * scale + bias) + identity)`` from fp32 NCHW ``c`` / ``identity`` [N, C, h, w] (C % 8 == 0)
+    and the folded norm's fp32 ``scale`` / ``bias`` [C] (constants: no gradient).  Bit-identical to the stock fp32 sequence
+    followed by ``.to(torch.bfloat16)``; the gradient to ``c`` / ``identity`` is the stock one computed from the bf16 ``dy``."""
+    return _SeamTailFn.apply(c, identity, scale, bias)
+
+
+# --------------------------------------------------------------------------------------------
 # materialising align-corners bilinear upsample (API-compat path)
 # --------------------------------------------------------------------------------------------
 class _UpsampleFn(torch.autograd.Function):
