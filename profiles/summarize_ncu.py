@@ -69,11 +69,11 @@ def write_bench_json(summary_csv, out_json, source):
     launch of each kernel below belongs to the train step unless it is the eval kernel."""
     import json
     keys = [("head_fwd_gemm", "gemm::gemm_bf16_kernel<0, 0, 2>", 0), ("head_dgrad_gemm", "gemm::gemm_bf16_kernel<0, 1, 1>", 0),
-            ("head_wgrad_gemm", "gemm::gemm_bf16_kernel<0, 1, 2>", 0), ("pack_features", "pack_features_kernel", 0),
+            ("head_wgrad_gemm", "gemm::gemm_bf16_kernel<0, 1, 2>", 0), ("pack_features", "nchw_to_nhwc_tile_kernel<false", 0),
             ("head_gather", "head_gather_kernel", 0), ("grad_im2col", "build_gprime", 0),
             ("upsample_ce_main", "k2_upsample_ce_main", 0), ("wgrad_reduce", "wgrad_reduce_kernel", 0),
             ("eval_argmax_confusion", "k4_upsample_argmax_confusion", 0), ("eval_head_fwd_gemm", "gemm::gemm_bf16_kernel<0, 0, 2>", 1),
-            ("eval_pack_features", "pack_features_kernel", 1), ("eval_head_gather", "head_gather_kernel", 1)]
+            ("eval_pack_features", "nchw_to_nhwc_tile_kernel<false", 1), ("eval_head_gather", "head_gather_kernel", 1)]
     rows = list(csv.DictReader(open(summary_csv)))
     out = {"source": source, "kernels": {}}
     for key, pat, nth in keys:

@@ -23,6 +23,7 @@
 
 namespace b200seg {
 namespace gemm { int overlap_sms(); }
+int nchw_to_nhwc_bf16(const float* src, int N, int C, int hw, void* dst, int pitch, cudaStream_t stream);   // seam_tail_kernels.cu
 
 constexpr int MAX_RATES = 8;
 constexpr int MAX_TAPS = 8 * MAX_RATES + 1;
@@ -122,32 +123,6 @@ __global__ void __launch_bounds__(256) pack_weights_kernel(PtrList w, PtrList b,
       w4[e] = *reinterpret_cast<const uint32_t*>(&v);
     }
     *reinterpret_cast<uint4*>(Wp + (long long)j * Cin + ci0) = make_uint4(w4[0], w4[1], w4[2], w4[3]);
-  }
-}
-
-// ------------------------------------------------------------------------------------------
-// pack features: x fp32 NCHW [N, Cin, hw] -> Xp bf16 [N*hw, Cin]  (64 ci x 64 px tiles through smem)
-// ------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) pack_features_kernel(const float* __restrict__ x, int Cin, int hw,
-                                                            __nv_bfloat16* __restrict__ Xp) {
-  __shared__ float tile[64][65];
-  const int s0 = blockIdx.x * 64, c0 = blockIdx.y * 64, n = blockIdx.z;
-  const int tx = threadIdx.x & 63, ty = threadIdx.x >> 6;          // 64 x 4
-  const float* src = x + ((long long)n * Cin + c0) * hw + s0;
-#pragma unroll
-  for (int i = 0; i < 16; ++i) {
-    const int ci = ty + i * 4;
-    tile[ci][tx] = (c0 + ci < Cin && s0 + tx < hw) ? __ldcs(src + (long long)ci * hw + tx) : 0.f;
-  }
-  __syncthreads();
-  const int cpair = threadIdx.x & 31, prow = threadIdx.x >> 5;     // 32 channel pairs x 8 pixel rows
-#pragma unroll
-  for (int i = 0; i < 8; ++i) {
-    const int s = prow + i * 8;
-    if (s0 + s < hw && c0 + 2 * cpair < Cin) {
-      const __nv_bfloat162 v = __floats2bfloat162_rn(tile[2 * cpair][s], tile[2 * cpair + 1][s]);
-      *reinterpret_cast<__nv_bfloat162*>(Xp + ((long long)n * hw + s0 + s) * Cin + c0 + 2 * cpair) = v;
-    }
   }
 }
 
@@ -460,12 +435,10 @@ int aspp_pack_weights(const float* const* w, const float* const* b, int R, int C
 int aspp_pack_features(const float* x, int N, int Cin, int h, int w, void* Xp, cudaStream_t stream) {
   B200SEG_CHECK_ARG(x && Xp && N > 0 && h > 0 && w > 0, "aspp_pack_features: bad arguments");
   B200SEG_CHECK_ARG(Cin % 8 == 0, "aspp: in_channels=%d must be a multiple of 8", Cin);
-  dim3 grid(ceil_div(h * w, 64), ceil_div(Cin, 64), N);
   profile_begin(3, stream);
-  pack_features_kernel<<<grid, 256, 0, stream>>>(x, Cin, h * w, (__nv_bfloat16*)Xp);
+  const int rc = nchw_to_nhwc_bf16(x, N, Cin, h * w, Xp, Cin, stream);      // Xp [N*hw, Cin] is NHWC with pitch Cin
   profile_end(3, stream);
-  B200SEG_LAUNCH_CHECK();
-  return B200SEG_OK;
+  return rc;
 }
 
 long long aspp_yt_bytes(int N, int C, int h, int w, int R) {

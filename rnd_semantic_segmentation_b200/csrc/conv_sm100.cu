@@ -684,23 +684,6 @@ __global__ void __launch_bounds__(256) conv_pack_weights_kernel(const PackTable 
   }
 }
 
-// fp32 NCHW [N][C][hw] -> bf16 NHWC [N*hw][pitch], channels >= C zero
-__global__ void __launch_bounds__(256) nchw_to_nhwc_bf16_kernel(const float* __restrict__ src, int C, int hw, int pitch,
-                                                                __nv_bfloat16* __restrict__ dst) {
-  const int s = blockIdx.x * 256 + threadIdx.x, c0 = blockIdx.y * 8, n = blockIdx.z;
-  if (s >= hw) return;
-  uint32_t w4[4];
-#pragma unroll
-  for (int e = 0; e < 4; ++e) {
-    const int c = c0 + 2 * e;
-    const float a = c < C ? __ldg(src + ((long long)n * C + c) * hw + s) : 0.f;
-    const float b = c + 1 < C ? __ldg(src + ((long long)n * C + c + 1) * hw + s) : 0.f;
-    const __nv_bfloat162 v = __floats2bfloat162_rn(a, b);
-    w4[e] = *reinterpret_cast<const uint32_t*>(&v);
-  }
-  *reinterpret_cast<uint4*>(dst + ((long long)n * hw + s) * pitch + c0) = make_uint4(w4[0], w4[1], w4[2], w4[3]);
-}
-
 // deterministic column sums of bf16 [P][pitch]: per-block partials, then a fixed-order final sum (bias gradients)
 constexpr int COLSUM_BLOCKS = 296;
 __global__ void __launch_bounds__(256) colsum_partial_kernel(const __nv_bfloat16* __restrict__ g, long long P, int pitch,
@@ -843,13 +826,6 @@ int conv3x3_pack_weights_stack(int n_layers, const float* const* weights, const 
   return pack_launch(t, stream);
 }
 
-int nchw_to_nhwc_bf16(const float* src, int N, int C, int hw, void* dst, int pitch, cudaStream_t stream) {
-  B200SEG_CHECK_ARG(src && dst && N > 0 && C > 0 && hw > 0 && pitch % 8 == 0 && pitch >= C, "nchw_to_nhwc_bf16: bad arguments");
-  dim3 grid(ceil_div(hw, 256), pitch / 8, N);
-  nchw_to_nhwc_bf16_kernel<<<grid, 256, 0, stream>>>(src, C, hw, pitch, (__nv_bfloat16*)dst);
-  B200SEG_LAUNCH_CHECK();
-  return B200SEG_OK;
-}
 
 long long nhwc_colsum_scratch_bytes(int pitch) { return (long long)COLSUM_BLOCKS * pitch * 4; }
 

@@ -13,6 +13,11 @@
 // (one warp streams a 512-byte channel row with 16-byte accesses) and the NHWC side (one thread moves 8 channels = 16 bytes of
 // one pixel; a warp covers 8 pixels x 64 contiguous bytes).  The tile's 4-pixel quads are XOR-swizzled with the channel's
 // 8-group so that both the row-wise float4 accesses and the column-wise scalar accesses are free of bank conflicts.
+//
+// The forward pass with the identity prologue is also the library's fp32 NCHW -> bf16 NHWC conversion (nchw_to_nhwc_bf16):
+// the head's feature pack (aspp_pack_features) and the discriminator's gradient layout, whose output pitch may exceed C (the
+// pad channels are written as zeros).  At the 2:1 read/write mix of the pack this tile runs at 6.5 TB/s where the 64 x 64
+// scalar-load tile it replaced ran at 5.6 (profiles/micro/nhwc_tile_micro.cu).
 #include "common.cuh"
 
 namespace b200seg {
@@ -29,11 +34,13 @@ __device__ __forceinline__ float tail_value(float c, float sc, float bi, float i
   return v <= 0.f ? 0.f : v;                                       // NaN passes through, as torch.relu
 }
 
+// y[n, s, ch] = bf16_rn(f(c[n, ch, s])) for ch < pitch, with f the seam tail (TAIL) or the identity (then identity, scale and
+// bias are not read); channels C <= ch < pitch are written as 0.
 // VEC: hw % 4 == 0 and c / identity 16-byte aligned (float4 rows); otherwise scalar loads
-template <bool VEC>
-__global__ void __launch_bounds__(ST_THREADS) seam_tail_forward_kernel(const float* __restrict__ c, const float* __restrict__ identity,
+template <bool TAIL, bool VEC>
+__global__ void __launch_bounds__(ST_THREADS) nchw_to_nhwc_tile_kernel(const float* __restrict__ c, const float* __restrict__ identity,
                                                                        const float* __restrict__ scale, const float* __restrict__ bias,
-                                                                       int C, int hw, __nv_bfloat16* __restrict__ y) {
+                                                                       int C, int hw, int pitch, __nv_bfloat16* __restrict__ y) {
   __shared__ __align__(16) float tile[ST_CH * ST_PX];
   const int s0 = blockIdx.x * ST_PX, c0 = blockIdx.y * ST_CH, n = blockIdx.z;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -48,23 +55,29 @@ __global__ void __launch_bounds__(ST_THREADS) seam_tail_forward_kernel(const flo
       if (VEC) {
         if (s < hw) {
           a[i] = __ldcs(reinterpret_cast<const float4*>(c + off));
-          b[i] = __ldcs(reinterpret_cast<const float4*>(identity + off));
+          if (TAIL) b[i] = __ldcs(reinterpret_cast<const float4*>(identity + off));
         }
       } else {
         float* av = &a[i].x;
         float* bv = &b[i].x;
 #pragma unroll
         for (int j = 0; j < 4; ++j)
-          if (s + j < hw) { av[j] = __ldcs(c + off + j); bv[j] = __ldcs(identity + off + j); }
+          if (s + j < hw) {
+            av[j] = __ldcs(c + off + j);
+            if (TAIL) bv[j] = __ldcs(identity + off + j);
+          }
       }
     }
   }
 #pragma unroll
   for (int i = 0; i < 4; ++i) {
     const int ch = warp + 8 * i, cg = c0 + ch;
-    const float sc = cg < C ? __ldg(scale + cg) : 0.f, bi = cg < C ? __ldg(bias + cg) : 0.f;
-    const float4 v = make_float4(tail_value(a[i].x, sc, bi, b[i].x), tail_value(a[i].y, sc, bi, b[i].y),
-                                 tail_value(a[i].z, sc, bi, b[i].z), tail_value(a[i].w, sc, bi, b[i].w));
+    float4 v = a[i];
+    if (TAIL) {
+      const float sc = cg < C ? __ldg(scale + cg) : 0.f, bi = cg < C ? __ldg(bias + cg) : 0.f;
+      v = make_float4(tail_value(a[i].x, sc, bi, b[i].x), tail_value(a[i].y, sc, bi, b[i].y), tail_value(a[i].z, sc, bi, b[i].z),
+                      tail_value(a[i].w, sc, bi, b[i].w));
+    }
     *reinterpret_cast<float4*>(tile + st_idx(ch, 4 * lane)) = v;
   }
   __syncthreads();
@@ -72,14 +85,14 @@ __global__ void __launch_bounds__(ST_THREADS) seam_tail_forward_kernel(const flo
 #pragma unroll
   for (int it = 0; it < 2; ++it) {
     const int sl = (lane >> 2) + 8 * warp + 64 * it;
-    if (s0 + sl < hw && cc < C) {
+    if (s0 + sl < hw && cc < pitch) {
       uint32_t w4[4];
 #pragma unroll
       for (int e = 0; e < 4; ++e) {
         const __nv_bfloat162 v = __floats2bfloat162_rn(tile[st_idx(8 * chunk + 2 * e, sl)], tile[st_idx(8 * chunk + 2 * e + 1, sl)]);
         w4[e] = *reinterpret_cast<const uint32_t*>(&v);
       }
-      *reinterpret_cast<uint4*>(y + ((long long)n * hw + s0 + sl) * C + cc) = make_uint4(w4[0], w4[1], w4[2], w4[3]);
+      *reinterpret_cast<uint4*>(y + ((long long)n * hw + s0 + sl) * pitch + cc) = make_uint4(w4[0], w4[1], w4[2], w4[3]);
     }
   }
 }
@@ -148,20 +161,35 @@ __global__ void __launch_bounds__(ST_THREADS) seam_tail_backward_kernel(const __
 
 static inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
 
+// identity may be null (TAIL = false)
+template <bool TAIL>
+static int nchw_to_nhwc_launch(const float* c, const float* identity, const float* scale, const float* bias, int N, int C, int hw,
+                               int pitch, void* y, cudaStream_t stream) {
+  const dim3 grid(ceil_div(hw, ST_PX), ceil_div(pitch, ST_CH), N);
+  __nv_bfloat16* yb = reinterpret_cast<__nv_bfloat16*>(y);
+  if (hw % 4 == 0 && aligned16(c) && aligned16(identity))         // (a null pointer counts as aligned)
+    nchw_to_nhwc_tile_kernel<TAIL, true><<<grid, ST_THREADS, 0, stream>>>(c, identity, scale, bias, C, hw, pitch, yb);
+  else
+    nchw_to_nhwc_tile_kernel<TAIL, false><<<grid, ST_THREADS, 0, stream>>>(c, identity, scale, bias, C, hw, pitch, yb);
+  B200SEG_LAUNCH_CHECK();
+  return B200SEG_OK;
+}
+
 int seam_tail_forward(const float* c, const float* identity, const float* scale, const float* bias, int N, int C, int hw, void* y,
                       cudaStream_t stream) {
   B200SEG_CHECK_ARG(c && identity && scale && bias && y && N > 0 && C > 0 && hw > 0, "seam_tail_forward: bad arguments");
   B200SEG_CHECK_ARG(C % 8 == 0, "seam_tail_forward: C = %d is not a multiple of 8", C);
   B200SEG_CHECK_ARG(N <= 65535 && ceil_div(C, ST_CH) <= 65535, "seam_tail_forward: N = %d / C = %d too large", N, C);
   B200SEG_CHECK_ARG(aligned16(y), "seam_tail_forward: y must be 16-byte aligned");
-  const dim3 grid(ceil_div(hw, ST_PX), ceil_div(C, ST_CH), N);
-  __nv_bfloat16* yb = reinterpret_cast<__nv_bfloat16*>(y);
-  if (hw % 4 == 0 && aligned16(c) && aligned16(identity))
-    seam_tail_forward_kernel<true><<<grid, ST_THREADS, 0, stream>>>(c, identity, scale, bias, C, hw, yb);
-  else
-    seam_tail_forward_kernel<false><<<grid, ST_THREADS, 0, stream>>>(c, identity, scale, bias, C, hw, yb);
-  B200SEG_LAUNCH_CHECK();
-  return B200SEG_OK;
+  return nchw_to_nhwc_launch<true>(c, identity, scale, bias, N, C, hw, C, y, stream);
+}
+
+// fp32 NCHW [N][C][hw] -> bf16 NHWC [N*hw][pitch], channels >= C zero
+int nchw_to_nhwc_bf16(const float* src, int N, int C, int hw, void* dst, int pitch, cudaStream_t stream) {
+  B200SEG_CHECK_ARG(src && dst && N > 0 && C > 0 && hw > 0 && pitch % 8 == 0 && pitch >= C, "nchw_to_nhwc_bf16: bad arguments");
+  B200SEG_CHECK_ARG(N <= 65535 && ceil_div(pitch, ST_CH) <= 65535, "nchw_to_nhwc_bf16: N = %d / pitch = %d too large", N, pitch);
+  B200SEG_CHECK_ARG(aligned16(dst), "nchw_to_nhwc_bf16: dst must be 16-byte aligned");
+  return nchw_to_nhwc_launch<false>(src, nullptr, nullptr, nullptr, N, C, hw, pitch, dst, stream);
 }
 
 int seam_tail_backward(const void* dy, const void* y, const float* scale, int N, int C, int hw, float* dc, float* didentity,
