@@ -330,6 +330,43 @@ B200SEG_API int b200seg_seam_tail_backward(const void* dy, const void* y, const 
                                            float* didentity, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * The same tail with bn3 a training-mode BatchNorm2d / SyncBatchNorm (batch statistics): the end of Bottleneck.forward,
+ * core/models/feature_extractor/resnet.py:106-113, in the self-distillation stage whose backbone train_distill.py:52-53 converts
+ * with SyncBatchNorm.convert_sync_batchnorm.  c / identity fp32 NCHW [N][C][hw], M = N * hw per rank.  No atomics (every reduction
+ * in a fixed order: bit-identical run to run) and no host synchronisation (capturable in a CUDA graph).
+ * b200seg_bn_stats  replaces  the per-rank statistics of F.batch_norm / torch.batch_norm_stats:
+ *   record fp64 [3][C] = (count, mean, M2 = sum (c - mean)^2) of this rank's c.  Scratch: b200seg_bn_stats_scratch_bytes.
+ * b200seg_bn_combine_stats  replaces  the statistics reduction of F.batch_norm / torch.batch_norm_gather_stats_with_counts:
+ *   combines R records [R][3][C] in rank order (R = 1 for BatchNorm2d; SyncBatchNorm: the all-gathered records of the group)
+ *   -> mean, invstd = 1 / sqrt(var + eps) fp32 [C] (var biased), count fp64 [1] = total M (may be NULL), and, when running_mean
+ *   and running_var are given, running = (1 - f) running + f * (mean | var * M / (M - 1)) with f = momentum, or
+ *   f = 1 / *num_batches_tracked (int64, read on the device) when num_batches_tracked is given (momentum=None).
+ * b200seg_seam_tail_bn_forward  replaces  out = self.bn3(out); out += identity; out = self.relu(out) in training mode, + bf16 cast:
+ *   y bf16 NHWC [N][hw][C] = bf16_rn(relu(((c - mean) * invstd * gamma + beta) + identity)); gamma / beta NULL for affine=False.
+ * b200seg_seam_tail_bn_backward_reduce  replaces  torch.batch_norm_backward_reduce of the same lines, with g = dy * (y > 0):
+ *   sums fp32 [2][C] = (sum g, sum g (c - mean)) over this rank; dbeta = sum g and dgamma = invstd * sum g (c - mean) (local
+ *   sums; either may be NULL).  Scratch: b200seg_seam_tail_bn_backward_reduce_scratch_bytes.
+ * b200seg_seam_tail_bn_backward  replaces  torch.batch_norm_backward_elemt and the residual / relu backward:
+ *   sum_g, sum_gx = the R records of sums [R][2][C] added in rank order (SyncBatchNorm: the all-gathered per-rank sums), M = *count;
+ *   dc = (g - sum_g / M - (c - mean) * invstd^2 * sum_gx / M) * invstd * gamma,  didentity = g   (fp32 NCHW; either may be NULL)
+ * C % 8 == 0, any hw >= 1, any N; y and dy 16-byte aligned.
+ * ------------------------------------------------------------------------------------------- */
+B200SEG_API int64_t b200seg_bn_stats_scratch_bytes(int N, int C);
+B200SEG_API int b200seg_bn_stats(const float* c, int N, int C, int hw, void* scratch, int64_t scratch_bytes, double* record, void* stream);
+B200SEG_API int b200seg_bn_combine_stats(const double* records, int R, int C, float eps, float momentum,
+                                         const int64_t* num_batches_tracked, float* running_mean, float* running_var, float* mean,
+                                         float* invstd, double* count, void* stream);
+B200SEG_API int b200seg_seam_tail_bn_forward(const float* c, const float* identity, const float* mean, const float* invstd,
+                                             const float* gamma, const float* beta, int N, int C, int hw, void* y, void* stream);
+B200SEG_API int64_t b200seg_seam_tail_bn_backward_reduce_scratch_bytes(int N, int C, int hw);
+B200SEG_API int b200seg_seam_tail_bn_backward_reduce(const void* dy, const void* y, const float* c, const float* mean,
+                                                     const float* invstd, int N, int C, int hw, void* scratch, int64_t scratch_bytes,
+                                                     float* sums, float* dgamma, float* dbeta, void* stream);
+B200SEG_API int b200seg_seam_tail_bn_backward(const void* dy, const void* y, const float* c, const float* mean, const float* invstd,
+                                              const float* gamma, const float* sums, int R, const double* count, int N, int C, int hw,
+                                              float* dc, float* didentity, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * K7  test-time augmentation fused with argmax + confusion matrix (SURVEY 8f rank 3).
  * Replaces inference(..., flip=True) (core/utils/utility.py:179-191), multi_scale_inference (utility.py:193-209), the
  * output.max(1)[1] / output.argmax(0) that follow (core/testers/aspp_tester.py:63,42) and confusion_matrix /

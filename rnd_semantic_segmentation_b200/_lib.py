@@ -103,6 +103,15 @@ SIGNATURES = {
     "b200seg_nchw_to_nhwc_bf16": (c_int, [c_vp, c_int, c_int, c_int, c_vp, c_int, c_vp]),
     "b200seg_seam_tail_forward": (c_int, [c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_vp, c_vp]),
     "b200seg_seam_tail_backward": (c_int, [c_vp, c_vp, c_vp, c_int, c_int, c_int, c_vp, c_vp, c_vp]),
+    "b200seg_bn_stats_scratch_bytes": (c_i64, [c_int, c_int]),
+    "b200seg_bn_stats": (c_int, [c_vp, c_int, c_int, c_int, c_vp, c_i64, c_vp, c_vp]),
+    "b200seg_bn_combine_stats": (c_int, [c_vp, c_int, c_int, c_f32, c_f32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
+    "b200seg_seam_tail_bn_forward": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_vp, c_vp]),
+    "b200seg_seam_tail_bn_backward_reduce_scratch_bytes": (c_i64, [c_int, c_int, c_int]),
+    "b200seg_seam_tail_bn_backward_reduce": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_vp, c_i64, c_vp, c_vp, c_vp,
+                                                     c_vp]),
+    "b200seg_seam_tail_bn_backward": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_vp, c_int, c_int, c_int, c_vp, c_vp,
+                                              c_vp]),
     "b200seg_nhwc_colsum_scratch_bytes": (c_i64, [c_int]),
     "b200seg_nhwc_bf16_colsum": (c_int, [c_vp, c_i64, c_int, c_int, c_vp, c_vp, c_vp]),
     "b200seg_gemm_set_overlap_sms": (None, [c_int]),
@@ -1250,6 +1259,139 @@ def seam_tail_backward(dy: torch.Tensor, y: torch.Tensor, scale: torch.Tensor, n
         return None, None
     with _on_device(y.device):
         _check(lib.b200seg_seam_tail_backward(dy.data_ptr(), y.data_ptr(), scale.data_ptr(), N, C, h * w, _ptr(dc), _ptr(di), _stream()))
+    return dc, di
+
+
+def _need_nchw_f32(t: torch.Tensor, name: str) -> torch.Tensor:
+    _need(t, torch.float32, name)
+    if t.dim() != 4:
+        raise B200SegError(f"{name}: expected an fp32 [N,C,h,w] tensor, got shape {tuple(t.shape)}")
+    return t
+
+
+def _optional_channel_vector(t: Optional[torch.Tensor], C: int, name: str) -> Optional[torch.Tensor]:
+    return None if t is None else _need_channel_vector(t, C, name)
+
+
+def bn_stats(c: torch.Tensor) -> torch.Tensor:
+    """fp64 [3, C] record (count, mean, M2 = sum (c - mean)^2) of fp32 NCHW ``c`` per channel: this rank's batch statistics."""
+    lib = load()
+    N, C, h, w = _need_nchw_f32(c, "c").shape
+    nbytes = lib.b200seg_bn_stats_scratch_bytes(N, C)
+    scratch = _scratch("bn_stats", nbytes, c.device)
+    record = torch.empty((3, C), dtype=torch.float64, device=c.device)
+    with _on_device(c.device):
+        _check(lib.b200seg_bn_stats(c.data_ptr(), N, C, h * w, scratch.data_ptr(), nbytes, record.data_ptr(), _stream()))
+    return record
+
+
+def bn_combine_stats(records: torch.Tensor, eps: float, momentum: Optional[float] = None, running_mean=None, running_var=None,
+                     num_batches_tracked=None):
+    """(mean, invstd, count): R records [R, 3, C] (or one [3, C]) combined in rank order; mean / invstd fp32 [C], count fp64 [1]
+    (the total M).  With running buffers, they are updated in place with factor ``momentum``, or 1 / num_batches_tracked (int64
+    [], read on the device) when ``momentum`` is None."""
+    lib = load()
+    _need(records, torch.float64, "records")
+    if records.dim() == 2:
+        records = records.unsqueeze(0)
+    if records.dim() != 3 or records.shape[1] != 3:
+        raise B200SegError(f"bn_combine_stats: expected records [R, 3, C], got {tuple(records.shape)}")
+    R, _, C = records.shape
+    if (running_mean is None) != (running_var is None):
+        raise B200SegError("bn_combine_stats: give both running buffers or neither")
+    _optional_channel_vector(running_mean, C, "running_mean")
+    _optional_channel_vector(running_var, C, "running_var")
+    nbt = None
+    if running_mean is not None and momentum is None:
+        nbt = _need(num_batches_tracked, torch.int64, "num_batches_tracked")
+        if nbt.numel() != 1:
+            raise B200SegError("bn_combine_stats: num_batches_tracked must hold one value")
+    mean = torch.empty(C, dtype=torch.float32, device=records.device)
+    invstd = torch.empty(C, dtype=torch.float32, device=records.device)
+    count = torch.empty(1, dtype=torch.float64, device=records.device)
+    with _on_device(records.device):
+        _check(lib.b200seg_bn_combine_stats(records.data_ptr(), R, C, float(eps), 0.0 if momentum is None else float(momentum),
+                                            _ptr(nbt), _ptr(running_mean), _ptr(running_var), mean.data_ptr(), invstd.data_ptr(),
+                                            count.data_ptr(), _stream()))
+    return mean, invstd, count
+
+
+def seam_tail_bn_forward(c: torch.Tensor, identity: torch.Tensor, mean: torch.Tensor, invstd: torch.Tensor,
+                         weight: Optional[torch.Tensor], bias: Optional[torch.Tensor]) -> torch.Tensor:
+    """bf16 channels_last y = bf16_rn(relu(((c - mean) * invstd * weight + bias) + identity)) from fp32 NCHW c / identity (the last
+    Bottleneck's training-mode bn3 + residual + relu, resnet.py:106-113); weight / bias None for affine=False.  C % 8 == 0."""
+    lib = load()
+    _need_nchw_f32(c, "c")
+    _need(identity, torch.float32, "identity")
+    if identity.shape != c.shape:
+        raise B200SegError(f"seam_tail_bn_forward: c {tuple(c.shape)} and identity {tuple(identity.shape)} must be equal [N,C,h,w]")
+    N, C, h, w = c.shape
+    for t, name in ((mean, "mean"), (invstd, "invstd")):
+        _need_channel_vector(t, C, name)
+    _optional_channel_vector(weight, C, "weight")
+    _optional_channel_vector(bias, C, "bias")
+    y = torch.empty((N, C, h, w), dtype=torch.bfloat16, device=c.device, memory_format=torch.channels_last)
+    with _on_device(c.device):
+        _check(lib.b200seg_seam_tail_bn_forward(c.data_ptr(), identity.data_ptr(), mean.data_ptr(), invstd.data_ptr(), _ptr(weight),
+                                                _ptr(bias), N, C, h * w, y.data_ptr(), _stream()))
+    return y
+
+
+def seam_tail_bn_backward_reduce(dy: torch.Tensor, y: torch.Tensor, c: torch.Tensor, mean: torch.Tensor, invstd: torch.Tensor,
+                                 need_weight: bool = False, need_bias: bool = False):
+    """(sums, grad_weight, grad_bias) with g = dy * (y > 0): sums fp32 [2, C] = (sum g, sum g * (c - mean)) over this rank, and the
+    local grad_bias = sum g, grad_weight = invstd * sum g * (c - mean) (None when not asked for)."""
+    lib = load()
+    _need_channels_last_bf16(dy, "dy")
+    _need_channels_last_bf16(y, "y")
+    _need_nchw_f32(c, "c")
+    if dy.shape != y.shape or c.shape != y.shape:
+        raise B200SegError(f"seam_tail_bn_backward_reduce: dy {tuple(dy.shape)}, y {tuple(y.shape)} and c {tuple(c.shape)} differ")
+    N, C, h, w = y.shape
+    _need_channel_vector(mean, C, "mean")
+    _need_channel_vector(invstd, C, "invstd")
+    nbytes = lib.b200seg_seam_tail_bn_backward_reduce_scratch_bytes(N, C, h * w)
+    scratch = _scratch("seam_bn_reduce", nbytes, y.device)
+    sums = torch.empty((2, C), dtype=torch.float32, device=y.device)
+    gw = torch.empty(C, dtype=torch.float32, device=y.device) if need_weight else None
+    gb = torch.empty(C, dtype=torch.float32, device=y.device) if need_bias else None
+    with _on_device(y.device):
+        _check(lib.b200seg_seam_tail_bn_backward_reduce(dy.data_ptr(), y.data_ptr(), c.data_ptr(), mean.data_ptr(), invstd.data_ptr(),
+                                                        N, C, h * w, scratch.data_ptr(), nbytes, sums.data_ptr(), _ptr(gw), _ptr(gb),
+                                                        _stream()))
+    return sums, gw, gb
+
+
+def seam_tail_bn_backward(dy: torch.Tensor, y: torch.Tensor, c: torch.Tensor, mean: torch.Tensor, invstd: torch.Tensor,
+                          weight: Optional[torch.Tensor], sums: torch.Tensor, count: torch.Tensor, need_c: bool = True,
+                          need_identity: bool = True):
+    """(dc, didentity), fp32 NCHW: g = dy * (y > 0); dc = (g - sum_g / M - (c - mean) * invstd^2 * sum_gx / M) * invstd * weight
+    with (sum_g, sum_gx) the R records of ``sums`` [R, 2, C] (or one [2, C]) added in rank order and M = count (fp64 [1], on the
+    device); didentity = g.  An output that is not needed is None (and not written)."""
+    lib = load()
+    _need_channels_last_bf16(dy, "dy")
+    _need_channels_last_bf16(y, "y")
+    _need_nchw_f32(c, "c")
+    if dy.shape != y.shape or c.shape != y.shape:
+        raise B200SegError(f"seam_tail_bn_backward: dy {tuple(dy.shape)}, y {tuple(y.shape)} and c {tuple(c.shape)} differ")
+    N, C, h, w = y.shape
+    _need_channel_vector(mean, C, "mean")
+    _need_channel_vector(invstd, C, "invstd")
+    _optional_channel_vector(weight, C, "weight")
+    _need(sums, torch.float32, "sums")
+    if sums.dim() == 2:
+        sums = sums.unsqueeze(0)
+    if sums.dim() != 3 or tuple(sums.shape[1:]) != (2, C):
+        raise B200SegError(f"seam_tail_bn_backward: expected sums [R, 2, {C}], got {tuple(sums.shape)}")
+    _need(count, torch.float64, "count")
+    dc = torch.empty((N, C, h, w), dtype=torch.float32, device=y.device) if need_c else None
+    di = torch.empty((N, C, h, w), dtype=torch.float32, device=y.device) if need_identity else None
+    if dc is None and di is None:
+        return None, None
+    with _on_device(y.device):
+        _check(lib.b200seg_seam_tail_bn_backward(dy.data_ptr(), y.data_ptr(), c.data_ptr(), mean.data_ptr(), invstd.data_ptr(),
+                                                 _ptr(weight), sums.data_ptr(), sums.shape[0], count.data_ptr(), N, C, h * w, _ptr(dc),
+                                                 _ptr(di), _stream()))
     return dc, di
 
 

@@ -96,6 +96,16 @@ int conv3x3_wgrad(const void*, int, long long, const void*, int, long long, int,
 int nchw_to_nhwc_bf16(const float*, int, int, int, void*, int, cudaStream_t);
 int seam_tail_forward(const float*, const float*, const float*, const float*, int, int, int, void*, cudaStream_t);
 int seam_tail_backward(const void*, const void*, const float*, int, int, int, float*, float*, cudaStream_t);
+long long bn_stats_scratch_bytes(int, int);
+int bn_stats(const float*, int, int, int, void*, long long, double*, cudaStream_t);
+int bn_combine_stats(const double*, int, int, float, float, const long long*, float*, float*, float*, float*, double*, cudaStream_t);
+int seam_tail_bn_forward(const float*, const float*, const float*, const float*, const float*, const float*, int, int, int, void*,
+                         cudaStream_t);
+long long seam_tail_bn_backward_reduce_scratch_bytes(int, int, int);
+int seam_tail_bn_backward_reduce(const void*, const void*, const float*, const float*, const float*, int, int, int, void*, long long,
+                                 float*, float*, float*, cudaStream_t);
+int seam_tail_bn_backward(const void*, const void*, const float*, const float*, const float*, const float*, const float*, int,
+                          const double*, int, int, int, float*, float*, cudaStream_t);
 long long nhwc_colsum_scratch_bytes(int);
 int nhwc_bf16_colsum(const void*, long long, int, int, void*, float*, cudaStream_t);
 int tta_launch(const float* const*, const int*, const int*, const int*, int, int, const void*, int, int, int, int, const float*, int, int,
@@ -540,6 +550,44 @@ int b200seg_seam_tail_backward(const void* dy, const void* y, const float* scale
                                void* stream) {
   REQUIRE_DEVICE();
   return seam_tail_backward(dy, y, scale, N, C, hw, dc, didentity, S(stream));
+}
+
+int64_t b200seg_bn_stats_scratch_bytes(int N, int C) { return bn_stats_scratch_bytes(N, C); }
+
+int b200seg_bn_stats(const float* c, int N, int C, int hw, void* scratch, int64_t scratch_bytes, double* record, void* stream) {
+  REQUIRE_DEVICE();
+  return bn_stats(c, N, C, hw, scratch, scratch_bytes, record, S(stream));
+}
+
+int b200seg_bn_combine_stats(const double* records, int R, int C, float eps, float momentum, const int64_t* num_batches_tracked,
+                             float* running_mean, float* running_var, float* mean, float* invstd, double* count, void* stream) {
+  REQUIRE_DEVICE();
+  return bn_combine_stats(records, R, C, eps, momentum, reinterpret_cast<const long long*>(num_batches_tracked), running_mean,
+                          running_var, mean, invstd, count, S(stream));
+}
+
+int b200seg_seam_tail_bn_forward(const float* c, const float* identity, const float* mean, const float* invstd, const float* gamma,
+                                 const float* beta, int N, int C, int hw, void* y, void* stream) {
+  REQUIRE_DEVICE();
+  return seam_tail_bn_forward(c, identity, mean, invstd, gamma, beta, N, C, hw, y, S(stream));
+}
+
+int64_t b200seg_seam_tail_bn_backward_reduce_scratch_bytes(int N, int C, int hw) {
+  return seam_tail_bn_backward_reduce_scratch_bytes(N, C, hw);
+}
+
+int b200seg_seam_tail_bn_backward_reduce(const void* dy, const void* y, const float* c, const float* mean, const float* invstd, int N,
+                                         int C, int hw, void* scratch, int64_t scratch_bytes, float* sums, float* dgamma, float* dbeta,
+                                         void* stream) {
+  REQUIRE_DEVICE();
+  return seam_tail_bn_backward_reduce(dy, y, c, mean, invstd, N, C, hw, scratch, scratch_bytes, sums, dgamma, dbeta, S(stream));
+}
+
+int b200seg_seam_tail_bn_backward(const void* dy, const void* y, const float* c, const float* mean, const float* invstd,
+                                  const float* gamma, const float* sums, int R, const double* count, int N, int C, int hw, float* dc,
+                                  float* didentity, void* stream) {
+  REQUIRE_DEVICE();
+  return seam_tail_bn_backward(dy, y, c, mean, invstd, gamma, sums, R, count, N, C, hw, dc, didentity, S(stream));
 }
 
 int b200seg_tta_argmax_confusion(const float* const* logits_lr, const int* h, const int* w, const int* flip, int n_members, int C,

@@ -10,7 +10,8 @@ scripts themselves stay unmodified (INTEGRATION.md).  ``install(optimizers=True)
 ``torch.optim.SGD`` / ``torch.optim.Adam`` constructions (aspp_trainer.py:25-26, fada_adapter.py:24) build FusedSGD / FusedAdam for
 parameter sets that live on a CUDA device (everything else keeps the stock classes).  ``install(seam=True)`` additionally wraps
 ``core.models.build.build_feature_extractor`` (same signature) so that the backbone it returns emits the head's seam format, bf16
-channels_last, from its last Bottleneck (seam.fuse_backbone_tail; INTEGRATION.md "Seam format").
+channels_last, from its last Bottleneck (seam.fuse_backbone_tail; INTEGRATION.md "Seam format"); with ``seam_train_bn=True`` also
+when that block's bn3 is a training-mode BatchNorm2d / SyncBatchNorm (batch statistics, the self-distillation stage).
 """
 from __future__ import annotations
 
@@ -76,7 +77,7 @@ def uninstall_optimizers():
         torch.optim.SGD, torch.optim.Adam = _stock_optimizers.pop("SGD"), _stock_optimizers.pop("Adam")
 
 
-def _install_seam(patched):
+def _install_seam(patched, train_bn=False):
     """core.models(.build).build_feature_extractor -> the same factory with fuse_backbone_tail applied to its result, also in
     modules that imported the name before."""
     wrapped = {}                     # id(stock function) -> wrapper (core.models re-exports core.models.build's function)
@@ -85,7 +86,7 @@ def _install_seam(patched):
         stock = getattr(mod, "build_feature_extractor", None) if mod is not None else None
         if stock is None:
             continue
-        fn = wrapped.setdefault(id(stock), _seam.wrap_feature_extractor_factory(stock))
+        fn = wrapped.setdefault(id(stock), _seam.wrap_feature_extractor_factory(stock, train_bn))
         wrapped[id(fn)] = fn
         setattr(mod, "build_feature_extractor", fn)
         patched.append(f"{modname}.build_feature_extractor")
@@ -99,9 +100,10 @@ def _install_seam(patched):
             patched.append(f"{name}.build_feature_extractor")
 
 
-def install(strict: bool = False, optimizers: bool = False, seam: bool = False):
+def install(strict: bool = False, optimizers: bool = False, seam: bool = False, seam_train_bn: bool = False):
     """Returns the list of 'module.attr' names that were patched.  ``seam=True``: the reference's build_feature_extractor returns
-    a backbone whose last Bottleneck emits bf16 channels_last features (seam.fuse_backbone_tail)."""
+    a backbone whose last Bottleneck emits bf16 channels_last features (seam.fuse_backbone_tail); ``seam_train_bn=True`` (with
+    ``seam=True``) extends that to a bn3 that trains with batch statistics (fuse_backbone_tail(fe, train_bn=True))."""
     patched = install_optimizers() if optimizers else []
     targets = (("core.models.build", _build, _BUILD_NAMES), ("core.models", _build, _BUILD_NAMES),
                ("core.utils.utility", _utility, _UTIL_NAMES), ("core.utils.adapt_lr", _optim, _LR_NAMES))
@@ -128,5 +130,5 @@ def install(strict: bool = False, optimizers: bool = False, seam: bool = False):
                     setattr(mod, n, getattr(src, n))
                     patched.append(f"{name}.{n}")
     if seam:
-        _install_seam(patched)
+        _install_seam(patched, seam_train_bn)
     return patched

@@ -261,12 +261,7 @@ class _SeamTailFn(torch.autograd.Function):
     def backward(ctx, dy):
         y, scale = ctx.saved_tensors
         need_c, need_id = ctx.needs_input_grad[0], ctx.needs_input_grad[1]
-        dy = dy.detach()
-        # the head's seam-format dgrad already writes bf16 channels_last; a sum of two consumers' gradients or the NCHW bf16
-        # gradient of the plain head call is converted once
-        if dy.dtype != torch.bfloat16 or not dy.is_contiguous(memory_format=torch.channels_last):
-            dy = dy.to(torch.bfloat16).contiguous(memory_format=torch.channels_last)
-        dc, di = _lib.seam_tail_backward(dy, y, scale.contiguous(), need_c, need_id)
+        dc, di = _lib.seam_tail_backward(_seam_dy(dy), y, scale.contiguous(), need_c, need_id)
         return dc, di, None, None
 
 
@@ -275,6 +270,77 @@ def seam_tail(c: torch.Tensor, identity: torch.Tensor, scale: torch.Tensor, bias
     and the folded norm's fp32 ``scale`` / ``bias`` [C] (constants: no gradient).  Bit-identical to the stock fp32 sequence
     followed by ``.to(torch.bfloat16)``; the gradient to ``c`` / ``identity`` is the stock one computed from the bf16 ``dy``."""
     return _SeamTailFn.apply(c, identity, scale, bias)
+
+
+def _seam_dy(dy: torch.Tensor) -> torch.Tensor:
+    """The incoming gradient of a seam-format output as bf16 channels_last: the head's seam-format dgrad already writes it; a sum
+    of two consumers' gradients or the NCHW bf16 gradient of the plain head call is converted once."""
+    dy = dy.detach()
+    if dy.dtype != torch.bfloat16 or not dy.is_contiguous(memory_format=torch.channels_last):
+        dy = dy.to(torch.bfloat16).contiguous(memory_format=torch.channels_last)
+    return dy
+
+
+def _gather_ranks(t: torch.Tensor, group) -> torch.Tensor:
+    """[R, *t.shape]: every rank's ``t`` in rank order (torch.distributed.all_gather_into_tensor, as torch's SyncBatchNorm)."""
+    import torch.distributed as dist
+    out = torch.empty((dist.get_world_size(group),) + tuple(t.shape), dtype=t.dtype, device=t.device)
+    dist.all_gather_into_tensor(out, t.contiguous(), group=group)
+    return out
+
+
+class _SeamTailBNFn(torch.autograd.Function):
+    """bf16 channels_last relu(batch_norm(c) + identity) with bn3 in training mode (resnet.py:106-113; BatchNorm2d, or
+    SyncBatchNorm over ``group``).  Saves c (which the stock BatchNorm saves too), y, mean, invstd and the total count: the stock
+    tail's fp32 relu output is not kept.  The running buffers are updated in place once per forward (under no_grad too)."""
+
+    @staticmethod
+    def forward(ctx, c, identity, weight, bias, running_mean, running_var, num_batches_tracked, momentum, eps, group):
+        cd = c.detach().contiguous()
+        w = None if weight is None else weight.detach().contiguous()
+        b = None if bias is None else bias.detach().contiguous()
+        records = _lib.bn_stats(cd)
+        if group is not None:
+            records = _gather_ranks(records, group)
+        if running_mean is not None and num_batches_tracked is not None:
+            num_batches_tracked.add_(1)
+        mean, invstd, count = _lib.bn_combine_stats(records, eps, momentum, running_mean, running_var, num_batches_tracked)
+        y = _lib.seam_tail_bn_forward(cd, identity.detach().contiguous(), mean, invstd, w, b)
+        ctx.group = group
+        ctx.save_for_backward(cd, y, mean, invstd, count, w)
+        return y
+
+    @staticmethod
+    def backward(ctx, dy):
+        c, y, mean, invstd, count, w = ctx.saved_tensors
+        need_c, need_id, need_w, need_b = ctx.needs_input_grad[:4]
+        dy = _seam_dy(dy)
+        dc = di = gw = gb = None
+        if need_c or need_w or need_b:
+            sums, gw, gb = _lib.seam_tail_bn_backward_reduce(dy, y, c, mean, invstd, need_w, need_b)
+            if need_c and ctx.group is not None:
+                sums = _gather_ranks(sums, ctx.group)       # dgamma / dbeta stay local: DDP averages them
+            dc, di = _lib.seam_tail_bn_backward(dy, y, c, mean, invstd, w, sums, count, need_c, need_id)
+        elif need_id:
+            _, di = _lib.seam_tail_backward(dy, y, invstd, False, True)     # didentity = g (the scale is not read)
+        return dc, di, gw, gb, None, None, None, None, None, None
+
+
+def seam_tail_bn(c: torch.Tensor, identity: torch.Tensor, weight: Optional[torch.Tensor], bias: Optional[torch.Tensor],
+                 running_mean: Optional[torch.Tensor], running_var: Optional[torch.Tensor],
+                 num_batches_tracked: Optional[torch.Tensor], momentum: Optional[float], eps: float, process_group=None) -> torch.Tensor:
+    """bf16 channels_last ``relu(batch_norm(c) + identity)`` with training-mode batch statistics, from fp32 NCHW ``c`` /
+    ``identity`` [N, C, h, w] (C % 8 == 0): the last Bottleneck's bn3 + residual + relu.  ``weight`` / ``bias`` are the norm's
+    affine parameters (None for affine=False) and receive gradients; ``running_mean`` / ``running_var`` / ``num_batches_tracked``
+    are updated in place as ``nn.BatchNorm2d`` does (factor ``momentum``, or the cumulative 1 / num_batches_tracked when it is
+    None).  ``process_group``: SyncBatchNorm statistics over that NCCL group -- the per-rank statistics in the forward and the
+    two per-channel sums in the backward are all-gathered and combined in rank order, so every rank computes bit-identical
+    statistics and c gradients.  The statistics match PyTorch's to fp32 rounding, not bit for bit (PyTorch's reduction order is
+    its own)."""
+    if process_group is None and c.numel() <= c.shape[1]:
+        raise ValueError(f"Expected more than 1 value per channel when training, got input size {tuple(c.shape)}")
+    return _SeamTailBNFn.apply(c, identity, weight, bias, running_mean, running_var, num_batches_tracked,
+                               None if momentum is None else float(momentum), float(eps), process_group)
 
 
 # --------------------------------------------------------------------------------------------

@@ -22,8 +22,17 @@ whose fold is verified: a FrozenBatchNorm2d (buffers only; ``weight * running_va
 an ``eps``), or an ``nn.BatchNorm2d`` in eval mode whose affine parameters need no gradient in the call.  The fold is checked
 against the module's own forward on a small seeded probe the first time and whenever the norm's tensors change (bit-equal for
 the frozen norm, within 4 fp32 ulp of the intermediates' magnitude for BatchNorm2d); the fold itself is recomputed from the
-norm's current tensors on every call.  Anything else -- a training-mode BatchNorm2d / SyncBatchNorm, another norm, a failed
-probe -- runs the block's stock forward.
+norm's current tensors on every call.  Anything else -- another norm, a failed probe, and by default a training-mode
+BatchNorm2d / SyncBatchNorm -- runs the block's stock forward.
+
+Batch statistics (opt-in: ``fuse_backbone_tail(fe, train_bn=True)`` / ``install(seam=True, seam_train_bn=True)``): a ``bn3`` that
+is exactly ``nn.BatchNorm2d`` or ``nn.SyncBatchNorm`` in training mode with running statistics runs ops.seam_tail_bn: the batch
+mean / variance, the running-statistics update and ``relu(((c - mean) * invstd * weight + bias) + identity)`` as bf16
+channels_last, with the gradient to c, identity and the norm's weight / bias.  A SyncBatchNorm whose group (``process_group`` or
+the world) has more than one rank exchanges its statistics over that group, which must be NCCL; otherwise it is per-rank, as
+in SyncBatchNorm.forward.  The statistics match PyTorch's to fp32 rounding, not bit for bit.  The flag also lets an eval-mode
+SyncBatchNorm with constant affine parameters take the fold.  Subclasses, ``track_running_stats=False``, another backend, a
+single value per channel, autocast and CPU input keep the stock forward.
 """
 from __future__ import annotations
 
@@ -31,6 +40,7 @@ import functools
 import warnings
 
 import torch
+import torch.distributed as dist
 import torch.nn as nn
 
 from . import ops
@@ -46,11 +56,13 @@ class _FusedForward:
     """What ``fuse_backbone_tail`` installs as the block's instance ``forward``: a plain picklable object (``torch.save`` of a
     whole fused extractor loads again; ``copy.deepcopy`` re-targets it to the copy).  It keeps the forward that was in the
     instance's __dict__ before (normally none) and the key (norm class, eps, data pointers and version counters of the norm's
-    tensors) under which the fold last passed or failed its probe."""
+    tensors) under which the fold last passed or failed its probe, and ``train_bn`` (fuse_backbone_tail's flag)."""
+    train_bn = False                    # (objects pickled before the flag existed load with the default)
 
-    def __init__(self, block, had_forward, old_forward):
+    def __init__(self, block, had_forward, old_forward, train_bn=False):
         self.block, self.had_forward, self.old_forward = block, had_forward, old_forward
         self.key, self.ok, self.warned = None, False, False
+        self.train_bn = bool(train_bn)
 
     def __getstate__(self):
         state = dict(self.__dict__)
@@ -69,9 +81,15 @@ def _last_bottleneck(feature_extractor: nn.Module):
     return last
 
 
-def _norm_kind(norm):
-    """'frozen', 'bn' (eval-mode BatchNorm2d with constant affine parameters in this call) or None (stays stock)."""
-    if isinstance(norm, nn.BatchNorm2d):
+def _norm_kind(norm, train_bn=False):
+    """'frozen', 'bn' (eval-mode BatchNorm2d with constant affine parameters in this call) or None (stays stock).  With
+    ``train_bn`` also 'batch' (exactly nn.BatchNorm2d / nn.SyncBatchNorm in training mode with running statistics), and an
+    eval-mode SyncBatchNorm is taken like an eval-mode BatchNorm2d."""
+    if train_bn and type(norm) in (nn.BatchNorm2d, nn.SyncBatchNorm) and norm.training:
+        if norm.track_running_stats and norm.running_mean is not None and norm.running_var is not None:
+            return "batch"
+        return None
+    if isinstance(norm, nn.BatchNorm2d) or (train_bn and isinstance(norm, nn.SyncBatchNorm)):
         if norm.training or norm.running_mean is None or norm.running_var is None:
             return None
         if norm.affine and torch.is_grad_enabled() and (norm.weight.requires_grad or norm.bias.requires_grad):
@@ -132,8 +150,8 @@ def _folded_norm(block, state, device):
     bumping their version counters, and writes through ``.data`` bypass them too, so no cached value could be trusted.  Only the
     probe, which checks that the module's forward IS ``x * scale + bias``, is keyed on the tensors' addresses and versions."""
     norm = block.bn3
-    kind = _norm_kind(norm)
-    if kind is None:
+    kind = _norm_kind(norm, state.train_bn)
+    if kind not in ("frozen", "bn"):
         return None
     tensors = _norm_tensors(norm, kind)
     if not all(isinstance(t, torch.Tensor) and t.device == device and t.dtype == torch.float32 for t in tensors):
@@ -149,6 +167,22 @@ def _folded_norm(block, state, device):
     return (scale, bias) if state.ok else None
 
 
+def _batch_group(norm, device):
+    """For a 'batch' norm: (group,) with the process group to exchange statistics over (None: this rank's batch only), or None
+    when the norm stays stock (tensors elsewhere or of another dtype, a group that is not NCCL)."""
+    tensors = [t for t in (norm.weight, norm.bias, norm.running_mean, norm.running_var) if t is not None]
+    if not all(t.device == device and t.dtype == torch.float32 for t in tensors):
+        return None
+    nbt = norm.num_batches_tracked
+    if nbt is not None and (nbt.device != device or nbt.dtype != torch.int64):
+        return None
+    if isinstance(norm, nn.SyncBatchNorm) and dist.is_available() and dist.is_initialized():
+        group = norm.process_group or dist.group.WORLD
+        if dist.get_world_size(group) > 1:
+            return (group,) if dist.get_backend(group) == "nccl" else None
+    return (None,)
+
+
 def _stock_forward(block, state, x):
     if state.had_forward:
         return state.old_forward(x)
@@ -157,10 +191,13 @@ def _stock_forward(block, state, x):
 
 def _fused_forward(block, state, x):
     """Bottleneck.forward with the tail after conv3 (resnet.py:106-113) as one seam-format kernel."""
-    fold = None
+    fold = batch = None
     if isinstance(x, torch.Tensor) and x.is_cuda and x.dtype == torch.float32 and block.conv3.out_channels % 8 == 0:
-        fold = _folded_norm(block, state, x.device)
-    if fold is None:
+        if _norm_kind(block.bn3, state.train_bn) == "batch":
+            batch = _batch_group(block.bn3, x.device)
+        else:
+            fold = _folded_norm(block, state, x.device)
+    if fold is None and batch is None:
         return _stock_forward(block, state, x)
     identity = x
     out = block.relu(block.bn1(block.conv1(x)))
@@ -168,11 +205,16 @@ def _fused_forward(block, state, x):
     c = block.conv3(out)
     if block.downsample is not None:
         identity = block.downsample(x)
-    if c.dtype != torch.float32 or identity.dtype != torch.float32 or identity.shape != c.shape:
-        # (autocast and friends) finish with the stock tail's own operations
+    single = batch is not None and batch[0] is None and c.numel() <= c.shape[1]
+    if c.dtype != torch.float32 or identity.dtype != torch.float32 or identity.shape != c.shape or single:
+        # (autocast and friends; one value per channel, which the stock norm rejects) finish with the stock tail's own operations
         out = block.bn3(c)
         out += identity
         return block.relu(out)
+    if batch is not None:
+        norm = block.bn3
+        return ops.seam_tail_bn(c, identity, norm.weight, norm.bias, norm.running_mean, norm.running_var, norm.num_batches_tracked,
+                                norm.momentum, norm.eps, batch[0])
     scale, bias = fold
     return ops.seam_tail(c, identity, scale, bias)
 
@@ -182,17 +224,21 @@ def _installed(block):
     return fwd if isinstance(fwd, _FusedForward) else None
 
 
-def fuse_backbone_tail(feature_extractor: nn.Module) -> nn.Module:
+def fuse_backbone_tail(feature_extractor: nn.Module, train_bn: bool = False) -> nn.Module:
     """Make the last Bottleneck of ``feature_extractor`` emit bf16 channels_last features (see the module docstring).  Returns
-    ``feature_extractor``; a second call is a no-op.  Raises ValueError when no Bottleneck-shaped module is found.
+    ``feature_extractor``; a second call only sets ``train_bn`` (a training-mode BatchNorm2d / SyncBatchNorm bn3 takes the
+    batch-statistics kernels).  Raises ValueError when no Bottleneck-shaped module is found.
     The hook lives in the block's instance __dict__: ``nn.DataParallel`` replicas (which copy that dict) would run it on the
     original block, so use one process per GPU (DistributedDataParallel), as the reference's trainers do."""
     block = _last_bottleneck(feature_extractor)
     if block is None:
         raise ValueError("fuse_backbone_tail: no module with conv1/bn1/conv2/bn2/conv3/bn3/relu/downsample (a Bottleneck) found")
-    if _installed(block) is None:
+    state = _installed(block)
+    if state is None:
         had = "forward" in block.__dict__
-        block.__dict__["forward"] = _FusedForward(block, had, block.__dict__.get("forward"))
+        block.__dict__["forward"] = _FusedForward(block, had, block.__dict__.get("forward"), train_bn)
+    else:
+        state.train_bn = bool(train_bn)
     return feature_extractor
 
 
@@ -214,17 +260,20 @@ def is_fused(feature_extractor: nn.Module) -> bool:
     return block is not None and _installed(block) is not None
 
 
-def wrap_feature_extractor_factory(stock):
-    """``build_feature_extractor`` with the same signature whose result goes through ``fuse_backbone_tail`` (install(seam=True))."""
+def wrap_feature_extractor_factory(stock, train_bn: bool = False):
+    """``build_feature_extractor`` with the same signature whose result goes through ``fuse_backbone_tail(fe, train_bn)``
+    (install(seam=True, seam_train_bn=...)).  Wrapping a wrapper returns it with its ``train_bn`` set to the new value."""
     if getattr(stock, "_b200seg_seam", False):
+        stock._b200seg_seam_train_bn = bool(train_bn)
         return stock
 
     @functools.wraps(stock)
     def build_feature_extractor(*args, **kwargs):
         fe = stock(*args, **kwargs)
         if isinstance(fe, nn.Module) and _last_bottleneck(fe) is not None:       # (a VGG backbone stays as built)
-            fuse_backbone_tail(fe)
+            fuse_backbone_tail(fe, train_bn=build_feature_extractor._b200seg_seam_train_bn)
         return fe
 
     build_feature_extractor._b200seg_seam = True
+    build_feature_extractor._b200seg_seam_train_bn = bool(train_bn)
     return build_feature_extractor
