@@ -330,6 +330,29 @@ B200SEG_API int b200seg_seam_tail_backward(const void* dy, const void* y, const 
                                            float* didentity, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * The same tail with conv3 fused in (opt-in): the last Bottleneck's 1x1 conv3 (stride 1, no bias) runs as a tcgen05 GEMM over
+ * pixels whose epilogue applies the folded bn3, the residual and the relu, so conv3's fp32 output is never materialised.
+ * b200seg_seam_conv3_forward  replaces  out = self.conv3(out); out = self.bn3(out); out += identity; out = self.relu(out)
+ *                                       (core/models/feature_extractor/resnet.py:106-113, bn3 folded to x * scale + bias) + bf16 cast:
+ *   y bf16 NHWC [N][hw][Cout] = bf16_rn(relu((acc * scale + bias) + identity)), acc = fp32 sum over ci of bf16(out2) * bf16(W3)
+ *   out2 fp32 NCHW [N][Cin][hw], identity fp32 NCHW [N][Cout][hw], W3 fp32 [Cout][Cin], scale / bias fp32 [Cout].
+ *   ws (b200seg_seam_conv3_workspace_bytes, 16-byte aligned) receives bf16(out2) NHWC and bf16(scale * W3)^T, which the backward
+ *   reads: keep it from the forward to the backward.
+ * b200seg_seam_conv3_backward  replaces  the autograd backward of the same lines (relu, add, bn3 and conv3's data and weight gradients):
+ *   g = dy * (y > 0);  didentity fp32 NCHW = g;  d_out2 fp32 NCHW [N][Cin][hw] = sum_co g[., co] * bf16(scale[co] W3[co, .]);
+ *   dW3 fp32 [Cout][Cin] = scale[co] * sum_p g[p, co] * bf16(out2)[p, ci] (split-K slabs summed in a fixed order, no atomics).
+ *   d_out2, dW3 and didentity may each be NULL.  Scratch: b200seg_seam_conv3_backward_scratch_bytes.
+ * Cin % 8 == 0, Cout % 8 == 0, any hw >= 1, any N; y and dy 16-byte aligned.
+ * ------------------------------------------------------------------------------------------- */
+B200SEG_API int64_t b200seg_seam_conv3_workspace_bytes(int N, int Cin, int Cout, int hw);
+B200SEG_API int b200seg_seam_conv3_forward(const float* out2, const float* identity, const float* w3, const float* scale, const float* bias,
+                                           int N, int Cin, int Cout, int hw, void* ws, int64_t ws_bytes, void* y, void* stream);
+B200SEG_API int64_t b200seg_seam_conv3_backward_scratch_bytes(int N, int Cin, int Cout, int hw);
+B200SEG_API int b200seg_seam_conv3_backward(const void* dy, const void* y, const void* ws, const float* scale, int N, int Cin, int Cout,
+                                            int hw, void* scratch, int64_t scratch_bytes, float* d_out2, float* dw3, float* didentity,
+                                            void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * The same tail with bn3 a training-mode BatchNorm2d / SyncBatchNorm (batch statistics): the end of Bottleneck.forward,
  * core/models/feature_extractor/resnet.py:106-113, in the self-distillation stage whose backbone train_distill.py:52-53 converts
  * with SyncBatchNorm.convert_sync_batchnorm.  c / identity fp32 NCHW [N][C][hw], M = N * hw per rank.  No atomics (every reduction

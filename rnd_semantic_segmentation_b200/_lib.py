@@ -103,6 +103,10 @@ SIGNATURES = {
     "b200seg_nchw_to_nhwc_bf16": (c_int, [c_vp, c_int, c_int, c_int, c_vp, c_int, c_vp]),
     "b200seg_seam_tail_forward": (c_int, [c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_vp, c_vp]),
     "b200seg_seam_tail_backward": (c_int, [c_vp, c_vp, c_vp, c_int, c_int, c_int, c_vp, c_vp, c_vp]),
+    "b200seg_seam_conv3_workspace_bytes": (c_i64, [c_int] * 4),
+    "b200seg_seam_conv3_forward": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_int, c_vp, c_i64, c_vp, c_vp]),
+    "b200seg_seam_conv3_backward_scratch_bytes": (c_i64, [c_int] * 4),
+    "b200seg_seam_conv3_backward": (c_int, [c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_int, c_vp, c_i64, c_vp, c_vp, c_vp, c_vp]),
     "b200seg_bn_stats_scratch_bytes": (c_i64, [c_int, c_int]),
     "b200seg_bn_stats": (c_int, [c_vp, c_int, c_int, c_int, c_vp, c_i64, c_vp, c_vp]),
     "b200seg_bn_combine_stats": (c_int, [c_vp, c_int, c_int, c_f32, c_f32, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp]),
@@ -1260,6 +1264,58 @@ def seam_tail_backward(dy: torch.Tensor, y: torch.Tensor, scale: torch.Tensor, n
     with _on_device(y.device):
         _check(lib.b200seg_seam_tail_backward(dy.data_ptr(), y.data_ptr(), scale.data_ptr(), N, C, h * w, _ptr(dc), _ptr(di), _stream()))
     return dc, di
+
+
+def seam_conv3_forward(out2: torch.Tensor, identity: torch.Tensor, weight: torch.Tensor, scale: torch.Tensor, bias: torch.Tensor):
+    """(y, ws): the last Bottleneck's conv3 + folded bn3 + residual + relu as one tcgen05 GEMM (resnet.py:106-113).  y bf16
+    channels_last [N, Cout, h, w] = bf16_rn(relu((acc * scale + bias) + identity)) with acc the fp32 sum of bf16(out2) * bf16(weight)
+    over Cin; out2 fp32 NCHW [N, Cin, h, w], identity fp32 NCHW [N, Cout, h, w], weight fp32 [Cout, Cin(, 1, 1)].  ``ws`` (uint8)
+    holds what seam_conv3_backward reads.  Cin % 8 == 0 and Cout % 8 == 0."""
+    lib = load()
+    N, Cin, h, w = _need_nchw_f32(out2, "out2").shape
+    _need(identity, torch.float32, "identity")
+    _need(weight, torch.float32, "weight")
+    Cout = weight.shape[0]
+    if weight.numel() != Cout * Cin or tuple(identity.shape) != (N, Cout, h, w):
+        raise B200SegError(f"seam_conv3_forward: out2 {tuple(out2.shape)}, weight {tuple(weight.shape)} and identity "
+                           f"{tuple(identity.shape)} do not form a 1x1 convolution")
+    _need_channel_vector(scale, Cout, "scale")
+    _need_channel_vector(bias, Cout, "bias")
+    nbytes = lib.b200seg_seam_conv3_workspace_bytes(N, Cin, Cout, h * w)
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=out2.device)
+    y = torch.empty((N, Cout, h, w), dtype=torch.bfloat16, device=out2.device, memory_format=torch.channels_last)
+    with _on_device(out2.device):
+        _check(lib.b200seg_seam_conv3_forward(out2.data_ptr(), identity.data_ptr(), weight.data_ptr(), scale.data_ptr(), bias.data_ptr(),
+                                              N, Cin, Cout, h * w, ws.data_ptr(), nbytes, y.data_ptr(), _stream()))
+    return y, ws
+
+
+def seam_conv3_backward(dy: torch.Tensor, y: torch.Tensor, ws: torch.Tensor, scale: torch.Tensor, Cin: int, need_out2: bool = True,
+                        need_weight: bool = True, need_identity: bool = True):
+    """(d_out2, d_weight, d_identity) of seam_conv3_forward from dy / y bf16 channels_last: g = dy * (y > 0); d_identity = g and
+    d_out2 = g . bf16(scale * weight) (fp32 NCHW); d_weight fp32 [Cout, Cin, 1, 1] = scale * (g^T . bf16(out2)).  An output that is
+    not needed is None (and not written)."""
+    lib = load()
+    _need_channels_last_bf16(dy, "dy")
+    _need_channels_last_bf16(y, "y")
+    if dy.shape != y.shape:
+        raise B200SegError(f"seam_conv3_backward: dy {tuple(dy.shape)} and y {tuple(y.shape)} differ")
+    N, Cout, h, w = y.shape
+    _need_channel_vector(scale, Cout, "scale")
+    _need(ws, torch.uint8, "ws")
+    if ws.numel() < lib.b200seg_seam_conv3_workspace_bytes(N, Cin, Cout, h * w):
+        raise B200SegError("seam_conv3_backward: workspace too small for this shape")
+    dx = torch.empty((N, Cin, h, w), dtype=torch.float32, device=y.device) if need_out2 else None
+    dw = torch.empty((Cout, Cin, 1, 1), dtype=torch.float32, device=y.device) if need_weight else None
+    di = torch.empty((N, Cout, h, w), dtype=torch.float32, device=y.device) if need_identity else None
+    if dx is None and dw is None and di is None:
+        return None, None, None
+    nbytes = lib.b200seg_seam_conv3_backward_scratch_bytes(N, Cin, Cout, h * w)
+    scratch = _scratch("seam_conv3", nbytes, y.device)
+    with _on_device(y.device):
+        _check(lib.b200seg_seam_conv3_backward(dy.data_ptr(), y.data_ptr(), ws.data_ptr(), scale.data_ptr(), N, Cin, Cout, h * w,
+                                               scratch.data_ptr(), nbytes, _ptr(dx), _ptr(dw), _ptr(di), _stream()))
+    return dx, dw, di
 
 
 def _need_nchw_f32(t: torch.Tensor, name: str) -> torch.Tensor:

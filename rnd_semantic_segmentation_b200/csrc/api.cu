@@ -96,6 +96,12 @@ int conv3x3_wgrad(const void*, int, long long, const void*, int, long long, int,
 int nchw_to_nhwc_bf16(const float*, int, int, int, void*, int, cudaStream_t);
 int seam_tail_forward(const float*, const float*, const float*, const float*, int, int, int, void*, cudaStream_t);
 int seam_tail_backward(const void*, const void*, const float*, int, int, int, float*, float*, cudaStream_t);
+long long seam_conv3_workspace_bytes(int, int, int, int);
+int seam_conv3_forward(const float*, const float*, const float*, const float*, const float*, int, int, int, int, void*, long long, void*,
+                       cudaStream_t);
+long long seam_conv3_backward_scratch_bytes(int, int, int, int);
+int seam_conv3_backward(const void*, const void*, const void*, const float*, int, int, int, int, void*, long long, float*, float*, float*,
+                        cudaStream_t);
 long long bn_stats_scratch_bytes(int, int);
 int bn_stats(const float*, int, int, int, void*, long long, double*, cudaStream_t);
 int bn_combine_stats(const double*, int, int, float, float, const long long*, float*, float*, float*, float*, double*, cudaStream_t);
@@ -550,6 +556,24 @@ int b200seg_seam_tail_backward(const void* dy, const void* y, const float* scale
                                void* stream) {
   REQUIRE_DEVICE();
   return seam_tail_backward(dy, y, scale, N, C, hw, dc, didentity, S(stream));
+}
+
+int64_t b200seg_seam_conv3_workspace_bytes(int N, int Cin, int Cout, int hw) { return seam_conv3_workspace_bytes(N, Cin, Cout, hw); }
+
+int b200seg_seam_conv3_forward(const float* out2, const float* identity, const float* w3, const float* scale, const float* bias, int N,
+                               int Cin, int Cout, int hw, void* ws, int64_t ws_bytes, void* y, void* stream) {
+  REQUIRE_DEVICE();
+  return seam_conv3_forward(out2, identity, w3, scale, bias, N, Cin, Cout, hw, ws, ws_bytes, y, S(stream));
+}
+
+int64_t b200seg_seam_conv3_backward_scratch_bytes(int N, int Cin, int Cout, int hw) {
+  return seam_conv3_backward_scratch_bytes(N, Cin, Cout, hw);
+}
+
+int b200seg_seam_conv3_backward(const void* dy, const void* y, const void* ws, const float* scale, int N, int Cin, int Cout, int hw,
+                                void* scratch, int64_t scratch_bytes, float* d_out2, float* dw3, float* didentity, void* stream) {
+  REQUIRE_DEVICE();
+  return seam_conv3_backward(dy, y, ws, scale, N, Cin, Cout, hw, scratch, scratch_bytes, d_out2, dw3, didentity, S(stream));
 }
 
 int64_t b200seg_bn_stats_scratch_bytes(int N, int C) { return bn_stats_scratch_bytes(N, C); }

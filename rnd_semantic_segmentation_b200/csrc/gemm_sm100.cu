@@ -56,15 +56,15 @@ int overlap_sms() { return g_overlap_sms; }
 static int g_share_enabled = 1;
 void set_sharing(int on) { g_share_enabled = on; }
 
-template <bool A_MN, bool B_MN, int SHARE, int BN = 256, bool RS = false>
+template <bool A_MN, bool B_MN, int SHARE, int BN = 256, bool RS = false, bool SEAM = false>
 static int launch_t(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& to, const Params& p, int grid, cudaStream_t stream) {
   static bool configured = false;
   if (!configured) {
-    B200SEG_CUDA(cudaFuncSetAttribute(gemm_bf16_kernel<A_MN, B_MN, SHARE, BN, RS>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+    B200SEG_CUDA(cudaFuncSetAttribute(gemm_bf16_kernel<A_MN, B_MN, SHARE, BN, RS, SEAM>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
     configured = true;
   }
   if (SHARE == SHARE_NONE) {
-    gemm_bf16_kernel<A_MN, B_MN, SHARE, BN, RS><<<grid, NUM_THREADS, SMEM_BYTES, stream>>>(ta, tb, to, p);
+    gemm_bf16_kernel<A_MN, B_MN, SHARE, BN, RS, SEAM><<<grid, NUM_THREADS, SMEM_BYTES, stream>>>(ta, tb, to, p);
   } else {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(grid);
@@ -78,7 +78,7 @@ static int launch_t(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensor
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    B200SEG_CUDA(cudaLaunchKernelEx(&cfg, gemm_bf16_kernel<A_MN, B_MN, SHARE, BN, RS>, ta, tb, to, p));
+    B200SEG_CUDA(cudaLaunchKernelEx(&cfg, gemm_bf16_kernel<A_MN, B_MN, SHARE, BN, RS, SEAM>, ta, tb, to, p));
   }
   B200SEG_LAUNCH_CHECK();
   return B200SEG_OK;
@@ -228,6 +228,46 @@ int launch(const Operand& a, const Operand& b, int M, int N, int K, int splits, 
   else if (a.mn_major && b.mn_major) rc = launch_s<true, true>(ta, tb, to, p, grid, share, stream);
   else if (a.mn_major && !b.mn_major) rc = launch_s<true, false>(ta, tb, to, p, grid, share, stream);
   else rc = launch_s<false, true>(ta, tb, to, p, grid, share, stream);
+  profile_end(prof_tag, stream);
+  return rc;
+}
+
+// Pixel-major forward with the seam epilogue (the fused conv3 + tail of the backbone's last Bottleneck): cta_group::2 pairs along
+// M walking along N, so a pair's two pixel tiles are read once for all N-tiles while the small weight operand stays in L2.
+int launch_seam(const Operand& a, const Operand& b, int M, int N, int K, __nv_bfloat16* out, const float* identity, const float* scale,
+                const float* bias, int hw, cudaStream_t stream, int prof_tag) {
+  B200SEG_CHECK_ARG(M > 0 && N > 0 && K > 0 && hw > 0 && (M % hw == 0 || M <= hw), "gemm seam: bad problem %dx%dx%d (hw %d)", M, N, K, hw);
+  B200SEG_CHECK_ARG(!a.mn_major && !b.mn_major, "gemm seam: K-major operands only");
+  B200SEG_CHECK_ARG(identity && scale && bias && N % 8 == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0,
+                    "gemm seam: N = %d must be a multiple of 8 and D 16-byte aligned", N);
+  Params p = {};
+  p.M = M; p.N = N; p.K = K;
+  p.m_tiles = ceil_div(M, BLOCK_M);
+  p.n_tiles = ceil_div(N, BLOCK_N);
+  p.kb_total = ceil_div(K, BLOCK_K);
+  p.splits = 1;
+  p.kb_per_split = p.kb_total;
+  p.out = reinterpret_cast<float*>(out);
+  p.row_stride = N;
+  p.col_hw = INT_MAX;
+  p.img_stride = (long long)N * hw;
+  p.out_bf16 = 1;
+  p.n_fastest = 1;
+  p.row_hw_px = hw;
+  p.seam_identity = identity;
+  p.seam_scale = scale;
+  p.seam_bias = bias;
+  const bool pair = g_share_enabled != 0 && p.m_tiles >= 2;
+  CUtensorMap ta, tb;
+  int rc = make_tmap(&ta, a.ptr, K, M, a.pitch, BLOCK_K, BLOCK_M);
+  if (rc) return rc;
+  rc = make_tmap(&tb, b.ptr, K, N, b.pitch, BLOCK_K, pair ? BLOCK_N / 2 : BLOCK_N);
+  if (rc) return rc;
+  const int sms = num_sms();
+  const int units = (pair ? (p.m_tiles + 1) / 2 : p.m_tiles) * p.n_tiles;
+  profile_begin(prof_tag, stream);
+  if (pair) rc = launch_t<false, false, SHARE_PAIR, 256, false, true>(ta, tb, ta, p, 2 * (units < sms / 2 ? units : sms / 2), stream);
+  else rc = launch_t<false, false, SHARE_NONE, 256, false, true>(ta, tb, ta, p, units < sms ? units : sms, stream);
   profile_end(prof_tag, stream);
   return rc;
 }

@@ -53,6 +53,11 @@ struct Params {
   int row_hw;               // > 0: ROWS of D are pixels of images with row_hw pixels each and D is fp32 NCHW: element (m, n)
                             // lives at out[(m / row_hw) * img_stride + n * row_hw + m % row_hw]; stored straight from registers
                             // (lane = pixel: a warp-level store is 32 consecutive pixels of one channel plane)
+  // seam epilogue (SEAM kernels only): D[m, n] = bf16_rn(relu((acc * scale[n] + bias[n]) + identity[m, n])), identity fp32 NCHW
+  // addressed as the row_hw map (row_hw_px pixels per image, img_stride elements between images), D bf16 row-major (out_bf16)
+  const float* seam_identity;
+  const float* seam_scale;
+  const float* seam_bias;
 };
 
 // ------------------------------------------------------------------------------------------
@@ -283,7 +288,9 @@ struct TileSched {
 // RS ("register stores"): the fp32 NCHW pixel-major epilogue only (Params::row_hw), which needs no shared-memory staging -- the
 // 32 KB go to a seventh ring stage instead (PAIR mode): the operand loads of this store-heavy problem see their latency inflated
 // by the epilogue's store bursts, and bytes in flight are what hides it.
-template <bool A_MN, bool B_MN, int SHARE, int BN = 256, bool RS = false>
+// SEAM: the bf16 row-major epilogue with the backbone tail applied to the accumulator first (Params::seam_*): M = pixels, so a
+// TMEM lane is a pixel and each identity column load is 32 consecutive pixels of one fp32 NCHW plane.  K-major operands only.
+template <bool A_MN, bool B_MN, int SHARE, int BN = 256, bool RS = false, bool SEAM = false>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
                  const __grid_constant__ CUtensorMap tmap_out, const Params p) {
@@ -297,6 +304,7 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
   constexpr int BLOCK_N = BN;                                       // shadows gemm::BLOCK_N below
   constexpr int B_BYTES = BN * BLOCK_K * 2;
   static_assert(!RS || (PAIR && BN == 256), "register-store variant: cta_group::2 pairs only");
+  static_assert(!SEAM || (!RS && !A_MN && !B_MN && BN == 256), "seam epilogue: K-major operands, 256-column tiles");
   constexpr int STAGES = PAIR ? (RS ? PAIR_STAGES + 1 : PAIR_STAGES) : gemm::STAGES;         // same total bytes either way
   constexpr int STAGE_BYTES = PAIR ? PAIR_STAGE_BYTES : gemm::STAGE_BYTES;     // ring stride (a narrow B tile leaves its tail unused)
   constexpr int STAGE_TX = PAIR ? PAIR_STAGE_BYTES : A_BYTES + B_BYTES;        // bytes that land in a stage per k-block
@@ -481,18 +489,40 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
       tc_fence_after();
       const uint32_t taddr = tmem_base + ((uint32_t)(wq * 32) << 16) + (uint32_t)(acc * gemm::BLOCK_N + half * (BLOCK_N / 2));
       const int rows = min(32, p.M - row_base);
-      if (!RS && p.out_bf16) {
+      if (SEAM || (!RS && p.out_bf16)) {
         // bf16 row-major D (the NHWC feature gradient): 32 columns per pass, converted before the smem transpose, every
         // store instruction writes 8 rows x 64 contiguous bytes
         if (rows > 0 && col_base < p.N) {
           __nv_bfloat16* outb = reinterpret_cast<__nv_bfloat16*>(p.out) + (long long)z * p.split_stride;
           uint32_t* stw = reinterpret_cast<uint32_t*>(stg);
+          const float* idp = nullptr;                  // SEAM: this lane's pixel in channel plane 0 of its image
+          if (SEAM) {
+            const int m = lane < rows ? row_base + lane : row_base;
+            const int img = m / p.row_hw_px;
+            idp = p.seam_identity + (long long)img * p.img_stride + (m - img * p.row_hw_px);
+          }
 #pragma unroll 1
           for (int c = 0; c < BLOCK_N / 2 / 32; ++c) {
             uint32_t r[32];
             tmem_ld16(taddr + (uint32_t)(c * 32), r);
             tmem_ld16(taddr + (uint32_t)(c * 32 + 16), r + 16);
-            tmem_ld_wait();
+            if (SEAM) {
+              // the 32 identity loads are in flight with the TMEM loads; the tail in the stock order (mul, add, add, relu)
+              const int cb = col_base + c * 32;
+              float id[32];
+#pragma unroll
+              for (int k = 0; k < 32; ++k)
+                id[k] = (lane < rows && cb + k < p.N) ? __ldcs(idp + (long long)(cb + k) * p.row_hw_px) : 0.f;
+              tmem_ld_wait();
+#pragma unroll
+              for (int k = 0; k < 32; ++k) {
+                const int n = min(cb + k, p.N - 1);
+                const float v = __fadd_rn(__fadd_rn(__fmul_rn(__uint_as_float(r[k]), __ldg(p.seam_scale + n)), __ldg(p.seam_bias + n)), id[k]);
+                r[k] = __float_as_uint(v <= 0.f ? 0.f : v);      // NaN passes through, as torch.relu
+              }
+            } else {
+              tmem_ld_wait();
+            }
 #pragma unroll
             for (int k = 0; k < 4; ++k) {
               uint32_t w4[4];
@@ -940,6 +970,10 @@ int launch_fwd_convert(const __nv_bfloat16* a, long long a_pitch, const float* x
 int launch(const Operand& a, const Operand& b, int M, int N, int K, int splits, float* out, long long row_stride,
            int col_hw, long long img_stride, long long split_stride, cudaStream_t stream, int* splits_used, int prof_tag = -1,
            int share = SHARE_NONE, bool out_bf16 = false, int sm_reserve = 0, int pair_fallback = SHARE_B, int row_hw = 0);
+// D bf16 [M][N] row-major = bf16_rn(relu((A B^T * scale + bias) + identity)) with M = n_img * hw pixels, identity fp32 NCHW
+// [n_img][N][hw]; A [M][K] and B [N][K] K-major.  N % 8 == 0, D 16-byte aligned.
+int launch_seam(const Operand& a, const Operand& b, int M, int N, int K, __nv_bfloat16* out, const float* identity, const float* scale,
+                const float* bias, int hw, cudaStream_t stream, int prof_tag = -1);
 // fp32 NCHW data gradient of the head: 0 = channels along M (shared-memory transpose epilogue), 1 = pixels along M as cta_group::2
 // pairs, stores straight from registers, seven ring stages
 void set_dgrad_mode(int mode);

@@ -1,0 +1,151 @@
+// Fused backbone tail with conv3: the last Bottleneck's 1x1 conv3 runs as a tcgen05 GEMM whose epilogue applies the folded bn3,
+// the residual add, the ReLU and the bf16 channels_last cast, so conv3's fp32 output c is never written nor read back.
+//
+// Replaces (reference file:line): core/models/feature_extractor/resnet.py:106-113
+//   out = self.conv3(out); out = self.bn3(out); out += identity; out = self.relu(out)
+// with conv3 a bias-free 1x1 stride-1 convolution (a plain GEMM over pixels) and bn3 folded to x * scale + bias:
+//   forward   Xp = bf16(out2) NHWC [P][Cin];  W3b = bf16(W3) [Cout][Cin];  W't = bf16(scale * W3)^T [Cin][Cout]
+//             y[p, co] = bf16_rn(relu((acc[p, co] * scale[co] + bias[co]) + identity[p, co])),  acc = sum_ci Xp[p, ci] W3b[co, ci]
+//   backward  g = dy * (y > 0) (bf16 NHWC, exact);  didentity = g (fp32 NCHW)
+//             d_out2[p, ci] = sum_co g[p, co] W'[co, ci]           (fp32 NCHW, register-store epilogue)
+//             dW3[co, ci] = scale[co] * sum_p g[p, co] Xp[p, ci]    (split-K fp32 slabs summed in a fixed order: no atomics)
+// bf16 operands, fp32 accumulation in TMEM: out2 and W3 are each rounded to bf16 once, the tail is applied to the fp32 accumulator
+// in the fold path's __fmul_rn / __fadd_rn order, then one bf16 rounding.  No host synchronisation (capturable in a CUDA graph).
+#include "gemm_sm100.cuh"
+
+namespace b200seg {
+
+int nchw_to_nhwc_bf16(const float* src, int N, int C, int hw, void* dst, int pitch, cudaStream_t stream);   // seam_tail_kernels.cu
+int seam_conv3_g(const void* dy, const void* y, int N, int C, int hw, void* g, float* didentity, cudaStream_t stream);
+
+// W3 fp32 [Cout][Cin] -> W3b bf16 [Cout][Cin] and W't bf16 [Cin][Cout] (W'[co, ci] = bf16_rn(scale[co] * W3[co, ci])), through a
+// 32 x 32 shared-memory tile
+__global__ void __launch_bounds__(256) seam_conv3_pack_weights_kernel(const float* __restrict__ w, const float* __restrict__ scale,
+                                                                      int Cout, int Cin, __nv_bfloat16* __restrict__ wb,
+                                                                      __nv_bfloat16* __restrict__ wt) {
+  __shared__ float tile[32][33];
+  const int ci0 = blockIdx.x * 32, co0 = blockIdx.y * 32;
+  const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const int co = co0 + ty + 8 * i, ci = ci0 + tx;
+    if (co < Cout && ci < Cin) {
+      const float v = w[(long long)co * Cin + ci];
+      wb[(long long)co * Cin + ci] = __float2bfloat16_rn(v);
+      tile[ty + 8 * i][tx] = __fmul_rn(__ldg(scale + co), v);
+    }
+  }
+  __syncthreads();
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    const int ci = ci0 + ty + 8 * i, co = co0 + tx;
+    if (co < Cout && ci < Cin) wt[(long long)ci * Cout + co] = __float2bfloat16_rn(tile[tx][ty + 8 * i]);
+  }
+}
+
+// dW[co, ci] = scale[co] * (part[0] + part[1] + ... + part[S-1])[co, ci], four consecutive ci per thread (Cin % 8 == 0)
+__global__ void __launch_bounds__(256) seam_conv3_wgrad_reduce_kernel(const float* __restrict__ part, int S, long long slab,
+                                                                      const float* __restrict__ scale, int Cin, float* __restrict__ dw) {
+  const long long i = ((long long)blockIdx.x * blockDim.x + threadIdx.x) * 4;
+  if (i >= slab) return;
+  float4 a = __ldcs(reinterpret_cast<const float4*>(part + i));
+  for (int s = 1; s < S; ++s) {
+    const float4 v = __ldcs(reinterpret_cast<const float4*>(part + s * slab + i));
+    a.x += v.x; a.y += v.y; a.z += v.z; a.w += v.w;
+  }
+  const float sc = __ldg(scale + i / Cin);
+  reinterpret_cast<float4*>(dw)[i / 4] = make_float4(__fmul_rn(a.x, sc), __fmul_rn(a.y, sc), __fmul_rn(a.z, sc), __fmul_rn(a.w, sc));
+}
+
+static long long align256(long long b) { return (b + 255) / 256 * 256; }
+static bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15) == 0; }
+
+// workspace (forward -> backward): Xp bf16 [P][Cin] | W't bf16 [Cin][Cout] | W3b bf16 [Cout][Cin]
+long long seam_conv3_workspace_bytes(int N, int Cin, int Cout, int hw) {
+  return align256((long long)N * hw * Cin * 2) + 2 * align256((long long)Cin * Cout * 2);
+}
+
+// split-K factor of the weight-gradient GEMM: one unit per CTA pair (Cout / 256 pairs of M-tiles x Cin / 256 N-tiles per split)
+static int wgrad_splits(int Cin, int Cout, long long P) {
+  const int units = ceil_div(ceil_div(Cout, gemm::BLOCK_M), 2) * ceil_div(Cin, gemm::BLOCK_N);
+  const int kb = (int)ceil_div_ll(P, gemm::BLOCK_K);
+  int s = (num_sms() / 2) / units;
+  if (s > 8) s = 8;
+  if (s > kb) s = kb;
+  return s < 1 ? 1 : s;
+}
+
+// scratch (backward only): g bf16 [P][Cout] | wgrad slabs fp32 [S][Cout][Cin]
+long long seam_conv3_backward_scratch_bytes(int N, int Cin, int Cout, int hw) {
+  const long long P = (long long)N * hw;
+  return align256(P * Cout * 2) + (long long)wgrad_splits(Cin, Cout, P) * Cout * Cin * 4;
+}
+
+static int check_shape(const char* who, int N, int Cin, int Cout, int hw) {
+  B200SEG_CHECK_ARG(N > 0 && Cin > 0 && Cout > 0 && hw > 0, "%s: bad shape", who);
+  B200SEG_CHECK_ARG(Cin % 8 == 0 && Cout % 8 == 0, "%s: Cin = %d and Cout = %d must be multiples of 8", who, Cin, Cout);
+  B200SEG_CHECK_ARG((long long)N * hw < (1LL << 31) - 256, "%s: too many pixels", who);
+  return B200SEG_OK;
+}
+
+int seam_conv3_forward(const float* out2, const float* identity, const float* w3, const float* scale, const float* bias, int N, int Cin,
+                       int Cout, int hw, void* ws, long long ws_bytes, void* y, cudaStream_t stream) {
+  B200SEG_CHECK_ARG(out2 && identity && w3 && scale && bias && ws && y, "seam_conv3_forward: null pointer");
+  if (int rc = check_shape("seam_conv3_forward", N, Cin, Cout, hw)) return rc;
+  B200SEG_CHECK_ARG(ws_bytes >= seam_conv3_workspace_bytes(N, Cin, Cout, hw) && aligned16(ws) && aligned16(y),
+                    "seam_conv3_forward: workspace too small, or workspace / y not 16-byte aligned");
+  const long long P = (long long)N * hw;
+  uint8_t* sp = reinterpret_cast<uint8_t*>(ws);
+  __nv_bfloat16* Xp = reinterpret_cast<__nv_bfloat16*>(sp);
+  __nv_bfloat16* Wt = reinterpret_cast<__nv_bfloat16*>(sp + align256(P * Cin * 2));
+  __nv_bfloat16* Wb = reinterpret_cast<__nv_bfloat16*>(sp + align256(P * Cin * 2) + align256((long long)Cin * Cout * 2));
+  int rc = nchw_to_nhwc_bf16(out2, N, Cin, hw, Xp, Cin, stream);
+  if (rc) return rc;
+  seam_conv3_pack_weights_kernel<<<dim3(ceil_div(Cin, 32), ceil_div(Cout, 32)), 256, 0, stream>>>(w3, scale, Cout, Cin, Wb, Wt);
+  B200SEG_LAUNCH_CHECK();
+  gemm::Operand a{Xp, false, Cin};
+  gemm::Operand b{Wb, false, Cin};
+  return gemm::launch_seam(a, b, (int)P, Cout, Cin, reinterpret_cast<__nv_bfloat16*>(y), identity, scale, bias, hw,
+                           stream);
+}
+
+int seam_conv3_backward(const void* dy, const void* y, const void* ws, const float* scale, int N, int Cin, int Cout, int hw,
+                        void* scratch, long long scratch_bytes, float* d_out2, float* dw3, float* didentity, cudaStream_t stream) {
+  B200SEG_CHECK_ARG(dy && y && ws && scale && scratch, "seam_conv3_backward: null pointer");
+  if (int rc = check_shape("seam_conv3_backward", N, Cin, Cout, hw)) return rc;
+  B200SEG_CHECK_ARG(scratch_bytes >= seam_conv3_backward_scratch_bytes(N, Cin, Cout, hw) && aligned16(scratch) && aligned16(ws) &&
+                        aligned16(dw3),
+                    "seam_conv3_backward: scratch too small, or scratch / workspace / dW3 not 16-byte aligned");
+  if (!d_out2 && !dw3 && !didentity) return B200SEG_OK;
+  const long long P = (long long)N * hw;
+  const uint8_t* wp = reinterpret_cast<const uint8_t*>(ws);
+  const __nv_bfloat16* Xp = reinterpret_cast<const __nv_bfloat16*>(wp);
+  const __nv_bfloat16* Wt = reinterpret_cast<const __nv_bfloat16*>(wp + align256(P * Cin * 2));
+  __nv_bfloat16* g = reinterpret_cast<__nv_bfloat16*>(scratch);
+  float* wpart = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(scratch) + align256(P * Cout * 2));
+  int rc = seam_conv3_g(dy, y, N, Cout, hw, g, didentity, stream);
+  if (rc) return rc;
+  if (dw3) {
+    // dW3[co, ci] = sum_p g[p, co] Xp[p, ci]: both operands MN-major as the forward left them, split-K over pixels
+    gemm::Operand a{g, true, Cout};
+    gemm::Operand b{Xp, true, Cin};
+    const long long slab = (long long)Cout * Cin;
+    int used = 1;
+    rc = gemm::launch(a, b, Cout, Cin, (int)P, wgrad_splits(Cin, Cout, P), wpart, Cin, 0, 0, slab, stream, &used, -1, gemm::SHARE_PAIR,
+                      false, 0, gemm::SHARE_A);
+    if (rc) return rc;
+    seam_conv3_wgrad_reduce_kernel<<<(unsigned)ceil_div_ll(slab / 4, 256), 256, 0, stream>>>(wpart, used, slab, scale, Cin, dw3);
+    B200SEG_LAUNCH_CHECK();
+  }
+  if (d_out2) {
+    // d_out2[p, ci] = sum_co g[p, co] W'[co, ci] with the pixels along M, fp32 NCHW straight from the accumulator registers
+    gemm::Operand a{g, false, Cout};
+    gemm::Operand b{Wt, false, Cout};
+    rc = gemm::launch(a, b, (int)P, Cin, Cout, 1, d_out2, 0, 0, (long long)Cin * hw, 0, stream, nullptr, -1, gemm::SHARE_PAIR, false, 0,
+                      gemm::SHARE_B, hw);
+    if (rc) return rc;
+  }
+  return B200SEG_OK;
+}
+
+}  // namespace b200seg

@@ -116,7 +116,9 @@ __global__ void __launch_bounds__(ST_THREADS) nchw_to_nhwc_tile_kernel(const flo
 //             (P = N * gridDim.x) and nothing else;
 //   BN_APPLY  writes dc = (g - sum_g / M - (c - mean) * invstd^2 * sum_gx / M) * invstd * gamma with the sums taken over the R
 //             records of sums [R][2][C] in rank order and M = *count (gamma may be null), and didentity = g.
-enum { BN_FOLD = 0, BN_REDUCE = 1, BN_APPLY = 2 };
+// BN_G (the fused conv3 tail, whose conv3 runs inside the tcgen05 GEMMs) writes g itself as bf16 NHWC (the GEMMs' operand; exact,
+// no rounding) and didentity = g; c, scale and dc are not used.
+enum { BN_FOLD = 0, BN_REDUCE = 1, BN_APPLY = 2, BN_G = 3 };
 struct BnBackward {
   const float* c;
   const float* mean;
@@ -126,6 +128,7 @@ struct BnBackward {
   int R;
   const double* count;
   float2* partial;
+  __nv_bfloat16* g;
 };
 
 // VEC: hw % 4 == 0 and the requested outputs (and c) 16-byte aligned (float4 rows); otherwise scalar accesses.  dc / didentity may
@@ -152,7 +155,7 @@ __global__ void __launch_bounds__(ST_THREADS) seam_tail_backward_kernel(const __
     }
   }
   float4 cv[4];                                                    // the c rows this thread owns after the barrier, also in flight
-  if (BN != BN_FOLD) {
+  if (BN != BN_FOLD && BN != BN_G) {
     const int s = s0 + 4 * lane;
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
@@ -181,6 +184,15 @@ __global__ void __launch_bounds__(ST_THREADS) seam_tail_backward_kernel(const __
       const float2 y2 = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(y32 + e));
       tile[st_idx(8 * chunk + 2 * e, sl)] = y2.x > 0.f ? g2.x : 0.f;
       tile[st_idx(8 * chunk + 2 * e + 1, sl)] = y2.y > 0.f ? g2.y : 0.f;
+    }
+    if (BN == BN_G && s0 + sl < hw && cc < C) {                    // the same values as bf16 NHWC: dy's bits where y > 0, else +0
+      uint32_t w4[4];
+#pragma unroll
+      for (int e = 0; e < 4; ++e) {
+        const float2 y2 = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(y32 + e));
+        w4[e] = (y2.x > 0.f ? (g32[e] & 0xffffu) : 0u) | (y2.y > 0.f ? (g32[e] & 0xffff0000u) : 0u);
+      }
+      *reinterpret_cast<uint4*>(bn.g + ((long long)n * hw + s0 + sl) * C + cc) = make_uint4(w4[0], w4[1], w4[2], w4[3]);
     }
   }
   __syncthreads();
@@ -214,9 +226,11 @@ __global__ void __launch_bounds__(ST_THREADS) seam_tail_backward_kernel(const __
       const float mdy = sg * norm, f1 = is * is * sx * norm, f2 = (bn.gamma ? __ldg(bn.gamma + cg) : 1.f) * is;
       d = make_float4((g.x - mdy - (cv[i].x - mu) * f1) * f2, (g.y - mdy - (cv[i].y - mu) * f1) * f2,
                       (g.z - mdy - (cv[i].z - mu) * f1) * f2, (g.w - mdy - (cv[i].w - mu) * f1) * f2);
-    } else {
+    } else if (BN == BN_FOLD) {
       const float sc = __ldg(scale + cg);
       d = make_float4(__fmul_rn(g.x, sc), __fmul_rn(g.y, sc), __fmul_rn(g.z, sc), __fmul_rn(g.w, sc));
+    } else {
+      d = g;                                                       // (BN_G: dc is null)
     }
     const long long off = ((long long)n * C + cg) * hw + s;
     if (VEC) {
@@ -438,6 +452,20 @@ int seam_tail_backward(const void* dy, const void* y, const float* scale, int N,
   B200SEG_CHECK_ARG(aligned16(dy) && aligned16(y), "seam_tail_backward: dy and y must be 16-byte aligned");
   if (!dc && !didentity) return B200SEG_OK;
   backward_launch<BN_FOLD>(dy, y, scale, N, C, hw, dc, didentity, BnBackward{}, stream);
+  B200SEG_LAUNCH_CHECK();
+  return B200SEG_OK;
+}
+
+// g = dy * (y > 0) as bf16 NHWC [N*hw][C] (the operand of the fused conv3's data- and weight-gradient GEMMs) and, when didentity is
+// not null, didentity = g as fp32 NCHW
+int seam_conv3_g(const void* dy, const void* y, int N, int C, int hw, void* g, float* didentity, cudaStream_t stream) {
+  B200SEG_CHECK_ARG(dy && y && g && N > 0 && C > 0 && hw > 0, "seam_conv3_g: bad arguments");
+  B200SEG_CHECK_ARG(C % 8 == 0, "seam_conv3_g: C = %d is not a multiple of 8", C);
+  B200SEG_CHECK_ARG(N <= 65535 && ceil_div(C, ST_CH) <= 65535, "seam_conv3_g: N = %d / C = %d too large", N, C);
+  B200SEG_CHECK_ARG(aligned16(dy) && aligned16(y) && aligned16(g), "seam_conv3_g: dy, y and g must be 16-byte aligned");
+  BnBackward bn{};
+  bn.g = reinterpret_cast<__nv_bfloat16*>(g);
+  backward_launch<BN_G>(dy, y, nullptr, N, C, hw, nullptr, didentity, bn, stream);
   B200SEG_LAUNCH_CHECK();
   return B200SEG_OK;
 }

@@ -272,6 +272,41 @@ def seam_tail(c: torch.Tensor, identity: torch.Tensor, scale: torch.Tensor, bias
     return _SeamTailFn.apply(c, identity, scale, bias)
 
 
+class _SeamConv3TailFn(torch.autograd.Function):
+    """bf16 channels_last relu((conv1x1(out2, W3) * scale + bias) + identity)  (resnet.py:106-113 with conv3 a bias-free 1x1
+    convolution and bn3 folded).  Saves y and the forward's workspace (bf16 out2 and bf16(scale * W3)^T), never conv3's fp32 output;
+    nothing when no input needs a gradient."""
+
+    @staticmethod
+    def forward(ctx, out2, identity, weight, scale, bias):
+        scale = scale.detach().contiguous()
+        y, ws = _lib.seam_conv3_forward(out2.detach().contiguous(), identity.detach().contiguous(), weight.detach().contiguous(), scale,
+                                        bias.detach().contiguous())
+        if any(ctx.needs_input_grad[:3]):
+            ctx.cin = out2.shape[1]
+            ctx.save_for_backward(y, ws, scale)
+        return y
+
+    @staticmethod
+    def backward(ctx, dy):
+        y, ws, scale = ctx.saved_tensors
+        need_x, need_id, need_w = ctx.needs_input_grad[:3]
+        dx, dw, di = _lib.seam_conv3_backward(_seam_dy(dy), y, ws, scale, ctx.cin, need_x, need_w, need_id)
+        return dx, di, dw, None, None
+
+
+def seam_conv3_tail(out2: torch.Tensor, identity: torch.Tensor, weight: torch.Tensor, scale: torch.Tensor,
+                    bias: torch.Tensor) -> torch.Tensor:
+    """bf16 channels_last ``relu((conv3(out2) * scale + bias) + identity)``: the last Bottleneck's 1x1 conv3 (stride 1, no bias,
+    fp32 ``weight`` [Cout, Cin, 1, 1]) and folded bn3 (fp32 ``scale`` / ``bias`` [Cout], constants) as one tcgen05 GEMM whose
+    epilogue adds the fp32 NCHW ``identity`` [N, Cout, h, w]; ``out2`` fp32 NCHW [N, Cin, h, w], Cin % 8 == 0, Cout % 8 == 0.
+    Numerics: out2 and weight are each rounded to bf16 once, the products are accumulated in fp32, the tail is applied to the
+    accumulator as ``relu((acc * scale + bias) + identity)`` (each step rounded in fp32, no FMA) and the result rounded once to
+    bf16 -- not bit-identical to the stock fp32 block.  Differentiable in out2, identity and weight; the data gradient uses
+    bf16(scale * weight) and the weight gradient bf16(out2), both with fp32 accumulation."""
+    return _SeamConv3TailFn.apply(out2, identity, weight, scale, bias)
+
+
 def _seam_dy(dy: torch.Tensor) -> torch.Tensor:
     """The incoming gradient of a seam-format output as bf16 channels_last: the head's seam-format dgrad already writes it; a sum
     of two consumers' gradients or the NCHW bf16 gradient of the plain head call is converted once."""

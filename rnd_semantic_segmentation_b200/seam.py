@@ -33,6 +33,17 @@ the world) has more than one rank exchanges its statistics over that group, whic
 in SyncBatchNorm.forward.  The statistics match PyTorch's to fp32 rounding, not bit for bit.  The flag also lets an eval-mode
 SyncBatchNorm with constant affine parameters take the fold.  Subclasses, ``track_running_stats=False``, another backend, a
 single value per channel, autocast and CPU input keep the stock forward.
+
+conv3 fused into the tail (opt-in: ``fuse_backbone_tail(fe, conv3=True)`` / ``install(seam=True, seam_conv3=True)``): when the fold
+applies (a 'frozen' or 'bn' bn3 as above) and ``conv3`` is exactly ``nn.Conv2d`` -- 1x1, stride 1, padding 0, groups 1, no bias,
+an fp32 weight on the input's device, Cin % 8 == 0 and Cout % 8 == 0 -- and conv2's output is fp32, the block runs
+ops.seam_conv3_tail: conv3 as a tcgen05 GEMM whose epilogue applies the fold, the residual and the relu and writes the bf16
+channels_last features, so conv3's fp32 output is neither written nor read back.  Numerics: conv2's output and conv3's weight are
+each rounded to bf16 once and accumulated in fp32 (the head's standing choice), the tail is applied to the fp32 accumulator in the
+fold's order and rounded once to bf16; the features are therefore NOT bit-identical to the stock block's, unlike the fold path.
+The backward computes conv3's data gradient from bf16(scale * weight) and its weight gradient from bf16(out2), with fp32
+accumulation.  Every other case (including a training-mode 'batch' bn3, whose statistics need conv3's output) takes the
+path above with a stock conv3.
 """
 from __future__ import annotations
 
@@ -56,13 +67,15 @@ class _FusedForward:
     """What ``fuse_backbone_tail`` installs as the block's instance ``forward``: a plain picklable object (``torch.save`` of a
     whole fused extractor loads again; ``copy.deepcopy`` re-targets it to the copy).  It keeps the forward that was in the
     instance's __dict__ before (normally none) and the key (norm class, eps, data pointers and version counters of the norm's
-    tensors) under which the fold last passed or failed its probe, and ``train_bn`` (fuse_backbone_tail's flag)."""
-    train_bn = False                    # (objects pickled before the flag existed load with the default)
+    tensors) under which the fold last passed or failed its probe, and ``train_bn`` / ``conv3`` (fuse_backbone_tail's flags)."""
+    train_bn = False                    # (objects pickled before a flag existed load with the default)
+    conv3 = False
 
-    def __init__(self, block, had_forward, old_forward, train_bn=False):
+    def __init__(self, block, had_forward, old_forward, train_bn=False, conv3=False):
         self.block, self.had_forward, self.old_forward = block, had_forward, old_forward
         self.key, self.ok, self.warned = None, False, False
         self.train_bn = bool(train_bn)
+        self.conv3 = bool(conv3)
 
     def __getstate__(self):
         state = dict(self.__dict__)
@@ -183,6 +196,14 @@ def _batch_group(norm, device):
     return (None,)
 
 
+def _conv3_fusable(conv, x):
+    """conv3 can run inside the fused GEMM: exactly nn.Conv2d, 1x1, stride 1, no padding, one group, no bias, an fp32 weight on x's
+    device, input and output channels multiples of 8."""
+    return (type(conv) is nn.Conv2d and conv.kernel_size == (1, 1) and conv.stride == (1, 1) and conv.padding in ((0, 0), "valid")
+            and conv.groups == 1 and conv.bias is None and conv.weight.dtype == torch.float32 and conv.weight.device == x.device
+            and conv.in_channels % 8 == 0 and conv.out_channels % 8 == 0)
+
+
 def _stock_forward(block, state, x):
     if state.had_forward:
         return state.old_forward(x)
@@ -202,9 +223,16 @@ def _fused_forward(block, state, x):
     identity = x
     out = block.relu(block.bn1(block.conv1(x)))
     out = block.relu(block.bn2(block.conv2(out)))
-    c = block.conv3(out)
-    if block.downsample is not None:
-        identity = block.downsample(x)
+    if fold is not None and state.conv3 and out.dtype == torch.float32 and _conv3_fusable(block.conv3, x):
+        if block.downsample is not None:
+            identity = block.downsample(x)
+        if identity.dtype == torch.float32 and tuple(identity.shape) == (out.shape[0], block.conv3.out_channels) + tuple(out.shape[2:]):
+            return ops.seam_conv3_tail(out, identity, block.conv3.weight, fold[0], fold[1])
+        c = block.conv3(out)
+    else:
+        c = block.conv3(out)
+        if block.downsample is not None:
+            identity = block.downsample(x)
     single = batch is not None and batch[0] is None and c.numel() <= c.shape[1]
     if c.dtype != torch.float32 or identity.dtype != torch.float32 or identity.shape != c.shape or single:
         # (autocast and friends; one value per channel, which the stock norm rejects) finish with the stock tail's own operations
@@ -224,10 +252,11 @@ def _installed(block):
     return fwd if isinstance(fwd, _FusedForward) else None
 
 
-def fuse_backbone_tail(feature_extractor: nn.Module, train_bn: bool = False) -> nn.Module:
+def fuse_backbone_tail(feature_extractor: nn.Module, train_bn: bool = False, conv3: bool = False) -> nn.Module:
     """Make the last Bottleneck of ``feature_extractor`` emit bf16 channels_last features (see the module docstring).  Returns
     ``feature_extractor``; a second call only sets ``train_bn`` (a training-mode BatchNorm2d / SyncBatchNorm bn3 takes the
-    batch-statistics kernels).  Raises ValueError when no Bottleneck-shaped module is found.
+    batch-statistics kernels) and ``conv3`` (an eligible conv3 runs inside the fused GEMM, with bf16 operands: see the module
+    docstring for what that changes numerically).  Raises ValueError when no Bottleneck-shaped module is found.
     The hook lives in the block's instance __dict__: ``nn.DataParallel`` replicas (which copy that dict) would run it on the
     original block, so use one process per GPU (DistributedDataParallel), as the reference's trainers do."""
     block = _last_bottleneck(feature_extractor)
@@ -236,9 +265,10 @@ def fuse_backbone_tail(feature_extractor: nn.Module, train_bn: bool = False) -> 
     state = _installed(block)
     if state is None:
         had = "forward" in block.__dict__
-        block.__dict__["forward"] = _FusedForward(block, had, block.__dict__.get("forward"), train_bn)
+        block.__dict__["forward"] = _FusedForward(block, had, block.__dict__.get("forward"), train_bn, conv3)
     else:
         state.train_bn = bool(train_bn)
+        state.conv3 = bool(conv3)
     return feature_extractor
 
 
@@ -260,20 +290,23 @@ def is_fused(feature_extractor: nn.Module) -> bool:
     return block is not None and _installed(block) is not None
 
 
-def wrap_feature_extractor_factory(stock, train_bn: bool = False):
-    """``build_feature_extractor`` with the same signature whose result goes through ``fuse_backbone_tail(fe, train_bn)``
-    (install(seam=True, seam_train_bn=...)).  Wrapping a wrapper returns it with its ``train_bn`` set to the new value."""
+def wrap_feature_extractor_factory(stock, train_bn: bool = False, conv3: bool = False):
+    """``build_feature_extractor`` with the same signature whose result goes through ``fuse_backbone_tail(fe, train_bn, conv3)``
+    (install(seam=True, seam_train_bn=..., seam_conv3=...)).  Wrapping a wrapper returns it with its flags set to the new values."""
     if getattr(stock, "_b200seg_seam", False):
         stock._b200seg_seam_train_bn = bool(train_bn)
+        stock._b200seg_seam_conv3 = bool(conv3)
         return stock
 
     @functools.wraps(stock)
     def build_feature_extractor(*args, **kwargs):
         fe = stock(*args, **kwargs)
         if isinstance(fe, nn.Module) and _last_bottleneck(fe) is not None:       # (a VGG backbone stays as built)
-            fuse_backbone_tail(fe, train_bn=build_feature_extractor._b200seg_seam_train_bn)
+            fuse_backbone_tail(fe, train_bn=build_feature_extractor._b200seg_seam_train_bn,
+                               conv3=build_feature_extractor._b200seg_seam_conv3)
         return fe
 
     build_feature_extractor._b200seg_seam = True
     build_feature_extractor._b200seg_seam_train_bn = bool(train_bn)
+    build_feature_extractor._b200seg_seam_conv3 = bool(conv3)
     return build_feature_extractor
