@@ -460,8 +460,8 @@ B200SEG_API void b200seg_profile_enable(int on);
 B200SEG_API int b200seg_profile_read(int tag, double* total_ms, int* count);
 
 /* on-device self-test of the tcgen05 GEMM core against a CUDA-core reference (synchronous).
- * share: 0 = one CTA per tile, 1 = 2-CTA cluster multicasting the shared B tile, 2 = ... the shared A tile,
- *        3 = 2 x 2 cluster multicasting both, 4 = CTA pair on one tcgen05.mma.cta_group::2 (M = 256). */
+ * share: 0 = one CTA per tile, 1 = 2-CTA cluster multicasting the shared B tile, 2 = ... the shared A tile, 3 = the same as 2
+ *        (it named 2 x 2 clusters, which were removed), 4 = CTA pair on one tcgen05.mma.cta_group::2 (M = 256). */
 B200SEG_API int b200seg_gemm_selftest(int M, int N, int K, int a_mn_major, int b_mn_major, int splits, int col_hw, int share,
                           double* max_err, double* max_ref);
 /* head forward GEMM: 1 (default) = the tile width (256 / 224 / 192 accumulator columns) is chosen per problem so that the tile
@@ -485,8 +485,10 @@ B200SEG_API int b200seg_gemm_fwd_convert_selftest(int M, int n_img, int hw, int 
 /* K6 conv kernel: 1 (default) = CTA pairs driving one tcgen05.mma.cta_group::2 (M = 256) wherever a layer has two M-tiles,
  * 0 = one CTA per tile (A/B experiments) */
 B200SEG_API void b200seg_conv_set_pair(int on);
-/* operand sharing inside the ASPP head GEMMs: 0 none, 1 (default) 2-CTA multicast pairs, 2 2 x 2 clusters sharing both
- * operands, 3 = 1, plus cta_group::2 pairs (one 2-SM MMA) for the GEMMs whose pairs lie along M (the data gradient) */
+/* operand sharing inside the ASPP head GEMMs: 0 none, 1 (default) the pairs each GEMM asks for (cta_group::2 pairs, 2-CTA
+ * multicast pairs for the fp32 NCHW data gradient), 2 = 1, 3 = 1 plus cta_group::2 pairs (one 2-SM MMA) for the GEMMs whose
+ * multicast pairs lie along M (the data gradient), 4 = every shared GEMM as cta_group::2 pairs, 5 = the head GEMMs
+ * without cta_group::2 (2-CTA multicast pairs instead) */
 B200SEG_API void b200seg_gemm_set_sharing(int on);
 /* SMs the data-gradient GEMM leaves free when b200seg_aspp_backward_packed_ex is given a weights_ready_event, so that the
  * caller's all-reduce kernel can be resident underneath it (the persistent GEMM otherwise fills every SM's shared memory);

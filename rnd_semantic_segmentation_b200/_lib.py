@@ -1513,7 +1513,8 @@ def conv_set_pair(on):
 
 
 def gemm_set_sharing(mode):
-    """0 / False: no multicast; 1 / True: 2-CTA pairs (default); 2: 2 x 2 clusters multicasting both operands (slower: kept for A/B)."""
+    """0 / False: one CTA per tile; 1 / True: the 2-CTA pairs each GEMM asks for (default); 2: the same as 1; 3: 1 with the
+    multicast pairs along M as cta_group::2 pairs; 4: every pair as cta_group::2; 5: the head GEMMs without cta_group::2 (multicast pairs)."""
     load().b200seg_gemm_set_sharing(int(mode))
 
 

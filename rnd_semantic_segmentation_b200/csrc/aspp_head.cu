@@ -464,10 +464,18 @@ int aspp_forward(const void* Xp, const void* Wp, const float* bias_sum, const in
     // MMA width 128 (half the cycles) instead of leaving half a CTA pair idle as the channel-major form does with its 5 M-tiles
     // on 3 pairs; the accumulator goes to Yt straight from registers (a lane is a pixel: 32 consecutive pixels of one row j per
     // store instruction)
-    rc = gemm::launch(b, a, (int)P, NJ, Cin, 1, Yt, 0, 0, 0, 0, stream, nullptr, 0, gemm::SHARE_PAIR, false, 0, gemm::SHARE_B,
-                      (int)ypitch);
+    // (one plane of ypitch pixels: Yt[j][p] = D[p, j])
+    gemm::Gemm g{b, a, (int)P, NJ, Cin, gemm::out_f32_nchw_rows(Yt, (int)ypitch, 0)};
+    g.share = gemm::SHARE_PAIR;
+    g.pair_fallback = gemm::SHARE_B;
+    g.prof_tag = 0;
+    rc = gemm::launch(g, stream);
   } else {
-    rc = gemm::launch(a, b, NJ, (int)P, Cin, 1, Yt, ypitch, 0, 0, 0, stream, nullptr, 0, gemm::SHARE_PAIR, false, 0, gemm::SHARE_A);
+    gemm::Gemm g{a, b, NJ, (int)P, Cin, gemm::out_f32(Yt, ypitch)};
+    g.share = gemm::SHARE_PAIR;
+    g.pair_fallback = gemm::SHARE_A;
+    g.prof_tag = 0;
+    rc = gemm::launch(g, stream);
   }
   if (rc) return rc;
   TapTable tt;
@@ -587,9 +595,13 @@ int aspp_backward_packed(const void* gOt_in, const void* Xp, const void* WpT, co
       gemm::Operand b{(const __nv_bfloat16*)Xp, true, Cin};
       int used = 1;
       const long long slab = (long long)NJ * Cin;
-      int rc = gemm::launch(a, b, NJ, Cin, (int)P, splits, wpart, Cin, 0, 0, slab, stream, &used, 2, gemm::SHARE_PAIR, false, 0,
-                            gemm::SHARE_A);                       // cta_group::2 pairs: 138 vs 165 us
-      if (rc) return rc;
+      gemm::Gemm g{a, b, NJ, Cin, (int)P, gemm::out_f32(wpart, Cin, slab)};
+      g.splits = splits;
+      g.splits_used = &used;
+      g.share = gemm::SHARE_PAIR;                                 // cta_group::2 pairs: 138 vs 165 us
+      g.pair_fallback = gemm::SHARE_A;
+      g.prof_tag = 2;
+      if (int rc = gemm::launch(g, stream)) return rc;
       dim3 grid(ceil_div(Cin, 256), C, R);
       profile_begin(10, stream);
       if (!wgrad_reduce_vec_launch(wpart, used, slab, R, C, Cin, gw, stream))
@@ -613,18 +625,22 @@ int aspp_backward_packed(const void* gOt_in, const void* Xp, const void* WpT, co
     // dX[ci, p] = WpT[ci, :] . G't[:, p]   -> fp32 NCHW: column p = (image, pixel), row = channel
     gemm::Operand a{(const __nv_bfloat16*)WpT, false, NJ};
     gemm::Operand b{Gp, true, Ppitch};
-    int rc = gemm::launch(a, b, Cin, (int)P, NJ, 1, grad_x, hw, hw, (long long)Cin * hw, 0, stream, nullptr, 1, gemm::SHARE_B, false,
-                          weights_ready ? gemm::overlap_sms() : 0);
-    if (rc) return rc;
+    gemm::Gemm g{a, b, Cin, (int)P, NJ, gemm::out_f32_nchw_cols(grad_x, hw, hw, (long long)Cin * hw)};
+    g.share = gemm::SHARE_B;
+    g.sm_reserve = weights_ready ? gemm::overlap_sms() : 0;
+    g.prof_tag = 1;
+    if (int rc = gemm::launch(g, stream)) return rc;
   } else if (grad_x) {
     // dXt[p, ci] = G't[:, p] . WpT[ci, :] with the PIXELS along M, written as fp32 NCHW straight from the accumulator registers:
     // a TMEM lane is a pixel, so one store instruction covers 32 consecutive pixels of a channel plane (no smem transpose)
     gemm::Operand a{Gp, true, Ppitch};
     gemm::Operand b{(const __nv_bfloat16*)WpT, false, NJ};
-    int rc = gemm::launch(a, b, (int)P, Cin, NJ, 1, grad_x, 0, 0, (long long)Cin * hw, 0, stream, nullptr, 1,
-                          gemm::SHARE_PAIR, false, weights_ready ? gemm::overlap_sms() : 0,
-                          gemm::SHARE_B, hw);
-    if (rc) return rc;
+    gemm::Gemm g{a, b, (int)P, Cin, NJ, gemm::out_f32_nchw_rows(grad_x, hw, (long long)Cin * hw)};
+    g.share = gemm::SHARE_PAIR;
+    g.pair_fallback = gemm::SHARE_B;
+    g.sm_reserve = weights_ready ? gemm::overlap_sms() : 0;
+    g.prof_tag = 1;
+    if (int rc = gemm::launch(g, stream)) return rc;
   }
   if (grad_x_nhwc_bf16) {
     // seam format: dXt[p, ci] = G't[:, p] . WpT[ci, :]  written as bf16 pixel-major [P][Cin] (= channels_last NHWC),
@@ -633,9 +649,11 @@ int aspp_backward_packed(const void* gOt_in, const void* Xp, const void* WpT, co
     gemm::Operand b{(const __nv_bfloat16*)WpT, false, NJ};
     // CTA pairs on one tcgen05.mma.cta_group::2 (M = 256 pixels): 164 vs 170 us with the multicast pairs.  (The fp32 NCHW
     // dgrad above is bound by its 537 MB store, where the 2-SM MMA measured 5 us SLOWER, so it keeps the multicast pairs.)
-    int rc = gemm::launch(a, b, (int)P, Cin, NJ, 1, reinterpret_cast<float*>(grad_x_nhwc_bf16), Cin, 0, 0, 0, stream, nullptr, 1,
-                          gemm::SHARE_PAIR, true, weights_ready ? gemm::overlap_sms() : 0);
-    if (rc) return rc;
+    gemm::Gemm g{a, b, (int)P, Cin, NJ, gemm::out_bf16(reinterpret_cast<__nv_bfloat16*>(grad_x_nhwc_bf16), Cin)};
+    g.share = gemm::SHARE_PAIR;
+    g.sm_reserve = weights_ready ? gemm::overlap_sms() : 0;
+    g.prof_tag = 1;
+    if (int rc = gemm::launch(g, stream)) return rc;
   }
   return B200SEG_OK;
 }

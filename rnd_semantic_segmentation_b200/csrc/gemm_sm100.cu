@@ -44,45 +44,16 @@ static int make_tmap(CUtensorMap* m, const __nv_bfloat16* ptr, long long inner, 
   return B200SEG_OK;
 }
 
-static int sms_total() { return num_sms(); }
 static int g_overlap_sms = 8;         // b200seg_gemm_set_overlap_sms(): SMs left free while an all-reduce overlaps the dgrad GEMM
 void set_overlap_sms(int n) { g_overlap_sms = n < 0 ? 0 : n; }
 int overlap_sms() { return g_overlap_sms; }
 // b200seg_gemm_set_sharing(): 0 one CTA per tile; 1 (default) what each caller asks for -- cta_group::2 pairs for the forward,
-// weight-gradient and seam-format data-gradient GEMMs, 2-CTA multicast pairs for the fp32 NCHW data gradient; 2 2 x 2 clusters
-// (measured ~1.9x slower: 37 four-CTA clusters do not all fit the GPCs); 3 = 1 with the fp32 data gradient as cta_group::2
-// pairs too (measured 5 us slower: it is store-bound); 4 = every shared GEMM as cta_group::2 pairs; 5 = no cta_group::2 (the
-// multicast pairs of the earlier rounds)
+// weight-gradient and seam-format data-gradient GEMMs, 2-CTA multicast pairs for the fp32 NCHW data gradient; 2 = 1 (it named
+// 2 x 2 clusters, which measured ~1.9x slower: 37 four-CTA clusters do not all fit the GPCs); 3 = 1 with the fp32 data gradient
+// as cta_group::2 pairs too (measured 5 us slower: it is store-bound); 4 = every shared GEMM as cta_group::2 pairs; 5 = no
+// cta_group::2 (each caller's pair_fallback: the multicast pairs of the earlier rounds)
 static int g_share_enabled = 1;
 void set_sharing(int on) { g_share_enabled = on; }
-
-template <bool A_MN, bool B_MN, int SHARE, int BN = 256, bool RS = false, bool SEAM = false>
-static int launch_t(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& to, const Params& p, int grid, cudaStream_t stream) {
-  static bool configured = false;
-  if (!configured) {
-    B200SEG_CUDA(cudaFuncSetAttribute(gemm_bf16_kernel<A_MN, B_MN, SHARE, BN, RS, SEAM>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
-    configured = true;
-  }
-  if (SHARE == SHARE_NONE) {
-    gemm_bf16_kernel<A_MN, B_MN, SHARE, BN, RS, SEAM><<<grid, NUM_THREADS, SMEM_BYTES, stream>>>(ta, tb, to, p);
-  } else {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(grid);
-    cfg.blockDim = dim3(NUM_THREADS);
-    cfg.dynamicSmemBytes = SMEM_BYTES;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = SHARE == SHARE_AB ? 4 : 2;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    B200SEG_CUDA(cudaLaunchKernelEx(&cfg, gemm_bf16_kernel<A_MN, B_MN, SHARE, BN, RS, SEAM>, ta, tb, to, p));
-  }
-  B200SEG_LAUNCH_CHECK();
-  return B200SEG_OK;
-}
 
 static int g_dgrad_mode = 1;         // b200seg_gemm_set_dgrad_mode(): see gemm_sm100.cuh
 void set_dgrad_mode(int mode) { g_dgrad_mode = mode; }
@@ -93,79 +64,109 @@ int fwd_mode() { return g_fwd_mode; }
 static int g_narrow_tiles = 1;        // b200seg_gemm_set_narrow_tiles(): 0 = always 256-column tiles
 void set_narrow_tiles(int on) { g_narrow_tiles = on; }
 
-// K-major x K-major, fp32 out, unshared B: tile width chosen by the caller (wave quantisation)
-static int launch_kk(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& to, const Params& p, int grid, int share, int bn,
-                     cudaStream_t stream) {
-  if (share == SHARE_A) {
-    if (bn == 224) return launch_t<false, false, SHARE_A, 224>(ta, tb, to, p, grid, stream);
-    if (bn == 192) return launch_t<false, false, SHARE_A, 192>(ta, tb, to, p, grid, stream);
-    return launch_t<false, false, SHARE_A, 256>(ta, tb, to, p, grid, stream);
+// Every instantiation of gemm_bf16_kernel that launch() can run
+typedef void (*KernelFn)(CUtensorMap, CUtensorMap, CUtensorMap, Params);
+struct Variant {
+  bool a_mn, b_mn;
+  int share, bn;
+  bool rs, seam;
+  KernelFn fn;
+  bool configured;
+};
+template <bool A_MN, bool B_MN, int SHARE, int BN = 256, bool RS = false, bool SEAM = false>
+static Variant variant() { return {A_MN, B_MN, SHARE, BN, RS, SEAM, gemm_bf16_kernel<A_MN, B_MN, SHARE, BN, RS, SEAM>, false}; }
+static Variant g_variants[] = {
+    // any operand layout, any sharing geometry, 256-column tiles
+    variant<false, false, SHARE_NONE>(), variant<false, false, SHARE_B>(), variant<false, false, SHARE_A>(), variant<false, false, SHARE_PAIR>(),
+    variant<true, true, SHARE_NONE>(), variant<true, true, SHARE_B>(), variant<true, true, SHARE_A>(), variant<true, true, SHARE_PAIR>(),
+    variant<true, false, SHARE_NONE>(), variant<true, false, SHARE_B>(), variant<true, false, SHARE_A>(), variant<true, false, SHARE_PAIR>(),
+    variant<false, true, SHARE_NONE>(), variant<false, true, SHARE_B>(), variant<false, true, SHARE_A>(), variant<false, true, SHARE_PAIR>(),
+    // narrow tiles: K-major operands, unshared B
+    variant<false, false, SHARE_NONE, 224>(), variant<false, false, SHARE_NONE, 192>(),
+    variant<false, false, SHARE_A, 224>(), variant<false, false, SHARE_A, 192>(),
+    // fp32 NCHW rows-as-pixels stored from registers, seven ring stages: cta_group::2 pairs, B K-major
+    variant<false, false, SHARE_PAIR, 256, true>(), variant<true, false, SHARE_PAIR, 256, true>(),
+    // seam epilogue: K-major operands
+    variant<false, false, SHARE_NONE, 256, false, true>(), variant<false, false, SHARE_PAIR, 256, false, true>(),
+};
+
+static int check(const Gemm& g) {
+  const Out& o = g.out;
+  const bool aligned = (reinterpret_cast<uintptr_t>(o.ptr) & 15) == 0;
+  if (o.layout == Out::SEAM) {
+    B200SEG_CHECK_ARG(g.M > 0 && g.N > 0 && g.K > 0 && o.hw > 0 && (g.M % o.hw == 0 || g.M <= o.hw) && g.splits <= 1,
+                      "gemm seam: bad problem %dx%dx%d (hw %d)", g.M, g.N, g.K, o.hw);
+    B200SEG_CHECK_ARG(!g.a.mn_major && !g.b.mn_major, "gemm seam: K-major operands only");
+    B200SEG_CHECK_ARG(o.identity && o.scale && o.bias && g.N % 8 == 0 && aligned,
+                      "gemm seam: N = %d must be a multiple of 8 and D 16-byte aligned", g.N);
+    return B200SEG_OK;
   }
-  if (bn == 224) return launch_t<false, false, SHARE_NONE, 224>(ta, tb, to, p, grid, stream);
-  if (bn == 192) return launch_t<false, false, SHARE_NONE, 192>(ta, tb, to, p, grid, stream);
-  return launch_t<false, false, SHARE_NONE, 256>(ta, tb, to, p, grid, stream);
-}
-
-template <bool A_MN, bool B_MN>
-static int launch_s(const CUtensorMap& ta, const CUtensorMap& tb, const CUtensorMap& to, const Params& p, int grid, int share,
-                    cudaStream_t stream) {
-  if (share == SHARE_PAIR) return launch_t<A_MN, B_MN, SHARE_PAIR>(ta, tb, to, p, grid, stream);
-  if (share == SHARE_B) return launch_t<A_MN, B_MN, SHARE_B>(ta, tb, to, p, grid, stream);
-  if (share == SHARE_A) return launch_t<A_MN, B_MN, SHARE_A>(ta, tb, to, p, grid, stream);
-  return launch_t<A_MN, B_MN, SHARE_NONE>(ta, tb, to, p, grid, stream);
-}
-
-int launch(const Operand& a, const Operand& b, int M, int N, int K, int splits, float* out, long long row_stride,
-           int col_hw, long long img_stride, long long split_stride, cudaStream_t stream, int* splits_used, int prof_tag,
-           int share, bool out_bf16, int sm_reserve, int pair_fallback, int row_hw) {
-  B200SEG_CHECK_ARG(M > 0 && N > 0 && K > 0, "gemm: empty problem %dx%dx%d", M, N, K);
-  B200SEG_CHECK_ARG(row_hw <= 0 || (!out_bf16 && col_hw <= 0 && splits <= 1 && (M % row_hw == 0 || M <= row_hw)),
+  B200SEG_CHECK_ARG(g.M > 0 && g.N > 0 && g.K > 0, "gemm: empty problem %dx%dx%d", g.M, g.N, g.K);
+  B200SEG_CHECK_ARG(o.layout != Out::F32_NCHW_COLS || o.hw > 0, "gemm: the NCHW column map needs hw > 0");
+  B200SEG_CHECK_ARG(o.layout != Out::F32_NCHW_ROWS || (o.hw > 0 && g.splits <= 1 && (g.M % o.hw == 0 || g.M <= o.hw)),
                     "gemm: the pixel-major epilogue needs fp32 output, no split-K and whole images (or one plane) along M");
-  B200SEG_CHECK_ARG(!out_bf16 || (col_hw <= 0 && N % 8 == 0 && row_stride % 8 == 0 && split_stride % 8 == 0 &&
-                                  (reinterpret_cast<uintptr_t>(out) & 15) == 0),
+  B200SEG_CHECK_ARG(o.layout != Out::BF16 || (g.N % 8 == 0 && o.row_stride % 8 == 0 && o.split_stride % 8 == 0 && aligned),
                     "gemm: bf16 output needs plain row-major D with N, row pitch multiples of 8 and a 16-byte aligned base");
+  return B200SEG_OK;
+}
+
+int launch(const Gemm& g, cudaStream_t stream) {
+  if (int rc = check(g)) return rc;
+  const Operand &a = g.a, &b = g.b;
+  const Out& o = g.out;
+  const int M = g.M, N = g.N, K = g.K;
+  const bool seam = o.layout == Out::SEAM;
   // callers name the sharing geometry they want; the global mode (A/B experiments) can veto or override it
+  int share = g.share;
   if (!g_share_enabled) share = SHARE_NONE;
-  if (share == SHARE_AB) share = SHARE_A;                                    // (the 2 x 2-cluster mode measured ~1.9x slower and was removed)
   if (g_share_enabled == 3 && share == SHARE_B) share = SHARE_PAIR;         // also the store-bound fp32 dgrad as 2-SM pairs
   if (g_share_enabled == 4 && (share == SHARE_A || share == SHARE_B)) share = SHARE_PAIR;
-  if (g_share_enabled == 5 && share == SHARE_PAIR) share = pair_fallback;   // no cta_group::2: the multicast pairs used before
-  Params p;
+  if (g_share_enabled == 5 && share == SHARE_PAIR) share = g.pair_fallback;
+  Params p = {};
   p.M = M; p.N = N; p.K = K;
   p.m_tiles = ceil_div(M, BLOCK_M);
   p.n_tiles = ceil_div(N, BLOCK_N);
   p.kb_total = ceil_div(K, BLOCK_K);
-  if (splits < 1) splits = 1;
-  if (splits > p.kb_total) splits = p.kb_total;
+  const int splits = g.splits < 1 ? 1 : (g.splits > p.kb_total ? p.kb_total : g.splits);
   p.kb_per_split = ceil_div(p.kb_total, splits);
   p.splits = ceil_div(p.kb_total, p.kb_per_split);     // every split non-empty
-  p.out = out;
-  p.row_stride = row_stride;
-  p.col_hw = col_hw > 0 ? col_hw : INT_MAX;
-  p.img_stride = img_stride;
-  p.split_stride = split_stride;
-  p.out_bf16 = out_bf16 ? 1 : 0;
-  p.row_hw_px = row_hw > 0 ? row_hw : 0;
-  p.row_hw = row_hw > 0 ? (g_dgrad_mode == 2 ? 2 : 1) : 0;
-  // optional pacing of the register-store epilogue (B200SEG_EPI_SLEEP=<ns> after each 16-column chunk's stores, default off): with a
-  // six-stage ring, spreading a tile's 128 KB of stores over the tile time took the data gradient from 161 to 150 us (the
-  // store bursts delay the operand requests queued behind them); with the seventh stage it no longer changes anything (154-156 us
-  // with 0 or 192 ns), so it stays an experiment knob
-  {
-    static int env_ns = -2;
-    if (env_ns == -2) { const char* e = getenv("B200SEG_EPI_SLEEP"); env_ns = e ? atoi(e) : 0; }
-    p.epi_sleep_ns = row_hw > 0 && env_ns > 0 ? env_ns : 0;
-  }
+  if (g.splits_used) *g.splits_used = p.splits;
+  p.out = reinterpret_cast<float*>(o.ptr);
+  p.row_stride = o.row_stride;
+  p.col_hw = o.layout == Out::F32_NCHW_COLS ? o.hw : INT_MAX;
+  p.img_stride = o.img_stride;
+  p.split_stride = o.split_stride;
+  p.out_bf16 = o.layout == Out::BF16 || seam ? 1 : 0;
   // tile order: the units running together should share the LARGER operand, so that it streams from HBM once and the small
   // one lives in L2.  Channel-major problems (M = channels / packed weight rows <= N = pixels) walk along M; pixel-major ones
   // (M = pixels: the seam-format and the register-store data gradients) walk along N -- M-fastest made them re-read the
   // 86 MB pixel operand once per N-tile (653 MB of DRAM reads per launch at the bench shape, ncu profiles/r2_dgrad_*).
   p.n_fastest = M > N ? 1 : 0;
-  if (splits_used) *splits_used = p.splits;
-  p.vec_ok = ((reinterpret_cast<uintptr_t>(out) & 15) == 0 && row_stride % 4 == 0 && split_stride % 4 == 0 &&
-              (col_hw <= 0 || (col_hw % 4 == 0 && img_stride % 4 == 0)))
-                 ? 1
-                 : 0;
+  p.vec_ok = (reinterpret_cast<uintptr_t>(o.ptr) & 15) == 0 && o.row_stride % 4 == 0 && o.split_stride % 4 == 0 &&
+             (p.col_hw == INT_MAX || (p.col_hw % 4 == 0 && o.img_stride % 4 == 0));
+  if (o.layout == Out::F32_NCHW_ROWS) {
+    // every rows-as-pixels launch (the head's pixel-major forward and data gradient, conv3's data gradient) takes
+    // b200seg_gemm_set_dgrad_mode(2)'s streaming stores and the B200SEG_EPI_SLEEP pacing (<ns> after each 16-column chunk's stores,
+    // default off): with a six-stage ring, spreading a tile's 128 KB of stores over the tile time took the data gradient from 161
+    // to 150 us (the store bursts delay the operand requests queued behind them); with the seventh stage it no longer changes
+    // anything (154-156 us with 0 or 192 ns), so it stays an experiment knob
+    static int env_ns = -2;
+    if (env_ns == -2) { const char* e = getenv("B200SEG_EPI_SLEEP"); env_ns = e ? atoi(e) : 0; }
+    p.row_hw_px = o.hw;
+    p.row_hw = g_dgrad_mode == 2 ? 2 : 1;
+    p.epi_sleep_ns = env_ns > 0 ? env_ns : 0;
+  } else if (seam) {
+    // the fused conv3 + tail of the backbone's last Bottleneck: pairs along M walking along N, so a pair's two pixel tiles are read
+    // once for all N-tiles while the small weight operand stays in L2
+    p.row_stride = N;
+    p.img_stride = (long long)N * o.hw;
+    p.row_hw_px = o.hw;
+    p.n_fastest = 1;
+    p.vec_ok = 0;
+    p.seam_identity = o.identity;
+    p.seam_scale = o.scale;
+    p.seam_bias = o.bias;
+  }
   // a pair needs two tiles along the paired dimension to be worth it
   if (share == SHARE_B && p.m_tiles < 2) share = SHARE_NONE;
   if (share == SHARE_PAIR && p.m_tiles < 2) share = SHARE_NONE;
@@ -174,8 +175,8 @@ int launch(const Operand& a, const Operand& b, int M, int N, int K, int splits, 
   // tile width: with K-major operands, fp32 output and an unshared B tile, a narrower tile that makes the tile count a
   // near-multiple of the worker count beats 256 columns (rounds x columns is the cost)
   int bn = BLOCK_N;
-  if (g_narrow_tiles && !a.mn_major && !b.mn_major && !out_bf16 && (share == SHARE_NONE || share == SHARE_A)) {
-    const int workers = share == SHARE_A ? sms_total() / 2 : sms_total();
+  if (g_narrow_tiles && !a.mn_major && !b.mn_major && !p.out_bf16 && (share == SHARE_NONE || share == SHARE_A)) {
+    const int workers = share == SHARE_A ? num_sms() / 2 : num_sms();
     long long best = -1;
     for (int cand : {256, 224, 192}) {
       const int nt = ceil_div(N, cand);
@@ -186,90 +187,59 @@ int launch(const Operand& a, const Operand& b, int M, int N, int K, int splits, 
     }
     p.n_tiles = ceil_div(N, bn);
   }
+  const bool rs = p.row_hw == 1 && share == SHARE_PAIR && !b.mn_major;        // register-store variant (7 ring stages)
+  Variant* v = nullptr;
+  for (Variant& c : g_variants)
+    if (c.a_mn == a.mn_major && c.b_mn == b.mn_major && c.share == share && c.bn == bn && c.rs == rs && c.seam == seam) { v = &c; break; }
+  B200SEG_CHECK_ARG(v, "gemm: no kernel for operands %d/%d, sharing %d, %d-column tiles, output layout %d", (int)a.mn_major,
+                    (int)b.mn_major, share, bn, (int)o.layout);
 
   // the shared operand is loaded in halves (one per CTA of the pair): halve its K-major box
   CUtensorMap ta, tb;
   int rc;
-  if (!a.mn_major) rc = make_tmap(&ta, a.ptr, K, M, a.pitch, BLOCK_K, (share == SHARE_A || share == SHARE_AB) ? BLOCK_M / 2 : BLOCK_M);
+  if (!a.mn_major) rc = make_tmap(&ta, a.ptr, K, M, a.pitch, BLOCK_K, share == SHARE_A ? BLOCK_M / 2 : BLOCK_M);
   else rc = make_tmap(&ta, a.ptr, M, K, a.pitch, 64, BLOCK_K);
   if (rc) return rc;
-  if (!b.mn_major) rc = make_tmap(&tb, b.ptr, K, N, b.pitch, BLOCK_K, (share == SHARE_B || share == SHARE_AB || share == SHARE_PAIR) ? BLOCK_N / 2 : bn);
+  if (!b.mn_major) rc = make_tmap(&tb, b.ptr, K, N, b.pitch, BLOCK_K, (share == SHARE_B || share == SHARE_PAIR) ? BLOCK_N / 2 : bn);
   else rc = make_tmap(&tb, b.ptr, N, K, b.pitch, 64, BLOCK_K);
   if (rc) return rc;
-
   CUtensorMap to = ta;            // third tensor-map slot: the 64-row B boxes of the register-store variant (below)
-
-  // persistent CTAs, one per SM, minus the SMs the caller wants left free for a concurrent kernel (the NCCL all-reduce
-  // of the weight gradients running underneath the data-gradient GEMM)
-  int sms = num_sms() - (sm_reserve > 0 ? sm_reserve : 0);
-  if (sms < 2) sms = 2;
-  int grid;
-  if (share == SHARE_NONE) {
-    const int units = p.m_tiles * p.n_tiles * p.splits;
-    grid = units < sms ? units : sms;
-  } else {
-    const int cs = share == SHARE_AB ? 4 : 2;
-    const int mt = (share == SHARE_B || share == SHARE_AB || share == SHARE_PAIR) ? (p.m_tiles + 1) / 2 : p.m_tiles;
-    const int nt = (share == SHARE_A || share == SHARE_AB) ? (p.n_tiles + 1) / 2 : p.n_tiles;
-    const int units = mt * nt * p.splits;
-    const int clusters = units < sms / cs ? units : sms / cs;
-    grid = cs * clusters;
-  }
-  const bool rs = p.row_hw == 1 && share == SHARE_PAIR && !b.mn_major;        // register-store variant (7 ring stages)
   if (rs) {
     rc = make_tmap(&to, b.ptr, K, N, b.pitch, BLOCK_K, BLOCK_N / 4);          // 64-row B boxes for a ragged last N-tile
     if (rc) return rc;
   }
-  profile_begin(prof_tag, stream);
-  if (rs && a.mn_major) rc = launch_t<true, false, SHARE_PAIR, 256, true>(ta, tb, to, p, grid, stream);
-  else if (rs) rc = launch_t<false, false, SHARE_PAIR, 256, true>(ta, tb, to, p, grid, stream);
-  else if (!a.mn_major && !b.mn_major && bn != BLOCK_N) rc = launch_kk(ta, tb, to, p, grid, share, bn, stream);
-  else if (!a.mn_major && !b.mn_major) rc = launch_s<false, false>(ta, tb, to, p, grid, share, stream);
-  else if (a.mn_major && b.mn_major) rc = launch_s<true, true>(ta, tb, to, p, grid, share, stream);
-  else if (a.mn_major && !b.mn_major) rc = launch_s<true, false>(ta, tb, to, p, grid, share, stream);
-  else rc = launch_s<false, true>(ta, tb, to, p, grid, share, stream);
-  profile_end(prof_tag, stream);
-  return rc;
-}
 
-// Pixel-major forward with the seam epilogue (the fused conv3 + tail of the backbone's last Bottleneck): cta_group::2 pairs along
-// M walking along N, so a pair's two pixel tiles are read once for all N-tiles while the small weight operand stays in L2.
-int launch_seam(const Operand& a, const Operand& b, int M, int N, int K, __nv_bfloat16* out, const float* identity, const float* scale,
-                const float* bias, int hw, cudaStream_t stream, int prof_tag) {
-  B200SEG_CHECK_ARG(M > 0 && N > 0 && K > 0 && hw > 0 && (M % hw == 0 || M <= hw), "gemm seam: bad problem %dx%dx%d (hw %d)", M, N, K, hw);
-  B200SEG_CHECK_ARG(!a.mn_major && !b.mn_major, "gemm seam: K-major operands only");
-  B200SEG_CHECK_ARG(identity && scale && bias && N % 8 == 0 && (reinterpret_cast<uintptr_t>(out) & 15) == 0,
-                    "gemm seam: N = %d must be a multiple of 8 and D 16-byte aligned", N);
-  Params p = {};
-  p.M = M; p.N = N; p.K = K;
-  p.m_tiles = ceil_div(M, BLOCK_M);
-  p.n_tiles = ceil_div(N, BLOCK_N);
-  p.kb_total = ceil_div(K, BLOCK_K);
-  p.splits = 1;
-  p.kb_per_split = p.kb_total;
-  p.out = reinterpret_cast<float*>(out);
-  p.row_stride = N;
-  p.col_hw = INT_MAX;
-  p.img_stride = (long long)N * hw;
-  p.out_bf16 = 1;
-  p.n_fastest = 1;
-  p.row_hw_px = hw;
-  p.seam_identity = identity;
-  p.seam_scale = scale;
-  p.seam_bias = bias;
-  const bool pair = g_share_enabled != 0 && p.m_tiles >= 2;
-  CUtensorMap ta, tb;
-  int rc = make_tmap(&ta, a.ptr, K, M, a.pitch, BLOCK_K, BLOCK_M);
-  if (rc) return rc;
-  rc = make_tmap(&tb, b.ptr, K, N, b.pitch, BLOCK_K, pair ? BLOCK_N / 2 : BLOCK_N);
-  if (rc) return rc;
-  const int sms = num_sms();
-  const int units = (pair ? (p.m_tiles + 1) / 2 : p.m_tiles) * p.n_tiles;
-  profile_begin(prof_tag, stream);
-  if (pair) rc = launch_t<false, false, SHARE_PAIR, 256, false, true>(ta, tb, ta, p, 2 * (units < sms / 2 ? units : sms / 2), stream);
-  else rc = launch_t<false, false, SHARE_NONE, 256, false, true>(ta, tb, ta, p, units < sms ? units : sms, stream);
-  profile_end(prof_tag, stream);
-  return rc;
+  // persistent CTAs, one per SM, minus the SMs the caller wants left free for a concurrent kernel (the NCCL all-reduce
+  // of the weight gradients running underneath the data-gradient GEMM)
+  int sms = num_sms() - (g.sm_reserve > 0 ? g.sm_reserve : 0);
+  if (sms < 2) sms = 2;
+  const int cs = share == SHARE_NONE ? 1 : 2;                                 // CTAs per cluster
+  const int mt = (share == SHARE_B || share == SHARE_PAIR) ? (p.m_tiles + 1) / 2 : p.m_tiles;
+  const int nt = share == SHARE_A ? (p.n_tiles + 1) / 2 : p.n_tiles;
+  const int units = mt * nt * p.splits;
+  const int grid = cs * (units < sms / cs ? units : sms / cs);
+
+  if (!v->configured) {
+    B200SEG_CUDA(cudaFuncSetAttribute(v->fn, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+    v->configured = true;
+  }
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(grid);
+  cfg.blockDim = dim3(NUM_THREADS);
+  cfg.dynamicSmemBytes = SMEM_BYTES;
+  cfg.stream = stream;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeClusterDimension;
+  attr[0].val.clusterDim.x = cs;
+  attr[0].val.clusterDim.y = 1;
+  attr[0].val.clusterDim.z = 1;
+  cfg.attrs = attr;
+  cfg.numAttrs = share == SHARE_NONE ? 0 : 1;
+  profile_begin(g.prof_tag, stream);
+  B200SEG_CUDA(cudaLaunchKernelEx(&cfg, v->fn, ta, tb, to, p));
+  B200SEG_LAUNCH_CHECK();
+  profile_end(g.prof_tag, stream);
+  return B200SEG_OK;
 }
 
 // ------------------------------------------------------------------------------------------
@@ -347,8 +317,6 @@ int launch_fwd_convert(const __nv_bfloat16* a, long long a_pitch, const float* x
   }
 }
 
-int fwd_convert_max_clusters(int mp) { (void)mp; return 0; }
-
 // ------------------------------------------------------------------------------------------
 // Self-test helpers
 // ------------------------------------------------------------------------------------------
@@ -421,7 +389,12 @@ int selftest(int M, int N, int K, int a_mn, int b_mn, int splits, int col_hw, in
   B200SEG_LAUNCH_CHECK();
   Operand oa{A, a_mn != 0, a_pitch}, ob{B, b_mn != 0, b_pitch};
   int used = 1;
-  int rc = launch(oa, ob, M, N, K, s, D, row_stride, col_hw, img_stride, out_elems, 0, &used, -1, share);
+  Gemm gm{oa, ob, M, N, K,
+          col_hw > 0 ? out_f32_nchw_cols(D, col_hw, row_stride, img_stride, out_elems) : out_f32(D, row_stride, out_elems)};
+  gm.splits = s;
+  gm.splits_used = &used;
+  gm.share = share == 3 ? SHARE_A : share;      // 3 named the 2 x 2-cluster geometry, which was removed: it runs as SHARE_A
+  int rc = launch(gm, 0);
   if (rc == B200SEG_OK) {
     compare_kernel<<<g, 128>>>(D, ref, M, N, used, out_elems, row_stride, col_hw > 0 ? col_hw : INT_MAX, img_stride, res);
     cudaError_t e = cudaDeviceSynchronize();

@@ -172,15 +172,11 @@ __host__ __device__ constexpr uint32_t make_idesc(bool a_mn, bool b_mn, int m, i
 //   SHARE_A    : the two CTAs own N-tiles (2i, 2i+1) of the SAME M-tile; each loads its own B tile and half of A (40 KB).
 // Each CTA still issues its own cta_group::1 MMAs into its own TMEM.  A shared-memory stage is released to BOTH
 // producers only when BOTH CTAs' MMAs have drained it (empty barriers count 2, tcgen05.commit multicast to both CTAs).
-//   SHARE_AB   : 2 x 2 cluster (rank = rm + 2 * rn): CTA (rm, rn) owns M-tile 2i+rm and N-tile 2j+rn, loads half rn of its A
-//                tile (multicast to the CTA with the same rm) and half rm of its B tile (multicast to the CTA with the same
-//                rn): 24 KB per k-block per SM.  The kernel is bound by the L2 -> SM rate (~6.3 KB/clk chip-wide: at 32-40 KB
-//                per k-block the loads of a k-block take longer than its four MMAs), so this is what buys tensor-pipe time.
 //   SHARE_PAIR : the two CTAs own M-tiles (2i, 2i+1) of the same N-tile and drive ONE tcgen05.mma.cta_group::2 (M = 256):
 //                each stages its own A tile and HALF of the B tile (the tensor core reads the other half from the peer's
 //                shared memory): 32 KB per k-block per SM, half the B operand reads per MMA, 6 stages instead of 4.  The
 //                leader CTA issues; both CTAs' TMA bytes complete on the leader's full barrier; commits are multicast.
-constexpr int SHARE_NONE = 0, SHARE_B = 1, SHARE_A = 2, SHARE_AB = 3, SHARE_PAIR = 4;
+constexpr int SHARE_NONE = 0, SHARE_B = 1, SHARE_A = 2, SHARE_PAIR = 4;
 constexpr int PAIR_STAGES = 6;
 constexpr int PAIR_STAGE_BYTES = A_BYTES + B_BYTES / 2;          // 32 KB; 6 x 32 KB = 4 x 48 KB
 
@@ -256,12 +252,12 @@ struct TileSched {
   int units, worker, nworkers, rank, m_tiles, n_tiles, per_split, n_fastest;
   __device__ TileSched(const Params& p) {
     n_fastest = p.n_fastest;
-    constexpr int CS = SHARE == SHARE_NONE ? 1 : (SHARE == SHARE_AB ? 4 : 2);      // CTAs per cluster
+    constexpr int CS = SHARE == SHARE_NONE ? 1 : 2;      // CTAs per cluster
     rank = SHARE != SHARE_NONE ? (int)cluster_cta_rank() : 0;
     worker = (int)blockIdx.x / CS;
     nworkers = (int)gridDim.x / CS;
-    m_tiles = (SHARE == SHARE_B || SHARE == SHARE_AB || SHARE == SHARE_PAIR) ? (p.m_tiles + 1) >> 1 : p.m_tiles;     // pairs along M
-    n_tiles = (SHARE == SHARE_A || SHARE == SHARE_AB) ? (p.n_tiles + 1) >> 1 : p.n_tiles;     // pairs along N
+    m_tiles = (SHARE == SHARE_B || SHARE == SHARE_PAIR) ? (p.m_tiles + 1) >> 1 : p.m_tiles;     // pairs along M
+    n_tiles = SHARE == SHARE_A ? (p.n_tiles + 1) >> 1 : p.n_tiles;     // pairs along N
     per_split = m_tiles * n_tiles;
     units = per_split * p.splits;
   }
@@ -277,7 +273,6 @@ struct TileSched {
     }
     if (SHARE == SHARE_B || SHARE == SHARE_PAIR) mt = mt * 2 + rank;
     if (SHARE == SHARE_A) nt = nt * 2 + rank;
-    if (SHARE == SHARE_AB) { mt = mt * 2 + (rank & 1); nt = nt * 2 + (rank >> 1); }
   }
 };
 
@@ -329,7 +324,7 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
   if (warp == 1 && lane == 0) {
     for (int s = 0; s < STAGES; ++s) {
       mbar_init(&full_bar[s], 1);
-      mbar_init(&empty_bar[s], PAIR ? 1 : (SHARE == SHARE_AB ? 3 : (CLUSTER ? 2 : 1)));   // multicast modes: every CTA this one writes into releases the stage
+      mbar_init(&empty_bar[s], PAIR ? 1 : (CLUSTER ? 2 : 1));   // multicast modes: both CTAs of the pair release the stage
     }
     for (int a = 0; a < 2; ++a) {
       mbar_init(&tfull_bar[a], 1);
@@ -389,12 +384,11 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
           }
           mbar_arrive_expect_tx(&full_bar[stage], STAGE_TX);      // own loads + the peer's multicast half
           // ---- A ----
-          if (SHARE == SHARE_A || SHARE == SHARE_AB) {
-            // shared A tile: this CTA loads rows [64*ha, +64) and multicasts them to the CTAs that own the same M-tile
-            const int ha = SHARE == SHARE_A ? sched.rank : (sched.rank >> 1);
-            const uint16_t am = SHARE == SHARE_A ? (uint16_t)0x3 : (uint16_t)((1u << (sched.rank & 1)) | (1u << ((sched.rank & 1) + 2)));
-            if (!A_MN) tma_load_2d_mc(sa + ha * (A_BYTES / 2), &tmap_a, &full_bar[stage], k0, m0 + ha * 64, am);
-            else tma_load_2d_mc(sa + ha * MN_BOX_BYTES, &tmap_a, &full_bar[stage], m0 + ha * 64, k0, am);
+          if (SHARE == SHARE_A) {
+            // shared A tile: this CTA loads rows [64*ha, +64) and multicasts them to both CTAs of the pair
+            const int ha = sched.rank;
+            if (!A_MN) tma_load_2d_mc(sa + ha * (A_BYTES / 2), &tmap_a, &full_bar[stage], k0, m0 + ha * 64, 0x3);
+            else tma_load_2d_mc(sa + ha * MN_BOX_BYTES, &tmap_a, &full_bar[stage], m0 + ha * 64, k0, 0x3);
           } else if (!A_MN) {
             tma_load_2d(sa, &tmap_a, &full_bar[stage], k0, m0);            // box {64 k, 128 rows}
           } else {
@@ -403,16 +397,15 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
               tma_load_2d(sa + b * MN_BOX_BYTES, &tmap_a, &full_bar[stage], m0 + b * 64, k0);
           }
           // ---- B ----
-          if (SHARE == SHARE_B || SHARE == SHARE_AB) {
-            // shared B tile: this CTA loads rows [128*hb, +128) and multicasts them to the CTAs that own the same N-tile
-            const int hb = SHARE == SHARE_B ? sched.rank : (sched.rank & 1);
-            const uint16_t bm = SHARE == SHARE_B ? (uint16_t)0x3 : (uint16_t)(0x3u << (2 * (sched.rank >> 1)));
+          if (SHARE == SHARE_B) {
+            // shared B tile: this CTA loads rows [128*hb, +128) and multicasts them to both CTAs of the pair
+            const int hb = sched.rank;
             if (!B_MN) {
-              tma_load_2d_mc(sb + hb * (B_BYTES / 2), &tmap_b, &full_bar[stage], k0, n0 + hb * 128, bm);
+              tma_load_2d_mc(sb + hb * (B_BYTES / 2), &tmap_b, &full_bar[stage], k0, n0 + hb * 128, 0x3);
             } else {
 #pragma unroll
               for (int b = 0; b < 2; ++b)
-                tma_load_2d_mc(sb + (hb * 2 + b) * MN_BOX_BYTES, &tmap_b, &full_bar[stage], n0 + (hb * 2 + b) * 64, k0, bm);
+                tma_load_2d_mc(sb + (hb * 2 + b) * MN_BOX_BYTES, &tmap_b, &full_bar[stage], n0 + (hb * 2 + b) * 64, k0, 0x3);
             }
           } else if (!B_MN) {
             tma_load_2d(sb, &tmap_b, &full_bar[stage], k0, n0);            // box {64 k, 256 rows}
@@ -462,7 +455,6 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
           }
           // frees the slot in every CTA that multicasts into this one (itself included) when these MMAs retire
           if (PAIR) umma_commit_2sm(&empty_bar[stage], 0x3);
-          else if (SHARE == SHARE_AB) umma_commit_mc(&empty_bar[stage], (uint16_t)((1u << sched.rank) | (1u << (sched.rank ^ 1)) | (1u << (sched.rank ^ 2))));
           else if (CLUSTER) umma_commit_mc(&empty_bar[stage], 0x3);
           else umma_commit(&empty_bar[stage]);
           if (++stage == STAGES) { stage = 0; phase ^= 1u; }
@@ -967,13 +959,44 @@ struct Operand {
 bool fwd_convert_eligible(const float* x, int K, int hw, int M);
 int launch_fwd_convert(const __nv_bfloat16* a, long long a_pitch, const float* x, int n_img, int hw, int M, int K, float* out,
                        long long row_stride, __nv_bfloat16* xn, cudaStream_t stream, int prof_tag);
-int launch(const Operand& a, const Operand& b, int M, int N, int K, int splits, float* out, long long row_stride,
-           int col_hw, long long img_stride, long long split_stride, cudaStream_t stream, int* splits_used, int prof_tag = -1,
-           int share = SHARE_NONE, bool out_bf16 = false, int sm_reserve = 0, int pair_fallback = SHARE_B, int row_hw = 0);
-// D bf16 [M][N] row-major = bf16_rn(relu((A B^T * scale + bias) + identity)) with M = n_img * hw pixels, identity fp32 NCHW
-// [n_img][N][hw]; A [M][K] and B [N][K] K-major.  N % 8 == 0, D 16-byte aligned.
-int launch_seam(const Operand& a, const Operand& b, int M, int N, int K, __nv_bfloat16* out, const float* identity, const float* scale,
-                const float* bias, int hw, cudaStream_t stream, int prof_tag = -1);
+// What the GEMM writes: one layout and the fields that layout takes.  Build it with the functions below.
+struct Out {
+  enum Layout {
+    F32,              // fp32 row-major: D[m, n] at ptr[m * row_stride + n]
+    F32_NCHW_COLS,    // fp32 NCHW with the columns as pixels: D[m, n] at ptr[(n / hw) * img_stride + m * row_stride + n % hw]
+    F32_NCHW_ROWS,    // fp32 NCHW with the rows as pixels, stored from registers: D[m, n] at ptr[(m / hw) * img_stride + n * hw + m % hw]
+    BF16,             // bf16 row-major [M][row_stride]: N and row_stride multiples of 8, ptr 16-byte aligned
+    SEAM,             // bf16 row-major [M][N] = bf16_rn(relu((D * scale[n] + bias[n]) + identity)), M = n_img * hw pixels,
+                      // identity fp32 NCHW [n_img][N][hw]; K-major operands, N % 8 == 0, ptr 16-byte aligned
+  } layout;
+  void* ptr;
+  long long row_stride, img_stride, split_stride;   // split_stride: elements between split-K slabs (F32, F32_NCHW_COLS, BF16)
+  int hw;                                           // pixels per image (F32_NCHW_COLS, F32_NCHW_ROWS, SEAM)
+  const float *identity, *scale, *bias;             // SEAM
+};
+inline Out out_f32(float* d, long long row_stride, long long split_stride = 0) { return {Out::F32, d, row_stride, 0, split_stride}; }
+inline Out out_f32_nchw_cols(float* d, int hw, long long row_stride, long long img_stride, long long split_stride = 0) {
+  return {Out::F32_NCHW_COLS, d, row_stride, img_stride, split_stride, hw};
+}
+inline Out out_f32_nchw_rows(float* d, int hw, long long img_stride) { return {Out::F32_NCHW_ROWS, d, 0, img_stride, 0, hw}; }
+inline Out out_bf16(__nv_bfloat16* d, long long row_stride, long long split_stride = 0) { return {Out::BF16, d, row_stride, 0, split_stride}; }
+inline Out out_seam(__nv_bfloat16* d, const float* identity, const float* scale, const float* bias, int hw) {
+  return {Out::SEAM, d, 0, 0, 0, hw, identity, scale, bias};
+}
+
+// D = A B^T, A [M][K] and B [N][K] (each K-major or MN-major), written as `out` says
+struct Gemm {
+  Operand a, b;
+  int M, N, K;
+  Out out;
+  int splits = 1;                // split-K (clamped so that every split is non-empty); the count used goes to *splits_used
+  int* splits_used = nullptr;
+  int share = SHARE_NONE;        // the sharing geometry the caller asks for; b200seg_gemm_set_sharing() may veto or override it
+  int pair_fallback = SHARE_B;   // what SHARE_PAIR becomes under sharing mode 5 (no cta_group::2)
+  int sm_reserve = 0;            // SMs left free for a concurrent kernel
+  int prof_tag = -1;
+};
+int launch(const Gemm& g, cudaStream_t stream);
 // fp32 NCHW data gradient of the head: 0 = channels along M (shared-memory transpose epilogue), 1 = pixels along M as cta_group::2
 // pairs, stores straight from registers, seven ring stages
 void set_dgrad_mode(int mode);

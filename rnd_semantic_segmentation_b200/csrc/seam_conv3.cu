@@ -105,8 +105,10 @@ int seam_conv3_forward(const float* out2, const float* identity, const float* w3
   B200SEG_LAUNCH_CHECK();
   gemm::Operand a{Xp, false, Cin};
   gemm::Operand b{Wb, false, Cin};
-  return gemm::launch_seam(a, b, (int)P, Cout, Cin, reinterpret_cast<__nv_bfloat16*>(y), identity, scale, bias, hw,
-                           stream);
+  gemm::Gemm gm{a, b, (int)P, Cout, Cin, gemm::out_seam(reinterpret_cast<__nv_bfloat16*>(y), identity, scale, bias, hw)};
+  gm.share = gemm::SHARE_PAIR;                // whenever sharing is on, under sharing mode 5 too: the pair is its own fallback
+  gm.pair_fallback = gemm::SHARE_PAIR;
+  return gemm::launch(gm, stream);
 }
 
 int seam_conv3_backward(const void* dy, const void* y, const void* ws, const float* scale, int N, int Cin, int Cout, int hw,
@@ -131,8 +133,12 @@ int seam_conv3_backward(const void* dy, const void* y, const void* ws, const flo
     gemm::Operand b{Xp, true, Cin};
     const long long slab = (long long)Cout * Cin;
     int used = 1;
-    rc = gemm::launch(a, b, Cout, Cin, (int)P, wgrad_splits(Cin, Cout, P), wpart, Cin, 0, 0, slab, stream, &used, -1, gemm::SHARE_PAIR,
-                      false, 0, gemm::SHARE_A);
+    gemm::Gemm gm{a, b, Cout, Cin, (int)P, gemm::out_f32(wpart, Cin, slab)};
+    gm.splits = wgrad_splits(Cin, Cout, P);
+    gm.splits_used = &used;
+    gm.share = gemm::SHARE_PAIR;
+    gm.pair_fallback = gemm::SHARE_A;
+    rc = gemm::launch(gm, stream);
     if (rc) return rc;
     seam_conv3_wgrad_reduce_kernel<<<(unsigned)ceil_div_ll(slab / 4, 256), 256, 0, stream>>>(wpart, used, slab, scale, Cin, dw3);
     B200SEG_LAUNCH_CHECK();
@@ -141,8 +147,10 @@ int seam_conv3_backward(const void* dy, const void* y, const void* ws, const flo
     // d_out2[p, ci] = sum_co g[p, co] W'[co, ci] with the pixels along M, fp32 NCHW straight from the accumulator registers
     gemm::Operand a{g, false, Cout};
     gemm::Operand b{Wt, false, Cout};
-    rc = gemm::launch(a, b, (int)P, Cin, Cout, 1, d_out2, 0, 0, (long long)Cin * hw, 0, stream, nullptr, -1, gemm::SHARE_PAIR, false, 0,
-                      gemm::SHARE_B, hw);
+    gemm::Gemm gm{a, b, (int)P, Cin, Cout, gemm::out_f32_nchw_rows(d_out2, hw, (long long)Cin * hw)};
+    gm.share = gemm::SHARE_PAIR;
+    gm.pair_fallback = gemm::SHARE_B;
+    rc = gemm::launch(gm, stream);
     if (rc) return rc;
   }
   return B200SEG_OK;

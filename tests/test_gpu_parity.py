@@ -37,8 +37,8 @@ def lib():
 ])
 @pytest.mark.parametrize("share", [0, 1, 2, 3, 4])
 def test_gemm_core_matches_cuda_core_reference(lib, M, N, K, a_mn, b_mn, splits, col_hw, share):
-    """share: 0 = one CTA per tile; 1 / 2 = 2-CTA clusters multicasting the shared B / A tile; 3 = 2 x 2 clusters, both;
-    4 = CTA pairs driving one tcgen05.mma.cta_group::2 (M = 256)."""
+    """share: 0 = one CTA per tile; 1 / 2 = 2-CTA clusters multicasting the shared B / A tile; 3 = the same as 2 (the ABI
+    value of the removed 2 x 2 clusters); 4 = CTA pairs driving one tcgen05.mma.cta_group::2 (M = 256)."""
     err, ref = lib.gemm_selftest(M, N, K, a_mn, b_mn, splits, col_hw, share)
     assert ref > 0
     assert err <= 2e-4 * ref * max(1.0, (K / 2048) ** 0.5), (err, ref)
