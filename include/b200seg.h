@@ -390,6 +390,35 @@ B200SEG_API int b200seg_seam_tail_bn_backward(const void* dy, const void* y, con
                                               float* dc, float* didentity, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * conv3 under batch statistics (opt-in): the last Bottleneck's 1x1 conv3 (stride 1, no bias) as a tcgen05 GEMM that writes conv3's
+ * output c once, as fp32 NCHW, and its per-rank BatchNorm statistics from the accumulator, so nothing reads c back for them; bn3 is
+ * a training-mode BatchNorm2d / SyncBatchNorm (core/models/feature_extractor/resnet.py:106-113, train_distill.py:52-53).
+ * b200seg_seam_conv3_bn_forward  replaces  out = self.conv3(out) and the per-rank statistics of self.bn3(out):
+ *   c fp32 NCHW [N][Cout][hw] = sum over ci of bf16(out2) * bf16(W3) (fp32 accumulation), record fp64 [3][Cout] = (count, mean, M2)
+ *   of the stored c in b200seg_bn_stats' format (per 32-pixel group two-pass in fp32, groups merged in a fixed order in fp64).
+ *   The record then goes through b200seg_bn_combine_stats and c through b200seg_seam_tail_bn_forward, both unchanged.
+ *   ws (b200seg_seam_conv3_bn_workspace_bytes, 16-byte aligned) receives bf16(out2) NHWC and bf16(W3)^T, which the backward reads.
+ *   Scratch: b200seg_seam_conv3_bn_forward_scratch_bytes.
+ * b200seg_seam_conv3_bn_backward  replaces  torch.batch_norm_backward_elemt, the residual / relu backward and conv3's data and
+ *   weight gradients, after b200seg_seam_tail_bn_backward_reduce (sums [R][2][Cout], count as for b200seg_seam_tail_bn_backward):
+ *   dc as b200seg_seam_tail_bn_backward computes it, rounded once to bf16 (never written as fp32);  didentity fp32 NCHW = g;
+ *   d_out2 fp32 NCHW [N][Cin][hw] = sum_co dc[., co] * bf16(W3[co, .]);  dW3 fp32 [Cout][Cin] = sum_p dc[p, co] * bf16(out2)[p, ci]
+ *   (split-K slabs summed in a fixed order, no atomics).  d_out2, dW3 and didentity may each be NULL.
+ *   Scratch: b200seg_seam_conv3_bn_backward_scratch_bytes.
+ * Cin % 8 == 0, Cout % 8 == 0, any hw >= 1, any N; y and dy 16-byte aligned.  No atomics, no host synchronisation.
+ * ------------------------------------------------------------------------------------------- */
+B200SEG_API int64_t b200seg_seam_conv3_bn_workspace_bytes(int N, int Cin, int Cout, int hw);
+B200SEG_API int64_t b200seg_seam_conv3_bn_forward_scratch_bytes(int N, int Cout, int hw);
+B200SEG_API int b200seg_seam_conv3_bn_forward(const float* out2, const float* w3, int N, int Cin, int Cout, int hw, void* ws,
+                                              int64_t ws_bytes, void* scratch, int64_t scratch_bytes, float* c, double* record,
+                                              void* stream);
+B200SEG_API int64_t b200seg_seam_conv3_bn_backward_scratch_bytes(int N, int Cin, int Cout, int hw);
+B200SEG_API int b200seg_seam_conv3_bn_backward(const void* dy, const void* y, const float* c, const float* mean, const float* invstd,
+                                               const float* gamma, const float* sums, int R, const double* count, const void* ws, int N,
+                                               int Cin, int Cout, int hw, void* scratch, int64_t scratch_bytes, float* d_out2,
+                                               float* dw3, float* didentity, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * K7  test-time augmentation fused with argmax + confusion matrix (SURVEY 8f rank 3).
  * Replaces inference(..., flip=True) (core/utils/utility.py:179-191), multi_scale_inference (utility.py:193-209), the
  * output.max(1)[1] / output.argmax(0) that follow (core/testers/aspp_tester.py:63,42) and confusion_matrix /

@@ -116,6 +116,12 @@ SIGNATURES = {
                                                      c_vp]),
     "b200seg_seam_tail_bn_backward": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_vp, c_int, c_int, c_int, c_vp, c_vp,
                                               c_vp]),
+    "b200seg_seam_conv3_bn_workspace_bytes": (c_i64, [c_int] * 4),
+    "b200seg_seam_conv3_bn_forward_scratch_bytes": (c_i64, [c_int] * 3),
+    "b200seg_seam_conv3_bn_forward": (c_int, [c_vp, c_vp, c_int, c_int, c_int, c_int, c_vp, c_i64, c_vp, c_i64, c_vp, c_vp, c_vp]),
+    "b200seg_seam_conv3_bn_backward_scratch_bytes": (c_i64, [c_int] * 4),
+    "b200seg_seam_conv3_bn_backward": (c_int, [c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_vp, c_vp, c_int, c_int, c_int, c_int,
+                                               c_vp, c_i64, c_vp, c_vp, c_vp, c_vp]),
     "b200seg_nhwc_colsum_scratch_bytes": (c_i64, [c_int]),
     "b200seg_nhwc_bf16_colsum": (c_int, [c_vp, c_i64, c_int, c_int, c_vp, c_vp, c_vp]),
     "b200seg_gemm_set_overlap_sms": (None, [c_int]),
@@ -1449,6 +1455,70 @@ def seam_tail_bn_backward(dy: torch.Tensor, y: torch.Tensor, c: torch.Tensor, me
                                                  _ptr(weight), sums.data_ptr(), sums.shape[0], count.data_ptr(), N, C, h * w, _ptr(dc),
                                                  _ptr(di), _stream()))
     return dc, di
+
+
+def seam_conv3_bn_forward(out2: torch.Tensor, weight: torch.Tensor):
+    """(c, record, ws): the last Bottleneck's conv3 as a tcgen05 GEMM (resnet.py:106-113) with bn3's per-rank batch statistics
+    computed from its accumulator.  c fp32 NCHW [N, Cout, h, w] = the fp32 sum over Cin of bf16(out2) * bf16(weight); record fp64
+    [3, Cout] = (count, mean, M2) of the stored c, in bn_stats' format; ``ws`` (uint8) holds bf16(out2) NHWC and bf16(weight)^T,
+    which seam_conv3_bn_backward reads.  out2 fp32 NCHW [N, Cin, h, w], weight fp32 [Cout, Cin(, 1, 1)], Cin % 8 == Cout % 8 == 0."""
+    lib = load()
+    N, Cin, h, w = _need_nchw_f32(out2, "out2").shape
+    _need(weight, torch.float32, "weight")
+    Cout = weight.shape[0]
+    if weight.numel() != Cout * Cin:
+        raise B200SegError(f"seam_conv3_bn_forward: out2 {tuple(out2.shape)} and weight {tuple(weight.shape)} do not form a 1x1 "
+                           "convolution")
+    nbytes = lib.b200seg_seam_conv3_bn_workspace_bytes(N, Cin, Cout, h * w)
+    ws = torch.empty(nbytes, dtype=torch.uint8, device=out2.device)
+    sbytes = lib.b200seg_seam_conv3_bn_forward_scratch_bytes(N, Cout, h * w)
+    scratch = _scratch("seam_conv3_bn_stats", sbytes, out2.device)
+    c = torch.empty((N, Cout, h, w), dtype=torch.float32, device=out2.device)
+    record = torch.empty((3, Cout), dtype=torch.float64, device=out2.device)
+    with _on_device(out2.device):
+        _check(lib.b200seg_seam_conv3_bn_forward(out2.data_ptr(), weight.data_ptr(), N, Cin, Cout, h * w, ws.data_ptr(), nbytes,
+                                                 scratch.data_ptr(), sbytes, c.data_ptr(), record.data_ptr(), _stream()))
+    return c, record, ws
+
+
+def seam_conv3_bn_backward(dy: torch.Tensor, y: torch.Tensor, c: torch.Tensor, mean: torch.Tensor, invstd: torch.Tensor,
+                           weight: Optional[torch.Tensor], sums: torch.Tensor, count: torch.Tensor, ws: torch.Tensor, Cin: int,
+                           need_out2: bool = True, need_conv_weight: bool = True, need_identity: bool = True):
+    """(d_out2, d_conv_weight, d_identity) of seam_conv3_bn_forward + seam_tail_bn_forward: dc as seam_tail_bn_backward computes it
+    (``weight`` the norm's gamma, ``sums`` [R, 2, C] from seam_tail_bn_backward_reduce, ``count`` fp64 [1]), rounded once to bf16;
+    d_out2 = dc . bf16(conv weight) (fp32 NCHW), d_conv_weight fp32 [Cout, Cin, 1, 1] = dc^T . bf16(out2), d_identity = g = dy * (y > 0)
+    (fp32 NCHW).  An output that is not needed is None (and not written)."""
+    lib = load()
+    _need_channels_last_bf16(dy, "dy")
+    _need_channels_last_bf16(y, "y")
+    _need_nchw_f32(c, "c")
+    if dy.shape != y.shape or c.shape != y.shape:
+        raise B200SegError(f"seam_conv3_bn_backward: dy {tuple(dy.shape)}, y {tuple(y.shape)} and c {tuple(c.shape)} differ")
+    N, Cout, h, w = y.shape
+    _need_channel_vector(mean, Cout, "mean")
+    _need_channel_vector(invstd, Cout, "invstd")
+    _optional_channel_vector(weight, Cout, "weight")
+    _need(sums, torch.float32, "sums")
+    if sums.dim() == 2:
+        sums = sums.unsqueeze(0)
+    if sums.dim() != 3 or tuple(sums.shape[1:]) != (2, Cout):
+        raise B200SegError(f"seam_conv3_bn_backward: expected sums [R, 2, {Cout}], got {tuple(sums.shape)}")
+    _need(count, torch.float64, "count")
+    _need(ws, torch.uint8, "ws")
+    if ws.numel() < lib.b200seg_seam_conv3_bn_workspace_bytes(N, Cin, Cout, h * w):
+        raise B200SegError("seam_conv3_bn_backward: workspace too small for this shape")
+    dx = torch.empty((N, Cin, h, w), dtype=torch.float32, device=y.device) if need_out2 else None
+    dw = torch.empty((Cout, Cin, 1, 1), dtype=torch.float32, device=y.device) if need_conv_weight else None
+    di = torch.empty((N, Cout, h, w), dtype=torch.float32, device=y.device) if need_identity else None
+    if dx is None and dw is None and di is None:
+        return None, None, None
+    nbytes = lib.b200seg_seam_conv3_bn_backward_scratch_bytes(N, Cin, Cout, h * w)
+    scratch = _scratch("seam_conv3", nbytes, y.device)
+    with _on_device(y.device):
+        _check(lib.b200seg_seam_conv3_bn_backward(dy.data_ptr(), y.data_ptr(), c.data_ptr(), mean.data_ptr(), invstd.data_ptr(),
+                                                  _ptr(weight), sums.data_ptr(), sums.shape[0], count.data_ptr(), ws.data_ptr(), N, Cin,
+                                                  Cout, h * w, scratch.data_ptr(), nbytes, _ptr(dx), _ptr(dw), _ptr(di), _stream()))
+    return dx, dw, di
 
 
 def nhwc_bf16_colsum(g: torch.Tensor, C: Optional[int] = None) -> torch.Tensor:

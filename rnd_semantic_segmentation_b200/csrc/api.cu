@@ -112,6 +112,11 @@ int seam_tail_bn_backward_reduce(const void*, const void*, const float*, const f
                                  float*, float*, float*, cudaStream_t);
 int seam_tail_bn_backward(const void*, const void*, const float*, const float*, const float*, const float*, const float*, int,
                           const double*, int, int, int, float*, float*, cudaStream_t);
+long long seam_conv3_bn_forward_scratch_bytes(int, int, int);
+long long seam_conv3_bn_backward_scratch_bytes(int, int, int, int);
+int seam_conv3_bn_forward(const float*, const float*, int, int, int, int, void*, long long, void*, long long, float*, double*, cudaStream_t);
+int seam_conv3_bn_backward(const void*, const void*, const float*, const float*, const float*, const float*, const float*, int,
+                           const double*, const void*, int, int, int, int, void*, long long, float*, float*, float*, cudaStream_t);
 long long nhwc_colsum_scratch_bytes(int);
 int nhwc_bf16_colsum(const void*, long long, int, int, void*, float*, cudaStream_t);
 int tta_launch(const float* const*, const int*, const int*, const int*, int, int, const void*, int, int, int, int, const float*, int, int,
@@ -612,6 +617,30 @@ int b200seg_seam_tail_bn_backward(const void* dy, const void* y, const float* c,
                                   float* didentity, void* stream) {
   REQUIRE_DEVICE();
   return seam_tail_bn_backward(dy, y, c, mean, invstd, gamma, sums, R, count, N, C, hw, dc, didentity, S(stream));
+}
+
+// conv3 under batch statistics (resnet.py:106-113): the workspace has the fused conv3's layout
+int64_t b200seg_seam_conv3_bn_workspace_bytes(int N, int Cin, int Cout, int hw) { return seam_conv3_workspace_bytes(N, Cin, Cout, hw); }
+
+int64_t b200seg_seam_conv3_bn_forward_scratch_bytes(int N, int Cout, int hw) { return seam_conv3_bn_forward_scratch_bytes(N, Cout, hw); }
+
+int b200seg_seam_conv3_bn_forward(const float* out2, const float* w3, int N, int Cin, int Cout, int hw, void* ws, int64_t ws_bytes,
+                                  void* scratch, int64_t scratch_bytes, float* c, double* record, void* stream) {
+  REQUIRE_DEVICE();
+  return seam_conv3_bn_forward(out2, w3, N, Cin, Cout, hw, ws, ws_bytes, scratch, scratch_bytes, c, record, S(stream));
+}
+
+int64_t b200seg_seam_conv3_bn_backward_scratch_bytes(int N, int Cin, int Cout, int hw) {
+  return seam_conv3_bn_backward_scratch_bytes(N, Cin, Cout, hw);
+}
+
+int b200seg_seam_conv3_bn_backward(const void* dy, const void* y, const float* c, const float* mean, const float* invstd,
+                                   const float* gamma, const float* sums, int R, const double* count, const void* ws, int N, int Cin,
+                                   int Cout, int hw, void* scratch, int64_t scratch_bytes, float* d_out2, float* dw3, float* didentity,
+                                   void* stream) {
+  REQUIRE_DEVICE();
+  return seam_conv3_bn_backward(dy, y, c, mean, invstd, gamma, sums, R, count, ws, N, Cin, Cout, hw, scratch, scratch_bytes, d_out2, dw3,
+                                didentity, S(stream));
 }
 
 int b200seg_tta_argmax_confusion(const float* const* logits_lr, const int* h, const int* w, const int* flip, int n_members, int C,

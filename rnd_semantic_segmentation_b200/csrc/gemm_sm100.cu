@@ -64,17 +64,24 @@ int fwd_mode() { return g_fwd_mode; }
 static int g_narrow_tiles = 1;        // b200seg_gemm_set_narrow_tiles(): 0 = always 256-column tiles
 void set_narrow_tiles(int on) { g_narrow_tiles = on; }
 
+// the register-store epilogue that also writes each 32-pixel lane group's per-column (mean, M2) (Out::F32_NCHW_ROWS_STATS)
+__global__ void __launch_bounds__(NUM_THREADS, 1)
+gemm_bf16_stats_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
+                       const __grid_constant__ CUtensorMap tmap_out, const Params p) {
+  gemm_bf16_body<false, false, SHARE_PAIR, 256, true, false, true>(tmap_a, tmap_b, tmap_out, p);
+}
+
 // Every instantiation of gemm_bf16_kernel that launch() can run
 typedef void (*KernelFn)(CUtensorMap, CUtensorMap, CUtensorMap, Params);
 struct Variant {
   bool a_mn, b_mn;
   int share, bn;
-  bool rs, seam;
+  bool rs, seam, stats;
   KernelFn fn;
   bool configured;
 };
 template <bool A_MN, bool B_MN, int SHARE, int BN = 256, bool RS = false, bool SEAM = false>
-static Variant variant() { return {A_MN, B_MN, SHARE, BN, RS, SEAM, gemm_bf16_kernel<A_MN, B_MN, SHARE, BN, RS, SEAM>, false}; }
+static Variant variant() { return {A_MN, B_MN, SHARE, BN, RS, SEAM, false, gemm_bf16_kernel<A_MN, B_MN, SHARE, BN, RS, SEAM>, false}; }
 static Variant g_variants[] = {
     // any operand layout, any sharing geometry, 256-column tiles
     variant<false, false, SHARE_NONE>(), variant<false, false, SHARE_B>(), variant<false, false, SHARE_A>(), variant<false, false, SHARE_PAIR>(),
@@ -88,6 +95,8 @@ static Variant g_variants[] = {
     variant<false, false, SHARE_PAIR, 256, true>(), variant<true, false, SHARE_PAIR, 256, true>(),
     // seam epilogue: K-major operands
     variant<false, false, SHARE_NONE, 256, false, true>(), variant<false, false, SHARE_PAIR, 256, false, true>(),
+    // fp32 NCHW rows-as-pixels with per-lane-group column statistics: cta_group::2 pairs, K-major operands
+    {false, false, SHARE_PAIR, 256, true, false, true, gemm_bf16_stats_kernel, false},
 };
 
 static int check(const Gemm& g) {
@@ -99,6 +108,13 @@ static int check(const Gemm& g) {
     B200SEG_CHECK_ARG(!g.a.mn_major && !g.b.mn_major, "gemm seam: K-major operands only");
     B200SEG_CHECK_ARG(o.identity && o.scale && o.bias && g.N % 8 == 0 && aligned,
                       "gemm seam: N = %d must be a multiple of 8 and D 16-byte aligned", g.N);
+    return B200SEG_OK;
+  }
+  if (o.layout == Out::F32_NCHW_ROWS_STATS) {
+    B200SEG_CHECK_ARG(g.M > 0 && g.N > 0 && g.K > 0 && o.hw > 0 && (g.M % o.hw == 0 || g.M <= o.hw) && g.splits <= 1,
+                      "gemm rows + stats: bad problem %dx%dx%d (hw %d)", g.M, g.N, g.K, o.hw);
+    B200SEG_CHECK_ARG(!g.a.mn_major && !g.b.mn_major, "gemm rows + stats: K-major operands only");
+    B200SEG_CHECK_ARG(o.stats && (reinterpret_cast<uintptr_t>(o.stats) & 7) == 0, "gemm rows + stats: stats must be 8-byte aligned");
     return B200SEG_OK;
   }
   B200SEG_CHECK_ARG(g.M > 0 && g.N > 0 && g.K > 0, "gemm: empty problem %dx%dx%d", g.M, g.N, g.K);
@@ -115,13 +131,14 @@ int launch(const Gemm& g, cudaStream_t stream) {
   const Operand &a = g.a, &b = g.b;
   const Out& o = g.out;
   const int M = g.M, N = g.N, K = g.K;
-  const bool seam = o.layout == Out::SEAM;
+  const bool seam = o.layout == Out::SEAM, stats = o.layout == Out::F32_NCHW_ROWS_STATS;
   // callers name the sharing geometry they want; the global mode (A/B experiments) can veto or override it
   int share = g.share;
   if (!g_share_enabled) share = SHARE_NONE;
   if (g_share_enabled == 3 && share == SHARE_B) share = SHARE_PAIR;         // also the store-bound fp32 dgrad as 2-SM pairs
   if (g_share_enabled == 4 && (share == SHARE_A || share == SHARE_B)) share = SHARE_PAIR;
   if (g_share_enabled == 5 && share == SHARE_PAIR) share = g.pair_fallback;
+  if (stats) share = SHARE_PAIR;          // its only kernel, under every sharing mode and for a single M-tile too
   Params p = {};
   p.M = M; p.N = N; p.K = K;
   p.m_tiles = ceil_div(M, BLOCK_M);
@@ -155,6 +172,11 @@ int launch(const Gemm& g, cudaStream_t stream) {
     p.row_hw_px = o.hw;
     p.row_hw = g_dgrad_mode == 2 ? 2 : 1;
     p.epi_sleep_ns = env_ns > 0 ? env_ns : 0;
+  } else if (stats) {
+    // conv3 under batch statistics: the register-store epilogue with plain stores, no pacing
+    p.row_hw_px = o.hw;
+    p.row_hw = 1;
+    p.stats = o.stats;
   } else if (seam) {
     // the fused conv3 + tail of the backbone's last Bottleneck: pairs along M walking along N, so a pair's two pixel tiles are read
     // once for all N-tiles while the small weight operand stays in L2
@@ -169,7 +191,7 @@ int launch(const Gemm& g, cudaStream_t stream) {
   }
   // a pair needs two tiles along the paired dimension to be worth it
   if (share == SHARE_B && p.m_tiles < 2) share = SHARE_NONE;
-  if (share == SHARE_PAIR && p.m_tiles < 2) share = SHARE_NONE;
+  if (share == SHARE_PAIR && p.m_tiles < 2 && !stats) share = SHARE_NONE;
   if (share == SHARE_A && p.n_tiles < 2) share = SHARE_NONE;
 
   // tile width: with K-major operands, fp32 output and an unshared B tile, a narrower tile that makes the tile count a
@@ -190,7 +212,8 @@ int launch(const Gemm& g, cudaStream_t stream) {
   const bool rs = p.row_hw == 1 && share == SHARE_PAIR && !b.mn_major;        // register-store variant (7 ring stages)
   Variant* v = nullptr;
   for (Variant& c : g_variants)
-    if (c.a_mn == a.mn_major && c.b_mn == b.mn_major && c.share == share && c.bn == bn && c.rs == rs && c.seam == seam) { v = &c; break; }
+    if (c.a_mn == a.mn_major && c.b_mn == b.mn_major && c.share == share && c.bn == bn && c.rs == rs && c.seam == seam &&
+        c.stats == stats) { v = &c; break; }
   B200SEG_CHECK_ARG(v, "gemm: no kernel for operands %d/%d, sharing %d, %d-column tiles, output layout %d", (int)a.mn_major,
                     (int)b.mn_major, share, bn, (int)o.layout);
 

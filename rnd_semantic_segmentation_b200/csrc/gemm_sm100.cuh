@@ -58,6 +58,9 @@ struct Params {
   const float* seam_identity;
   const float* seam_scale;
   const float* seam_bias;
+  // statistics epilogue (gemm_bf16_stats_kernel only): for every 32-pixel TMEM lane group gi = m / 32 and column n < N,
+  // stats[gi * N + n] = (mean, M2) of the fp32 D values the register-store epilogue writes for those pixels
+  float2* stats;
 };
 
 // ------------------------------------------------------------------------------------------
@@ -276,6 +279,22 @@ struct TileSched {
   }
 };
 
+// Sum over the warp's 32 lanes of each of 16 values, by halving exchanges (8 + 4 + 2 + 1 + 1 shuffles, not 16 x 5): lane l
+// returns the total of value l / 2 (lanes 2j and 2j + 1 get the same bits).  v is consumed.  A fixed order: deterministic.
+__device__ __forceinline__ float warp_sum_scatter16(float (&v)[16], int lane) {
+#pragma unroll
+  for (int st = 0; st < 4; ++st) {
+    const int w = 8 >> st, o = 16 >> st;
+    const bool hi = (lane & o) != 0;
+#pragma unroll
+    for (int i = 0; i < w; ++i) {
+      const float keep = hi ? v[i + w] : v[i], send = hi ? v[i] : v[i + w];
+      v[i] = keep + __shfl_xor_sync(0xffffffffu, send, o);
+    }
+  }
+  return v[0] + __shfl_xor_sync(0xffffffffu, v[0], 1);
+}
+
 // BN = accumulator columns per tile (256 by default).  A narrower tile (224 / 192) is picked by the host when it makes the
 // tile count a near-multiple of the SM count: 5 M-tiles x 128 N-tiles of 256 on 148 SMs are 4.3 waves = 5 rounds; the same
 // problem in 224-column tiles is 5 x 147 = 4.97 waves = 5 rounds of 12.5 % less work each.  K-major operands, fp32 output,
@@ -285,10 +304,11 @@ struct TileSched {
 // by the epilogue's store bursts, and bytes in flight are what hides it.
 // SEAM: the bf16 row-major epilogue with the backbone tail applied to the accumulator first (Params::seam_*): M = pixels, so a
 // TMEM lane is a pixel and each identity column load is 32 consecutive pixels of one fp32 NCHW plane.  K-major operands only.
-template <bool A_MN, bool B_MN, int SHARE, int BN = 256, bool RS = false, bool SEAM = false>
-__global__ void __launch_bounds__(NUM_THREADS, 1)
-gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
-                 const __grid_constant__ CUtensorMap tmap_out, const Params p) {
+// STATS (gemm_bf16_stats_kernel): the RS epilogue also writes each lane group's per-column (mean, M2) (Params::stats).
+template <bool A_MN, bool B_MN, int SHARE, int BN, bool RS, bool SEAM, bool STATS>
+__device__ __forceinline__ void gemm_bf16_body(const CUtensorMap& tmap_a, const CUtensorMap& tmap_b, const CUtensorMap& tmap_out,
+                                               const Params& p) {
+  __builtin_assume(threadIdx.x < NUM_THREADS);      // what __launch_bounds__ tells the compiler in the kernel itself
   extern __shared__ uint8_t smem_raw[];
   const uint32_t raw_addr = smem_u32(smem_raw);
   const uint32_t pad = (1024u - (raw_addr & 1023u)) & 1023u;
@@ -300,6 +320,7 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
   constexpr int B_BYTES = BN * BLOCK_K * 2;
   static_assert(!RS || (PAIR && BN == 256), "register-store variant: cta_group::2 pairs only");
   static_assert(!SEAM || (!RS && !A_MN && !B_MN && BN == 256), "seam epilogue: K-major operands, 256-column tiles");
+  static_assert(!STATS || (RS && !SEAM && !A_MN && !B_MN), "statistics epilogue: the register-store variant, K-major operands");
   constexpr int STAGES = PAIR ? (RS ? PAIR_STAGES + 1 : PAIR_STAGES) : gemm::STAGES;         // same total bytes either way
   constexpr int STAGE_BYTES = PAIR ? PAIR_STAGE_BYTES : gemm::STAGE_BYTES;     // ring stride (a narrow B tile leaves its tail unused)
   constexpr int STAGE_TX = PAIR ? PAIR_STAGE_BYTES : A_BYTES + B_BYTES;        // bytes that land in a stage per k-block
@@ -574,6 +595,29 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
                   if (k < ncols) d[(long long)k * hw] = __uint_as_float(r[k]);
               }
             }
+            if (STATS && ncols > 0) {
+              // the chunk's 16 channels over this warp's `rows` pixels, corrected two-pass (no shift is available here to keep
+              // |mean| >> sigma accurate): the group mean m, then M2 = sum (v - m)^2 - (sum (v - m))^2 / n about m + sum (v - m) / n;
+              // lanes past the last pixel contribute nothing
+              const float cnt = (float)rows;
+              float v[16], sq[16];
+#pragma unroll
+              for (int k = 0; k < 16; ++k) v[k] = ok ? __uint_as_float(r[k]) : 0.f;
+#pragma unroll
+              for (int k = 0; k < 16; ++k) sq[k] = v[k];
+              const float mean = warp_sum_scatter16(sq, lane) / cnt;            // of channel lane / 2
+#pragma unroll
+              for (int k = 0; k < 16; ++k) {
+                const float mk = __shfl_sync(0xffffffffu, mean, 2 * k);
+                v[k] = ok ? v[k] - mk : 0.f;
+                sq[k] = v[k] * v[k];
+              }
+              const float sd = warp_sum_scatter16(v, lane);
+              const float m2 = warp_sum_scatter16(sq, lane) - sd * sd / cnt;
+              const int j = lane >> 1;
+              if ((lane & 1) == 0 && j < ncols)                              // (the mean the corrected M2 is taken about)
+                p.stats[(long long)(row_base >> 5) * p.N + col_base + c * 16 + j] = make_float2(mean + sd / cnt, m2);
+            }
             if (p.epi_sleep_ns > 0) __nanosleep((unsigned)p.epi_sleep_ns);
           }
         }
@@ -645,6 +689,13 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
     if (PAIR) tmem_dealloc_2sm(tmem_base, TMEM_COLS);
     else tmem_dealloc(tmem_base, TMEM_COLS);
   }
+}
+
+template <bool A_MN, bool B_MN, int SHARE, int BN = 256, bool RS = false, bool SEAM = false>
+__global__ void __launch_bounds__(NUM_THREADS, 1)
+gemm_bf16_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
+                 const __grid_constant__ CUtensorMap tmap_out, const Params p) {
+  gemm_bf16_body<A_MN, B_MN, SHARE, BN, RS, SEAM, false>(tmap_a, tmap_b, tmap_out, p);
 }
 
 // ------------------------------------------------------------------------------------------
@@ -968,11 +1019,14 @@ struct Out {
     BF16,             // bf16 row-major [M][row_stride]: N and row_stride multiples of 8, ptr 16-byte aligned
     SEAM,             // bf16 row-major [M][N] = bf16_rn(relu((D * scale[n] + bias[n]) + identity)), M = n_img * hw pixels,
                       // identity fp32 NCHW [n_img][N][hw]; K-major operands, N % 8 == 0, ptr 16-byte aligned
+    F32_NCHW_ROWS_STATS,  // F32_NCHW_ROWS, and stats[(m / 32) * N + n] = (mean, M2) over the (up to) 32 pixels m of each lane
+                          // group: always cta_group::2 pairs, K-major operands, no split-K
   } layout;
   void* ptr;
   long long row_stride, img_stride, split_stride;   // split_stride: elements between split-K slabs (F32, F32_NCHW_COLS, BF16)
-  int hw;                                           // pixels per image (F32_NCHW_COLS, F32_NCHW_ROWS, SEAM)
+  int hw;                                           // pixels per image (F32_NCHW_COLS, F32_NCHW_ROWS, SEAM, F32_NCHW_ROWS_STATS)
   const float *identity, *scale, *bias;             // SEAM
+  float2* stats;                                    // F32_NCHW_ROWS_STATS: [ceil(M / 32)][N]
 };
 inline Out out_f32(float* d, long long row_stride, long long split_stride = 0) { return {Out::F32, d, row_stride, 0, split_stride}; }
 inline Out out_f32_nchw_cols(float* d, int hw, long long row_stride, long long img_stride, long long split_stride = 0) {
@@ -982,6 +1036,9 @@ inline Out out_f32_nchw_rows(float* d, int hw, long long img_stride) { return {O
 inline Out out_bf16(__nv_bfloat16* d, long long row_stride, long long split_stride = 0) { return {Out::BF16, d, row_stride, 0, split_stride}; }
 inline Out out_seam(__nv_bfloat16* d, const float* identity, const float* scale, const float* bias, int hw) {
   return {Out::SEAM, d, 0, 0, 0, hw, identity, scale, bias};
+}
+inline Out out_f32_nchw_rows_stats(float* d, int hw, long long img_stride, float2* stats) {
+  return {Out::F32_NCHW_ROWS_STATS, d, 0, img_stride, 0, hw, nullptr, nullptr, nullptr, stats};
 }
 
 // D = A B^T, A [M][K] and B [N][K] (each K-major or MN-major), written as `out` says

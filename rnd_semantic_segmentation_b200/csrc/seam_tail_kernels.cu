@@ -118,7 +118,9 @@ __global__ void __launch_bounds__(ST_THREADS) nchw_to_nhwc_tile_kernel(const flo
 //             records of sums [R][2][C] in rank order and M = *count (gamma may be null), and didentity = g.
 // BN_G (the fused conv3 tail, whose conv3 runs inside the tcgen05 GEMMs) writes g itself as bf16 NHWC (the GEMMs' operand; exact,
 // no rounding) and didentity = g; c, scale and dc are not used.
-enum { BN_FOLD = 0, BN_REDUCE = 1, BN_APPLY = 2, BN_G = 3 };
+// BN_APPLY_G (conv3 under batch statistics) computes dc as BN_APPLY does and writes it rounded once to bf16 NHWC into g (the operand
+// of conv3's backward GEMMs) instead of fp32 NCHW dc; didentity = g as in BN_APPLY.
+enum { BN_FOLD = 0, BN_REDUCE = 1, BN_APPLY = 2, BN_G = 3, BN_APPLY_G = 4 };
 struct BnBackward {
   const float* c;
   const float* mean;
@@ -215,7 +217,7 @@ __global__ void __launch_bounds__(ST_THREADS) seam_tail_backward_kernel(const __
       continue;
     }
     float4 d;
-    if (BN == BN_APPLY) {
+    if (BN == BN_APPLY || BN == BN_APPLY_G) {
       float sg = 0.f, sx = 0.f;
       for (int r = 0; r < bn.R; ++r) {                             // rank order: every rank computes the same sums
         sg += __ldg(bn.sums + (long long)r * 2 * C + cg);
@@ -232,6 +234,7 @@ __global__ void __launch_bounds__(ST_THREADS) seam_tail_backward_kernel(const __
     } else {
       d = g;                                                       // (BN_G: dc is null)
     }
+    if (BN == BN_APPLY_G) *reinterpret_cast<float4*>(tile + st_idx(ch, 4 * lane)) = d;    // (this thread's own slot)
     const long long off = ((long long)n * C + cg) * hw + s;
     if (VEC) {
       if (s < hw) {
@@ -246,6 +249,22 @@ __global__ void __launch_bounds__(ST_THREADS) seam_tail_backward_kernel(const __
         if (s + j >= hw) break;
         if (didentity) __stcs(didentity + off + j, gp[j]);
         if (dc) __stcs(dc + off + j, dp[j]);
+      }
+    }
+  }
+  if (BN == BN_APPLY_G) {                                          // dc through the tile to bf16 NHWC, as the forward's y
+    __syncthreads();
+#pragma unroll
+    for (int it = 0; it < 2; ++it) {
+      const int sl = (lane >> 2) + 8 * warp + 64 * it;
+      if (s0 + sl < hw && cc < C) {
+        uint32_t w4[4];
+#pragma unroll
+        for (int e = 0; e < 4; ++e) {
+          const __nv_bfloat162 v = __floats2bfloat162_rn(tile[st_idx(8 * chunk + 2 * e, sl)], tile[st_idx(8 * chunk + 2 * e + 1, sl)]);
+          w4[e] = *reinterpret_cast<const uint32_t*>(&v);
+        }
+        *reinterpret_cast<uint4*>(bn.g + ((long long)n * hw + s0 + sl) * C + cc) = make_uint4(w4[0], w4[1], w4[2], w4[3]);
       }
     }
   }
@@ -541,6 +560,22 @@ int seam_tail_bn_backward(const void* dy, const void* y, const float* c, const f
   if (!dc && !didentity) return B200SEG_OK;
   BnBackward bn{c, mean, invstd, gamma, sums, R, count, nullptr};
   backward_launch<BN_APPLY>(dy, y, nullptr, N, C, hw, dc, didentity, bn, stream);
+  B200SEG_LAUNCH_CHECK();
+  return B200SEG_OK;
+}
+
+// conv3 under batch statistics: dc as seam_tail_bn_backward computes it, rounded once to bf16 NHWC [N*hw][C] (the operand of conv3's
+// data- and weight-gradient GEMMs; fp32 dc is never written), and, when didentity is not null, didentity = g as fp32 NCHW
+int seam_tail_bn_backward_g(const void* dy, const void* y, const float* c, const float* mean, const float* invstd, const float* gamma,
+                            const float* sums, int R, const double* count, int N, int C, int hw, void* g, float* didentity,
+                            cudaStream_t stream) {
+  B200SEG_CHECK_ARG(dy && y && c && mean && invstd && sums && count && g && R > 0 && N > 0 && C > 0 && hw > 0,
+                    "seam_tail_bn_backward_g: bad arguments");
+  B200SEG_CHECK_ARG(C % 8 == 0, "seam_tail_bn_backward_g: C = %d is not a multiple of 8", C);
+  B200SEG_CHECK_ARG(N <= 65535 && ceil_div(C, ST_CH) <= 65535, "seam_tail_bn_backward_g: N = %d / C = %d too large", N, C);
+  B200SEG_CHECK_ARG(aligned16(dy) && aligned16(y) && aligned16(g), "seam_tail_bn_backward_g: dy, y and g must be 16-byte aligned");
+  BnBackward bn{c, mean, invstd, gamma, sums, R, count, nullptr, reinterpret_cast<__nv_bfloat16*>(g)};
+  backward_launch<BN_APPLY_G>(dy, y, nullptr, N, C, hw, nullptr, didentity, bn, stream);
   B200SEG_LAUNCH_CHECK();
   return B200SEG_OK;
 }

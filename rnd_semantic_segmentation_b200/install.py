@@ -12,7 +12,8 @@ parameter sets that live on a CUDA device (everything else keeps the stock class
 ``core.models.build.build_feature_extractor`` (same signature) so that the backbone it returns emits the head's seam format, bf16
 channels_last, from its last Bottleneck (seam.fuse_backbone_tail; INTEGRATION.md "Seam format"); with ``seam_train_bn=True`` also
 when that block's bn3 is a training-mode BatchNorm2d / SyncBatchNorm (batch statistics, the self-distillation stage); with
-``seam_conv3=True`` the block's conv3 runs inside the fused GEMM (bf16 operands, fp32 accumulation: see seam.py).
+``seam_conv3=True`` the block's conv3 runs inside the fused GEMM (bf16 operands, fp32 accumulation: see seam.py); with
+``seam_train_bn=True, seam_conv3_batch=True`` a batch-statistics bn3's conv3 runs as a tcgen05 GEMM that also computes the statistics.
 """
 from __future__ import annotations
 
@@ -78,7 +79,7 @@ def uninstall_optimizers():
         torch.optim.SGD, torch.optim.Adam = _stock_optimizers.pop("SGD"), _stock_optimizers.pop("Adam")
 
 
-def _install_seam(patched, train_bn=False, conv3=False):
+def _install_seam(patched, train_bn=False, conv3=False, conv3_batch=False):
     """core.models(.build).build_feature_extractor -> the same factory with fuse_backbone_tail applied to its result, also in
     modules that imported the name before."""
     wrapped = {}                     # id(stock function) -> wrapper (core.models re-exports core.models.build's function)
@@ -87,7 +88,7 @@ def _install_seam(patched, train_bn=False, conv3=False):
         stock = getattr(mod, "build_feature_extractor", None) if mod is not None else None
         if stock is None:
             continue
-        fn = wrapped.setdefault(id(stock), _seam.wrap_feature_extractor_factory(stock, train_bn, conv3))
+        fn = wrapped.setdefault(id(stock), _seam.wrap_feature_extractor_factory(stock, train_bn, conv3, conv3_batch))
         wrapped[id(fn)] = fn
         setattr(mod, "build_feature_extractor", fn)
         patched.append(f"{modname}.build_feature_extractor")
@@ -101,12 +102,15 @@ def _install_seam(patched, train_bn=False, conv3=False):
             patched.append(f"{name}.build_feature_extractor")
 
 
-def install(strict: bool = False, optimizers: bool = False, seam: bool = False, seam_train_bn: bool = False, seam_conv3: bool = False):
+def install(strict: bool = False, optimizers: bool = False, seam: bool = False, seam_train_bn: bool = False, seam_conv3: bool = False,
+            seam_conv3_batch: bool = False):
     """Returns the list of 'module.attr' names that were patched.  ``seam=True``: the reference's build_feature_extractor returns
     a backbone whose last Bottleneck emits bf16 channels_last features (seam.fuse_backbone_tail); ``seam_train_bn=True`` (with
     ``seam=True``) extends that to a bn3 that trains with batch statistics (fuse_backbone_tail(fe, train_bn=True));
     ``seam_conv3=True`` (with ``seam=True``) fuses an eligible conv3 into the tail's GEMM (fuse_backbone_tail(fe, conv3=True)),
-    which rounds conv3's operands to bf16."""
+    which rounds conv3's operands to bf16; ``seam_conv3_batch=True`` (with ``seam=True, seam_train_bn=True``) runs an eligible conv3
+    of a batch-statistics bn3 as a tcgen05 GEMM that writes its output and statistics (fuse_backbone_tail(fe, train_bn=True,
+    conv3_batch=True)), also with bf16 operands."""
     patched = install_optimizers() if optimizers else []
     targets = (("core.models.build", _build, _BUILD_NAMES), ("core.models", _build, _BUILD_NAMES),
                ("core.utils.utility", _utility, _UTIL_NAMES), ("core.utils.adapt_lr", _optim, _LR_NAMES))
@@ -133,5 +137,5 @@ def install(strict: bool = False, optimizers: bool = False, seam: bool = False, 
                     setattr(mod, n, getattr(src, n))
                     patched.append(f"{name}.{n}")
     if seam:
-        _install_seam(patched, seam_train_bn, seam_conv3)
+        _install_seam(patched, seam_train_bn, seam_conv3, seam_conv3_batch)
     return patched

@@ -378,6 +378,63 @@ def seam_tail_bn(c: torch.Tensor, identity: torch.Tensor, weight: Optional[torch
                                None if momentum is None else float(momentum), float(eps), process_group)
 
 
+class _SeamConv3TailBNFn(torch.autograd.Function):
+    """bf16 channels_last relu(batch_norm(conv1x1(out2, W3)) + identity) with bn3 in training mode (resnet.py:106-113; BatchNorm2d,
+    or SyncBatchNorm over ``group``): conv3 as a tcgen05 GEMM that writes c and its statistics, then the batch tail.  Saves the
+    workspace (bf16 out2, bf16 W3 and its transpose), c, y, mean, invstd and the count; nothing under no_grad.  The running
+    buffers are updated in place once per forward (under no_grad too)."""
+
+    @staticmethod
+    def forward(ctx, out2, identity, conv_weight, weight, bias, running_mean, running_var, num_batches_tracked, momentum, eps, group):
+        w = None if weight is None else weight.detach().contiguous()
+        b = None if bias is None else bias.detach().contiguous()
+        c, records, ws = _lib.seam_conv3_bn_forward(out2.detach().contiguous(), conv_weight.detach().contiguous())
+        if group is not None:
+            records = _gather_ranks(records, group)
+        if running_mean is not None and num_batches_tracked is not None:
+            num_batches_tracked.add_(1)
+        mean, invstd, count = _lib.bn_combine_stats(records, eps, momentum, running_mean, running_var, num_batches_tracked)
+        y = _lib.seam_tail_bn_forward(c, identity.detach().contiguous(), mean, invstd, w, b)
+        if any(ctx.needs_input_grad[:5]):
+            ctx.group, ctx.cin = group, out2.shape[1]
+            ctx.save_for_backward(ws, c, y, mean, invstd, count, w)
+        return y
+
+    @staticmethod
+    def backward(ctx, dy):
+        ws, c, y, mean, invstd, count, w = ctx.saved_tensors
+        need_x, need_id, need_cw, need_w, need_b = ctx.needs_input_grad[:5]
+        dy = _seam_dy(dy)
+        dx = di = dcw = gw = gb = None
+        if need_x or need_cw or need_w or need_b:
+            sums, gw, gb = _lib.seam_tail_bn_backward_reduce(dy, y, c, mean, invstd, need_w, need_b)
+            if (need_x or need_cw) and ctx.group is not None:
+                sums = _gather_ranks(sums, ctx.group)       # dgamma / dbeta stay local: DDP averages them
+            dx, dcw, di = _lib.seam_conv3_bn_backward(dy, y, c, mean, invstd, w, sums, count, ws, ctx.cin, need_x, need_cw, need_id)
+        elif need_id:
+            _, di = _lib.seam_tail_backward(dy, y, invstd, False, True)     # didentity = g (the scale is not read)
+        return dx, di, dcw, gw, gb, None, None, None, None, None, None
+
+
+def seam_conv3_tail_bn(out2: torch.Tensor, identity: torch.Tensor, conv_weight: torch.Tensor, weight: Optional[torch.Tensor],
+                       bias: Optional[torch.Tensor], running_mean: Optional[torch.Tensor], running_var: Optional[torch.Tensor],
+                       num_batches_tracked: Optional[torch.Tensor], momentum: Optional[float], eps: float,
+                       process_group=None) -> torch.Tensor:
+    """bf16 channels_last ``relu(batch_norm(conv3(out2)) + identity)`` with training-mode batch statistics: the last Bottleneck's
+    1x1 conv3 (stride 1, no bias, fp32 ``conv_weight`` [Cout, Cin, 1, 1]) as a tcgen05 GEMM that writes conv3's output c (fp32
+    NCHW) and its per-rank statistics from the accumulator, then bn3 + residual + relu as ``seam_tail_bn`` (same arguments, same
+    running-buffer update and SyncBatchNorm exchange over ``process_group``).  ``out2`` fp32 NCHW [N, Cin, h, w], ``identity`` fp32
+    NCHW [N, Cout, h, w], Cin % 8 == 0, Cout % 8 == 0.
+    Numerics: out2 and conv_weight are each rounded to bf16 once and the products accumulated in fp32 (as the fold's fused conv3);
+    the statistics are those of the stored fp32 c; in the backward, dc is rounded once to bf16 before conv3's data and weight
+    gradient GEMMs (fp32 accumulation).  Differentiable in out2, identity, conv_weight, weight and bias."""
+    if process_group is None and out2.shape[0] * out2.shape[2] * out2.shape[3] <= 1:
+        raise ValueError(f"Expected more than 1 value per channel when training, got input size "
+                         f"{(out2.shape[0], conv_weight.shape[0]) + tuple(out2.shape[2:])}")
+    return _SeamConv3TailBNFn.apply(out2, identity, conv_weight, weight, bias, running_mean, running_var, num_batches_tracked,
+                                    None if momentum is None else float(momentum), float(eps), process_group)
+
+
 # --------------------------------------------------------------------------------------------
 # materialising align-corners bilinear upsample (API-compat path)
 # --------------------------------------------------------------------------------------------

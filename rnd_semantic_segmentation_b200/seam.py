@@ -42,8 +42,16 @@ channels_last features, so conv3's fp32 output is neither written nor read back.
 each rounded to bf16 once and accumulated in fp32 (the head's standing choice), the tail is applied to the fp32 accumulator in the
 fold's order and rounded once to bf16; the features are therefore NOT bit-identical to the stock block's, unlike the fold path.
 The backward computes conv3's data gradient from bf16(scale * weight) and its weight gradient from bf16(out2), with fp32
-accumulation.  Every other case (including a training-mode 'batch' bn3, whose statistics need conv3's output) takes the
-path above with a stock conv3.
+accumulation.  Every other case (a training-mode 'batch' bn3 included: see below) takes the path above with a stock conv3.
+
+conv3 under batch statistics (opt-in: ``fuse_backbone_tail(fe, train_bn=True, conv3_batch=True)`` / ``install(seam=True,
+seam_train_bn=True, seam_conv3_batch=True)``): when bn3 takes the batch-statistics path above and conv3 is eligible as for
+``conv3=True``, conv2's output and the identity are fp32 of the expected shape and there is more than one value per channel, the
+block runs ops.seam_conv3_tail_bn: conv3 as a tcgen05 GEMM that writes its fp32 NCHW output c once and computes the per-rank
+statistics from its accumulator (no pass reads c back for them), then the batch tail above, unchanged.  Numerics: conv2's output
+and conv3's weight are each rounded to bf16 once with fp32 accumulation; the statistics are those of the stored c; in the
+backward, the gradient into c is rounded once to bf16 before conv3's data and weight gradient GEMMs.  ``conv3=True`` keeps its
+meaning (the fold only); everything else keeps the batch path with a stock conv3.
 """
 from __future__ import annotations
 
@@ -67,15 +75,18 @@ class _FusedForward:
     """What ``fuse_backbone_tail`` installs as the block's instance ``forward``: a plain picklable object (``torch.save`` of a
     whole fused extractor loads again; ``copy.deepcopy`` re-targets it to the copy).  It keeps the forward that was in the
     instance's __dict__ before (normally none) and the key (norm class, eps, data pointers and version counters of the norm's
-    tensors) under which the fold last passed or failed its probe, and ``train_bn`` / ``conv3`` (fuse_backbone_tail's flags)."""
+    tensors) under which the fold last passed or failed its probe, and ``train_bn`` / ``conv3`` / ``conv3_batch``
+    (fuse_backbone_tail's flags)."""
     train_bn = False                    # (objects pickled before a flag existed load with the default)
     conv3 = False
+    conv3_batch = False
 
-    def __init__(self, block, had_forward, old_forward, train_bn=False, conv3=False):
+    def __init__(self, block, had_forward, old_forward, train_bn=False, conv3=False, conv3_batch=False):
         self.block, self.had_forward, self.old_forward = block, had_forward, old_forward
         self.key, self.ok, self.warned = None, False, False
         self.train_bn = bool(train_bn)
         self.conv3 = bool(conv3)
+        self.conv3_batch = bool(conv3_batch)
 
     def __getstate__(self):
         state = dict(self.__dict__)
@@ -229,6 +240,16 @@ def _fused_forward(block, state, x):
         if identity.dtype == torch.float32 and tuple(identity.shape) == (out.shape[0], block.conv3.out_channels) + tuple(out.shape[2:]):
             return ops.seam_conv3_tail(out, identity, block.conv3.weight, fold[0], fold[1])
         c = block.conv3(out)
+    elif batch is not None and state.conv3_batch and out.dtype == torch.float32 and _conv3_fusable(block.conv3, x):
+        if block.downsample is not None:
+            identity = block.downsample(x)
+        shape = (out.shape[0], block.conv3.out_channels) + tuple(out.shape[2:])
+        single = batch[0] is None and out.shape[0] * out.shape[2] * out.shape[3] <= 1
+        if identity.dtype == torch.float32 and tuple(identity.shape) == shape and not single:
+            norm = block.bn3
+            return ops.seam_conv3_tail_bn(out, identity, block.conv3.weight, norm.weight, norm.bias, norm.running_mean,
+                                          norm.running_var, norm.num_batches_tracked, norm.momentum, norm.eps, batch[0])
+        c = block.conv3(out)
     else:
         c = block.conv3(out)
         if block.downsample is not None:
@@ -252,11 +273,13 @@ def _installed(block):
     return fwd if isinstance(fwd, _FusedForward) else None
 
 
-def fuse_backbone_tail(feature_extractor: nn.Module, train_bn: bool = False, conv3: bool = False) -> nn.Module:
+def fuse_backbone_tail(feature_extractor: nn.Module, train_bn: bool = False, conv3: bool = False,
+                       conv3_batch: bool = False) -> nn.Module:
     """Make the last Bottleneck of ``feature_extractor`` emit bf16 channels_last features (see the module docstring).  Returns
     ``feature_extractor``; a second call only sets ``train_bn`` (a training-mode BatchNorm2d / SyncBatchNorm bn3 takes the
-    batch-statistics kernels) and ``conv3`` (an eligible conv3 runs inside the fused GEMM, with bf16 operands: see the module
-    docstring for what that changes numerically).  Raises ValueError when no Bottleneck-shaped module is found.
+    batch-statistics kernels), ``conv3`` (an eligible conv3 runs inside the fused GEMM, with bf16 operands: see the module
+    docstring for what that changes numerically) and ``conv3_batch`` (with ``train_bn``: an eligible conv3 of a batch-statistics
+    bn3 runs as a tcgen05 GEMM that writes its output and statistics, also with bf16 operands).  Raises ValueError when no Bottleneck-shaped module is found.
     The hook lives in the block's instance __dict__: ``nn.DataParallel`` replicas (which copy that dict) would run it on the
     original block, so use one process per GPU (DistributedDataParallel), as the reference's trainers do."""
     block = _last_bottleneck(feature_extractor)
@@ -265,10 +288,11 @@ def fuse_backbone_tail(feature_extractor: nn.Module, train_bn: bool = False, con
     state = _installed(block)
     if state is None:
         had = "forward" in block.__dict__
-        block.__dict__["forward"] = _FusedForward(block, had, block.__dict__.get("forward"), train_bn, conv3)
+        block.__dict__["forward"] = _FusedForward(block, had, block.__dict__.get("forward"), train_bn, conv3, conv3_batch)
     else:
         state.train_bn = bool(train_bn)
         state.conv3 = bool(conv3)
+        state.conv3_batch = bool(conv3_batch)
     return feature_extractor
 
 
@@ -290,12 +314,14 @@ def is_fused(feature_extractor: nn.Module) -> bool:
     return block is not None and _installed(block) is not None
 
 
-def wrap_feature_extractor_factory(stock, train_bn: bool = False, conv3: bool = False):
-    """``build_feature_extractor`` with the same signature whose result goes through ``fuse_backbone_tail(fe, train_bn, conv3)``
-    (install(seam=True, seam_train_bn=..., seam_conv3=...)).  Wrapping a wrapper returns it with its flags set to the new values."""
+def wrap_feature_extractor_factory(stock, train_bn: bool = False, conv3: bool = False, conv3_batch: bool = False):
+    """``build_feature_extractor`` with the same signature whose result goes through ``fuse_backbone_tail(fe, train_bn, conv3,
+    conv3_batch)`` (install(seam=True, seam_train_bn=..., seam_conv3=..., seam_conv3_batch=...)).  Wrapping a wrapper returns it
+    with its flags set to the new values."""
     if getattr(stock, "_b200seg_seam", False):
         stock._b200seg_seam_train_bn = bool(train_bn)
         stock._b200seg_seam_conv3 = bool(conv3)
+        stock._b200seg_seam_conv3_batch = bool(conv3_batch)
         return stock
 
     @functools.wraps(stock)
@@ -303,10 +329,12 @@ def wrap_feature_extractor_factory(stock, train_bn: bool = False, conv3: bool = 
         fe = stock(*args, **kwargs)
         if isinstance(fe, nn.Module) and _last_bottleneck(fe) is not None:       # (a VGG backbone stays as built)
             fuse_backbone_tail(fe, train_bn=build_feature_extractor._b200seg_seam_train_bn,
-                               conv3=build_feature_extractor._b200seg_seam_conv3)
+                               conv3=build_feature_extractor._b200seg_seam_conv3,
+                               conv3_batch=build_feature_extractor._b200seg_seam_conv3_batch)
         return fe
 
     build_feature_extractor._b200seg_seam = True
     build_feature_extractor._b200seg_seam_train_bn = bool(train_bn)
     build_feature_extractor._b200seg_seam_conv3 = bool(conv3)
+    build_feature_extractor._b200seg_seam_conv3_batch = bool(conv3_batch)
     return build_feature_extractor
