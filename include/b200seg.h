@@ -493,6 +493,31 @@ B200SEG_API int b200seg_profile_read(int tag, double* total_ms, int* count);
  *        (it named 2 x 2 clusters, which were removed), 4 = CTA pair on one tcgen05.mma.cta_group::2 (M = 256). */
 B200SEG_API int b200seg_gemm_selftest(int M, int N, int K, int a_mn_major, int b_mn_major, int splits, int col_hw, int share,
                           double* max_err, double* max_ref);
+/* The tcgen05 GEMM's production launch path on caller-provided device buffers (tests, A/B experiments): D = A B^T with
+ * A [M][K] and B [N][K] bf16, each K-major (pitch = elements between rows) or MN-major ([K][rows], pitch = elements between
+ * k-rows); pointers 16-byte aligned, pitches multiples of 8.  No allocation, no synchronisation.  layout:
+ *   0 F32                  fp32 D[m, n] at out[z * split_stride + m * row_stride + n]            (z = split-K slab)
+ *   1 F32_NCHW_COLS        fp32 D[m, n] at out[z * split_stride + (n / hw) * img_stride + m * row_stride + n % hw]
+ *   2 F32_NCHW_ROWS        fp32 D[m, n] at out[(m / hw) * img_stride + n * hw + m % hw]; no split-K, M % hw == 0 or M <= hw
+ *   3 BF16                 bf16 D[m, n] at out[z * split_stride + m * row_stride + n]; N, row_stride, split_stride multiples of 8
+ *   4 SEAM                 bf16 out[m * N + n] = bf16_rn(relu((D * scale[n] + bias[n]) + identity[(m / hw) * N * hw + n * hw + m % hw]))
+ *                          (fp32 identity / scale / bias); K-major operands, no split-K, N % 8 == 0
+ *   5 F32_NCHW_ROWS_STATS  layout 2, and float2 stats[(m / 32) * N + n] = (mean, M2) of each 32-row group's stored values;
+ *                          K-major operands, no split-K, stats 8-byte aligned
+ * share: the geometry the caller asks for (0 one CTA per tile, 1 2-CTA pairs sharing B, 2 sharing A, 4 cta_group::2 pairs),
+ * vetoed or overridden by b200seg_gemm_set_sharing() exactly as for the head; pair_fallback: what 4 becomes under sharing mode 5;
+ * sm_reserve: SMs left out of the persistent grid.  *splits_used_host gets the split count after clamping (every split non-empty),
+ * *variant_host the index of the kernel launched (-1 when the arguments are rejected, B200SEG_ERR_ARG). */
+B200SEG_API int b200seg_gemm_run(const void* a, int a_mn_major, long long a_pitch, const void* b, int b_mn_major, long long b_pitch,
+                                 int M, int N, int K, int layout, void* out, long long row_stride, long long img_stride,
+                                 long long split_stride, int hw, const float* identity, const float* scale, const float* bias,
+                                 void* stats, int splits, int share, int pair_fallback, int sm_reserve, int* splits_used_host,
+                                 int* variant_host, void* stream);
+/* the table of GEMM kernels b200seg_gemm_run() / the head choose from: its size, and entry i's template arguments (host
+ * pointers; share as above, bn = accumulator columns per tile, rs = register-store epilogue, seam / stats = layouts 4 / 5) */
+B200SEG_API int b200seg_gemm_variant_count(void);
+B200SEG_API int b200seg_gemm_variant_info(int i, int* a_mn_major, int* b_mn_major, int* share, int* bn, int* rs, int* seam,
+                                          int* stats);
 /* head forward GEMM: 1 (default) = the tile width (256 / 224 / 192 accumulator columns) is chosen per problem so that the tile
  * count is a near-multiple of the SM count (wave quantisation), 0 = always 256 */
 B200SEG_API void b200seg_gemm_set_narrow_tiles(int on);

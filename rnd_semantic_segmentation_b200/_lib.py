@@ -129,6 +129,10 @@ SIGNATURES = {
     "b200seg_profile_enable": (None, [c_int]),
     "b200seg_profile_read": (c_int, [c_int, ctypes.POINTER(ctypes.c_double), ctypes.POINTER(c_int)]),
     "b200seg_gemm_selftest": (c_int, [c_int] * 8 + [ctypes.POINTER(ctypes.c_double), ctypes.POINTER(ctypes.c_double)]),
+    "b200seg_gemm_run": (c_int, [c_vp, c_int, c_i64, c_vp, c_int, c_i64, c_int, c_int, c_int, c_int, c_vp, c_i64, c_i64, c_i64, c_int,
+                                 c_vp, c_vp, c_vp, c_vp, c_int, c_int, c_int, c_int, ctypes.POINTER(c_int), ctypes.POINTER(c_int), c_vp]),
+    "b200seg_gemm_variant_count": (c_int, []),
+    "b200seg_gemm_variant_info": (c_int, [c_int] + [ctypes.POINTER(c_int)] * 7),
     "b200seg_gemm_set_sharing": (None, [c_int]),
     "b200seg_conv_set_pair": (None, [c_int]),
     "b200seg_gemm_set_narrow_tiles": (None, [c_int]),
@@ -1559,6 +1563,47 @@ def gemm_selftest(M, N, K, a_mn=False, b_mn=False, splits=1, col_hw=0, share=0):
     err, ref = ctypes.c_double(0), ctypes.c_double(0)
     _check(lib.b200seg_gemm_selftest(M, N, K, int(a_mn), int(b_mn), splits, col_hw, int(share), ctypes.byref(err), ctypes.byref(ref)))
     return err.value, ref.value
+
+
+GEMM_LAYOUTS = {"f32": 0, "f32_nchw_cols": 1, "f32_nchw_rows": 2, "bf16": 3, "seam": 4, "f32_nchw_rows_stats": 5}
+GEMM_SHARE = {"none": 0, "b": 1, "a": 2, "pair": 4}
+
+
+def gemm_run(a, b, M, N, K, layout, out, *, a_mn=False, a_pitch=None, b_mn=False, b_pitch=None, row_stride=0, img_stride=0,
+             split_stride=0, hw=0, identity=None, scale=None, bias=None, stats=None, splits=1, share=0, pair_fallback=1,
+             sm_reserve=0, check=True):
+    """The tcgen05 GEMM's production launch path (gemm::launch) on the current stream: D = A B^T written into ``out`` as ``layout``
+    (a key of GEMM_LAYOUTS or its value) says.  ``a`` / ``b`` / ``out`` / ``identity`` / ``scale`` / ``bias`` / ``stats`` are CUDA
+    tensors or views whose data_ptr() is the matrix origin; the pitches default to the operands' row strides.  Returns
+    (rc, splits_used, variant index); with check=True a non-zero rc raises."""
+    for name, t in (("a", a), ("b", b)):
+        if t.dtype != torch.bfloat16 or not t.is_cuda:
+            raise B200SegError(f"gemm_run: {name} must be a bf16 CUDA tensor")
+    for name, t in (("identity", identity), ("scale", scale), ("bias", bias)):
+        if t is not None and (t.dtype != torch.float32 or not t.is_cuda):
+            raise B200SegError(f"gemm_run: {name} must be an fp32 CUDA tensor")
+    lay = GEMM_LAYOUTS[layout] if isinstance(layout, str) else int(layout)
+    used, var = c_int(0), c_int(-1)
+    with _on_device(out.device):
+        rc = load().b200seg_gemm_run(
+            a.data_ptr(), int(a_mn), int(a.stride(0) if a_pitch is None else a_pitch), b.data_ptr(), int(b_mn),
+            int(b.stride(0) if b_pitch is None else b_pitch), M, N, K, lay, out.data_ptr(), row_stride, img_stride, split_stride, hw,
+            _ptr(identity), _ptr(scale), _ptr(bias), _ptr(stats), splits, int(share), int(pair_fallback), sm_reserve,
+            ctypes.byref(used), ctypes.byref(var), _stream(out.device))
+    if check:
+        _check(rc)
+    return rc, used.value, var.value
+
+
+def gemm_variants():
+    """The table of GEMM kernels launch() chooses from: one dict of template arguments per entry, in index order."""
+    lib = load()
+    rows = []
+    for i in range(lib.b200seg_gemm_variant_count()):
+        f = [c_int(0) for _ in range(7)]
+        _check(lib.b200seg_gemm_variant_info(i, *[ctypes.byref(x) for x in f]))
+        rows.append(dict(zip(("a_mn", "b_mn", "share", "bn", "rs", "seam", "stats"), (x.value for x in f))))
+    return rows
 
 
 def gemm_set_dgrad_mode(mode: int):

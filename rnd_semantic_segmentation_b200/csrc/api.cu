@@ -138,6 +138,10 @@ void set_dgrad_mode(int);
 void set_fwd_mode(int);
 void set_fwd_convert(int);
 int selftest_fwd_convert(int, int, int, int, int, double*, double*, double*);
+int run(const void*, int, long long, const void*, int, long long, int, int, int, int, void*, long long, long long, long long, int,
+        const float*, const float*, const float*, void*, int, int, int, int, int*, int*, cudaStream_t);
+int variant_count();
+int variant_info(int, int*, int*, int*, int*, int*, int*, int*);
 }
 
 static int require_device() {
@@ -735,6 +739,19 @@ int b200seg_gemm_selftest(int M, int N, int K, int a_mn_major, int b_mn_major, i
     return B200SEG_ERR_ARG;
   }
   return gemm::selftest(M, N, K, a_mn_major, b_mn_major, splits, col_hw, share, max_err, max_ref);
+}
+
+int b200seg_gemm_run(const void* a, int a_mn_major, long long a_pitch, const void* b, int b_mn_major, long long b_pitch, int M, int N,
+                     int K, int layout, void* out, long long row_stride, long long img_stride, long long split_stride, int hw,
+                     const float* identity, const float* scale, const float* bias, void* stats, int splits, int share,
+                     int pair_fallback, int sm_reserve, int* splits_used_host, int* variant_host, void* stream) {
+  REQUIRE_DEVICE();
+  return gemm::run(a, a_mn_major, a_pitch, b, b_mn_major, b_pitch, M, N, K, layout, out, row_stride, img_stride, split_stride, hw,
+                   identity, scale, bias, stats, splits, share, pair_fallback, sm_reserve, splits_used_host, variant_host, S(stream));
+}
+int b200seg_gemm_variant_count(void) { return gemm::variant_count(); }
+int b200seg_gemm_variant_info(int i, int* a_mn_major, int* b_mn_major, int* share, int* bn, int* rs, int* seam, int* stats) {
+  return gemm::variant_info(i, a_mn_major, b_mn_major, share, bn, rs, seam, stats);
 }
 
 }  // extern "C"

@@ -99,6 +99,20 @@ static Variant g_variants[] = {
     {false, false, SHARE_PAIR, 256, true, false, true, gemm_bf16_stats_kernel, false},
 };
 
+int variant_count() { return (int)(sizeof(g_variants) / sizeof(g_variants[0])); }
+int variant_info(int i, int* a_mn, int* b_mn, int* share, int* bn, int* rs, int* seam, int* stats) {
+  B200SEG_CHECK_ARG(i >= 0 && i < variant_count(), "gemm: variant %d out of range [0, %d)", i, variant_count());
+  const Variant& v = g_variants[i];
+  if (a_mn) *a_mn = v.a_mn;
+  if (b_mn) *b_mn = v.b_mn;
+  if (share) *share = v.share;
+  if (bn) *bn = v.bn;
+  if (rs) *rs = v.rs;
+  if (seam) *seam = v.seam;
+  if (stats) *stats = v.stats;
+  return B200SEG_OK;
+}
+
 static int check(const Gemm& g) {
   const Out& o = g.out;
   const bool aligned = (reinterpret_cast<uintptr_t>(o.ptr) & 15) == 0;
@@ -258,11 +272,41 @@ int launch(const Gemm& g, cudaStream_t stream) {
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = share == SHARE_NONE ? 0 : 1;
+  if (g.variant_used) *g.variant_used = (int)(v - g_variants);
   profile_begin(g.prof_tag, stream);
   B200SEG_CUDA(cudaLaunchKernelEx(&cfg, v->fn, ta, tb, to, p));
   B200SEG_LAUNCH_CHECK();
   profile_end(g.prof_tag, stream);
   return B200SEG_OK;
+}
+
+// b200seg_gemm_run(): launch() on caller-provided buffers, the Out built by the out_* function of `layout`
+int run(const void* a, int a_mn, long long a_pitch, const void* b, int b_mn, long long b_pitch, int M, int N, int K, int layout,
+        void* out, long long row_stride, long long img_stride, long long split_stride, int hw, const float* identity,
+        const float* scale, const float* bias, void* stats, int splits, int share, int pair_fallback, int sm_reserve,
+        int* splits_used, int* variant, cudaStream_t stream) {
+  if (variant) *variant = -1;
+  const auto geometry = [](int s) { return s == SHARE_NONE || s == SHARE_B || s == SHARE_A || s == SHARE_PAIR; };
+  B200SEG_CHECK_ARG(a && b && out && geometry(share) && geometry(pair_fallback),
+                    "gemm_run: null operand / output, or sharing geometry %d / fallback %d not one of 0, 1, 2, 4", share, pair_fallback);
+  Out o;
+  switch (layout) {
+    case Out::F32: o = out_f32((float*)out, row_stride, split_stride); break;
+    case Out::F32_NCHW_COLS: o = out_f32_nchw_cols((float*)out, hw, row_stride, img_stride, split_stride); break;
+    case Out::F32_NCHW_ROWS: o = out_f32_nchw_rows((float*)out, hw, img_stride); break;
+    case Out::BF16: o = out_bf16((__nv_bfloat16*)out, row_stride, split_stride); break;
+    case Out::SEAM: o = out_seam((__nv_bfloat16*)out, identity, scale, bias, hw); break;
+    case Out::F32_NCHW_ROWS_STATS: o = out_f32_nchw_rows_stats((float*)out, hw, img_stride, (float2*)stats); break;
+    default: set_error("gemm_run: unknown output layout %d", layout); return B200SEG_ERR_ARG;
+  }
+  Gemm g{{(const __nv_bfloat16*)a, a_mn != 0, a_pitch}, {(const __nv_bfloat16*)b, b_mn != 0, b_pitch}, M, N, K, o};
+  g.splits = splits;
+  g.splits_used = splits_used;
+  g.share = share;
+  g.pair_fallback = pair_fallback;
+  g.sm_reserve = sm_reserve;
+  g.variant_used = variant;
+  return launch(g, stream);
 }
 
 // ------------------------------------------------------------------------------------------

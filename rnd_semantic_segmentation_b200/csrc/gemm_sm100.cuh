@@ -1052,8 +1052,12 @@ struct Gemm {
   int pair_fallback = SHARE_B;   // what SHARE_PAIR becomes under sharing mode 5 (no cta_group::2)
   int sm_reserve = 0;            // SMs left free for a concurrent kernel
   int prof_tag = -1;
+  int* variant_used = nullptr;   // the index of the kernel launched, in the table variant_info() reads
 };
 int launch(const Gemm& g, cudaStream_t stream);
+// the kernels launch() chooses from: their count, and entry i's template arguments (B200SEG_ERR_ARG for i out of range)
+int variant_count();
+int variant_info(int i, int* a_mn, int* b_mn, int* share, int* bn, int* rs, int* seam, int* stats);
 // fp32 NCHW data gradient of the head: 0 = channels along M (shared-memory transpose epilogue), 1 = pixels along M as cta_group::2
 // pairs, stores straight from registers, seven ring stages
 void set_dgrad_mode(int mode);
