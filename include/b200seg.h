@@ -126,7 +126,7 @@ B200SEG_API int b200seg_soft_ce_forward(const float* pred, const float* soft, co
                             void* workspace, int64_t workspace_bytes, float* loss_out, void* stream);
 B200SEG_API int b200seg_soft_ce_backward(const float* pred, const float* soft, const float* weights, const float* grad_out, int N,
                              int K, int H, int W, float* grad_pred, void* stream);
-/* Same loss, with the forward saving per-pixel statistics {log-sum-exp, sum_k q_k} (two f32 planes [N*H*W], needs
+/* Same loss, with the forward saving per-pixel statistics {max_k p_k, sum_k q_k / sum_k exp(p_k - max)} (two f32 planes [N*H*W], needs
  * H*W % 4 == 0 and 16-byte aligned tensors) so that the backward is ONE 128-bit-vectorised streaming pass
  * (12*K + 8 bytes per pixel) instead of recomputing the softmax normaliser from a second read. */
 B200SEG_API int64_t b200seg_soft_ce_stats_bytes(int N, int H, int W);

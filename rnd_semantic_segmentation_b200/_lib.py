@@ -568,8 +568,8 @@ def upsample_bilinear_backward(grad_out: torch.Tensor, in_hw) -> torch.Tensor:
 # K3
 # --------------------------------------------------------------------------------------------
 def soft_ce_forward(pred, soft, weights=None, want_stats: bool = False):
-    """loss (0-d); with ``want_stats`` also the per-pixel {lse, sum q} planes for soft_ce_backward (None when the shapes do
-    not allow the vectorised path)."""
+    """loss (0-d); with ``want_stats`` also the per-pixel {max p, sum q / sum exp(p - max)} planes for soft_ce_backward (None
+    when the shapes do not allow the vectorised path)."""
     lib = load()
     _need(pred, torch.float32, "pred")
     _need(soft, torch.float32, "soft_label")

@@ -490,7 +490,7 @@ __global__ void __launch_bounds__(256) k2_finalize_loss(const float* loss_part, 
   }
 }
 
-// grad[n,c,i,j] = grad_out * inv_T / n_valid * sum over the tiles touching (i,j) of their partial block.
+// grad[n,c,i,j] = grad_out * inv_T / n_valid * sum over the tiles touching (i,j) of their partial block (0 when n_valid = 0).
 // PACKED = false: fp32 NCHW grad_logits (the autograd contract of the stand-alone loss op).
 // PACKED = true : bf16 class planes gOc[n][c][hw] (what the head's backward consumes) + per-block fp32 partial sums
 //                 of the gradient per class (-> bias gradient), skipping the NCHW round trip.
@@ -504,7 +504,8 @@ __global__ void __launch_bounds__(128) k2_finalize_grad(const K2Geom g, const fl
   const int n = blockIdx.z;
   const bool active = j < g.w;
   const float n_valid = loss_out2[1];
-  const float scale = (grad_out ? grad_out[0] : 1.f) * inv_T / n_valid;
+  // no valid label: every accumulator is 0 and so is the gradient (as in ATen); 1 / n_valid would make it 0 * inf = NaN
+  const float scale = n_valid > 0.f ? (grad_out ? grad_out[0] : 1.f) * inv_T / n_valid : 0.f;
   float acc[32];
 #pragma unroll
   for (int c = 0; c < 32; ++c) acc[c] = 0.f;

@@ -3,6 +3,9 @@
 // Replaces (reference file:line):
 //   soft_label_cross_entropy(pred, soft_label, pixel_weights=None)   core/utils/utility.py:172-177
 //     loss = mean_{N,H,W}( [w *] sum_c( -q_c * log_softmax(p)_c ) )
+//          per pixel as  log(s) * sum_k q_k - sum_k q_k * (p_k - r),  s = sum_k exp(p_k - m),  with m the pixel's maximum and r
+//          one of its own logits (m, or the first class on the online path): every term is a difference of logits, so a logit
+//          offset common to all classes (which cancels in the loss) costs no precision
 //     d loss / d p_c = ( softmax(p)_c * sum_k q_k - q_c ) * w / (N*H*W)
 //   callers: core/combos/aspp_fada.py:111,120,124 on [N, 2C, H, W] fp32 operands.
 //
@@ -33,17 +36,17 @@ __global__ void __launch_bounds__(K3_THREADS) k3_softce_fwd(const float* __restr
 #pragma unroll
     for (int k = 0; k < KT; ++k)
       if (k < K) m = fmaxf(m, p[k]);
-    float s = 0.f, sq = 0.f, sqp = 0.f;
-    const float mneg = -m * 1.4426950408889634f;
+    float s = 0.f, sq = 0.f, sqd = 0.f;
 #pragma unroll
     for (int k = 0; k < KT; ++k)
       if (k < K) {
         const float q = __ldcs(soft + base + k * HW);
-        s += fast_exp2(fmaf(p[k], 1.4426950408889634f, mneg));
+        const float d = p[k] - m;
+        s += fast_exp2(d * 1.4426950408889634f);
         sq += q;
-        sqp = fmaf(q, p[k], sqp);
+        sqd = fmaf(q, d, sqd);
       }
-    float l = (m + __logf(s)) * sq - sqp;
+    float l = __logf(s) * sq - sqd;
     if (wts) l *= __ldcs(wts + i);
     acc += l;
   }
@@ -93,11 +96,10 @@ __global__ void __launch_bounds__(K3_THREADS) k3_softce_bwd(const float* __restr
     for (int k = 0; k < KT; ++k)
       if (k < K) { m = fmaxf(m, p[k]); sq += q[k]; }
     float s = 0.f;
-    const float mneg = -m * 1.4426950408889634f;
 #pragma unroll
     for (int k = 0; k < KT; ++k)
       if (k < K) {
-        p[k] = fast_exp2(fmaf(p[k], 1.4426950408889634f, mneg));
+        p[k] = fast_exp2((p[k] - m) * 1.4426950408889634f);
         s += p[k];
       }
     const float wgt = (wts ? __ldcs(wts + i) : 1.f) * go;
@@ -110,7 +112,8 @@ __global__ void __launch_bounds__(K3_THREADS) k3_softce_bwd(const float* __restr
 
 // ---- 128-bit vectorised variants: one thread per 4 consecutive pixels (HW % 4 == 0, 16-byte aligned tensors) --------
 // forward: online softmax over chunks of K3_CH class planes (2 * K3_CH independent 16-byte loads in flight per thread),
-// optionally saving {lse, sum_k q_k} per pixel so that the backward is ONE streaming pass with no register arrays.
+// optionally saving {m, sum_k q_k / s} per pixel (the maximum and the softmax scale of the soft-label mass) so that the backward
+// is ONE streaming pass with no register arrays.
 #ifndef K3_CH_DEF
 #define K3_CH_DEF 4
 #endif
@@ -133,7 +136,8 @@ __global__ void __launch_bounds__(K3_THREADS, K3_MINB) k3_softce_fwd_v4(const fl
     const float* pp = pred + n * K * HW + (i - n * HW);
     const float* qp = soft + n * K * HW + (i - n * HW);
     float m[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
-    float sden[4] = {0.f, 0.f, 0.f, 0.f}, sq[4] = {0.f, 0.f, 0.f, 0.f}, sqp[4] = {0.f, 0.f, 0.f, 0.f};
+    float sden[4] = {0.f, 0.f, 0.f, 0.f}, sq[4] = {0.f, 0.f, 0.f, 0.f}, sqd[4] = {0.f, 0.f, 0.f, 0.f};
+    float r[4];                                      // reference logit of sqd = sum q * (p - r): the pixel's first class
     auto load_chunk = [&](float4 (&P)[K3_CH], float4 (&Q)[K3_CH], int k0) {
 #pragma unroll
       for (int k = 0; k < K3_CH; ++k) {
@@ -153,14 +157,14 @@ __global__ void __launch_bounds__(K3_THREADS, K3_MINB) k3_softce_fwd_v4(const fl
 #pragma unroll
         for (int k = 0; k < K3_CH; ++k) cm = fmaxf(cm, (&P[k].x)[e]);
         const float mn = fmaxf(m[e], cm);
-        const float mneg = -mn * K3_L2E;
-        float sd = sden[e] * fast_exp2(fmaf(m[e], K3_L2E, mneg));         // m = -inf on the first chunk -> ex2(-inf) = 0
+        float sd = sden[e] * fast_exp2((m[e] - mn) * K3_L2E);             // m = -inf on the first chunk -> ex2(-inf) = 0
+        if (k0 == 0) r[e] = (&P[0].x)[e];
 #pragma unroll
         for (int k = 0; k < K3_CH; ++k) {
           const float pv = (&P[k].x)[e], qv = (&Q[k].x)[e];
-          sd += fast_exp2(fmaf(pv, K3_L2E, mneg));                          // padding planes: ex2(-inf) = 0
+          sd += fast_exp2((pv - mn) * K3_L2E);                             // padding planes: ex2(-inf) = 0
           sq[e] += qv;
-          sqp[e] = fmaf(qv, (k0 + k < K) ? pv : 0.f, sqp[e]);
+          sqd[e] = fmaf(qv, (k0 + k < K) ? pv - r[e] : 0.f, sqd[e]);
         }
         sden[e] = sd;
         m[e] = mn;
@@ -175,16 +179,17 @@ __global__ void __launch_bounds__(K3_THREADS, K3_MINB) k3_softce_fwd_v4(const fl
       if (k0 + 2 * K3_CH < K) load_chunk(PA, QA, k0 + 2 * K3_CH);
       if (k0 + K3_CH < K) fold_chunk(PB, QB, k0 + K3_CH);
     }
-    float lse[4];
+    float l[4];                                      // lse - r = (m - r) + log(s)
 #pragma unroll
-    for (int e = 0; e < 4; ++e) lse[e] = fmaf(__log2f(sden[e]), K3_LN2, m[e]);
+    for (int e = 0; e < 4; ++e) l[e] = (m[e] - r[e]) + __log2f(sden[e]) * K3_LN2;
     float4 wv = make_float4(1.f, 1.f, 1.f, 1.f);
     if (wts) wv = ld_stream_f4(wts + i);
-    acc += (lse[0] * sq[0] - sqp[0]) * wv.x + (lse[1] * sq[1] - sqp[1]) * wv.y + (lse[2] * sq[2] - sqp[2]) * wv.z +
-           (lse[3] * sq[3] - sqp[3]) * wv.w;
+    acc += (l[0] * sq[0] - sqd[0]) * wv.x + (l[1] * sq[1] - sqd[1]) * wv.y + (l[2] * sq[2] - sqd[2]) * wv.z +
+           (l[3] * sq[3] - sqd[3]) * wv.w;
     if (stats) {
-      st_stream_f4(stats + i, make_float4(lse[0], lse[1], lse[2], lse[3]));
-      st_stream_f4(stats + total_px + i, make_float4(sq[0], sq[1], sq[2], sq[3]));
+      st_stream_f4(stats + i, make_float4(m[0], m[1], m[2], m[3]));
+      st_stream_f4(stats + total_px + i, make_float4(__fdividef(sq[0], sden[0]), __fdividef(sq[1], sden[1]),
+                                                     __fdividef(sq[2], sden[2]), __fdividef(sq[3], sden[3])));
     }
   }
   acc = warp_sum(acc);
@@ -198,7 +203,7 @@ __global__ void __launch_bounds__(K3_THREADS, K3_MINB) k3_softce_fwd_v4(const fl
   }
 }
 
-// backward from the saved per-pixel {lse, sum q}: grad_k = w * go / (NHW) * (exp(p_k - lse) * sum_q - q_k), one streaming pass
+// backward from the saved per-pixel {m, sum q / s}: grad_k = w * go / (NHW) * (exp(p_k - m) * sum_q / s - q_k), one streaming pass
 __global__ void __launch_bounds__(K3_THREADS, K3_MINB) k3_softce_bwd_stats_v4(const float* __restrict__ pred, const float* __restrict__ soft,
                                                                      const float* __restrict__ wts, const float* __restrict__ stats,
                                                                      const float* __restrict__ grad_out, int K, long long HW,
@@ -209,11 +214,10 @@ __global__ void __launch_bounds__(K3_THREADS, K3_MINB) k3_softce_bwd_stats_v4(co
     const long long i = qi << 2;
     const long long n = i / HW;
     const long long base = n * K * HW + (i - n * HW);
-    const float4 lse = ld_stream_f4(stats + i), sq = ld_stream_f4(stats + total_px + i);
+    const float4 m = ld_stream_f4(stats + i), sqs = ld_stream_f4(stats + total_px + i);
     float4 a = make_float4(go, go, go, go);
     if (wts) { const float4 wv = ld_stream_f4(wts + i); a = make_float4(go * wv.x, go * wv.y, go * wv.z, go * wv.w); }
-    const float4 as = make_float4(a.x * sq.x, a.y * sq.y, a.z * sq.z, a.w * sq.w);
-    const float4 ln = make_float4(-lse.x * K3_L2E, -lse.y * K3_L2E, -lse.z * K3_L2E, -lse.w * K3_L2E);
+    const float4 as = make_float4(a.x * sqs.x, a.y * sqs.y, a.z * sqs.z, a.w * sqs.w);
     for (int k0 = 0; k0 < K; k0 += K3_CH) {
       float4 P[K3_CH], Q[K3_CH];
 #pragma unroll
@@ -226,10 +230,10 @@ __global__ void __launch_bounds__(K3_THREADS, K3_MINB) k3_softce_bwd_stats_v4(co
       for (int k = 0; k < K3_CH; ++k)
         if (k0 + k < K) {
           float4 gv;
-          gv.x = fmaf(as.x, fast_exp2(fmaf(P[k].x, K3_L2E, ln.x)), -a.x * Q[k].x);
-          gv.y = fmaf(as.y, fast_exp2(fmaf(P[k].y, K3_L2E, ln.y)), -a.y * Q[k].y);
-          gv.z = fmaf(as.z, fast_exp2(fmaf(P[k].z, K3_L2E, ln.z)), -a.z * Q[k].z);
-          gv.w = fmaf(as.w, fast_exp2(fmaf(P[k].w, K3_L2E, ln.w)), -a.w * Q[k].w);
+          gv.x = fmaf(as.x, fast_exp2((P[k].x - m.x) * K3_L2E), -a.x * Q[k].x);
+          gv.y = fmaf(as.y, fast_exp2((P[k].y - m.y) * K3_L2E), -a.y * Q[k].y);
+          gv.z = fmaf(as.z, fast_exp2((P[k].z - m.z) * K3_L2E), -a.z * Q[k].z);
+          gv.w = fmaf(as.w, fast_exp2((P[k].w - m.w) * K3_L2E), -a.w * Q[k].w);
           st_stream_f4(grad + base + (long long)(k0 + k) * HW, gv);
         }
     }

@@ -481,7 +481,10 @@ class _UpsampleCEFn(torch.autograd.Function):
 def upsample_cross_entropy(logits_lr: torch.Tensor, labels: torch.Tensor, ignore_index: int = 255,
                            temperature: float = 1.0) -> torch.Tensor:
     """CrossEntropyLoss(ignore_index)(interpolate(logits_lr, labels.shape[-2:]) / temperature, labels) without
-    materialising the full-resolution logits (aspp_trainer.py:88-92, aspp_fada.py:91-96)."""
+    materialising the full-resolution logits (aspp_trainer.py:88-92, aspp_fada.py:91-96).
+    ``labels``: int64 or uint8 [N, H, W].  A label outside [0, C) -- negative or >= C -- counts like ``ignore_index``: it adds
+    nothing to the loss sum or to the number of valid pixels the mean divides by, in every kernel and for both label widths
+    (PyTorch raises on such a label instead).  With no valid pixel the loss is NaN and the gradient is zero, as in PyTorch."""
     labels = _lib.as_label_tensor(labels)
     return _UpsampleCEFn.apply(logits_lr, labels, int(ignore_index), float(temperature))
 
