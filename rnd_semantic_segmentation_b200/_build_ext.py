@@ -21,9 +21,12 @@ OBJ_DIR = os.path.join(PKG_DIR, "_obj")
 SOURCES = ["api.cu", "eval_kernels.cu", "ce_kernels.cu", "ce_v2_kernels.cu", "softce_kernels.cu",
            "gemm_sm100.cu", "aspp_head.cu", "conv_sm100.cu", "tta_kernels.cu", "optim_kernels.cu", "p2p_allreduce.cu",
            "seam_tail_kernels.cu", "seam_conv3.cu"]
-HEADERS = ["common.cuh", "ce_geom.cuh", "gemm_sm100.cuh", os.path.join(ROOT, "include", "b200seg.h")]
+HEADERS = ["common.cuh", "ce_geom.cuh", "gemm_sm100.cuh", "host_api.h", os.path.join(ROOT, "include", "b200seg.h")]
+# -Werror=missing-declarations: every non-static host function is defined after a declaration (host_api.h for those shared
+# between files), so a definition whose parameters drift from its declaration fails to compile instead of becoming an overload
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
-              "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "--expt-relaxed-constexpr"]
+              "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "-Xcompiler", "-Werror=missing-declarations",
+              "--expt-relaxed-constexpr"]
 
 
 def _nvcc() -> str:
@@ -75,8 +78,9 @@ def build(force: bool = False, verbose: bool = False) -> str:
 
     with ThreadPoolExecutor(max_workers=min(8, len(srcs))) as ex:
         objs = list(ex.map(compile_one, srcs))
+    # --no-undefined: a declared function nothing defines fails here, not when the library is loaded
     link = [nvcc, "-shared", "-o", LIB_PATH] + objs + ["-gencode", "arch=compute_100a,code=sm_100a",
-                                                       "-cudart", "static", "-Xcompiler", "-fPIC"]
+                                                       "-cudart", "static", "-Xcompiler", "-fPIC", "-Xlinker", "--no-undefined"]
     r = subprocess.run(link, capture_output=True, text=True)
     if r.returncode != 0:
         raise RuntimeError(f"link failed:\n{r.stdout}\n{r.stderr}")

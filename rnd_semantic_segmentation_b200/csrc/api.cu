@@ -4,6 +4,7 @@
 #include <string.h>
 #include "../../include/b200seg.h"
 #include "common.cuh"
+#include "host_api.h"
 
 namespace b200seg {
 
@@ -47,101 +48,6 @@ int num_sms() {
       return 148;
   }
   return cached;
-}
-
-// kernels' host launchers (defined in the other translation units)
-int k4_launch(const float*, int, int, int, int, const void*, int, int, int, int, long long*, long long, void*, int, int, cudaStream_t);
-int k4_launch_frames(const float* const*, int, int, int, int, const void* const*, int, int, int, int, long long*, long long, void* const*,
-                     int, int, cudaStream_t);
-int confusion_pairs_launch_ex(void*, int, const void*, int, long long, int, int, int, long long*, cudaStream_t);
-long long k2_workspace_bytes(int, int, int, int, int, int);
-int k2_forward(const float*, int, int, int, int, const void*, int, int, int, int, float, int, void*, long long, float*, cudaStream_t,
-               float* loss_copy = nullptr);
-int k2_backward_packed_multi(void*, int, int, int, int, int, int, float, const float*, const float*, void*, float* const*, int, cudaStream_t);
-void* aspp_bwd_gOt_ptr(void*);
-int k2_backward(const void*, int, int, int, int, int, int, float, const float*, const float*, float*, cudaStream_t);
-int k2_backward_packed(void*, int, int, int, int, int, int, float, const float*, const float*, void*, float*, cudaStream_t);
-int aspp_backward_packed(const void*, const void*, const void*, const int*, int, int, int, int, int, int, void*, long long, int, float*,
-                         float* const*, cudaStream_t, void*, cudaEvent_t);
-int upsample_fwd_launch(const float*, float*, int, int, int, int, int, int, cudaStream_t);
-int upsample_bwd_launch(const float*, float*, int, int, int, int, int, cudaStream_t);
-long long k3_workspace_bytes();
-long long k3_stats_bytes(int, int, int);
-int k3_forward(const float*, const float*, const float*, int, int, int, int, void*, long long, float*, cudaStream_t, float*);
-int k3_backward(const float*, const float*, const float*, const float*, int, int, int, int, float*, cudaStream_t, const float*);
-int aspp_nj(int, int);
-int aspp_pack_weights(const float* const*, const float* const*, int, int, int, void*, void*, float*, cudaStream_t);
-int aspp_pack_features(const float*, int, int, int, int, void*, cudaStream_t);
-long long aspp_yt_bytes(int, int, int, int, int);
-int aspp_forward(const void*, const void*, const float*, const int*, int, int, int, int, int, int, float*, float*, cudaStream_t);
-int aspp_forward_f32(const float*, const void*, const float*, const int*, int, int, int, int, int, int, float*, float*, void*, cudaStream_t);
-int aspp_forward_f32_supported(const float*, int, int, int, int, int);
-long long aspp_bwd_scratch_bytes(int, int, int, int, int, int, int);
-int aspp_backward(const float*, const void*, const void*, const int*, int, int, int, int, int, int, void*, long long, int, float*,
-                  float* const*, float* const*, cudaStream_t);
-long long k5_workspace_bytes(int, int, int, int, int, int);
-int k5_forward(const float*, const float*, int, int, int, int, int, int, float, float, int, int, void*, long long, float*, cudaStream_t);
-int k5_backward(const void*, int, int, int, int, int, int, const float*, const float*, float*, cudaStream_t);
-int conv3x3_pack_weights(const float* const*, const int*, int, int, void*, void*, int, cudaStream_t);
-int conv3x3_pack_weights_stack(int, const float* const*, const int*, const int*, const int*, void* const*, void* const*, const int*,
-                               const float* const*, const int*, int, float*, cudaStream_t);
-int conv3x3_forward(const void*, int, int, int, int, long long, const void*, int, int, const float*, int, float, void*, long long, float*,
-                    cudaStream_t);
-int conv3x3_dgrad(const void*, int, int, int, int, long long, const void*, int, int, const void*, float, void*, long long, float*,
-                  cudaStream_t, void*, long long, float*);
-long long conv3x3_dgrad_colsum_scratch_bytes(int, int, int, long long);
-long long conv3x3_wgrad_scratch_bytes(int, int, int, int, int, int);
-int conv3x3_wgrad(const void*, int, long long, const void*, int, long long, int, int, int, int, int, void*, long long, float* const*,
-                  const int*, int, cudaStream_t);
-int nchw_to_nhwc_bf16(const float*, int, int, int, void*, int, cudaStream_t);
-int seam_tail_forward(const float*, const float*, const float*, const float*, int, int, int, void*, cudaStream_t);
-int seam_tail_backward(const void*, const void*, const float*, int, int, int, float*, float*, cudaStream_t);
-long long seam_conv3_workspace_bytes(int, int, int, int);
-int seam_conv3_forward(const float*, const float*, const float*, const float*, const float*, int, int, int, int, void*, long long, void*,
-                       cudaStream_t);
-long long seam_conv3_backward_scratch_bytes(int, int, int, int);
-int seam_conv3_backward(const void*, const void*, const void*, const float*, int, int, int, int, void*, long long, float*, float*, float*,
-                        cudaStream_t);
-long long bn_stats_scratch_bytes(int, int);
-int bn_stats(const float*, int, int, int, void*, long long, double*, cudaStream_t);
-int bn_combine_stats(const double*, int, int, float, float, const long long*, float*, float*, float*, float*, double*, cudaStream_t);
-int seam_tail_bn_forward(const float*, const float*, const float*, const float*, const float*, const float*, int, int, int, void*,
-                         cudaStream_t);
-long long seam_tail_bn_backward_reduce_scratch_bytes(int, int, int);
-int seam_tail_bn_backward_reduce(const void*, const void*, const float*, const float*, const float*, int, int, int, void*, long long,
-                                 float*, float*, float*, cudaStream_t);
-int seam_tail_bn_backward(const void*, const void*, const float*, const float*, const float*, const float*, const float*, int,
-                          const double*, int, int, int, float*, float*, cudaStream_t);
-long long seam_conv3_bn_forward_scratch_bytes(int, int, int);
-long long seam_conv3_bn_backward_scratch_bytes(int, int, int, int);
-int seam_conv3_bn_forward(const float*, const float*, int, int, int, int, void*, long long, void*, long long, float*, double*, cudaStream_t);
-int seam_conv3_bn_backward(const void*, const void*, const float*, const float*, const float*, const float*, const float*, int,
-                           const double*, const void*, int, int, int, int, void*, long long, float*, float*, float*, cudaStream_t);
-long long nhwc_colsum_scratch_bytes(int);
-int nhwc_bf16_colsum(const void*, long long, int, int, void*, float*, cudaStream_t);
-int tta_launch(const float* const*, const int*, const int*, const int*, int, int, const void*, int, int, int, int, const float*, int, int,
-               long long*, void*, int, float*, cudaStream_t);
-void tta_set_row_walk(int);
-void k2_set_variant(int);
-int p2p_allreduce_mean(void* const*, void*, void* const*, int, int, long long, int, int, cudaStream_t);
-int sgd_step(int, float* const*, const float* const*, float* const*, const long long*, float, float, float, float, int, int, float,
-             cudaStream_t);
-int adam_step(int, float* const*, const float* const*, float* const*, float* const*, const long long*, float, float, float, float,
-              float, long long, float, cudaStream_t);
-namespace gemm { namespace conv { void set_pair(int); } }
-namespace gemm {
-int selftest(int, int, int, int, int, int, int, int, double*, double*);
-void set_sharing(int);
-void set_overlap_sms(int);
-void set_narrow_tiles(int);
-void set_dgrad_mode(int);
-void set_fwd_mode(int);
-void set_fwd_convert(int);
-int selftest_fwd_convert(int, int, int, int, int, double*, double*, double*);
-int run(const void*, int, long long, const void*, int, long long, int, int, int, int, void*, long long, long long, long long, int,
-        const float*, const float*, const float*, void*, int, int, int, int, int*, int*, cudaStream_t);
-int variant_count();
-int variant_info(int, int*, int*, int*, int*, int*, int*, int*);
 }
 
 static int require_device() {

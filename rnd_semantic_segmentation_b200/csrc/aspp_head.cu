@@ -22,8 +22,6 @@
 #include "gemm_sm100.cuh"
 
 namespace b200seg {
-namespace gemm { int overlap_sms(); }
-int nchw_to_nhwc_bf16(const float* src, int N, int C, int hw, void* dst, int pitch, cudaStream_t stream);   // seam_tail_kernels.cu
 
 constexpr int MAX_RATES = 8;
 constexpr int MAX_TAPS = 8 * MAX_RATES + 1;

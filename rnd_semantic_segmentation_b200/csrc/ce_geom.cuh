@@ -76,6 +76,5 @@ constexpr int K2V2_SPAN = 8;          // source columns a 32-column warp tile ma
 bool k2v2_eligible(int N, int C, int h, int w, int H, int W);
 void k2v2_geometry(K2Geom& g, int N, int C, int h, int w, int H, int W);
 int k2v2_main_launch(const K2Params& p, bool grad, cudaStream_t stream);
-void k2_set_variant(int v);           // A/B: 0 = always the CTA-tile kernel, 1 = warp-tile kernel where eligible (default)
 
 }  // namespace b200seg

@@ -20,6 +20,7 @@
 // Also here: materialising align-corners upsample forward / backward (the API-compat path for
 // callers that want the full-resolution tensor, e.g. PixelDiscriminator.forward(x, size)).
 #include "ce_geom.cuh"
+#include "host_api.h"
 
 namespace b200seg {
 

@@ -492,9 +492,9 @@ static int launch_conv(const CUtensorMap& ta, const CUtensorMap& tb, const ConvP
 }
 
 // D[pixel, co] = sum_t sum_ck act[pixel + sign*d_t, ck] * wt[t][co][ck]  (+ epilogue), see the header comment
-int conv3x3_run(const void* act, int N, int h, int w, int Ck, long long act_pitch, const void* wt, int Co, int dilation, int sign,
-                const float* bias, int lrelu, float slope, const void* mask, void* out, int out_mode, long long out_pitch,
-                cudaStream_t stream, int prof_tag, float* colsum_part = nullptr) {
+static int conv3x3_run(const void* act, int N, int h, int w, int Ck, long long act_pitch, const void* wt, int Co, int dilation, int sign,
+                       const float* bias, int lrelu, float slope, const void* mask, void* out, int out_mode, long long out_pitch,
+                       cudaStream_t stream, int prof_tag, float* colsum_part = nullptr) {
   B200SEG_CHECK_ARG(act && wt && out, "conv3x3: null pointer");
   B200SEG_CHECK_ARG(!colsum_part || out_mode == OUT_BF16_NHWC, "conv3x3: fused column sums need the bf16 NHWC output");
   B200SEG_CHECK_ARG(N > 0 && h > 0 && w > 0 && Ck > 0 && Co > 0 && dilation > 0, "conv3x3: bad geometry");
@@ -545,13 +545,13 @@ int conv3x3_run(const void* act, int N, int h, int w, int Ck, long long act_pitc
 }
 
 // rows of the fused column-sum partials: one per (M-tile, epilogue warp quarter)
-int conv3x3_colsum_rows(int N, int h, int w) {
+static int conv3x3_colsum_rows(int N, int h, int w) {
   int TW = 64, TH = 1;
   pick_rect(h, w, BLOCK_M, &TW, &TH);
   return N * ceil_div(w, TW) * ceil_div(h, TH) * 4;
 }
 
-int conv3x3_wgrad_splits(int N, int h, int w, int Co, int Ci) {
+static int conv3x3_wgrad_splits(int N, int h, int w, int Co, int Ci) {
   int TW = 64, TH = 1;
   pick_rect(h, w, BLOCK_K, &TW, &TH);
   const int kb_total = N * ceil_div(w, TW) * ceil_div(h, TH);
@@ -566,8 +566,8 @@ int conv3x3_wgrad_splits(int N, int h, int w, int Co, int Ci) {
 }
 
 // slabs[z][t][Co][Ci] = sum over the pixels of split z of g[pixel, co] * x[pixel + d_t, ci]
-int conv3x3_wgrad_run(const void* g, int Co, long long g_pitch, const void* x, int Ci, long long x_pitch, int N, int h, int w,
-                      int dilation, int splits, float* slabs, int* splits_used, cudaStream_t stream, int prof_tag) {
+static int conv3x3_wgrad_run(const void* g, int Co, long long g_pitch, const void* x, int Ci, long long x_pitch, int N, int h, int w,
+                             int dilation, int splits, float* slabs, int* splits_used, cudaStream_t stream, int prof_tag) {
   B200SEG_CHECK_ARG(g && x && slabs, "conv3x3_wgrad: null pointer");
   B200SEG_CHECK_ARG(N > 0 && h > 0 && w > 0 && Co > 0 && Ci > 0 && dilation > 0, "conv3x3_wgrad: bad geometry");
   B200SEG_CHECK_ARG(g_pitch % 8 == 0 && x_pitch % 8 == 0 && Ci % 4 == 0 && x_pitch >= Ci, "conv3x3_wgrad: channel pitches must be multiples of 8");
@@ -893,7 +893,7 @@ long long conv3x3_dgrad_colsum_scratch_bytes(int N, int h, int w, long long out_
 // below, accumulated in the GEMM epilogue (per M-tile and warp quarter) and finished by one small fixed-order reduction
 int conv3x3_dgrad(const void* g, int N, int h, int w, int Cg, long long g_pitch, const void* Wb, int Ci, int dilation, const void* mask,
                   float slope, void* out_bf16_nhwc, long long out_pitch, float* out_f32_nchw, cudaStream_t stream,
-                  void* colsum_scratch = nullptr, long long colsum_scratch_bytes = 0, float* colsum_out = nullptr) {
+                  void* colsum_scratch, long long colsum_scratch_bytes, float* colsum_out) {
   B200SEG_CHECK_ARG((out_bf16_nhwc != nullptr) != (out_f32_nchw != nullptr), "conv3x3_dgrad: give exactly one output");
   B200SEG_CHECK_ARG(!mask || out_bf16_nhwc, "conv3x3_dgrad: the activation mask needs the bf16 NHWC output");
   if (colsum_out) {

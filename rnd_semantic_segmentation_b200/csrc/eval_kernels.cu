@@ -28,6 +28,7 @@
 // even for i.i.d. labels), folded with dp4a into an int32 CTA histogram before a counter could overflow and into
 // the int64 global matrix once per frame per CTA.
 #include "common.cuh"
+#include "host_api.h"
 
 namespace b200seg {
 
@@ -881,10 +882,7 @@ static int confusion_pairs_any_launch(PdT* pd, const GtT* gt, long long n, int C
   return B200SEG_OK;
 }
 
-int confusion_pairs_launch_ex(void* pd, int pd_bytes, const void* gt, int gt_bytes, long long n, int C, int ignore_index, int mutate_pd,
-                              long long* cm, cudaStream_t stream);
-
-int confusion_pairs_launch(long long* pd, const long long* gt, long long n, int C, int ignore_index, int mutate_pd,
+static int confusion_pairs_launch(long long* pd, const long long* gt, long long n, int C, int ignore_index, int mutate_pd,
                            long long* cm, cudaStream_t stream) {
   B200SEG_CHECK_ARG(pd && gt && cm, "confusion_from_pred: null pointer");
   B200SEG_CHECK_ARG(C > 0 && C <= 104, "confusion_from_pred: num_classes=%d unsupported (1..104)", C);

@@ -55,10 +55,10 @@ int overlap_sms() { return g_overlap_sms; }
 static int g_share_enabled = 1;
 void set_sharing(int on) { g_share_enabled = on; }
 
-static int g_dgrad_mode = 1;         // b200seg_gemm_set_dgrad_mode(): see gemm_sm100.cuh
+static int g_dgrad_mode = 1;         // b200seg_gemm_set_dgrad_mode(): see host_api.h
 void set_dgrad_mode(int mode) { g_dgrad_mode = mode; }
 int dgrad_mode() { return g_dgrad_mode; }
-static int g_fwd_mode = 1;           // b200seg_gemm_set_fwd_mode(): see gemm_sm100.cuh
+static int g_fwd_mode = 1;           // b200seg_gemm_set_fwd_mode(): see host_api.h
 void set_fwd_mode(int mode) { g_fwd_mode = mode; }
 int fwd_mode() { return g_fwd_mode; }
 static int g_narrow_tiles = 1;        // b200seg_gemm_set_narrow_tiles(): 0 = always 256-column tiles

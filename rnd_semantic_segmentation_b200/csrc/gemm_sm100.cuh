@@ -16,6 +16,7 @@
 #pragma once
 #include <cuda.h>
 #include "common.cuh"
+#include "host_api.h"
 
 namespace b200seg {
 namespace gemm {
@@ -1055,17 +1056,6 @@ struct Gemm {
   int* variant_used = nullptr;   // the index of the kernel launched, in the table variant_info() reads
 };
 int launch(const Gemm& g, cudaStream_t stream);
-// the kernels launch() chooses from: their count, and entry i's template arguments (B200SEG_ERR_ARG for i out of range)
-int variant_count();
-int variant_info(int i, int* a_mn, int* b_mn, int* share, int* bn, int* rs, int* seam, int* stats);
-// fp32 NCHW data gradient of the head: 0 = channels along M (shared-memory transpose epilogue), 1 = pixels along M as cta_group::2
-// pairs, stores straight from registers, seven ring stages
-void set_dgrad_mode(int mode);
-int dgrad_mode();
-// forward GEMM of the head: 0 = channel-major (M = packed weight rows, shared-memory transpose epilogue), 1 = pixel-major
-// (M = pixels, register stores, ragged last N-tile at half MMA width)
-void set_fwd_mode(int mode);
-int fwd_mode();
 
 }  // namespace gemm
 }  // namespace b200seg

@@ -22,6 +22,7 @@
 // Tests hold the result to 1e-6 relative of torch.optim on the same inputs (one-ulp differences where a backend of the reference
 // rounds an intermediate the other way).
 #include "common.cuh"
+#include "host_api.h"
 
 namespace b200seg {
 

@@ -18,6 +18,7 @@
 // Here every byte crosses the switch once per direction in ONE step: a handful of CTAs suffice, so the persistent data-gradient
 // GEMM cedes 4 SMs instead of 32.
 #include "common.cuh"
+#include "host_api.h"
 
 namespace b200seg {
 

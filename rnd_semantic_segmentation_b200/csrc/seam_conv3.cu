@@ -24,9 +24,6 @@
 
 namespace b200seg {
 
-int nchw_to_nhwc_bf16(const float* src, int N, int C, int hw, void* dst, int pitch, cudaStream_t stream);   // seam_tail_kernels.cu
-int seam_conv3_g(const void* dy, const void* y, int N, int C, int hw, void* g, float* didentity, cudaStream_t stream);
-
 // W3 fp32 [Cout][Cin] -> W3b bf16 [Cout][Cin] and W't bf16 [Cin][Cout] (W'[co, ci] = bf16_rn(scale[co] * W3[co, ci]); SCALE false:
 // bf16_rn(W3[co, ci]), scale not read), through a 32 x 32 shared-memory tile
 template <bool SCALE>
@@ -300,12 +297,6 @@ int seam_conv3_bn_forward(const float* out2, const float* w3, int N, int Cin, in
   B200SEG_LAUNCH_CHECK();
   return B200SEG_OK;
 }
-
-int seam_tail_bn_backward_g(const void* dy, const void* y, const float* c, const float* mean, const float* invstd, const float* gamma,
-                            const float* sums, int R, const double* count, int N, int C, int hw, void* g, float* didentity,
-                            cudaStream_t stream);      // seam_tail_kernels.cu
-int seam_tail_backward(const void* dy, const void* y, const float* scale, int N, int C, int hw, float* dc, float* didentity,
-                       cudaStream_t stream);
 
 int seam_conv3_bn_backward(const void* dy, const void* y, const float* c, const float* mean, const float* invstd, const float* gamma,
                            const float* sums, int R, const double* count, const void* ws, int N, int Cin, int Cout, int hw, void* scratch,

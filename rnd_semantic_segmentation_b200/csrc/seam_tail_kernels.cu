@@ -19,6 +19,7 @@
 // pad channels are written as zeros).  At the 2:1 read/write mix of the pack this tile runs at 6.5 TB/s where the 64 x 64
 // scalar-load tile it replaced ran at 5.6 (profiles/micro/nhwc_tile_micro.cu).
 #include "common.cuh"
+#include "host_api.h"
 
 namespace b200seg {
 

@@ -14,6 +14,7 @@
 // (NCHW), so every load/store instruction of a warp is one fully coalesced 128-byte line, and all K
 // loads of a thread are issued before the first use (K independent requests in flight per thread).
 #include "common.cuh"
+#include "host_api.h"
 
 namespace b200seg {
 

@@ -25,6 +25,7 @@
 // Mapping: one thread per label pixel; a CTA owns a run of consecutive rows of one 128-column strip (consecutive rows share
 // source rows, which stay in L1).  Confusion counts go to a shared-memory int32 histogram (atomics), published once per CTA.
 #include "common.cuh"
+#include "host_api.h"
 
 namespace b200seg {
 
