@@ -268,6 +268,23 @@ B200SEG_API int b200seg_disc_backward(const float* grad_out, const void* Xp, con
                                     float slope, void* G3, void* dZ2, void* dZ1, void* scratch, int64_t scratch_bytes, float* gw1,
                                     float* gb1, float* gw2, float* gb2, float* gwc1, float* gwc2, float* gb3, float* gx_f32_nchw,
                                     void* gx_bf16_nhwc, void* stream);
+/* The same stack with TF32 tensor-core operands (tcgen05.mma.kind::tf32) and fp32 activations / gradients -- the numeric class of
+ * cuDNN under torch.backends.cudnn.allow_tf32.  Same arguments as the bf16 entries; what those take as bf16 is fp32 here:
+ *   Wf_l / Wb_l fp32 [9][Co_l][Ci_l] / [9][Ci_l][round8(Co_l)] rounded to TF32; Xp / A1 / A2 / G3 / dZ2 / dZ1 fp32 NHWC, every value
+ *   rounded to TF32 (nearest-even, low 13 mantissa bits zero).  Xp is required for both x_kinds (fp32 NCHW rounded, or bf16 NHWC
+ *   widened exactly).  Bias gradients are column sums of the unrounded fp32 gradients; gx_bf16_nhwc is the bf16 NHWC feature
+ *   gradient of bf16 features.  scratch: b200seg_disc_backward_tf32_scratch_bytes(...) bytes */
+B200SEG_API int b200seg_disc_forward_tf32(const void* x, int x_kind, int N, int Cin, int h, int w, int ndf1, int ndf2, int C,
+                                         const float* w1, const float* b1, const float* w2, const float* b2, const float* wc1,
+                                         const float* bc1, const float* wc2, const float* bc2, float slope, int do_pack, float* Wf1,
+                                         float* Wb1, float* Wf2, float* Wb2, float* Wf3, float* Wb3, float* b3, float* Xp, float* A1,
+                                         float* A2, float* out, void* stream);
+B200SEG_API int64_t b200seg_disc_backward_tf32_scratch_bytes(int N, int Cin, int h, int w, int ndf1, int ndf2, int C);
+B200SEG_API int b200seg_disc_backward_tf32(const float* grad_out, const float* Xp, const float* A1, const float* A2, const float* Wb1,
+                                          const float* Wb2, const float* Wb3, int N, int Cin, int h, int w, int ndf1, int ndf2, int C,
+                                          float slope, float* G3, float* dZ2, float* dZ1, void* scratch, int64_t scratch_bytes,
+                                          float* gw1, float* gb1, float* gw2, float* gb2, float* gwc1, float* gwc2, float* gb3,
+                                          float* gx_f32_nchw, void* gx_bf16_nhwc, void* stream);
 /* n_parts weight tensors fp32 [part_co[i]][Ci][3][3], concatenated along the output-channel axis (cls1 | cls2 = torch.cat(dim=1)):
  *   Wf bf16 [9][Co][Ci]        forward operand (Co = sum part_co)           (may be NULL)
  *   Wb bf16 [9][Ci][co_pitch]  data-gradient operand, caller zero-fills the padding columns co_pitch > Co   (may be NULL) */
@@ -305,6 +322,25 @@ B200SEG_API int64_t b200seg_conv3x3_wgrad_scratch_bytes(int N, int h, int w, int
 B200SEG_API int b200seg_conv3x3_wgrad(const void* g_nhwc_bf16, int Co, int64_t g_pitch, const void* x_nhwc_bf16, int Ci, int64_t x_pitch,
                                       int N, int h, int w, int dilation, int splits, void* scratch, int64_t scratch_bytes,
                                       float* const* grad_w, const int* part_co_host, int n_parts, void* stream);
+/* The single layers of the TF32 stack: the entries above with fp32 operands holding TF32 values (b200seg_conv3x3_pack_weights_stack_tf32
+ * writes them) and an fp32 NHWC output (out_nhwc) whose values are rounded to TF32; out_f32_nchw and the weight gradients are not
+ * rounded.  The data gradient's mask is fp32 NHWC; colsum_out (optional, with colsum_scratch of
+ * b200seg_conv3x3_dgrad_colsum_scratch_bytes bytes) sums the NHWC output's values before their rounding.  The weight-gradient scratch
+ * is b200seg_conv3x3_wgrad_scratch_bytes. */
+B200SEG_API int b200seg_conv3x3_pack_weights_stack_tf32(int n_layers, const float* const* weights, const int* part_co_host,
+                                                        const int* parts_per_layer_host, const int* Ci_host, float* const* Wf,
+                                                        float* const* Wb, const int* co_pitch_host, const float* const* bias_parts,
+                                                        const int* bias_len_host, int n_bias, float* bias_out, void* stream);
+B200SEG_API int b200seg_conv3x3_forward_tf32(const float* act_nhwc, int N, int h, int w, int Ci, int64_t act_pitch, const float* Wf, int Co,
+                                             int dilation, const float* bias, int lrelu, float slope, float* out_nhwc, int64_t out_pitch,
+                                             float* out_f32_nchw, void* stream);
+B200SEG_API int b200seg_conv3x3_dgrad_tf32(const float* g_nhwc, int N, int h, int w, int Cg, int64_t g_pitch, const float* Wb, int Ci,
+                                           int dilation, const float* mask_nhwc, float slope, float* out_nhwc, int64_t out_pitch,
+                                           float* out_f32_nchw, void* colsum_scratch, int64_t colsum_scratch_bytes, float* colsum_out,
+                                           void* stream);
+B200SEG_API int b200seg_conv3x3_wgrad_tf32(const float* g_nhwc, int Co, int64_t g_pitch, const float* x_nhwc, int Ci, int64_t x_pitch,
+                                           int N, int h, int w, int dilation, int splits, void* scratch, int64_t scratch_bytes,
+                                           float* const* grad_w, const int* part_co_host, int n_parts, void* stream);
 /* fp32 NCHW [N,C,hw] -> bf16 NHWC [N*hw][pitch] (channels >= C zero): the output gradient of the last layer */
 B200SEG_API int b200seg_nchw_to_nhwc_bf16(const float* src, int N, int C, int hw, void* dst, int pitch, void* stream);
 /* bias gradient: out[c] = sum_pixels g[pixel][c], deterministic (fixed-order two-phase sum) */

@@ -86,6 +86,16 @@ SIGNATURES = {
     "b200seg_disc_backward_scratch_bytes": (c_i64, [c_int] * 7),
     "b200seg_disc_forward": (c_int, [c_vp, c_int] + [c_int] * 7 + [c_vp] * 8 + [c_f32, c_int] + [c_vp] * 11 + [c_vp]),
     "b200seg_disc_backward": (c_int, [c_vp] * 7 + [c_int] * 7 + [c_f32] + [c_vp] * 4 + [c_i64] + [c_vp] * 9 + [c_vp]),
+    "b200seg_disc_backward_tf32_scratch_bytes": (c_i64, [c_int] * 7),
+    "b200seg_disc_forward_tf32": (c_int, [c_vp, c_int] + [c_int] * 7 + [c_vp] * 8 + [c_f32, c_int] + [c_vp] * 11 + [c_vp]),
+    "b200seg_disc_backward_tf32": (c_int, [c_vp] * 7 + [c_int] * 7 + [c_f32] + [c_vp] * 4 + [c_i64] + [c_vp] * 9 + [c_vp]),
+    "b200seg_conv3x3_pack_weights_stack_tf32": (c_int, [c_int, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_vp, c_int, c_vp, c_vp]),
+    "b200seg_conv3x3_forward_tf32": (c_int, [c_vp, c_int, c_int, c_int, c_int, c_i64, c_vp, c_int, c_int, c_vp, c_int, c_f32, c_vp,
+                                             c_i64, c_vp, c_vp]),
+    "b200seg_conv3x3_dgrad_tf32": (c_int, [c_vp, c_int, c_int, c_int, c_int, c_i64, c_vp, c_int, c_int, c_vp, c_f32, c_vp, c_i64,
+                                           c_vp, c_vp, c_i64, c_vp, c_vp]),
+    "b200seg_conv3x3_wgrad_tf32": (c_int, [c_vp, c_int, c_i64, c_vp, c_int, c_i64, c_int, c_int, c_int, c_int, c_int, c_vp, c_i64,
+                                           c_vp, c_vp, c_int, c_vp]),
     "b200seg_set_step_graphs": (None, [c_int]),
     "b200seg_step_graph_stats": (None, [c_vp, c_vp]),
     "b200seg_conv3x3_pack_weights": (c_int, [c_vp, c_vp, c_int, c_int, c_vp, c_vp, c_int, c_vp]),
@@ -960,10 +970,11 @@ def head_loss_backward(ws: torch.Tensor, x_bf16: Optional[torch.Tensor], x_kind:
 # --------------------------------------------------------------------------------------------
 # K6 in one foreign call per direction (the PixelDiscriminator conv stack, graph-replayed like the head entries)
 # --------------------------------------------------------------------------------------------
-def disc_forward(x: torch.Tensor, x_kind: int, shape, weights, biases, slope: float, packed=None):
+def disc_forward(x: torch.Tensor, x_kind: int, shape, weights, biases, slope: float, packed=None, tf32: bool = False):
     """cat(cls1, cls2)(LReLU(conv(LReLU(conv(x))))) in ONE call (weight pack, feature pack, three conv layers).  ``x``: fp32 NCHW
     (x_kind 0) or bf16 NHWC [N,h,w,Cin] (x_kind 1); ``shape`` = (N, Cin, h, w); ``weights`` = (w1, w2, wc1, wc2), ``biases`` =
     (b1, b2, bc1, bc2).  ``packed`` = ((Wf1,Wb1),(Wf2,Wb2),(Wf3,Wb3),b3) to reuse an existing pack (eval), None to pack inside the call.
+    ``tf32``: TF32 tensor-core operands, the packed weights, Xp, A1 and A2 fp32 (b200seg_disc_forward_tf32).
     Returns (out fp32 [N,2C,h,w], Xp, A1, A2, packed)."""
     lib = load()
     N, Cin, h, w = shape
@@ -981,22 +992,25 @@ def disc_forward(x: torch.Tensor, x_kind: int, shape, weights, biases, slope: fl
     if Cin % 8 or ndf1 % 8 or ndf2 % 8:
         raise B200SegError("PixelDiscriminator: in_channels, ndf and ndf/2 must be multiples of 8")
     do_pack = packed is None
+    bf = torch.float32 if tf32 else torch.bfloat16
     if do_pack:
-        bf = torch.bfloat16
         packed = ((torch.empty((9, ndf1, Cin), dtype=bf, device=dev), torch.empty((9, Cin, ndf1), dtype=bf, device=dev)),
                   (torch.empty((9, ndf2, ndf1), dtype=bf, device=dev), torch.empty((9, ndf1, ndf2), dtype=bf, device=dev)),
                   (torch.empty((9, 2 * C, ndf2), dtype=bf, device=dev), torch.empty((9, ndf2, _round8(2 * C)), dtype=bf, device=dev)),
                   torch.empty(2 * C, dtype=torch.float32, device=dev))
     (Wf1, Wb1), (Wf2, Wb2), (Wf3, Wb3), b3 = packed
-    Xp = x if x_kind == 1 else torch.empty((N, h, w, Cin), dtype=torch.bfloat16, device=dev)
-    A1 = torch.empty((N, h, w, ndf1), dtype=torch.bfloat16, device=dev)
-    A2 = torch.empty((N, h, w, ndf2), dtype=torch.bfloat16, device=dev)
+    if any(t.dtype != bf for t in (Wf1, Wb1, Wf2, Wb2, Wf3, Wb3)):
+        raise B200SegError(f"disc_forward: packed weights must be {bf} for tf32={bool(tf32)}")
+    Xp = x if (x_kind == 1 and not tf32) else torch.empty((N, h, w, Cin), dtype=bf, device=dev)
+    A1 = torch.empty((N, h, w, ndf1), dtype=bf, device=dev)
+    A2 = torch.empty((N, h, w, ndf2), dtype=bf, device=dev)
     out = torch.empty((N, 2 * C, h, w), dtype=torch.float32, device=dev)
+    entry = lib.b200seg_disc_forward_tf32 if tf32 else lib.b200seg_disc_forward
     with _on_device(dev):
-        _check(lib.b200seg_disc_forward(x.data_ptr(), x_kind, N, Cin, h, w, ndf1, ndf2, C, w1.data_ptr(), _ptr(b1), w2.data_ptr(), _ptr(b2),
+        _check(entry(x.data_ptr(), x_kind, N, Cin, h, w, ndf1, ndf2, C, w1.data_ptr(), _ptr(b1), w2.data_ptr(), _ptr(b2),
                                         wc1.data_ptr(), _ptr(bc1), wc2.data_ptr(), _ptr(bc2), float(slope), 1 if do_pack else 0,
                                         Wf1.data_ptr(), Wb1.data_ptr(), Wf2.data_ptr(), Wb2.data_ptr(), Wf3.data_ptr(), Wb3.data_ptr(),
-                                        b3.data_ptr(), None if x_kind == 1 else Xp.data_ptr(), A1.data_ptr(), A2.data_ptr(),
+                                        b3.data_ptr(), None if Xp is x else Xp.data_ptr(), A1.data_ptr(), A2.data_ptr(),
                                         out.data_ptr(), _stream()))
     return out, Xp, A1, A2, packed
 
@@ -1004,7 +1018,7 @@ def disc_forward(x: torch.Tensor, x_kind: int, shape, weights, biases, slope: fl
 def disc_backward(grad_out: torch.Tensor, Xp, A1, A2, Wb1, Wb2, Wb3, C: int, slope: float, need, x_bf16: bool):
     """Backward of disc_forward in ONE call.  ``need`` = (x, w1, b1, w2, b2, wc1, bc1, wc2, bc2) booleans.  Returns
     (gx | None, gw1, gb1, gw2, gb2, gwc1, gbc1, gwc2, gbc2) with None where not needed; gx is fp32 NCHW, or with ``x_bf16`` a bf16
-    channels_last tensor of logical shape [N,Cin,h,w]."""
+    channels_last tensor of logical shape [N,Cin,h,w].  fp32 Xp / A1 / A2 / Wb (disc_forward(tf32=True)) take the TF32 entry."""
     lib = load()
     N, h, w, Cin = (int(v) for v in Xp.shape)
     ndf1, ndf2 = int(A1.shape[3]), int(A2.shape[3])
@@ -1014,11 +1028,13 @@ def disc_backward(grad_out: torch.Tensor, Xp, A1, A2, Wb1, Wb2, Wb3, C: int, slo
         raise B200SegError(f"disc_backward: grad_out shape {tuple(grad_out.shape)} != {(N, 2 * C, h, w)}")
     nx, nw1, nb1, nw2, nb2, nwc1, nbc1, nwc2, nbc2 = (bool(v) for v in need)
     f32, bf = torch.float32, torch.bfloat16
+    tf32 = A1.dtype == f32
+    act = f32 if tf32 else bf
     need_l1 = nx or nw1 or nb1
     need_l2 = need_l1 or nw2 or nb2
-    G3 = torch.empty((N, h, w, _round8(2 * C)), dtype=bf, device=dev)
-    dZ2 = torch.empty((N, h, w, ndf2), dtype=bf, device=dev) if need_l2 else None
-    dZ1 = torch.empty((N, h, w, ndf1), dtype=bf, device=dev) if need_l1 else None
+    G3 = torch.empty((N, h, w, _round8(2 * C)), dtype=act, device=dev)
+    dZ2 = torch.empty((N, h, w, ndf2), dtype=act, device=dev) if need_l2 else None
+    dZ1 = torch.empty((N, h, w, ndf1), dtype=act, device=dev) if need_l1 else None
     gw1 = torch.empty((ndf1, Cin, 3, 3), dtype=f32, device=dev) if nw1 else None
     gb1 = torch.empty(ndf1, dtype=f32, device=dev) if nb1 else None
     gw2 = torch.empty((ndf2, ndf1, 3, 3), dtype=f32, device=dev) if nw2 else None
@@ -1033,9 +1049,12 @@ def disc_backward(grad_out: torch.Tensor, Xp, A1, A2, Wb1, Wb2, Wb3, C: int, slo
         else:
             gx = torch.empty((N, Cin, h, w), dtype=f32, device=dev)
     with _on_device(dev):
-        nbytes = int(lib.b200seg_disc_backward_scratch_bytes(N, Cin, h, w, ndf1, ndf2, C))
+        if tf32:
+            nbytes, entry = int(lib.b200seg_disc_backward_tf32_scratch_bytes(N, Cin, h, w, ndf1, ndf2, C)), lib.b200seg_disc_backward_tf32
+        else:
+            nbytes, entry = int(lib.b200seg_disc_backward_scratch_bytes(N, Cin, h, w, ndf1, ndf2, C)), lib.b200seg_disc_backward
         scratch = _scratch("disc_bwd", nbytes, dev)
-        _check(lib.b200seg_disc_backward(grad_out.data_ptr(), Xp.data_ptr(), A1.data_ptr(), A2.data_ptr(), Wb1.data_ptr(), Wb2.data_ptr(),
+        _check(entry(grad_out.data_ptr(), Xp.data_ptr(), A1.data_ptr(), A2.data_ptr(), Wb1.data_ptr(), Wb2.data_ptr(),
                                          Wb3.data_ptr(), N, Cin, h, w, ndf1, ndf2, C, float(slope), G3.data_ptr(), _ptr(dZ2), _ptr(dZ1),
                                          scratch.data_ptr(), scratch.numel(), _ptr(gw1), _ptr(gb1), _ptr(gw2), _ptr(gb2), _ptr(gwc1),
                                          _ptr(gwc2), _ptr(gb3), _ptr(gx), _ptr(gx_nhwc), _stream()))
@@ -1075,9 +1094,10 @@ def conv3x3_pack_weights(weights: Sequence[torch.Tensor]):
 
 
 def conv3x3_pack_weights_stack(layers: Sequence[Sequence[torch.Tensor]], bias_parts: Sequence[Optional[torch.Tensor]] = (),
-                               bias_lens: Sequence[int] = ()):
+                               bias_lens: Sequence[int] = (), tf32: bool = False):
     """Every layer of a conv stack in ONE launch: ``layers[l]`` = the [Co_i,Ci_l,3,3] fp32 tensors concatenated along Co for layer
-    l.  Returns ([(Wf_l, Wb_l)], bias) with bias = the concatenation of ``bias_parts`` (None = zeros of ``bias_lens[i]``)."""
+    l.  Returns ([(Wf_l, Wb_l)], bias) with bias = the concatenation of ``bias_parts`` (None = zeros of ``bias_lens[i]``).
+    ``tf32``: Wf / Wb are fp32 holding the weights rounded to TF32 (the operands of the TF32 layers) instead of bf16."""
     lib = load()
     flat, parts, ppl, cis, Wfs, Wbs, pitches = [], [], [], [], [], [], []
     dev = layers[0][0].device
@@ -1094,8 +1114,9 @@ def conv3x3_pack_weights_stack(layers: Sequence[Sequence[torch.Tensor]], bias_pa
         parts += [int(wt.shape[0]) for wt in ws]
         ppl.append(len(ws))
         cis.append(Ci)
-        Wfs.append(torch.empty((9, Co, Ci), dtype=torch.bfloat16, device=dev))
-        Wbs.append(torch.empty((9, Ci, _round8(Co)), dtype=torch.bfloat16, device=dev))
+        wdt = torch.float32 if tf32 else torch.bfloat16
+        Wfs.append(torch.empty((9, Co, Ci), dtype=wdt, device=dev))
+        Wbs.append(torch.empty((9, Ci, _round8(Co)), dtype=wdt, device=dev))
         pitches.append(_round8(Co))
     bias = None
     if bias_lens:
@@ -1105,26 +1126,29 @@ def conv3x3_pack_weights_stack(layers: Sequence[Sequence[torch.Tensor]], bias_pa
         bias = torch.empty(int(sum(bias_lens)), dtype=torch.float32, device=dev)
     ia = lambda v: (c_int * len(v))(*[int(x) for x in v])  # noqa: E731
     with _on_device(dev):
-        _check(lib.b200seg_conv3x3_pack_weights_stack(len(layers), _ptr_array(flat), ia(parts), ia(ppl), ia(cis), _ptr_array(Wfs),
+        entry = lib.b200seg_conv3x3_pack_weights_stack_tf32 if tf32 else lib.b200seg_conv3x3_pack_weights_stack
+        _check(entry(len(layers), _ptr_array(flat), ia(parts), ia(ppl), ia(cis), _ptr_array(Wfs),
                                                       _ptr_array(Wbs), ia(pitches), _ptr_array(list(bias_parts)) if bias_lens else None,
                                                       ia(bias_lens) if bias_lens else None, len(bias_lens), _ptr(bias), _stream()))
     return list(zip(Wfs, Wbs)), bias
 
 
-def _need_nhwc(t: torch.Tensor, name: str):
-    _need(t, torch.bfloat16, name)
+def _need_nhwc(t: torch.Tensor, name: str, dtype=torch.bfloat16):
+    _need(t, dtype, name)
     if t.dim() != 4 or t.shape[3] % 8 != 0:
-        raise B200SegError(f"{name}: expected bf16 NHWC [N,h,w,C] with C a multiple of 8, got {tuple(t.shape)}")
+        raise B200SegError(f"{name}: expected {dtype} NHWC [N,h,w,C] with C a multiple of 8, got {tuple(t.shape)}")
     return t.shape
 
 
 def conv3x3_forward(act: torch.Tensor, Wf: torch.Tensor, bias: Optional[torch.Tensor], lrelu_slope: Optional[float] = None,
                     dilation: int = 1, out_f32_nchw: bool = False) -> torch.Tensor:
     """[LeakyReLU](conv3x3(act) + bias) with padding == dilation.  act bf16 NHWC [N,h,w,Ci]; returns bf16 NHWC [N,h,w,round8(Co)]
-    (requires Co % 8 == 0) or, with ``out_f32_nchw``, fp32 NCHW [N,Co,h,w]."""
+    (requires Co % 8 == 0) or, with ``out_f32_nchw``, fp32 NCHW [N,Co,h,w].  fp32 ``act`` and ``Wf`` (TF32 values) run the TF32
+    layer, whose NHWC output is fp32 rounded to TF32."""
     lib = load()
-    N, h, w, pitch = _need_nhwc(act, "act")
-    _need(Wf, torch.bfloat16, "Wf")
+    dt = torch.float32 if act.dtype == torch.float32 else torch.bfloat16
+    N, h, w, pitch = _need_nhwc(act, "act", dt)
+    _need(Wf, dt, "Wf")
     Co, Ci = int(Wf.shape[1]), int(Wf.shape[2])
     if Ci != pitch:
         raise B200SegError(f"conv3x3_forward: activations have {pitch} channels, weights expect {Ci}")
@@ -1136,9 +1160,10 @@ def conv3x3_forward(act: torch.Tensor, Wf: torch.Tensor, bias: Optional[torch.Te
     else:
         if Co % 8 != 0:
             raise B200SegError(f"conv3x3_forward: bf16 NHWC output needs out_channels={Co} to be a multiple of 8")
-        out_b = torch.empty((N, h, w, Co), dtype=torch.bfloat16, device=act.device)
+        out_b = torch.empty((N, h, w, Co), dtype=dt, device=act.device)
+    entry = lib.b200seg_conv3x3_forward_tf32 if dt == torch.float32 else lib.b200seg_conv3x3_forward
     with _on_device(act.device):
-        _check(lib.b200seg_conv3x3_forward(act.data_ptr(), N, h, w, Ci, pitch, Wf.data_ptr(), Co, int(dilation), _ptr(bias),
+        _check(entry(act.data_ptr(), N, h, w, Ci, pitch, Wf.data_ptr(), Co, int(dilation), _ptr(bias),
                                            0 if lrelu_slope is None else 1, 0.0 if lrelu_slope is None else float(lrelu_slope),
                                            _ptr(out_b), Co, _ptr(out_f), _stream()))
     return out_f if out_f32_nchw else out_b
@@ -1149,10 +1174,13 @@ def conv3x3_dgrad(g: torch.Tensor, Wb: torch.Tensor, mask: Optional[torch.Tensor
     """Data gradient of conv3x3 (padding == dilation): g bf16 NHWC [N,h,w,round8(Co)], Wb bf16 [9,Ci,round8(Co)].  ``mask`` (bf16
     NHWC [N,h,w,Ci], the saved LeakyReLU output of the layer below) fuses the activation's backward into the epilogue.
     ``want_colsum`` (bf16 NHWC output only) returns (gradient, fp32 [Ci] per-channel sums of the gradient) -- the bias gradient of
-    the layer below, accumulated in the same epilogue."""
+    the layer below, accumulated in the same epilogue.  fp32 ``g`` / ``Wb`` / ``mask`` run the TF32 layer: NHWC output fp32 rounded
+    to TF32, column sums of the values before that rounding."""
     lib = load()
-    N, h, w, gp = _need_nhwc(g, "g")
-    _need(Wb, torch.bfloat16, "Wb")
+    dt = torch.float32 if g.dtype == torch.float32 else torch.bfloat16
+    tf32 = dt == torch.float32
+    N, h, w, gp = _need_nhwc(g, "g", dt)
+    _need(Wb, dt, "Wb")
     Ci, Cg = int(Wb.shape[1]), int(Wb.shape[2])
     if Cg != gp:
         raise B200SegError(f"conv3x3_dgrad: gradient has {gp} channels, Wb expects {Cg}")
@@ -1164,8 +1192,8 @@ def conv3x3_dgrad(g: torch.Tensor, Wb: torch.Tensor, mask: Optional[torch.Tensor
     else:
         if Ci % 8 != 0:
             raise B200SegError(f"conv3x3_dgrad: bf16 NHWC output needs in_channels={Ci} to be a multiple of 8")
-        out_b = torch.empty((N, h, w, Ci), dtype=torch.bfloat16, device=g.device)
-        if mask is not None and tuple(_need_nhwc(mask, "mask")) != (N, h, w, Ci):
+        out_b = torch.empty((N, h, w, Ci), dtype=dt, device=g.device)
+        if mask is not None and tuple(_need_nhwc(mask, "mask", dt)) != (N, h, w, Ci):
             raise B200SegError(f"conv3x3_dgrad: mask shape {tuple(mask.shape)} != {(N, h, w, Ci)}")
     if want_colsum:
         if out_f32_nchw:
@@ -1174,22 +1202,33 @@ def conv3x3_dgrad(g: torch.Tensor, Wb: torch.Tensor, mask: Optional[torch.Tensor
         scratch = _scratch("dgrad_colsum", nbytes, g.device)
         colsum = torch.empty(Ci, dtype=torch.float32, device=g.device)
         with _on_device(g.device):
+            if tf32:
+                _check(lib.b200seg_conv3x3_dgrad_tf32(g.data_ptr(), N, h, w, Cg, gp, Wb.data_ptr(), Ci, int(dilation), _ptr(mask),
+                                                      float(slope), out_b.data_ptr(), Ci, None, scratch.data_ptr(), nbytes,
+                                                      colsum.data_ptr(), _stream()))
+                return out_b, colsum
             _check(lib.b200seg_conv3x3_dgrad_colsum(g.data_ptr(), N, h, w, Cg, gp, Wb.data_ptr(), Ci, int(dilation), _ptr(mask),
                                                     float(slope), out_b.data_ptr(), Ci, scratch.data_ptr(), nbytes,
                                                     colsum.data_ptr(), _stream()))
         return out_b, colsum
     with _on_device(g.device):
-        _check(lib.b200seg_conv3x3_dgrad(g.data_ptr(), N, h, w, Cg, gp, Wb.data_ptr(), Ci, int(dilation), _ptr(mask), float(slope),
-                                         _ptr(out_b), Ci, _ptr(out_f), _stream()))
+        if tf32:
+            _check(lib.b200seg_conv3x3_dgrad_tf32(g.data_ptr(), N, h, w, Cg, gp, Wb.data_ptr(), Ci, int(dilation), _ptr(mask), float(slope),
+                                                  _ptr(out_b), Ci, _ptr(out_f), None, 0, None, _stream()))
+        else:
+            _check(lib.b200seg_conv3x3_dgrad(g.data_ptr(), N, h, w, Cg, gp, Wb.data_ptr(), Ci, int(dilation), _ptr(mask), float(slope),
+                                             _ptr(out_b), Ci, _ptr(out_f), _stream()))
     return out_f if out_f32_nchw else out_b
 
 
 def conv3x3_wgrad(g: torch.Tensor, x: torch.Tensor, parts: Sequence[int], dilation: int = 1, splits: int = 0,
                   out: Optional[Sequence[Optional[torch.Tensor]]] = None):
-    """Weight gradients [parts[i],Ci,3,3] fp32 from the bf16 NHWC output gradient g [N,h,w,round8(sum parts)] and input x."""
+    """Weight gradients [parts[i],Ci,3,3] fp32 from the bf16 NHWC output gradient g [N,h,w,round8(sum parts)] and input x (fp32
+    g and x holding TF32 values: the TF32 layer)."""
     lib = load()
-    N, h, w, gp = _need_nhwc(g, "g")
-    if tuple(_need_nhwc(x, "x"))[:3] != (N, h, w):
+    dt = torch.float32 if g.dtype == torch.float32 else torch.bfloat16
+    N, h, w, gp = _need_nhwc(g, "g", dt)
+    if tuple(_need_nhwc(x, "x", dt))[:3] != (N, h, w):
         raise B200SegError("conv3x3_wgrad: g and x must share [N,h,w]")
     Ci = int(x.shape[3])
     Co = int(sum(parts))
@@ -1203,7 +1242,8 @@ def conv3x3_wgrad(g: torch.Tensor, x: torch.Tensor, parts: Sequence[int], dilati
         if t is not None and (tuple(_need(t, torch.float32, "grad_w").shape) != (int(pc), Ci, 3, 3)):
             raise B200SegError("conv3x3_wgrad: bad output buffer shape")
     with _on_device(g.device):
-        _check(lib.b200seg_conv3x3_wgrad(g.data_ptr(), Co, gp, x.data_ptr(), Ci, Ci, N, h, w, int(dilation), int(splits),
+        entry = lib.b200seg_conv3x3_wgrad_tf32 if dt == torch.float32 else lib.b200seg_conv3x3_wgrad
+        _check(entry(g.data_ptr(), Co, gp, x.data_ptr(), Ci, Ci, N, h, w, int(dilation), int(splits),
                                          scratch.data_ptr(), nbytes, _ptr_array(out), (c_int * len(parts))(*[int(v) for v in parts]),
                                          len(parts), _stream()))
     return list(out)

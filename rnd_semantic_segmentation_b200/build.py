@@ -5,10 +5,12 @@ are read, exactly as the reference does.
 """
 from __future__ import annotations
 
+import functools
+
 from .classifier import ASPP_Classifier_V2
 from .discriminator import PixelDiscriminator
 
-__all__ = ["build_feature_extractor", "build_classifier", "build_adversarial_discriminator"]
+__all__ = ["build_feature_extractor", "build_classifier", "build_adversarial_discriminator", "wrap_discriminator_factory"]
 
 _ASPP_RATES = [6, 12, 18, 24]
 
@@ -49,3 +51,22 @@ def build_adversarial_discriminator(cfg, num_features=None, mid_nc=256):
                 num_features = feats
             return PixelDiscriminator(num_features, mid_nc, num_classes=cfg.MODEL.NUM_CLASSES)
     raise NotImplementedError
+
+
+def wrap_discriminator_factory(stock, tf32: bool = False):
+    """``build_adversarial_discriminator`` with the same signature whose PixelDiscriminator results get ``tf32`` set
+    (install(disc_tf32=True)).  Wrapping a wrapper returns it with its flag set to the new value."""
+    if getattr(stock, "_b200seg_disc", False):
+        stock._b200seg_disc_tf32 = bool(tf32)
+        return stock
+
+    @functools.wraps(stock)
+    def build_adversarial_discriminator(*args, **kwargs):
+        D = stock(*args, **kwargs)
+        if isinstance(D, PixelDiscriminator):
+            D.tf32 = build_adversarial_discriminator._b200seg_disc_tf32
+        return D
+
+    build_adversarial_discriminator._b200seg_disc = True
+    build_adversarial_discriminator._b200seg_disc_tf32 = bool(tf32)
+    return build_adversarial_discriminator

@@ -456,6 +456,40 @@ int b200seg_conv3x3_wgrad(const void* g, int Co, int64_t g_pitch, const void* x,
                        n_parts, S(stream));
 }
 
+int b200seg_conv3x3_pack_weights_stack_tf32(int n_layers, const float* const* weights, const int* part_co_host,
+                                            const int* parts_per_layer_host, const int* Ci_host, float* const* Wf, float* const* Wb,
+                                            const int* co_pitch_host, const float* const* bias_parts, const int* bias_len_host, int n_bias,
+                                            float* bias_out, void* stream) {
+  REQUIRE_DEVICE();
+  return conv3x3_pack_weights_stack_tf32(n_layers, weights, part_co_host, parts_per_layer_host, Ci_host, reinterpret_cast<void* const*>(Wf),
+                                         reinterpret_cast<void* const*>(Wb), co_pitch_host, bias_parts, bias_len_host, n_bias, bias_out,
+                                         S(stream));
+}
+
+int b200seg_conv3x3_forward_tf32(const float* act, int N, int h, int w, int Ci, int64_t act_pitch, const float* Wf, int Co, int dilation,
+                                 const float* bias, int lrelu, float slope, float* out_nhwc, int64_t out_pitch, float* out_f32_nchw,
+                                 void* stream) {
+  REQUIRE_DEVICE();
+  return conv3x3_forward(act, N, h, w, Ci, act_pitch, Wf, Co, dilation, bias, lrelu, slope, out_nhwc, out_pitch, out_f32_nchw, S(stream),
+                         1);
+}
+
+int b200seg_conv3x3_dgrad_tf32(const float* g, int N, int h, int w, int Cg, int64_t g_pitch, const float* Wb, int Ci, int dilation,
+                               const float* mask, float slope, float* out_nhwc, int64_t out_pitch, float* out_f32_nchw,
+                               void* colsum_scratch, int64_t colsum_scratch_bytes, float* colsum_out, void* stream) {
+  REQUIRE_DEVICE();
+  return conv3x3_dgrad(g, N, h, w, Cg, g_pitch, Wb, Ci, dilation, mask, slope, out_nhwc, out_pitch, out_f32_nchw, S(stream),
+                       colsum_scratch, colsum_scratch_bytes, colsum_out, 1);
+}
+
+int b200seg_conv3x3_wgrad_tf32(const float* g, int Co, int64_t g_pitch, const float* x, int Ci, int64_t x_pitch, int N, int h, int w,
+                               int dilation, int splits, void* scratch, int64_t scratch_bytes, float* const* grad_w,
+                               const int* part_co_host, int n_parts, void* stream) {
+  REQUIRE_DEVICE();
+  return conv3x3_wgrad(g, Co, g_pitch, x, Ci, x_pitch, N, h, w, dilation, splits, scratch, scratch_bytes, grad_w, part_co_host,
+                       n_parts, S(stream), 1);
+}
+
 int b200seg_nchw_to_nhwc_bf16(const float* src, int N, int C, int hw, void* dst, int pitch, void* stream) {
   REQUIRE_DEVICE();
   return nchw_to_nhwc_bf16(src, N, C, hw, dst, pitch, S(stream));
@@ -922,6 +956,127 @@ int b200seg_disc_backward(const float* grad_out, const void* Xp, const void* A1,
     }
     if (need_x)
       rc = conv3x3_dgrad(dZ1, N, h, w, ndf1, ndf1, Wb1, Cin, 1, nullptr, slope, gx_bf16_nhwc, Cin, gx_f32_nchw, st, nullptr, 0, nullptr);
+    return rc;
+  });
+}
+
+// The same stack with TF32 tensor-core operands (conv_sm100.cu OP_TF32): weights packed to fp32 TF32 values, features converted to
+// fp32 NHWC (fp32 NCHW rounded to TF32, or bf16 NHWC widened exactly), activations and inter-layer gradients stored as fp32 NHWC
+// rounded to TF32, bias gradients summed from unrounded fp32 values.  Same arguments as the bf16 entries, fp32 where those are bf16.
+int64_t b200seg_disc_backward_tf32_scratch_bytes(int N, int Cin, int h, int w, int ndf1, int ndf2, int C) {
+  if (N <= 0 || Cin <= 0 || h <= 0 || w <= 0 || ndf1 <= 0 || ndf2 <= 0 || C <= 0) return 0;
+  long long m = 0;
+  const long long cands[] = {conv3x3_wgrad_scratch_bytes(N, h, w, 2 * C, ndf2, 0), conv3x3_wgrad_scratch_bytes(N, h, w, ndf2, ndf1, 0),
+                             conv3x3_wgrad_scratch_bytes(N, h, w, ndf1, Cin, 0), conv3x3_dgrad_colsum_scratch_bytes(N, h, w, ndf2),
+                             conv3x3_dgrad_colsum_scratch_bytes(N, h, w, ndf1)};
+  for (long long v : cands) m = v > m ? v : m;
+  return m + 256;
+}
+
+int b200seg_disc_forward_tf32(const void* x, int x_kind, int N, int Cin, int h, int w, int ndf1, int ndf2, int C, const float* w1,
+                              const float* b1, const float* w2, const float* b2, const float* wc1, const float* bc1, const float* wc2,
+                              const float* bc2, float slope, int do_pack, float* Wf1, float* Wb1, float* Wf2, float* Wb2, float* Wf3,
+                              float* Wb3, float* b3, float* Xp, float* A1, float* A2, float* out, void* stream) {
+  REQUIRE_DEVICE();
+  B200SEG_CHECK_ARG(x && Wf1 && Wb1 && Wf2 && Wb2 && Wf3 && Wb3 && b3 && Xp && A1 && A2 && out, "disc_forward_tf32: null pointer");
+  B200SEG_CHECK_ARG(x_kind == 0 || x_kind == 1, "disc_forward_tf32: x_kind must be 0 (fp32 NCHW) or 1 (bf16 NHWC), got %d", x_kind);
+  B200SEG_CHECK_ARG(!do_pack || (w1 && w2 && wc1 && wc2), "disc_forward_tf32: null weight pointer");
+  B200SEG_CHECK_ARG(N > 0 && Cin > 0 && h > 0 && w > 0 && ndf1 > 0 && ndf2 > 0 && C > 0 && Cin % 8 == 0 && ndf1 % 8 == 0 && ndf2 % 8 == 0,
+                    "disc_forward_tf32: bad shape (channel counts must be multiples of 8)");
+  StepKey key = {};
+  int np = 0, ni = 0;
+  const void* ptrs[] = {x, w1, b1, w2, b2, wc1, bc1, wc2, bc2, Wf1, Wb1, Wf2, Wb2, Wf3, Wb3, b3, Xp, A1, A2, out};
+  for (const void* q : ptrs) key.p[np++] = q;
+  int dev = 0;
+  cudaGetDevice(&dev);
+  const long long ints[] = {5, x_kind, N, Cin, h, w, ndf1, ndf2, C, do_pack, dev};
+  for (long long v : ints) key.i[ni++] = v;
+  key.f[0] = slope;
+  return run_step(key, S(stream), true, [&](cudaStream_t st) -> int {
+    int rc;
+    if (do_pack) {
+      const float* weights[4] = {w1, w2, wc1, wc2};
+      const int part_co[4] = {ndf1, ndf2, C, C}, parts_per_layer[3] = {1, 1, 2}, cis[3] = {Cin, ndf1, ndf2};
+      void* Wfs[3] = {Wf1, Wf2, Wf3};
+      void* Wbs[3] = {Wb1, Wb2, Wb3};
+      const int pitches[3] = {round8i(ndf1), round8i(ndf2), round8i(2 * C)};
+      const float* bias_parts[2] = {bc1, bc2};
+      const int bias_lens[2] = {C, C};
+      rc = conv3x3_pack_weights_stack_tf32(3, weights, part_co, parts_per_layer, cis, Wfs, Wbs, pitches, bias_parts, bias_lens, 2, b3, st);
+      if (rc) return rc;
+    }
+    rc = x_kind == 0 ? nchw_to_nhwc_tf32(reinterpret_cast<const float*>(x), N, Cin, h * w, Xp, Cin, st)
+                     : widen_bf16(x, (long long)N * h * w * Cin, Xp, st);
+    if (rc) return rc;
+    rc = conv3x3_forward(Xp, N, h, w, Cin, Cin, Wf1, ndf1, 1, b1, 1, slope, A1, ndf1, nullptr, st, 1);
+    if (rc) return rc;
+    rc = conv3x3_forward(A1, N, h, w, ndf1, ndf1, Wf2, ndf2, 1, b2, 1, slope, A2, ndf2, nullptr, st, 1);
+    if (rc) return rc;
+    return conv3x3_forward(A2, N, h, w, ndf2, ndf2, Wf3, 2 * C, 1, b3, 0, 0.f, nullptr, 2 * C, out, st, 1);
+  });
+}
+
+int b200seg_disc_backward_tf32(const float* grad_out, const float* Xp, const float* A1, const float* A2, const float* Wb1, const float* Wb2,
+                               const float* Wb3, int N, int Cin, int h, int w, int ndf1, int ndf2, int C, float slope, float* G3, float* dZ2,
+                               float* dZ1, void* scratch, int64_t scratch_bytes, float* gw1, float* gb1, float* gw2, float* gb2,
+                               float* gwc1, float* gwc2, float* gb3, float* gx_f32_nchw, void* gx_bf16_nhwc, void* stream) {
+  REQUIRE_DEVICE();
+  B200SEG_CHECK_ARG(grad_out && Xp && A1 && A2 && Wb1 && Wb2 && Wb3 && G3 && scratch, "disc_backward_tf32: null pointer");
+  B200SEG_CHECK_ARG(N > 0 && Cin > 0 && h > 0 && w > 0 && ndf1 > 0 && ndf2 > 0 && C > 0, "disc_backward_tf32: bad shape");
+  B200SEG_CHECK_ARG(!(gx_f32_nchw && gx_bf16_nhwc), "disc_backward_tf32: give at most one feature-gradient destination");
+  const bool need_x = gx_f32_nchw || gx_bf16_nhwc;
+  const bool need_l1 = need_x || gw1 || gb1;
+  const bool need_l2 = need_l1 || gw2 || gb2;
+  B200SEG_CHECK_ARG(!need_l2 || dZ2, "disc_backward_tf32: dZ2 buffer missing");
+  B200SEG_CHECK_ARG(!need_l1 || dZ1, "disc_backward_tf32: dZ1 buffer missing");
+  B200SEG_CHECK_ARG(scratch_bytes >= b200seg_disc_backward_tf32_scratch_bytes(N, Cin, h, w, ndf1, ndf2, C),
+                    "disc_backward_tf32: scratch too small");
+  StepKey key = {};
+  int np = 0, ni = 0;
+  const void* ptrs[] = {grad_out, Xp, A1, A2, Wb1, Wb2, Wb3, G3, dZ2, dZ1, scratch, gw1, gb1, gw2, gb2, gwc1, gwc2, gb3, gx_f32_nchw, gx_bf16_nhwc};
+  for (const void* q : ptrs) key.p[np++] = q;
+  int dev = 0;
+  cudaGetDevice(&dev);
+  const long long ints[] = {6, N, Cin, h, w, ndf1, ndf2, C, scratch_bytes, dev};
+  for (long long v : ints) key.i[ni++] = v;
+  key.f[0] = slope;
+  return run_step(key, S(stream), true, [&](cudaStream_t st) -> int {
+    const int p3 = round8i(2 * C);
+    int rc = nchw_to_nhwc_tf32(grad_out, N, 2 * C, h * w, G3, p3, st);
+    if (rc) return rc;
+    if (gb3) {                                                // cls1 | cls2 bias gradient from the unrounded loss gradient
+      rc = nchw_channel_sum(grad_out, N, 2 * C, h * w, gb3, st);
+      if (rc) return rc;
+    }
+    if (gwc1 || gwc2) {
+      float* outs[2] = {gwc1, gwc2};
+      const int parts[2] = {C, C};
+      rc = conv3x3_wgrad(G3, 2 * C, p3, A2, ndf2, ndf2, N, h, w, 1, 0, scratch, scratch_bytes, outs, parts, 2, st, 1);
+      if (rc) return rc;
+    }
+    if (!need_l2) return B200SEG_OK;
+    rc = conv3x3_dgrad(G3, N, h, w, p3, p3, Wb3, ndf2, 1, A2, slope, dZ2, ndf2, nullptr, st, gb2 ? scratch : nullptr,
+                       gb2 ? scratch_bytes : 0, gb2, 1);
+    if (rc) return rc;
+    if (gw2) {
+      float* outs[1] = {gw2};
+      const int parts[1] = {ndf2};
+      rc = conv3x3_wgrad(dZ2, ndf2, ndf2, A1, ndf1, ndf1, N, h, w, 1, 0, scratch, scratch_bytes, outs, parts, 1, st, 1);
+      if (rc) return rc;
+    }
+    if (!need_l1) return B200SEG_OK;
+    rc = conv3x3_dgrad(dZ2, N, h, w, ndf2, ndf2, Wb2, ndf1, 1, A1, slope, dZ1, ndf1, nullptr, st, gb1 ? scratch : nullptr,
+                       gb1 ? scratch_bytes : 0, gb1, 1);
+    if (rc) return rc;
+    if (gw1) {
+      float* outs[1] = {gw1};
+      const int parts[1] = {ndf1};
+      rc = conv3x3_wgrad(dZ1, ndf1, ndf1, Xp, Cin, Cin, N, h, w, 1, 0, scratch, scratch_bytes, outs, parts, 1, st, 1);
+      if (rc) return rc;
+    }
+    if (need_x)
+      rc = conv3x3_dgrad(dZ1, N, h, w, ndf1, ndf1, Wb1, Cin, 1, nullptr, slope, nullptr, Cin, gx_f32_nchw, st, nullptr, 0, nullptr, 1,
+                         gx_bf16_nhwc);
     return rc;
   });
 }

@@ -172,6 +172,15 @@ __device__ __forceinline__ void cp_async_8s(unsigned smem_dst, const void* gmem_
   asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(smem_dst), "l"(gmem_src) : "memory");
 }
 
+// fp32 -> the nearest TF32 value (10 explicit mantissa bits), ties to even: the low 13 mantissa bits cleared.  Values a tensor
+// core reads as TF32 operands are stored this way, so the product does not depend on how the hardware treats the dropped bits.
+// Inf / NaN pass unchanged.
+__device__ __forceinline__ float tf32_rn(float x) {
+  uint32_t u = __float_as_uint(x);
+  if ((u & 0x7f800000u) != 0x7f800000u) u = (u + 0xfffu + ((u >> 13) & 1u)) & ~0x1fffu;
+  return __uint_as_float(u);
+}
+
 // ---- warp / block reductions ----------------------------------------------------------------
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll

@@ -25,6 +25,13 @@
 //
 // Pipeline / roles are those of gemm_sm100.cuh (4-stage 48 KB TMA ring, one MMA-issuing thread, two 256-column TMEM
 // accumulators, persistent CTAs, 8 epilogue warps).
+//
+// OP_TF32: the same GEMMs with fp32 operands read by tcgen05.mma.kind::tf32.  A 128-byte swizzle row then holds 32 channels, so a
+// k-block is 32 channels (CONV) or 32 pixels (WGRAD), an MMA covers K = 8 (still 32 bytes of a K-major row, 8 k-rows of an
+// MN-major box) and the stage sizes are those of bf16.  MN-major tf32 boxes use the 32-byte-chunk swizzle (SWIZZLE_128B_BASE32B),
+// the one swizzled layout tcgen05 reads MN-major 32-bit operands from.  Activations and inter-layer gradients are fp32 NHWC (OUT_F32_NHWC) rounded
+// to TF32 (nearest-even) when stored, so every operand the tensor core reads is exact; the fused column sums are taken from the
+// unrounded values, and the LeakyReLU' mask is read as fp32.
 #include <limits.h>
 #include "common.cuh"
 #include "gemm_sm100.cuh"
@@ -35,7 +42,18 @@ namespace conv {
 
 constexpr int MAX_T = 9;
 constexpr int MODE_CONV = 0, MODE_WGRAD = 1;
-constexpr int OUT_BF16_NHWC = 0, OUT_F32_NCHW = 1;
+constexpr int OUT_BF16_NHWC = 0, OUT_F32_NCHW = 1, OUT_F32_NHWC = 2;
+constexpr int OP_BF16 = 0, OP_TF32 = 1;
+// channels per 128-byte swizzle row = channels (CONV) or pixels (WGRAD) per k-block
+__host__ __device__ constexpr int op_kb(int op) { return op == OP_TF32 ? 32 : 64; }
+__host__ __device__ constexpr int op_bytes(int op) { return op == OP_TF32 ? 4 : 2; }
+// the kernel's k-block geometry: KB channels or pixels per k-block, UK = the K of one MMA, MN_BOX = bytes of one MN-major box.
+// MN-major tf32 operands take the 32-byte-chunk swizzle (TMA CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B), whose atom is 4 rows of 128 B:
+// MN_SBO = the stride between 4-row k groups, MN_LAYOUT its descriptor layout type.
+template <int OP> struct OpGeom {
+  static constexpr int KB = op_kb(OP), UK = OP == OP_TF32 ? 8 : UMMA_K, MN_BOX = KB * 128;
+  static constexpr uint32_t MN_SBO = OP == OP_TF32 ? 512 : 1024, MN_LAYOUT = OP == OP_TF32 ? SMEM_SW128_BASE32B : SMEM_SW128;
+};
 // BN = accumulator columns per tile: 256, or 128 for layers with <= 128 output channels (half the MMA work of a padded 256)
 // PAIR = two CTAs of a cluster drive ONE tcgen05.mma.cta_group::2 (M = 256: 128 rows per CTA, N = BN): each CTA stages its own
 // A tile and only HALF of the B tile (the tensor core reads the other half from the peer's shared memory), so the bytes a
@@ -86,8 +104,9 @@ struct ConvParams {
   float slope;
   const __nv_bfloat16* mask;   // saved post-activation output of the layer below ([pixels][out_pitch]): multiply by LeakyReLU'
   long long split_stride;  // WGRAD: elements between split-K slabs
-  float* colsum_part;      // CONV + bf16 NHWC output: per (M-tile, warp row quarter) column sums of the STORED (bf16-rounded) values,
+  float* colsum_part;      // CONV + NHWC output: per (M-tile, warp row quarter) column sums of the STORED (bf16-rounded) values,
   int m_tiles_real;        //   [m_tiles_real * 4][out_pitch] -> the bias gradient without another pass over the tensor
+                           //   (OP_TF32 + OUT_F32_NHWC: of the values before their TF32 rounding)
 };
 
 __device__ __forceinline__ void tma_load_3d(uint32_t smem_dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1, int c2) {
@@ -141,7 +160,7 @@ __device__ __forceinline__ Unit decode_unit(const ConvParams& p, int unit, int r
   return u;
 }
 
-template <int MODE, int BN, bool PAIR>
+template <int MODE, int BN, bool PAIR, int OP>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 conv_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b, const ConvParams p) {
   extern __shared__ uint8_t smem_raw[];
@@ -208,17 +227,17 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
           const uint32_t fb = PAIR ? mapa_u32(smem_u32(&full_bar[stage]), 0) : smem_u32(&full_bar[stage]);
           if (MODE == MODE_CONV) {
             const int t = kb / p.KC, kc = kb - t * p.KC;
-            tma_ld4<PAIR>(sa, &tmap_a, fb, kc * BLOCK_K, x0 + p.dx[t], y0 + p.dy[t], img);
-            tma_ld3<PAIR>(sb, &tmap_b, fb, kc * BLOCK_K, u.nt * BLOCK_N + rank * B_ROWS, t);
+            tma_ld4<PAIR>(sa, &tmap_a, fb, kc * OpGeom<OP>::KB, x0 + p.dx[t], y0 + p.dy[t], img);
+            tma_ld3<PAIR>(sb, &tmap_b, fb, kc * OpGeom<OP>::KB, u.nt * BLOCK_N + rank * B_ROWS, t);
           } else {
             rect_origin(p, kb, img, y0, x0);
 #pragma unroll
-            for (int b = 0; b < BLOCK_M / 64; ++b)
-              tma_ld4<PAIR>(sa + b * MN_BOX_BYTES, &tmap_a, fb, u.mt * BLOCK_M + b * 64, x0, y0, img);
+            for (int b = 0; b < BLOCK_M / OpGeom<OP>::KB; ++b)
+              tma_ld4<PAIR>(sa + b * OpGeom<OP>::MN_BOX, &tmap_a, fb, u.mt * BLOCK_M + b * OpGeom<OP>::KB, x0, y0, img);
             const int xs = x0 + p.dx[u.t], ys = y0 + p.dy[u.t];
 #pragma unroll
-            for (int b = 0; b < B_ROWS / 64; ++b)
-              tma_ld4<PAIR>(sb + b * MN_BOX_BYTES, &tmap_b, fb, u.nt * BLOCK_N + rank * B_ROWS + b * 64, xs, ys, img);
+            for (int b = 0; b < B_ROWS / OpGeom<OP>::KB; ++b)
+              tma_ld4<PAIR>(sb + b * OpGeom<OP>::MN_BOX, &tmap_b, fb, u.nt * BLOCK_N + rank * B_ROWS + b * OpGeom<OP>::KB, xs, ys, img);
           }
           if (++stage == STAGES) { stage = 0; phase ^= 1u; }
         }
@@ -227,8 +246,9 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
   } else if (warp == 1) {
     // ================= MMA issuer =================
     if (lane == 0 && rank == 0) {                                    // PAIR: the leader CTA issues for both
-      constexpr uint32_t idesc = make_idesc(MN, MN, BLOCK_M * NCTA, BLOCK_N);
-      constexpr uint32_t lbo = MN ? MN_BOX_BYTES : 16, sbo = 1024, step = MN ? 2048 : 32;
+      constexpr uint32_t idesc = make_idesc(MN, MN, BLOCK_M * NCTA, BLOCK_N, OP == OP_TF32 ? IDESC_TF32 : IDESC_BF16);
+      constexpr uint32_t lbo = MN ? OpGeom<OP>::MN_BOX : 16, sbo = MN ? OpGeom<OP>::MN_SBO : 1024, step = MN ? OpGeom<OP>::UK * 128 : 32;
+      constexpr uint32_t layout = MN ? OpGeom<OP>::MN_LAYOUT : SMEM_SW128;
       int stage = 0;
       uint32_t phase = 0;
       int acc = 0;
@@ -244,11 +264,16 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
           const uint32_t sa = smem_u32(smem + stage * STAGE_BYTES);
           const uint32_t sb = sa + A_BYTES;
 #pragma unroll
-          for (int k = 0; k < BLOCK_K / UMMA_K; ++k) {
-            const uint64_t adesc = make_smem_desc(sa + k * step, lbo, sbo);
-            const uint64_t bdesc = make_smem_desc(sb + k * step, lbo, sbo);
-            if (PAIR) umma_bf16_2sm(tmem_d, adesc, bdesc, idesc, (kb > u.kb0 || k > 0) ? 1u : 0u);
-            else umma_bf16(tmem_d, adesc, bdesc, idesc, (kb > u.kb0 || k > 0) ? 1u : 0u);
+          for (int k = 0; k < OpGeom<OP>::KB / OpGeom<OP>::UK; ++k) {
+            const uint64_t adesc = make_smem_desc(sa + k * step, lbo, sbo, layout);
+            const uint64_t bdesc = make_smem_desc(sb + k * step, lbo, sbo, layout);
+            if constexpr (OP == OP_TF32) {
+              if (PAIR) umma_tf32_2sm(tmem_d, adesc, bdesc, idesc, (kb > u.kb0 || k > 0) ? 1u : 0u);
+              else umma_tf32(tmem_d, adesc, bdesc, idesc, (kb > u.kb0 || k > 0) ? 1u : 0u);
+            } else {
+              if (PAIR) umma_bf16_2sm(tmem_d, adesc, bdesc, idesc, (kb > u.kb0 || k > 0) ? 1u : 0u);
+              else umma_bf16(tmem_d, adesc, bdesc, idesc, (kb > u.kb0 || k > 0) ? 1u : 0u);
+            }
           }
           if (PAIR) umma_commit_2sm(&empty_bar[stage], 0x3);         // frees the stage in both CTAs
           else umma_commit(&empty_bar[stage]);
@@ -296,7 +321,47 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
 #pragma unroll
             for (int j = 0; j < 32; ++j) v[j] = v[j] > 0.f ? v[j] : v[j] * p.slope;
           }
-          if (p.mask && valid) {
+          if constexpr (OP == OP_TF32) {
+            if (p.mask && valid) {
+              const float4* mp = reinterpret_cast<const float4*>(reinterpret_cast<const float*>(p.mask) + pix * p.out_pitch + col0);
+#pragma unroll
+              for (int k = 0; k < 8; ++k) {
+                if (col0 + 4 * k < p.Co) {
+                  const float4 m4 = __ldg(mp + k);
+                  v[4 * k] *= m4.x > 0.f ? 1.f : p.slope;                 // ATen's x > 0 test: LeakyReLU'(0) = slope
+                  v[4 * k + 1] *= m4.y > 0.f ? 1.f : p.slope;
+                  v[4 * k + 2] *= m4.z > 0.f ? 1.f : p.slope;
+                  v[4 * k + 3] *= m4.w > 0.f ? 1.f : p.slope;
+                }
+              }
+            }
+            if (p.out_mode == OUT_F32_NHWC) {
+              if (valid) {
+                float4* op = reinterpret_cast<float4*>(reinterpret_cast<float*>(p.out) + pix * p.out_pitch + col0);
+#pragma unroll
+                for (int k = 0; k < 8; ++k)
+                  if (col0 + 4 * k < p.Co)
+                    op[k] = make_float4(tf32_rn(v[4 * k]), tf32_rn(v[4 * k + 1]), tf32_rn(v[4 * k + 2]), tf32_rn(v[4 * k + 3]));
+              }
+              if (p.colsum_part) {                                 // the unrounded values (a bias gradient never passes through TF32)
+#pragma unroll
+                for (int j = 0; j < 32; ++j) v[j] = valid ? v[j] : 0.f;
+#pragma unroll
+                for (int sft = 16; sft >= 1; sft >>= 1) {          // the exchange of the bf16 path below
+                  const bool up = (lane & sft) != 0;
+#pragma unroll
+                  for (int i = 0; i < sft; ++i) {
+                    const float send = up ? v[i] : v[i + sft];
+                    const float keep = up ? v[i + sft] : v[i];
+                    v[i] = keep + __shfl_xor_sync(0xffffffffu, send, sft);
+                  }
+                }
+                if (u.mt < p.m_tiles_real && col0 + lane < p.Co)
+                  p.colsum_part[((long long)u.mt * 4 + wq) * p.out_pitch + col0 + lane] = v[0];
+              }
+              continue;
+            }
+          } else if (p.mask && valid) {
             const uint4* mp = reinterpret_cast<const uint4*>(p.mask + pix * p.out_pitch + col0);
 #pragma unroll
             for (int k = 0; k < 4; ++k) {
@@ -402,7 +467,7 @@ conv_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_consta
 // host: tensor maps
 // ------------------------------------------------------------------------------------------
 static int make_tmap_nd(CUtensorMap* m, const void* ptr, int rank, const cuuint64_t* gdim, const cuuint64_t* gstride_bytes,
-                        const cuuint32_t* box) {
+                        const cuuint32_t* box, int op, bool mn = false) {
   EncodeTiledFn fn = encode_fn();
   if (!fn) {
     set_error("cuTensorMapEncodeTiled entry point not available (driver too old or no GPU)");
@@ -413,8 +478,9 @@ static int make_tmap_nd(CUtensorMap* m, const void* ptr, int rank, const cuuint6
     B200SEG_CHECK_ARG(gstride_bytes[i] % 16 == 0, "conv: TMA stride %d (%llu bytes) must be a multiple of 16", i,
                       (unsigned long long)gstride_bytes[i]);
   cuuint32_t estr[5] = {1, 1, 1, 1, 1};
-  CUresult r = fn(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, (cuuint32_t)rank, const_cast<void*>(ptr), gdim, gstride_bytes, box, estr,
-                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+  CUresult r = fn(m, op == OP_TF32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, (cuuint32_t)rank, const_cast<void*>(ptr), gdim, gstride_bytes, box, estr,
+                  CU_TENSOR_MAP_INTERLEAVE_NONE,
+                  (mn && op == OP_TF32) ? CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B : CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
     set_error("conv: cuTensorMapEncodeTiled (rank %d) failed with CUresult %d", rank, (int)r);
@@ -423,12 +489,15 @@ static int make_tmap_nd(CUtensorMap* m, const void* ptr, int rank, const cuuint6
   return B200SEG_OK;
 }
 
-// activation map over bf16 NHWC [N][h][w][pitch] exposing `C` channels, box {64, TW, TH, 1}
-static int make_act_tmap(CUtensorMap* m, const void* ptr, int N, int h, int w, int C, long long pitch, int TW, int TH) {
+// activation map over NHWC [N][h][w][pitch] (bf16, or fp32 with OP_TF32) exposing `C` channels, box {64 | 32, TW, TH, 1};
+// mn: the box is an MN-major operand (weight-gradient mode)
+static int make_act_tmap(CUtensorMap* m, const void* ptr, int N, int h, int w, int C, long long pitch, int TW, int TH, int op,
+                         bool mn = false) {
+  const cuuint64_t es = (cuuint64_t)op_bytes(op);
   cuuint64_t gdim[4] = {(cuuint64_t)C, (cuuint64_t)w, (cuuint64_t)h, (cuuint64_t)N};
-  cuuint64_t gstr[3] = {(cuuint64_t)pitch * 2, (cuuint64_t)pitch * 2 * w, (cuuint64_t)pitch * 2 * w * h};
-  cuuint32_t box[4] = {64, (cuuint32_t)TW, (cuuint32_t)TH, 1};
-  return make_tmap_nd(m, ptr, 4, gdim, gstr, box);
+  cuuint64_t gstr[3] = {(cuuint64_t)pitch * es, (cuuint64_t)pitch * es * w, (cuuint64_t)pitch * es * w * h};
+  cuuint32_t box[4] = {(cuuint32_t)op_kb(op), (cuuint32_t)TW, (cuuint32_t)TH, 1};
+  return make_tmap_nd(m, ptr, 4, gdim, gstr, box, op, mn);
 }
 
 // pixel rectangle of `area` pixels (power of two) with the least padding over an h x w image; ties -> widest
@@ -455,17 +524,17 @@ static int ilog2(int v) { int s = 0; while ((1 << s) < v) ++s; return s; }
 static int g_pair = 1;                 // b200seg_conv_set_pair(): 0 = one CTA per tile, 1 = CTA pairs (cta_group::2) where two M-tiles exist
 void set_pair(int on) { g_pair = on; }
 
-template <int MODE, int BN, bool PAIR>
+template <int MODE, int BN, bool PAIR, int OP>
 static int launch_conv_t(const CUtensorMap& ta, const CUtensorMap& tb, const ConvParams& p, cudaStream_t stream) {
   static bool configured = false;
   if (!configured) {
-    B200SEG_CUDA(cudaFuncSetAttribute(conv_gemm_kernel<MODE, BN, PAIR>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg<BN, PAIR>::SMEM));
+    B200SEG_CUDA(cudaFuncSetAttribute(conv_gemm_kernel<MODE, BN, PAIR, OP>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg<BN, PAIR>::SMEM));
     configured = true;
   }
   const int sms = num_sms();
   if (!PAIR) {
     const int grid = p.units < sms ? p.units : sms;
-    conv_gemm_kernel<MODE, BN, PAIR><<<grid, NUM_THREADS, Cfg<BN, PAIR>::SMEM, stream>>>(ta, tb, p);
+    conv_gemm_kernel<MODE, BN, PAIR, OP><<<grid, NUM_THREADS, Cfg<BN, PAIR>::SMEM, stream>>>(ta, tb, p);
   } else {
     const int pairs = p.units < sms / 2 ? p.units : sms / 2;
     cudaLaunchConfig_t cfg = {};
@@ -480,30 +549,36 @@ static int launch_conv_t(const CUtensorMap& ta, const CUtensorMap& tb, const Con
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    B200SEG_CUDA(cudaLaunchKernelEx(&cfg, conv_gemm_kernel<MODE, BN, PAIR>, ta, tb, p));
+    B200SEG_CUDA(cudaLaunchKernelEx(&cfg, conv_gemm_kernel<MODE, BN, PAIR, OP>, ta, tb, p));
   }
   B200SEG_LAUNCH_CHECK();
   return B200SEG_OK;
 }
+template <int MODE, int OP>
+static int launch_conv_op(const CUtensorMap& ta, const CUtensorMap& tb, const ConvParams& p, int BN, bool pair, cudaStream_t stream) {
+  if (BN == 128) return pair ? launch_conv_t<MODE, 128, true, OP>(ta, tb, p, stream) : launch_conv_t<MODE, 128, false, OP>(ta, tb, p, stream);
+  return pair ? launch_conv_t<MODE, 256, true, OP>(ta, tb, p, stream) : launch_conv_t<MODE, 256, false, OP>(ta, tb, p, stream);
+}
 template <int MODE>
-static int launch_conv(const CUtensorMap& ta, const CUtensorMap& tb, const ConvParams& p, int BN, bool pair, cudaStream_t stream) {
-  if (BN == 128) return pair ? launch_conv_t<MODE, 128, true>(ta, tb, p, stream) : launch_conv_t<MODE, 128, false>(ta, tb, p, stream);
-  return pair ? launch_conv_t<MODE, 256, true>(ta, tb, p, stream) : launch_conv_t<MODE, 256, false>(ta, tb, p, stream);
+static int launch_conv(const CUtensorMap& ta, const CUtensorMap& tb, const ConvParams& p, int BN, bool pair, int op, cudaStream_t stream) {
+  return op == OP_TF32 ? launch_conv_op<MODE, OP_TF32>(ta, tb, p, BN, pair, stream) : launch_conv_op<MODE, OP_BF16>(ta, tb, p, BN, pair, stream);
 }
 
-// D[pixel, co] = sum_t sum_ck act[pixel + sign*d_t, ck] * wt[t][co][ck]  (+ epilogue), see the header comment
+// D[pixel, co] = sum_t sum_ck act[pixel + sign*d_t, ck] * wt[t][co][ck]  (+ epilogue), see the header comment.  act, wt and
+// mask are bf16 (OP_BF16) or fp32 holding TF32 values (OP_TF32)
 static int conv3x3_run(const void* act, int N, int h, int w, int Ck, long long act_pitch, const void* wt, int Co, int dilation, int sign,
                        const float* bias, int lrelu, float slope, const void* mask, void* out, int out_mode, long long out_pitch,
-                       cudaStream_t stream, int prof_tag, float* colsum_part = nullptr) {
+                       cudaStream_t stream, int prof_tag, float* colsum_part, int op) {
   B200SEG_CHECK_ARG(act && wt && out, "conv3x3: null pointer");
-  B200SEG_CHECK_ARG(!colsum_part || out_mode == OUT_BF16_NHWC, "conv3x3: fused column sums need the bf16 NHWC output");
+  B200SEG_CHECK_ARG(out_mode != OUT_F32_NHWC || op == OP_TF32, "conv3x3: the fp32 NHWC output belongs to the TF32 layers");
+  B200SEG_CHECK_ARG(!colsum_part || out_mode != OUT_F32_NCHW, "conv3x3: fused column sums need an NHWC output");
   B200SEG_CHECK_ARG(N > 0 && h > 0 && w > 0 && Ck > 0 && Co > 0 && dilation > 0, "conv3x3: bad geometry");
   B200SEG_CHECK_ARG(Ck % 8 == 0 && act_pitch % 8 == 0 && act_pitch >= Ck, "conv3x3: input channels (%d, pitch %lld) must be multiples of 8", Ck, act_pitch);
   B200SEG_CHECK_ARG((long long)N * h * w < (1LL << 31), "conv3x3: too many pixels");
-  if (out_mode == OUT_BF16_NHWC || mask)
+  if (out_mode != OUT_F32_NCHW || mask)
     B200SEG_CHECK_ARG(Co % 8 == 0 && out_pitch % 8 == 0 && out_pitch >= Co && (reinterpret_cast<uintptr_t>(out) & 15) == 0 &&
                           (reinterpret_cast<uintptr_t>(mask) & 15) == 0,
-                      "conv3x3: bf16 NHWC output / mask need channel counts that are multiples of 8 and 16-byte aligned bases");
+                      "conv3x3: NHWC output / mask need channel counts that are multiples of 8 and 16-byte aligned bases");
   ConvParams p = {};
   p.N = N; p.h = h; p.w = w;
   pick_rect(h, w, BLOCK_M, &p.TW, &p.TH);
@@ -511,7 +586,7 @@ static int conv3x3_run(const void* act, int N, int h, int w, int Ck, long long a
   p.tiles_x = ceil_div(w, p.TW);
   p.tiles_y = ceil_div(h, p.TH);
   fill_taps(p, dilation, sign);
-  p.KC = ceil_div(Ck, BLOCK_K);
+  p.KC = ceil_div(Ck, op_kb(op));
   p.Co = Co; p.Ci = 0;
   const int BN = Co <= 128 ? 128 : 256;
   p.m_tiles = N * p.tiles_x * p.tiles_y;
@@ -529,17 +604,18 @@ static int conv3x3_run(const void* act, int N, int h, int w, int Ck, long long a
   p.mask = reinterpret_cast<const __nv_bfloat16*>(mask);
   p.split_stride = 0;
   CUtensorMap ta, tb;
-  int rc = make_act_tmap(&ta, act, N, h, w, Ck, act_pitch, p.TW, p.TH);
+  int rc = make_act_tmap(&ta, act, N, h, w, Ck, act_pitch, p.TW, p.TH, op);
   if (rc) return rc;
   {
+    const cuuint64_t es = (cuuint64_t)op_bytes(op);
     cuuint64_t gdim[3] = {(cuuint64_t)Ck, (cuuint64_t)Co, (cuuint64_t)p.T};
-    cuuint64_t gstr[2] = {(cuuint64_t)Ck * 2, (cuuint64_t)Ck * 2 * Co};
-    cuuint32_t box[3] = {64, (cuuint32_t)(pair ? BN / 2 : BN), 1};
-    rc = make_tmap_nd(&tb, wt, 3, gdim, gstr, box);
+    cuuint64_t gstr[2] = {(cuuint64_t)Ck * es, (cuuint64_t)Ck * es * Co};
+    cuuint32_t box[3] = {(cuuint32_t)op_kb(op), (cuuint32_t)(pair ? BN / 2 : BN), 1};
+    rc = make_tmap_nd(&tb, wt, 3, gdim, gstr, box, op);
     if (rc) return rc;
   }
   profile_begin(prof_tag, stream);
-  rc = launch_conv<MODE_CONV>(ta, tb, p, BN, pair, stream);
+  rc = launch_conv<MODE_CONV>(ta, tb, p, BN, pair, op, stream);
   profile_end(prof_tag, stream);
   return rc;
 }
@@ -565,16 +641,17 @@ static int conv3x3_wgrad_splits(int N, int h, int w, int Co, int Ci) {
   return s;
 }
 
-// slabs[z][t][Co][Ci] = sum over the pixels of split z of g[pixel, co] * x[pixel + d_t, ci]
+// slabs[z][t][Co][Ci] = sum over the pixels of split z of g[pixel, co] * x[pixel + d_t, ci].  The split count is planned on 64-pixel
+// chunks for both operand types (OP_TF32 runs 32-pixel k-blocks: the same splits, twice the k-blocks each)
 static int conv3x3_wgrad_run(const void* g, int Co, long long g_pitch, const void* x, int Ci, long long x_pitch, int N, int h, int w,
-                             int dilation, int splits, float* slabs, int* splits_used, cudaStream_t stream, int prof_tag) {
+                             int dilation, int splits, float* slabs, int* splits_used, cudaStream_t stream, int prof_tag, int op) {
   B200SEG_CHECK_ARG(g && x && slabs, "conv3x3_wgrad: null pointer");
   B200SEG_CHECK_ARG(N > 0 && h > 0 && w > 0 && Co > 0 && Ci > 0 && dilation > 0, "conv3x3_wgrad: bad geometry");
   B200SEG_CHECK_ARG(g_pitch % 8 == 0 && x_pitch % 8 == 0 && Ci % 4 == 0 && x_pitch >= Ci, "conv3x3_wgrad: channel pitches must be multiples of 8");
   B200SEG_CHECK_ARG((reinterpret_cast<uintptr_t>(slabs) & 15) == 0, "conv3x3_wgrad: slabs must be 16-byte aligned");
   ConvParams p = {};
   p.N = N; p.h = h; p.w = w;
-  pick_rect(h, w, BLOCK_K, &p.TW, &p.TH);
+  pick_rect(h, w, op_kb(op), &p.TW, &p.TH);
   p.tw_shift = ilog2(p.TW);
   p.tiles_x = ceil_div(w, p.TW);
   p.tiles_y = ceil_div(h, p.TH);
@@ -598,12 +675,12 @@ static int conv3x3_wgrad_run(const void* g, int Co, long long g_pitch, const voi
   CUtensorMap ta, tb;
   // the gradient map exposes min(g_pitch, ...) channels: the zero padding of a padded gradient tensor is harmless, channels
   // beyond the pitch are zero-filled by TMA
-  int rc = make_act_tmap(&ta, g, N, h, w, (int)g_pitch, g_pitch, p.TW, p.TH);
+  int rc = make_act_tmap(&ta, g, N, h, w, (int)g_pitch, g_pitch, p.TW, p.TH, op, true);
   if (rc) return rc;
-  rc = make_act_tmap(&tb, x, N, h, w, Ci, x_pitch, p.TW, p.TH);
+  rc = make_act_tmap(&tb, x, N, h, w, Ci, x_pitch, p.TW, p.TH, op, true);
   if (rc) return rc;
   profile_begin(prof_tag, stream);
-  rc = launch_conv<MODE_WGRAD>(ta, tb, p, BN, pair, stream);
+  rc = launch_conv<MODE_WGRAD>(ta, tb, p, BN, pair, op, stream);
   profile_end(prof_tag, stream);
   return rc;
 }
@@ -614,7 +691,8 @@ static int conv3x3_wgrad_run(const void* g, int Co, long long g_pitch, const voi
 // ------------------------------------------------------------------------------------------
 // helper kernels
 // ------------------------------------------------------------------------------------------
-// w fp32 [Co_part][Ci][3][3] -> Wf bf16 [9][Co_total][Ci] (rows co0 + co) and Wb bf16 [9][Ci][co_pitch] (columns co0 + co).
+// w fp32 [Co_part][Ci][3][3] -> Wf bf16 [9][Co_total][Ci] (rows co0 + co) and Wb bf16 [9][Ci][co_pitch] (columns co0 + co);
+// with TF32 the same layouts in fp32, every value rounded to TF32.
 // ONE launch packs every weight tensor of a layer -- or of the whole discriminator stack -- from a job table in the kernel
 // parameters (training re-packs every step: four launches + three memsets + a concatenation cost ~70 us of device time, mostly
 // dependency latency between tiny nodes).  A block owns 16 output x 64 input channels of one job: 16 contiguous runs of 576 floats
@@ -625,8 +703,8 @@ constexpr int CPW_CO = 16, CPW_CI = 64, CPW_PITCH = CPW_CI * 9 + 1;      // odd 
 constexpr int CPW_MAX_JOBS = 8, CPW_MAX_BIAS = 4;
 struct PackJob {
   const float* w;
-  __nv_bfloat16* Wf;
-  __nv_bfloat16* Wb;
+  void* Wf;                // __nv_bfloat16, or float with TF32
+  void* Wb;
   int Co_part, Ci, co0, Co_total, co_pitch, tiles_ci, tile0, zero_pad;
 };
 struct PackTable {
@@ -637,6 +715,12 @@ struct PackTable {
   int n_bias;
   float* bias_dst;
 };
+template <bool TF32>
+__device__ __forceinline__ void pack_store(void* base, long long i, float v) {
+  if (TF32) reinterpret_cast<float*>(base)[i] = tf32_rn(v);
+  else reinterpret_cast<__nv_bfloat16*>(base)[i] = __float2bfloat16(v);
+}
+template <bool TF32>
 __global__ void __launch_bounds__(256) conv_pack_weights_kernel(const PackTable t) {
   __shared__ float sm[CPW_CO * CPW_PITCH];
   if (blockIdx.x == 0 && t.bias_dst) {
@@ -665,20 +749,20 @@ __global__ void __launch_bounds__(256) conv_pack_weights_kernel(const PackTable 
     for (int i = threadIdx.x; i < 9 * CPW_CO * CPW_CI; i += 256) {         // ci fastest
       const int ci_l = i & (CPW_CI - 1), co_l = (i >> 6) & (CPW_CO - 1), k = i >> 10;
       if (ci_l < nci && co_l < nco)
-        j.Wf[((long long)k * j.Co_total + j.co0 + cop0 + co_l) * j.Ci + ci0 + ci_l] = __float2bfloat16(sm[co_l * CPW_PITCH + ci_l * 9 + k]);
+        pack_store<TF32>(j.Wf, ((long long)k * j.Co_total + j.co0 + cop0 + co_l) * j.Ci + ci0 + ci_l, sm[co_l * CPW_PITCH + ci_l * 9 + k]);
     }
   }
   if (j.Wb) {
     for (int i = threadIdx.x; i < 9 * CPW_CI * CPW_CO; i += 256) {         // co fastest
       const int co_l = i & (CPW_CO - 1), ci_l = (i >> 4) & (CPW_CI - 1), k = i >> 10;
       if (ci_l < nci && co_l < nco)
-        j.Wb[((long long)k * j.Ci + ci0 + ci_l) * j.co_pitch + j.co0 + cop0 + co_l] = __float2bfloat16(sm[co_l * CPW_PITCH + ci_l * 9 + k]);
+        pack_store<TF32>(j.Wb, ((long long)k * j.Ci + ci0 + ci_l) * j.co_pitch + j.co0 + cop0 + co_l, sm[co_l * CPW_PITCH + ci_l * 9 + k]);
     }
     const int npad = j.co_pitch - j.Co_total;
     if (j.zero_pad && cop0 == 0 && npad > 0) {
       for (int i = threadIdx.x; i < 9 * nci * npad; i += 256) {
         const int c = i % npad, kc = i / npad, ci_l = kc % nci, k = kc / nci;
-        j.Wb[((long long)k * j.Ci + ci0 + ci_l) * j.co_pitch + j.Co_total + c] = __float2bfloat16(0.f);
+        pack_store<TF32>(j.Wb, ((long long)k * j.Ci + ci0 + ci_l) * j.co_pitch + j.Co_total + c, 0.f);
       }
     }
   }
@@ -718,6 +802,42 @@ __global__ void __launch_bounds__(256) colsum_final_kernel(const float* __restri
   for (int b = lane; b < blocks; b += 32) s += (double)part[(long long)b * pitch + c];
   s = warp_sum_d(s);
   if (lane == 0) out[c] = (float)s;
+}
+
+// out[c] = sum over n, s of src[n][c][s] (fp32 NCHW): the bias gradient of the TF32 cls1 | cls2 layer straight from the unrounded
+// loss gradient.  One block per channel, fixed order (per-thread strided sums, then a double warp / block tree): deterministic
+__global__ void __launch_bounds__(256) nchw_channel_sum_kernel(const float* __restrict__ src, int N, int C, int hw, float* __restrict__ out) {
+  __shared__ double red[8];
+  const int c = blockIdx.x;
+  float acc = 0.f;
+  for (int n = 0; n < N; ++n) {
+    const float* row = src + ((long long)n * C + c) * hw;
+    for (int s = threadIdx.x; s < hw; s += 256) acc += __ldg(row + s);
+  }
+  double d = warp_sum_d((double)acc);
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = d;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    double t = 0.0;
+    for (int i = 0; i < 8; ++i) t += red[i];
+    out[c] = (float)t;
+  }
+}
+
+// bf16 [n] -> fp32 [n] (exact; n a multiple of 8, 16-byte aligned): seam-format features as the TF32 layers' operand
+__global__ void __launch_bounds__(256) widen_bf16_kernel(const uint4* __restrict__ src, long long n8, float4* __restrict__ dst) {
+  for (long long i = blockIdx.x * 256LL + threadIdx.x; i < n8; i += (long long)gridDim.x * 256) {
+    const uint4 q = __ldcs(src + i);
+    const uint32_t wv[4] = {q.x, q.y, q.z, q.w};
+    float f[8];
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+      f[2 * e] = __uint_as_float(wv[e] << 16);
+      f[2 * e + 1] = __uint_as_float(wv[e] & 0xFFFF0000u);
+    }
+    dst[2 * i] = make_float4(f[0], f[1], f[2], f[3]);
+    dst[2 * i + 1] = make_float4(f[4], f[5], f[6], f[7]);
+  }
 }
 
 // split-K slabs [S][9][Co_total][Ci] -> gw [Co_part][Ci][3][3] for rows co0 .. co0 + Co_part
@@ -778,7 +898,7 @@ static int pack_add_layer(PackTable& t, const float* const* weights, const int* 
   int co0 = 0;
   for (int i = 0; i < n_parts; ++i) {
     PackJob& j = t.job[t.n++];
-    j.w = weights[i]; j.Wf = (__nv_bfloat16*)Wf; j.Wb = (__nv_bfloat16*)Wb;
+    j.w = weights[i]; j.Wf = Wf; j.Wb = Wb;
     j.Co_part = part_co[i]; j.Ci = Ci; j.co0 = co0; j.Co_total = Co_total; j.co_pitch = co_pitch;
     j.tiles_ci = ceil_div(Ci, CPW_CI);
     j.tile0 = t.total_tiles;
@@ -789,8 +909,9 @@ static int pack_add_layer(PackTable& t, const float* const* weights, const int* 
   return B200SEG_OK;
 }
 
-static int pack_launch(const PackTable& t, cudaStream_t stream) {
-  conv_pack_weights_kernel<<<t.total_tiles, 256, 0, stream>>>(t);
+static int pack_launch(const PackTable& t, cudaStream_t stream, bool tf32 = false) {
+  if (tf32) conv_pack_weights_kernel<true><<<t.total_tiles, 256, 0, stream>>>(t);
+  else conv_pack_weights_kernel<false><<<t.total_tiles, 256, 0, stream>>>(t);
   B200SEG_LAUNCH_CHECK();
   return B200SEG_OK;
 }
@@ -806,9 +927,9 @@ int conv3x3_pack_weights(const float* const* weights, const int* part_co, int n_
 
 // a whole stack of layers in one launch: layer l owns parts [first, first + parts_per_layer[l]) of the flattened weights / part_co
 // arrays; bias_parts (optional, n_bias <= 4 device pointers, NULL = zeros) are concatenated into bias_out
-int conv3x3_pack_weights_stack(int n_layers, const float* const* weights, const int* part_co, const int* parts_per_layer,
-                               const int* Ci, void* const* Wf, void* const* Wb, const int* co_pitch, const float* const* bias_parts,
-                               const int* bias_len, int n_bias, float* bias_out, cudaStream_t stream) {
+static int pack_weights_stack(int n_layers, const float* const* weights, const int* part_co, const int* parts_per_layer, const int* Ci,
+                              void* const* Wf, void* const* Wb, const int* co_pitch, const float* const* bias_parts, const int* bias_len,
+                              int n_bias, float* bias_out, cudaStream_t stream, bool tf32) {
   B200SEG_CHECK_ARG(n_layers >= 1 && weights && part_co && parts_per_layer && Ci && Wf && Wb && co_pitch,
                     "conv3x3_pack_weights_stack: bad arguments");
   B200SEG_CHECK_ARG(n_bias >= 0 && n_bias <= CPW_MAX_BIAS && (n_bias == 0 || (bias_parts && bias_len && bias_out)),
@@ -823,7 +944,41 @@ int conv3x3_pack_weights_stack(int n_layers, const float* const* weights, const 
   t.n_bias = n_bias;
   t.bias_dst = n_bias ? bias_out : nullptr;
   for (int i = 0; i < n_bias; ++i) { t.bias_src[i] = bias_parts[i]; t.bias_len[i] = bias_len[i]; }
-  return pack_launch(t, stream);
+  return pack_launch(t, stream, tf32);
+}
+
+int conv3x3_pack_weights_stack(int n_layers, const float* const* weights, const int* part_co, const int* parts_per_layer,
+                               const int* Ci, void* const* Wf, void* const* Wb, const int* co_pitch, const float* const* bias_parts,
+                               const int* bias_len, int n_bias, float* bias_out, cudaStream_t stream) {
+  return pack_weights_stack(n_layers, weights, part_co, parts_per_layer, Ci, Wf, Wb, co_pitch, bias_parts, bias_len, n_bias, bias_out,
+                            stream, false);
+}
+
+// the same layouts in fp32, rounded to TF32: the operands of the TF32 layers
+int conv3x3_pack_weights_stack_tf32(int n_layers, const float* const* weights, const int* part_co, const int* parts_per_layer,
+                                    const int* Ci, void* const* Wf, void* const* Wb, const int* co_pitch, const float* const* bias_parts,
+                                    const int* bias_len, int n_bias, float* bias_out, cudaStream_t stream) {
+  return pack_weights_stack(n_layers, weights, part_co, parts_per_layer, Ci, Wf, Wb, co_pitch, bias_parts, bias_len, n_bias, bias_out,
+                            stream, true);
+}
+
+int nchw_channel_sum(const float* src, int N, int C, int hw, float* out, cudaStream_t stream) {
+  B200SEG_CHECK_ARG(src && out && N > 0 && C > 0 && hw > 0, "nchw_channel_sum: bad arguments");
+  nchw_channel_sum_kernel<<<C, 256, 0, stream>>>(src, N, C, hw, out);
+  B200SEG_LAUNCH_CHECK();
+  return B200SEG_OK;
+}
+
+int widen_bf16(const void* src, long long n, float* dst, cudaStream_t stream) {
+  B200SEG_CHECK_ARG(src && dst && n > 0 && n % 8 == 0 && (reinterpret_cast<uintptr_t>(src) & 15) == 0 &&
+                        (reinterpret_cast<uintptr_t>(dst) & 15) == 0,
+                    "widen_bf16: bad arguments (n a multiple of 8, 16-byte aligned buffers)");
+  const long long n8 = n / 8;
+  const long long blocks = ceil_div_ll(n8, 256);
+  widen_bf16_kernel<<<(int)(blocks < 4L * num_sms() ? blocks : 4L * num_sms()), 256, 0, stream>>>(
+      reinterpret_cast<const uint4*>(src), n8, reinterpret_cast<float4*>(dst));
+  B200SEG_LAUNCH_CHECK();
+  return B200SEG_OK;
 }
 
 
@@ -846,7 +1001,7 @@ long long conv3x3_wgrad_scratch_bytes(int N, int h, int w, int Co, int Ci, int s
 
 int conv3x3_wgrad(const void* g, int Co, long long g_pitch, const void* x, int Ci, long long x_pitch, int N, int h, int w, int dilation,
                   int splits, void* scratch, long long scratch_bytes, float* const* grad_w, const int* part_co, int n_parts,
-                  cudaStream_t stream) {
+                  cudaStream_t stream, int tf32) {
   B200SEG_CHECK_ARG(grad_w && part_co && n_parts >= 1 && scratch, "conv3x3_wgrad: bad arguments");
   int Co_total = 0;
   for (int i = 0; i < n_parts; ++i) Co_total += part_co[i];
@@ -854,7 +1009,8 @@ int conv3x3_wgrad(const void* g, int Co, long long g_pitch, const void* x, int C
   if (splits < 1) splits = gemm::conv::conv3x3_wgrad_splits(N, h, w, Co, Ci);
   B200SEG_CHECK_ARG(scratch_bytes >= (long long)splits * 9 * Co * Ci * 4, "conv3x3_wgrad: scratch too small");
   int used = 1;
-  int rc = gemm::conv::conv3x3_wgrad_run(g, Co, g_pitch, x, Ci, x_pitch, N, h, w, dilation, splits, (float*)scratch, &used, stream, 14);
+  int rc = gemm::conv::conv3x3_wgrad_run(g, Co, g_pitch, x, Ci, x_pitch, N, h, w, dilation, splits, (float*)scratch, &used, stream, 14,
+                                         tf32 ? gemm::conv::OP_TF32 : gemm::conv::OP_BF16);
   if (rc) return rc;
   int co0 = 0;
   for (int i = 0; i < n_parts; ++i) {
@@ -874,14 +1030,16 @@ int conv3x3_wgrad(const void* g, int Co, long long g_pitch, const void* x, int C
 }
 
 int conv3x3_forward(const void* act, int N, int h, int w, int Ck, long long act_pitch, const void* Wf, int Co, int dilation,
-                    const float* bias, int lrelu, float slope, void* out_bf16_nhwc, long long out_pitch, float* out_f32_nchw,
-                    cudaStream_t stream) {
-  B200SEG_CHECK_ARG((out_bf16_nhwc != nullptr) != (out_f32_nchw != nullptr), "conv3x3_forward: give exactly one output");
-  if (out_bf16_nhwc)
-    return gemm::conv::conv3x3_run(act, N, h, w, Ck, act_pitch, Wf, Co, dilation, 1, bias, lrelu, slope, nullptr, out_bf16_nhwc,
-                                   gemm::conv::OUT_BF16_NHWC, out_pitch, stream, 12);
-  return gemm::conv::conv3x3_run(act, N, h, w, Ck, act_pitch, Wf, Co, dilation, 1, bias, lrelu, slope, nullptr, out_f32_nchw,
-                                 gemm::conv::OUT_F32_NCHW, 0, stream, 12);
+                    const float* bias, int lrelu, float slope, void* out_nhwc, long long out_pitch, float* out_f32_nchw,
+                    cudaStream_t stream, int tf32) {
+  using namespace gemm::conv;
+  B200SEG_CHECK_ARG((out_nhwc != nullptr) != (out_f32_nchw != nullptr), "conv3x3_forward: give exactly one output");
+  const int op = tf32 ? OP_TF32 : OP_BF16;
+  if (out_nhwc)
+    return conv3x3_run(act, N, h, w, Ck, act_pitch, Wf, Co, dilation, 1, bias, lrelu, slope, nullptr, out_nhwc,
+                       tf32 ? OUT_F32_NHWC : OUT_BF16_NHWC, out_pitch, stream, 12, nullptr, op);
+  return conv3x3_run(act, N, h, w, Ck, act_pitch, Wf, Co, dilation, 1, bias, lrelu, slope, nullptr, out_f32_nchw, OUT_F32_NCHW, 0,
+                     stream, 12, nullptr, op);
 }
 
 // data gradient: gin[pixel, ci] = (sum_t sum_co g[pixel - d_t, co] * Wb[t][ci][co]) * LeakyReLU'(mask[pixel, ci])
@@ -889,29 +1047,39 @@ long long conv3x3_dgrad_colsum_scratch_bytes(int N, int h, int w, long long out_
   return (long long)gemm::conv::conv3x3_colsum_rows(N, h, w) * out_pitch * 4;
 }
 
-// colsum_out (optional, with colsum_scratch): fp32 [Ci] column sums of the stored bf16 gradient = the bias gradient of the layer
-// below, accumulated in the GEMM epilogue (per M-tile and warp quarter) and finished by one small fixed-order reduction
+// colsum_out (optional, with colsum_scratch): fp32 [Ci] column sums of the NHWC gradient = the bias gradient of the layer below,
+// accumulated in the GEMM epilogue (per M-tile and warp quarter) and finished by one small fixed-order reduction: the sums of the
+// stored bf16 values, or with tf32 of the fp32 values before their TF32 rounding.  With tf32 the NHWC output (out_nhwc, and the
+// mask) is fp32, and out_bf16_nhwc is the bf16 NHWC output of the same fp32 result (no mask, no column sums).
 int conv3x3_dgrad(const void* g, int N, int h, int w, int Cg, long long g_pitch, const void* Wb, int Ci, int dilation, const void* mask,
-                  float slope, void* out_bf16_nhwc, long long out_pitch, float* out_f32_nchw, cudaStream_t stream,
-                  void* colsum_scratch, long long colsum_scratch_bytes, float* colsum_out) {
-  B200SEG_CHECK_ARG((out_bf16_nhwc != nullptr) != (out_f32_nchw != nullptr), "conv3x3_dgrad: give exactly one output");
-  B200SEG_CHECK_ARG(!mask || out_bf16_nhwc, "conv3x3_dgrad: the activation mask needs the bf16 NHWC output");
+                  float slope, void* out_nhwc, long long out_pitch, float* out_f32_nchw, cudaStream_t stream,
+                  void* colsum_scratch, long long colsum_scratch_bytes, float* colsum_out, int tf32, void* out_bf16_nhwc) {
+  using namespace gemm::conv;
+  B200SEG_CHECK_ARG((out_nhwc != nullptr) + (out_f32_nchw != nullptr) + (out_bf16_nhwc != nullptr) == 1,
+                    "conv3x3_dgrad: give exactly one output");
+  B200SEG_CHECK_ARG(!out_bf16_nhwc || (tf32 && !mask && !colsum_out), "conv3x3_dgrad: the bf16 output of the TF32 layers takes no mask or sums");
+  B200SEG_CHECK_ARG(!mask || out_nhwc, "conv3x3_dgrad: the activation mask needs the NHWC output");
+  const int op = tf32 ? OP_TF32 : OP_BF16;
+  const int nhwc_mode = tf32 ? OUT_F32_NHWC : OUT_BF16_NHWC;
   if (colsum_out) {
-    B200SEG_CHECK_ARG(out_bf16_nhwc && colsum_scratch, "conv3x3_dgrad: fused column sums need the bf16 NHWC output and a scratch buffer");
+    B200SEG_CHECK_ARG(out_nhwc && colsum_scratch, "conv3x3_dgrad: fused column sums need the NHWC output and a scratch buffer");
     B200SEG_CHECK_ARG(colsum_scratch_bytes >= conv3x3_dgrad_colsum_scratch_bytes(N, h, w, out_pitch), "conv3x3_dgrad: column-sum scratch too small");
-    int rc = gemm::conv::conv3x3_run(g, N, h, w, Cg, g_pitch, Wb, Ci, dilation, -1, nullptr, 0, slope, mask, out_bf16_nhwc,
-                                     gemm::conv::OUT_BF16_NHWC, out_pitch, stream, 13, (float*)colsum_scratch);
+    int rc = conv3x3_run(g, N, h, w, Cg, g_pitch, Wb, Ci, dilation, -1, nullptr, 0, slope, mask, out_nhwc, nhwc_mode, out_pitch, stream, 13,
+                         (float*)colsum_scratch, op);
     if (rc) return rc;
-    colsum_final_kernel<<<ceil_div(Ci, 8), 256, 0, stream>>>((const float*)colsum_scratch, gemm::conv::conv3x3_colsum_rows(N, h, w),
-                                                            (int)out_pitch, Ci, colsum_out);
+    colsum_final_kernel<<<ceil_div(Ci, 8), 256, 0, stream>>>((const float*)colsum_scratch, conv3x3_colsum_rows(N, h, w), (int)out_pitch,
+                                                            Ci, colsum_out);
     B200SEG_LAUNCH_CHECK();
     return B200SEG_OK;
   }
+  if (out_nhwc)
+    return conv3x3_run(g, N, h, w, Cg, g_pitch, Wb, Ci, dilation, -1, nullptr, 0, slope, mask, out_nhwc, nhwc_mode, out_pitch, stream, 13,
+                       nullptr, op);
   if (out_bf16_nhwc)
-    return gemm::conv::conv3x3_run(g, N, h, w, Cg, g_pitch, Wb, Ci, dilation, -1, nullptr, 0, slope, mask, out_bf16_nhwc,
-                                   gemm::conv::OUT_BF16_NHWC, out_pitch, stream, 13);
-  return gemm::conv::conv3x3_run(g, N, h, w, Cg, g_pitch, Wb, Ci, dilation, -1, nullptr, 0, slope, nullptr, out_f32_nchw,
-                                 gemm::conv::OUT_F32_NCHW, 0, stream, 13);
+    return conv3x3_run(g, N, h, w, Cg, g_pitch, Wb, Ci, dilation, -1, nullptr, 0, slope, nullptr, out_bf16_nhwc, OUT_BF16_NHWC, out_pitch,
+                       stream, 13, nullptr, op);
+  return conv3x3_run(g, N, h, w, Cg, g_pitch, Wb, Ci, dilation, -1, nullptr, 0, slope, nullptr, out_f32_nchw, OUT_F32_NCHW, 0, stream, 13,
+                     nullptr, op);
 }
 
 }  // namespace b200seg

@@ -121,6 +121,13 @@ __device__ __forceinline__ void umma_bf16(uint32_t tmem_d, uint64_t adesc, uint6
       "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+// the same with tf32 operands (fp32 in shared memory, the tensor core reads the top 19 bits): K = 8 per instruction
+__device__ __forceinline__ void umma_tf32(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n .reg .pred p;\n setp.ne.b32 p, %4, 0;\n tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n}" ::"r"(tmem_d),
+      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
@@ -149,20 +156,23 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t* r) {
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
 // Shared-memory matrix descriptor (sm_100 format): start>>4 [0,14), LBO>>4 [16,30),
-// SBO>>4 [32,46), version=1 [46,48), layout type [61,64) (2 = SWIZZLE_128B).
-__device__ __forceinline__ uint64_t make_smem_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
+// SBO>>4 [32,46), version=1 [46,48), layout type [61,64) (2 = SWIZZLE_128B; 1 = SWIZZLE_128B_BASE32B, 32-byte chunks swizzled
+// over 4-row atoms: the only swizzled layout of MN-major 32-bit (tf32) operands).
+constexpr uint32_t SMEM_SW128 = 2, SMEM_SW128_BASE32B = 1;
+__device__ __forceinline__ uint64_t make_smem_desc(uint32_t saddr, uint32_t lbo_bytes, uint32_t sbo_bytes, uint32_t layout = SMEM_SW128) {
   uint64_t d = 0;
   d |= (uint64_t)((saddr >> 4) & 0x3FFF);
   d |= (uint64_t)((lbo_bytes >> 4) & 0x3FFF) << 16;
   d |= (uint64_t)((sbo_bytes >> 4) & 0x3FFF) << 32;
   d |= (uint64_t)1 << 46;
-  d |= (uint64_t)2 << 61;
+  d |= (uint64_t)layout << 61;
   return d;
 }
-// Instruction descriptor for kind::f16: D=f32 [4,6)=1, A=bf16 [7,10)=1, B=bf16 [10,13)=1,
-// a_major bit 15, b_major bit 16 (1 = MN-major), N>>3 [17,23), M>>4 [24,29).
-__host__ __device__ constexpr uint32_t make_idesc(bool a_mn, bool b_mn, int m, int n) {
-  return (1u << 4) | (1u << 7) | (1u << 10) | ((a_mn ? 1u : 0u) << 15) | ((b_mn ? 1u : 0u) << 16) |
+// Instruction descriptor: D=f32 [4,6)=1, A format [7,10), B format [10,13) (IDESC_BF16 = 1 for kind::f16, IDESC_TF32 = 2 for
+// kind::tf32), a_major bit 15, b_major bit 16 (1 = MN-major), N>>3 [17,23), M>>4 [24,29).
+constexpr uint32_t IDESC_BF16 = 1, IDESC_TF32 = 2;
+__host__ __device__ constexpr uint32_t make_idesc(bool a_mn, bool b_mn, int m, int n, uint32_t fmt = IDESC_BF16) {
+  return (1u << 4) | (fmt << 7) | (fmt << 10) | ((a_mn ? 1u : 0u) << 15) | ((b_mn ? 1u : 0u) << 16) |
          ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
 }
 
@@ -220,6 +230,12 @@ __device__ __forceinline__ void tmem_dealloc_2sm(uint32_t taddr, uint32_t ncols)
 __device__ __forceinline__ void umma_bf16_2sm(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
   asm volatile(
       "{\n .reg .pred p;\n setp.ne.b32 p, %4, 0;\n tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n}" ::"r"(tmem_d),
+      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
+__device__ __forceinline__ void umma_tf32_2sm(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n .reg .pred p;\n setp.ne.b32 p, %4, 0;\n tcgen05.mma.cta_group::2.kind::tf32 [%0], %1, %2, %3, p;\n}" ::"r"(tmem_d),
       "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }

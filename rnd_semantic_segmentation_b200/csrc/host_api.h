@@ -64,24 +64,31 @@ int aspp_backward(const float* grad_logits, const void* Xp, const void* WpT, con
                   float* const* grad_b, cudaStream_t stream);
 
 // ---- conv_sm100.cu ----
+// tf32 != 0: the TF32 layers -- act / g / x / mask / Wf / Wb and the NHWC outputs are fp32 (TF32 values) instead of bf16
 int conv3x3_pack_weights(const float* const* weights, const int* part_co, int n_parts, int Ci, void* Wf, void* Wb, int co_pitch,
                          cudaStream_t stream);
 int conv3x3_pack_weights_stack(int n_layers, const float* const* weights, const int* part_co, const int* parts_per_layer,
                                const int* Ci, void* const* Wf, void* const* Wb, const int* co_pitch, const float* const* bias_parts,
                                const int* bias_len, int n_bias, float* bias_out, cudaStream_t stream);
+int conv3x3_pack_weights_stack_tf32(int n_layers, const float* const* weights, const int* part_co, const int* parts_per_layer,
+                                    const int* Ci, void* const* Wf, void* const* Wb, const int* co_pitch, const float* const* bias_parts,
+                                    const int* bias_len, int n_bias, float* bias_out, cudaStream_t stream);
 int conv3x3_forward(const void* act, int N, int h, int w, int Ck, long long act_pitch, const void* Wf, int Co, int dilation,
-                    const float* bias, int lrelu, float slope, void* out_bf16_nhwc, long long out_pitch, float* out_f32_nchw,
-                    cudaStream_t stream);
+                    const float* bias, int lrelu, float slope, void* out_nhwc, long long out_pitch, float* out_f32_nchw,
+                    cudaStream_t stream, int tf32 = 0);
+// out_bf16_nhwc: with tf32 only, the layer's result as bf16 NHWC (the feature gradient of bf16 channels_last features)
 int conv3x3_dgrad(const void* g, int N, int h, int w, int Cg, long long g_pitch, const void* Wb, int Ci, int dilation,
-                  const void* mask, float slope, void* out_bf16_nhwc, long long out_pitch, float* out_f32_nchw, cudaStream_t stream,
-                  void* colsum_scratch, long long colsum_scratch_bytes, float* colsum_out);
+                  const void* mask, float slope, void* out_nhwc, long long out_pitch, float* out_f32_nchw, cudaStream_t stream,
+                  void* colsum_scratch, long long colsum_scratch_bytes, float* colsum_out, int tf32 = 0, void* out_bf16_nhwc = nullptr);
 long long conv3x3_dgrad_colsum_scratch_bytes(int N, int h, int w, long long out_pitch);
 long long conv3x3_wgrad_scratch_bytes(int N, int h, int w, int Co, int Ci, int splits);
 int conv3x3_wgrad(const void* g, int Co, long long g_pitch, const void* x, int Ci, long long x_pitch, int N, int h, int w,
                   int dilation, int splits, void* scratch, long long scratch_bytes, float* const* grad_w, const int* part_co,
-                  int n_parts, cudaStream_t stream);
+                  int n_parts, cudaStream_t stream, int tf32 = 0);
 long long nhwc_colsum_scratch_bytes(int pitch);
 int nhwc_bf16_colsum(const void* g, long long P, int C, int pitch, void* scratch, float* out, cudaStream_t stream);
+int nchw_channel_sum(const float* src, int N, int C, int hw, float* out, cudaStream_t stream);       // out[c] = sum src[n][c][:]
+int widen_bf16(const void* src, long long n, float* dst, cudaStream_t stream);                       // bf16 [n] -> fp32 [n], exact
 namespace gemm { namespace conv {
 void set_pair(int on);                // 0 = one CTA per tile, 1 = CTA pairs (cta_group::2) where two M-tiles exist
 } }
@@ -116,6 +123,7 @@ int variant_info(int i, int* a_mn, int* b_mn, int* share, int* bn, int* rs, int*
 int seam_tail_forward(const float* c, const float* identity, const float* scale, const float* bias, int N, int C, int hw, void* y,
                       cudaStream_t stream);
 int nchw_to_nhwc_bf16(const float* src, int N, int C, int hw, void* dst, int pitch, cudaStream_t stream);
+int nchw_to_nhwc_tf32(const float* src, int N, int C, int hw, float* dst, int pitch, cudaStream_t stream);   // fp32 NHWC, TF32-rounded
 int seam_tail_backward(const void* dy, const void* y, const float* scale, int N, int C, int hw, float* dc, float* didentity,
                        cudaStream_t stream);
 int seam_conv3_g(const void* dy, const void* y, int N, int C, int hw, void* g, float* didentity, cudaStream_t stream);

@@ -42,15 +42,15 @@ __device__ __forceinline__ float bn_tail_value(float c, float mean, float invstd
 }
 
 // y[n, s, ch] = bf16_rn(f(c[n, ch, s])) for ch < pitch, with f the seam tail (TAIL) or the identity (then identity, scale and
-// bias are not read); channels C <= ch < pitch are written as 0.
+// bias are not read); channels C <= ch < pitch are written as 0.  OUT = float: y is fp32 rounded to TF32 (tf32_rn) instead.
 // BATCH (with TAIL): f is the batch-statistics tail bn_tail_value; scale / bias carry mean / invstd, and gamma / beta may be null
 // (affine=False).  Without BATCH, gamma and beta are not read.
 // VEC: hw % 4 == 0 and c / identity 16-byte aligned (float4 rows); otherwise scalar loads
-template <bool TAIL, bool VEC, bool BATCH = false>
+template <bool TAIL, bool VEC, bool BATCH = false, typename OUT = __nv_bfloat16>
 __global__ void __launch_bounds__(ST_THREADS) nchw_to_nhwc_tile_kernel(const float* __restrict__ c, const float* __restrict__ identity,
                                                                        const float* __restrict__ scale, const float* __restrict__ bias,
                                                                        const float* __restrict__ gamma, const float* __restrict__ beta,
-                                                                       int C, int hw, int pitch, __nv_bfloat16* __restrict__ y) {
+                                                                       int C, int hw, int pitch, OUT* __restrict__ y) {
   __shared__ __align__(16) float tile[ST_CH * ST_PX];
   const int s0 = blockIdx.x * ST_PX, c0 = blockIdx.y * ST_CH, n = blockIdx.z;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -100,7 +100,16 @@ __global__ void __launch_bounds__(ST_THREADS) nchw_to_nhwc_tile_kernel(const flo
 #pragma unroll
   for (int it = 0; it < 2; ++it) {
     const int sl = (lane >> 2) + 8 * warp + 64 * it;
-    if (s0 + sl < hw && cc < pitch) {
+    if constexpr (sizeof(OUT) == 4) {
+      if (s0 + sl < hw && cc < pitch) {
+        float f[8];
+#pragma unroll
+        for (int e = 0; e < 8; ++e) f[e] = tf32_rn(tile[st_idx(8 * chunk + e, sl)]);
+        float4* yp = reinterpret_cast<float4*>(y + ((long long)n * hw + s0 + sl) * pitch + cc);
+        yp[0] = make_float4(f[0], f[1], f[2], f[3]);
+        yp[1] = make_float4(f[4], f[5], f[6], f[7]);
+      }
+    } else if (s0 + sl < hw && cc < pitch) {
       uint32_t w4[4];
 #pragma unroll
       for (int e = 0; e < 4; ++e) {
@@ -450,6 +459,22 @@ int nchw_to_nhwc_bf16(const float* src, int N, int C, int hw, void* dst, int pit
   B200SEG_CHECK_ARG(N <= 65535 && ceil_div(pitch, ST_CH) <= 65535, "nchw_to_nhwc_bf16: N = %d / pitch = %d too large", N, pitch);
   B200SEG_CHECK_ARG(aligned16(dst), "nchw_to_nhwc_bf16: dst must be 16-byte aligned");
   return nchw_to_nhwc_launch<false>(src, nullptr, nullptr, nullptr, nullptr, nullptr, N, C, hw, pitch, dst, stream);
+}
+
+// fp32 NCHW [N][C][hw] -> fp32 NHWC [N*hw][pitch] rounded to TF32, channels >= C zero (the operands of the TF32 discriminator)
+int nchw_to_nhwc_tf32(const float* src, int N, int C, int hw, float* dst, int pitch, cudaStream_t stream) {
+  B200SEG_CHECK_ARG(src && dst && N > 0 && C > 0 && hw > 0 && pitch % 8 == 0 && pitch >= C, "nchw_to_nhwc_tf32: bad arguments");
+  B200SEG_CHECK_ARG(N <= 65535 && ceil_div(pitch, ST_CH) <= 65535, "nchw_to_nhwc_tf32: N = %d / pitch = %d too large", N, pitch);
+  B200SEG_CHECK_ARG(aligned16(dst), "nchw_to_nhwc_tf32: dst must be 16-byte aligned");
+  const dim3 grid(ceil_div(hw, ST_PX), ceil_div(pitch, ST_CH), N);
+  if (hw % 4 == 0 && aligned16(src))
+    nchw_to_nhwc_tile_kernel<false, true, false, float><<<grid, ST_THREADS, 0, stream>>>(src, nullptr, nullptr, nullptr, nullptr, nullptr,
+                                                                                          C, hw, pitch, dst);
+  else
+    nchw_to_nhwc_tile_kernel<false, false, false, float><<<grid, ST_THREADS, 0, stream>>>(src, nullptr, nullptr, nullptr, nullptr, nullptr,
+                                                                                           C, hw, pitch, dst);
+  B200SEG_LAUNCH_CHECK();
+  return B200SEG_OK;
 }
 
 template <int BN>

@@ -14,6 +14,8 @@ channels_last, from its last Bottleneck (seam.fuse_backbone_tail; INTEGRATION.md
 when that block's bn3 is a training-mode BatchNorm2d / SyncBatchNorm (batch statistics, the self-distillation stage); with
 ``seam_conv3=True`` the block's conv3 runs inside the fused GEMM (bf16 operands, fp32 accumulation: see seam.py); with
 ``seam_train_bn=True, seam_conv3_batch=True`` a batch-statistics bn3's conv3 runs as a tcgen05 GEMM that also computes the statistics.
+``install(disc_tf32=True)`` makes the patched ``build_adversarial_discriminator`` (same signature) return discriminators with
+``tf32=True``: TF32 tensor-core operands and fp32 activations / gradients in the conv stack (INTEGRATION.md "TF32 discriminator").
 """
 from __future__ import annotations
 
@@ -32,6 +34,7 @@ _UTIL_NAMES = ("soft_label_cross_entropy", "inference", "multi_scale_inference",
                "AverageMeter", "get_color_palette")
 _LR_NAMES = ("adjust_learning_rate",)
 _stock_optimizers = {}
+_disc_factory = []                   # the one wrapper install(disc_tf32=True) hands out (re-flagged by later calls)
 
 
 def _optimizer_factory(stock, fused):
@@ -102,15 +105,24 @@ def _install_seam(patched, train_bn=False, conv3=False, conv3_batch=False):
             patched.append(f"{name}.build_feature_extractor")
 
 
+def _build_attr(src, n, disc_tf32):
+    if src is _build and n == "build_adversarial_discriminator" and disc_tf32:
+        if not _disc_factory:
+            _disc_factory.append(_build.wrap_discriminator_factory(_build.build_adversarial_discriminator))
+        return _build.wrap_discriminator_factory(_disc_factory[0], True)
+    return getattr(src, n)
+
+
 def install(strict: bool = False, optimizers: bool = False, seam: bool = False, seam_train_bn: bool = False, seam_conv3: bool = False,
-            seam_conv3_batch: bool = False):
+            seam_conv3_batch: bool = False, disc_tf32: bool = False):
     """Returns the list of 'module.attr' names that were patched.  ``seam=True``: the reference's build_feature_extractor returns
     a backbone whose last Bottleneck emits bf16 channels_last features (seam.fuse_backbone_tail); ``seam_train_bn=True`` (with
     ``seam=True``) extends that to a bn3 that trains with batch statistics (fuse_backbone_tail(fe, train_bn=True));
     ``seam_conv3=True`` (with ``seam=True``) fuses an eligible conv3 into the tail's GEMM (fuse_backbone_tail(fe, conv3=True)),
     which rounds conv3's operands to bf16; ``seam_conv3_batch=True`` (with ``seam=True, seam_train_bn=True``) runs an eligible conv3
     of a batch-statistics bn3 as a tcgen05 GEMM that writes its output and statistics (fuse_backbone_tail(fe, train_bn=True,
-    conv3_batch=True)), also with bf16 operands."""
+    conv3_batch=True)), also with bf16 operands.  ``disc_tf32=True``: build_adversarial_discriminator returns PixelDiscriminators with
+    ``tf32=True`` (build.wrap_discriminator_factory)."""
     patched = install_optimizers() if optimizers else []
     targets = (("core.models.build", _build, _BUILD_NAMES), ("core.models", _build, _BUILD_NAMES),
                ("core.utils.utility", _utility, _UTIL_NAMES), ("core.utils.adapt_lr", _optim, _LR_NAMES))
@@ -124,7 +136,7 @@ def install(strict: bool = False, optimizers: bool = False, seam: bool = False, 
                     raise
                 continue
         for n in names:
-            setattr(mod, n, getattr(src, n))
+            setattr(mod, n, _build_attr(src, n, disc_tf32))
             patched.append(f"{modname}.{n}")
     # modules that did `from core.utils.utility import X` / `from core.models import build_*` before install()
     for mod in list(sys.modules.values()):
@@ -134,7 +146,7 @@ def install(strict: bool = False, optimizers: bool = False, seam: bool = False, 
         for src, names in ((_build, _BUILD_NAMES), (_utility, _UTIL_NAMES), (_optim, _LR_NAMES)):
             for n in names:
                 if n in getattr(mod, "__dict__", {}):
-                    setattr(mod, n, getattr(src, n))
+                    setattr(mod, n, _build_attr(src, n, disc_tf32))
                     patched.append(f"{name}.{n}")
     if seam:
         _install_seam(patched, seam_train_bn, seam_conv3, seam_conv3_batch)

@@ -193,31 +193,38 @@ def aspp_head_loss(x, labels, weights, biases, rates, ignore_index=255, temperat
 # --------------------------------------------------------------------------------------------
 # K6  PixelDiscriminator conv stack (three 3x3 layers as tcgen05 implicit GEMMs, bf16 NHWC activations)
 # --------------------------------------------------------------------------------------------
-def pack_discriminator_weights(w1, w2, wc1, wc2, bc1, bc2):
+def pack_discriminator_weights(w1, w2, wc1, wc2, bc1, bc2, tf32: bool = False):
     """((Wf1, Wb1), (Wf2, Wb2), (Wf3, Wb3), bias3) -- cls1 | cls2 are packed as ONE layer with 2C output channels (the
-    torch.cat of discriminator.py:47 costs nothing)."""
+    torch.cat of discriminator.py:47 costs nothing).  bf16, or with ``tf32`` fp32 holding TF32 values."""
     C = wc1.shape[0]
     (l1, l2, l3), b3 = _lib.conv3x3_pack_weights_stack(
         [[w1.detach()], [w2.detach()], [wc1.detach(), wc2.detach()]],
-        bias_parts=[None if bc1 is None else bc1.detach(), None if bc2 is None else bc2.detach()], bias_lens=[C, C])     # ONE launch
+        bias_parts=[None if bc1 is None else bc1.detach(), None if bc2 is None else bc2.detach()], bias_lens=[C, C], tf32=tf32)  # ONE launch
     return l1, l2, l3, b3
 
 
 class _PixelDiscriminatorFn(torch.autograd.Function):
     """cat(cls1(mid), cls2(mid)) with mid = LReLU(conv(LReLU(conv(x))))  (discriminator.py:34-47), fp32 NCHW [N,2C,h,w].
-    ONE foreign call per direction (b200seg_disc_forward / _backward, graph-replayed in a steady-state loop)."""
+    ONE foreign call per direction (b200seg_disc_forward / _backward, graph-replayed in a steady-state loop; with ``tf32`` the
+    _tf32 entries: TF32 tensor-core operands, fp32 activations and gradients)."""
 
     @staticmethod
-    def forward(ctx, x, slope, packed, w1, b1, w2, b2, wc1, bc1, wc2, bc2):
+    def forward(ctx, x, slope, packed, tf32, w1, b1, w2, b2, wc1, bc1, wc2, bc2):
         N, Cin, h, w = x.shape
         xd = x.detach()
         if not xd.is_cuda:
             raise _lib.B200SegError("PixelDiscriminator: expected CUDA features (b200seg has no CPU fallback)")
-        if xd.dtype == torch.bfloat16 or _PACK_CACHE_SLOTS > 0:
+        if tf32:                                                              # fp32 NCHW, or bf16 features taken as NHWC
+            if xd.dtype == torch.bfloat16:
+                xk, x_kind = _pixel_major_bf16(xd).view(N, h, w, Cin), 1
+            else:
+                xk, x_kind = (xd if xd.dtype == torch.float32 else xd.float()).contiguous(), 0
+        elif xd.dtype == torch.bfloat16 or _PACK_CACHE_SLOTS > 0:
             xk, x_kind = _pixel_major_bf16(xd).view(N, h, w, Cin), 1          # bf16 channels_last input is taken zero-copy
         else:
             xk, x_kind = (xd if xd.dtype == torch.float32 else xd.float()).contiguous(), 0
-        out, Xp, A1, A2, packed = _lib.disc_forward(xk, x_kind, (N, Cin, h, w), (w1, w2, wc1, wc2), (b1, b2, bc1, bc2), slope, packed)
+        out, Xp, A1, A2, packed = _lib.disc_forward(xk, x_kind, (N, Cin, h, w), (w1, w2, wc1, wc2), (b1, b2, bc1, bc2), slope, packed,
+                                                    tf32=bool(tf32))
         (_, Wb1), (_, Wb2), (_, Wb3), _ = packed
         ctx.meta = (float(slope), x.dtype, int(wc1.shape[0]))
         ctx.save_for_backward(Xp, A1, A2, Wb1, Wb2, Wb3)
@@ -227,19 +234,21 @@ class _PixelDiscriminatorFn(torch.autograd.Function):
     def backward(ctx, grad_out):
         Xp, A1, A2, Wb1, Wb2, Wb3 = ctx.saved_tensors
         slope, x_dtype, C = ctx.meta
-        need = ctx.needs_input_grad          # x, slope, packed, w1, b1, w2, b2, wc1, bc1, wc2, bc2
+        need = ctx.needs_input_grad          # x, slope, packed, tf32, w1, b1, w2, b2, wc1, bc1, wc2, bc2
         go = grad_out.detach()
         if go.dtype != torch.float32:
             go = go.float()
         gx, gw1, gb1, gw2, gb2, gwc1, gbc1, gwc2, gbc2 = _lib.disc_backward(
-            go.contiguous(), Xp, A1, A2, Wb1, Wb2, Wb3, C, slope, (need[0],) + tuple(need[3:11]), x_bf16=(x_dtype == torch.bfloat16))
+            go.contiguous(), Xp, A1, A2, Wb1, Wb2, Wb3, C, slope, (need[0],) + tuple(need[4:12]), x_bf16=(x_dtype == torch.bfloat16))
         if gx is not None and gx.dtype != x_dtype:
             gx = gx.to(x_dtype)
-        return gx, None, None, gw1, gb1, gw2, gb2, gwc1, gbc1, gwc2, gbc2
+        return gx, None, None, None, gw1, gb1, gw2, gb2, gwc1, gbc1, gwc2, gbc2
 
 
-def pixel_discriminator_logits(x, w1, b1, w2, b2, wc1, bc1, wc2, bc2, slope: float = 0.2, packed=None) -> torch.Tensor:
-    return _PixelDiscriminatorFn.apply(x, float(slope), packed, w1, b1, w2, b2, wc1, bc1, wc2, bc2)
+def pixel_discriminator_logits(x, w1, b1, w2, b2, wc1, bc1, wc2, bc2, slope: float = 0.2, packed=None, tf32: bool = False) -> torch.Tensor:
+    """``tf32``: TF32 tensor-core operands with fp32 activations and gradients (``packed`` then from
+    pack_discriminator_weights(..., tf32=True)); otherwise bf16 operands, activations and gradients."""
+    return _PixelDiscriminatorFn.apply(x, float(slope), packed, bool(tf32), w1, b1, w2, b2, wc1, bc1, wc2, bc2)
 
 
 # --------------------------------------------------------------------------------------------
